@@ -2,6 +2,7 @@
 """bench.py — throughput of the hot path on B200 (and the reference's CPU path beside it).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload all|train|infer]
+                    [--dump-outputs DIR]
 
 ONE JSON line (rank 0). The top-level record is BASELINE.json's metric on configs[1]: one "step" = one soft-Dice
 training step (fwd + loss + bwd + Keras-Adam) of the depth-4 / 16-filter 3D U-Net on a batch of 8 synthetic 64^3
@@ -21,7 +22,16 @@ communicator). Nested records cover the rest of the metric:
 
 `value` is timed with CUDA events on the stream the kernels are launched on, inputs already resident in HBM; `e2e` goes
 through the reference-facing Python API (Model.train_on_batch / patch_wise_prediction) with host buffers, H2D + D2H inside
-the timed region. `--impl reference` times the oracle port of the reference's CPU path on the host cores.
+the timed region. `--impl reference` times the oracle port of the reference's CPU path on the host cores. Every timed
+loop of every record runs exactly `--steps` iterations (reported as `steps`); the warm-up calls before it are untimed.
+
+`--dump-outputs DIR` writes, after the timed steps, what the caller of each timed path received from its last step as
+DIR/<name>.npy: train_metrics (loss, binary_accuracy, vod_coefficient, dice_coefficient as fm_train_step_device returns
+them) and infer_prediction (the float64 patch_wise_prediction result of the last timed call, bit for bit). The inputs
+are seeded, so two builds can be compared output for output. The model's weights are not dumped: a training pass is not
+bit-reproducible (fp32 red.add of the weight gradients, three-issuer marching kernels; DESIGN.md §5), and Adam turns a
+last-bit difference of a near-zero gradient into an update of the size of the learning rate, so after a few steps the
+weights of two runs differ far beyond rounding while the metrics agree to it.
 """
 import argparse
 import json
@@ -35,6 +45,8 @@ PKG = os.path.join(ROOT, "fetal-mri-segmentation_b200")
 for p in (ROOT, PKG):
     if p not in sys.path:
         sys.path.insert(0, p)
+# the benchmark leaves the source tree as it found it (it may be read-only): no bytecode caches next to the modules
+sys.dont_write_bytecode = True
 
 import numpy as np  # noqa: E402
 
@@ -63,6 +75,20 @@ def peaks():
         return dict(hbm=float(d["hbm_gbs"]), tf_burst=float(d["bf16_tflops"]),
                     tf_sustained=float(d.get("bf16_tflops_sustained", d["bf16_tflops"])), src="measured")
     return dict(hbm=6650.0, tf_burst=1590.0, tf_sustained=1400.0, src="fallback")
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def write_dump(path, arrays):
+    """Writes {name: array} as path/<name>.npy (float64 stays float64, everything else becomes float32)."""
+    out = {k: np.ascontiguousarray(a, dtype=np.float64 if np.asarray(a).dtype == np.float64 else np.float32)
+           for k, a in arrays.items()}
+    total = sum(a.nbytes for a in out.values())
+    assert total <= DUMP_LIMIT_BYTES, "dump of %d bytes exceeds %d" % (total, DUMP_LIMIT_BYTES)
+    os.makedirs(path, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 def ncu_traffic():
@@ -321,8 +347,9 @@ def make_batch(rank, shape, batch=BATCH):
     return x, t
 
 
-def bench_train(e, args, patch, fwd_gf, first_gf, steps, warmup, with_profile):
-    """The data-parallel (or single-GPU) training step on `patch`; returns the record dict (rank 0) or None."""
+def bench_train(e, args, patch, fwd_gf, first_gf, steps, warmup, with_profile, dump=None):
+    """The data-parallel (or single-GPU) training step on `patch`; returns the record dict (rank 0) or None. With a
+    `dump` dict, rank 0 puts the metrics of the last timed step into it."""
     torch, _lib, lib, ctx = e.torch, e._lib, e.lib, e.ctx
     from fetal_net.distributed import DataParallelTrainer
     from fetal_net.model import unet_model_3d
@@ -359,6 +386,8 @@ def bench_train(e, args, patch, fwd_gf, first_gf, steps, warmup, with_profile):
     ms = timed_device(e, step_device, steps)
     clocks = sampler.stop() if e.rank == 0 else None
     launches = ctx.launch_count() - launches0
+    if dump is not None and e.rank == 0:
+        dump["train_metrics"] = np.asarray(last["m"] if dp is not None else m4, np.float32).copy()
     ms_step = ms / steps
     vox_step = BATCH * int(np.prod(patch)) * e.world
     rec = dict(value=vox_step / (ms_step * 1e-3), ms_per_step=ms_step, clocks=clocks, gpu_launches=int(launches))
@@ -433,7 +462,7 @@ def bench_train_sampled(e, steps, plain_ms):
     return dict(value=vox / sec, unit=UNIT, ms_per_step=sec * 1e3, fraction_of_device_step_rate=plain_ms / (sec * 1e3),
                 config=dict(workload="DeviceSampler.train_on_next_batch: 6 resident cases of 160x160x96, batch 8 x 64^3 "
                                      "cut on the device (skip_blank=True, shuffled index list), same model as the "
-                                     "headline step", host_bytes_per_step=32 * BATCH))
+                                     "headline step", host_bytes_per_step=32 * BATCH), steps=steps)
 
 
 def bench_allreduce(e, rec_train, steps):
@@ -458,7 +487,7 @@ def bench_allreduce(e, rec_train, steps):
     dp.set_comm_enabled(True)
     dp.broadcast_weights(0)                  # the replicas drifted apart while the collectives were off
     n = e.world
-    return dict(bytes=int(nbytes), buckets=int(e.lib.fm_model_num_buckets(model._h)), standalone_ms=ms,
+    return dict(steps=steps, bytes=int(nbytes), buckets=int(e.lib.fm_model_num_buckets(model._h)), standalone_ms=ms,
                 bus_gbs=2.0 * (n - 1) / n * nbytes / (ms * 1e-3) / 1e9, bus_peak_gbs=900.0,
                 frac_of_nvlink=2.0 * (n - 1) / n * nbytes / (ms * 1e-3) / 1e9 / 900.0,
                 step_ms_with_comm=on, step_ms_without_comm=off, exposed_ms=max(on - off, 0.0),
@@ -501,8 +530,9 @@ def bench_dp_parity(e):
     return out
 
 
-def bench_infer(e, args, steps, warmup):
-    """configs[0]: patch_wise_prediction of one 256x256x64 volume (49 patches), single GPU."""
+def bench_infer(e, args, steps, warmup, dump=None):
+    """configs[0]: patch_wise_prediction of one 256x256x64 volume (49 patches), single GPU. With a `dump` dict, the
+    result of the last timed call goes into it."""
     torch, ctx = e.torch, e.ctx
     from fetal_net.model import unet_model_3d
     from fetal_net.prediction import patch_wise_prediction
@@ -526,6 +556,8 @@ def bench_infer(e, args, steps, warmup):
         return r, ts
     out, t_page = timed_calls(vol)
     clocks = sampler.stop()
+    if dump is not None:
+        dump["infer_prediction"] = np.array(out, np.float64)
     launches = int((ctx.launch_count() - l0) // steps)
     for _ in range(2):
         call(volp)
@@ -599,7 +631,7 @@ def bench_infer_sharded(e, steps):
     nvox = int(np.prod(VOLUME5))
     if e.rank != 0:
         return None
-    return dict(metric="U-Net sharded infer voxels/sec", value=nvox / sec, unit=UNIT, ms_per_volume=sec * 1e3,
+    return dict(metric="U-Net sharded infer voxels/sec", steps=steps, value=nvox / sec, unit=UNIT, ms_per_volume=sec * 1e3,
                 config=dict(workload="sharded_patch_wise_prediction 1x512x512x128, patch 128x128x64, overlap_factor 0.5, "
                                      "147 patches split contiguously over the ranks, one ncclReduce of the float64 "
                                      "partial sums (BASELINE configs[4])", patches=147, ranks=e.world),
@@ -672,7 +704,7 @@ def bench_family(e, kind, steps):
                 predict=dict(value=units / s_pred, ms_per_call=s_pred * 1e3, conv_tflops=B * fwd_gf / (s_pred * 1e3),
                              note="Model.predict with host buffers (H2D + forward + D2H)"),
                 roofline=roofline_of(top[0], top[1], 2, total_ms, pk, clocks, {}, kind), kernel_breakdown=breakdown,
-                loss=float(m4[0]))
+                loss=float(m4[0]), steps=steps)
 
 
 def run_b200(args):
@@ -680,8 +712,9 @@ def run_b200(args):
     want_train = args.workload in ("all", "train")
     want_infer = args.workload in ("all", "infer")
     line = None
+    dump = {} if args.dump_outputs else None
     if want_train:
-        rec = bench_train(e, args, PATCH, FWD_GF_PER_PATCH, FIRST_CONV_GF, args.steps, args.warmup, True)
+        rec = bench_train(e, args, PATCH, FWD_GF_PER_PATCH, FIRST_CONV_GF, args.steps, args.warmup, True, dump)
         cpu_base = None
         if e.rank == 0 and e.world == 1 and not args.no_cpu_baseline:
             times, threads = cpu_train_steps(BATCH, 3, 1, budget_s=40)
@@ -691,17 +724,18 @@ def run_b200(args):
                                    "after 1 warm-up, %d threads" % (len(times), threads))
         extra = {}
         if e.world > 1:
-            extra["allreduce"] = bench_allreduce(e, rec, max(args.steps, 10))
+            extra["allreduce"] = bench_allreduce(e, rec, args.steps)
         model, dp = rec.pop("_model"), rec.pop("_dp")
         del model, dp
         if e.world > 1:
-            r5 = bench_train(e, args, PATCH5, FWD_GF_PER_PATCH5, FIRST_CONV_GF5, max(3, args.steps // 4), 3, False)
+            r5 = bench_train(e, args, PATCH5, FWD_GF_PER_PATCH5, FIRST_CONV_GF5, args.steps, 3, False)
             r5.pop("_model"), r5.pop("_dp")
             r5["config"] = dict(workload="same step on BASELINE configs[4]'s patch shape: batch 8 x 1x128x128x64 per GPU",
                                 global_batch=BATCH * e.world, patch=list(PATCH5))
             r5["unit"] = UNIT
+            r5["steps"] = args.steps
             extra["train_cfg5"] = r5
-            extra["infer_sharded"] = bench_infer_sharded(e, 3)
+            extra["infer_sharded"] = bench_infer_sharded(e, args.steps)
             extra["dp_parity"] = bench_dp_parity(e)
         if e.rank == 0:
             line = dict(metric=METRIC, value=rec["value"], unit=UNIT, n_gpus=e.world, steps=args.steps,
@@ -717,10 +751,10 @@ def run_b200(args):
             line.update(extra)
     if args.workload == "all" and e.rank == 0 and e.world == 1 and line is not None:
         line["train_sampled"] = bench_train_sampled(e, args.steps, line["ms_per_step"])
-        line["families"] = dict(isensee=bench_family(e, "isensee", max(3, args.steps // 4)),
-                                unet2d=bench_family(e, "unet2d", max(3, args.steps // 4)))
+        line["families"] = dict(isensee=bench_family(e, "isensee", args.steps),
+                                unet2d=bench_family(e, "unet2d", args.steps))
     if want_infer and e.rank == 0:
-        inf = bench_infer(e, args, max(5, args.steps // 2), 3)
+        inf = bench_infer(e, args, args.steps, 3, dump)
         if not args.no_cpu_baseline and e.world == 1:
             inf["cpu_baseline"] = cpu_infer_sample()
         if line is None:
@@ -730,6 +764,8 @@ def run_b200(args):
             line["infer"] = inf
     barrier(e)
     if e.rank == 0:
+        if dump is not None:
+            write_dump(args.dump_outputs, dump)
         print(json.dumps(line))
     if e.world > 1:
         e.lib.fm_comm_destroy(e.ctx.handle)
@@ -744,7 +780,13 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="all", choices=["all", "train", "infer"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step of each workload as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs records the outputs of --impl b200")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -100,6 +100,9 @@ def test_oracle_matches_live_reference():
                                          batch_size=bs)
         out = po.patch_wise_prediction(FunctionModel(fn, oshape), vol, patch, overlap_factor=f, batch_size=bs)
         assert np.array_equal(out, ref)
+
+
+def test_oracle_identity_model_returns_the_volume():
     # identity-model goldens of SURVEY.md §8c (1)-(2)
     for vshape in [(1, 96, 80, 40), (1, 70, 70, 20)]:
         vol = np.random.default_rng(0).standard_normal(vshape).astype(np.float32)
