@@ -64,6 +64,7 @@ extern "C" int fm_ctx_destroy(fm_ctx* ctx) {
   if (ctx->comm_stream) cudaStreamDestroy(ctx->comm_stream);
   if (ctx->comm_ev) cudaEventDestroy(ctx->comm_ev);
   if (ctx->red_scratch) cudaFree(ctx->red_scratch);
+  if (ctx->pp_ws) cudaFree(ctx->pp_ws);
   for (auto& r : ctx->prof) {
     cudaEventDestroy(r.e0);
     cudaEventDestroy(r.e1);
@@ -1955,17 +1956,85 @@ extern "C" int fm_reassemble(fm_ctx* ctx, const float* preds, const int32_t* idx
   return r;
 }
 
+// ---------------------------------------------------------------------------------------------
+// post-processing (postprocess.cu)
+// ---------------------------------------------------------------------------------------------
+static int check_pp_spec(const fm_postprocess_spec* spec, const int32_t dims[3]) {
+  FM_CHECK(spec && spec->weights && spec->radius >= 0, FM_EINVAL, "post-processing: bad spec");
+  FM_CHECK(dims[0] > 0 && dims[1] > 0 && dims[2] > 0, FM_EINVAL, "post-processing: dims %d x %d x %d", dims[0],
+           dims[1], dims[2]);
+  FM_CHECK((int64_t)dims[0] * dims[1] * dims[2] <= INT32_MAX, FM_EINVAL,
+           "post-processing: %d x %d x %d voxels exceed 2^31 - 1", dims[0], dims[1], dims[2]);
+  return FM_OK;
+}
+
+// mask (and the component count) of the last k_postprocess to the host, through the pinned staging area at `pin`
+static int pp_download(fm_ctx* ctx, const PostprocBuffers& b, size_t nvox, const fm_postprocess_spec* spec, char* pin,
+                       uint8_t* mask, int64_t* n_components) {
+  FM_CUDA(cudaMemcpyAsync(pin, b.stats, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
+  FM_CUDA(cudaMemcpyAsync(pin + 256, b.mask, nvox, cudaMemcpyDeviceToHost, ctx->stream));
+  FM_CUDA(cudaStreamSynchronize(ctx->stream));
+  host_copy(mask, pin + 256, nvox);
+  if (n_components) *n_components = spec->connected_component ? (int64_t)((unsigned long long*)pin)[0] : -1;
+  return FM_OK;
+}
+
+extern "C" int fm_postprocess(fm_ctx* ctx, const void* pred, int dtype, const int32_t dims[3],
+                              const fm_postprocess_spec* spec, uint8_t* mask, int64_t* n_components) {
+  FM_CHECK(ctx && pred && dims && mask, FM_EINVAL, "fm_postprocess: bad argument");
+  FM_CHECK(dtype == FM_DTYPE_FLOAT32 || dtype == FM_DTYPE_FLOAT64, FM_EINVAL, "fm_postprocess: dtype %d", dtype);
+  FM_TRY(check_pp_spec(spec, dims));
+  FM_CUDA(cudaSetDevice(ctx->device));
+  const size_t nvox = (size_t)dims[0] * dims[1] * dims[2], es = dtype == FM_DTYPE_FLOAT64 ? 8 : 4;
+  PostprocBuffers b;
+  FM_TRY(pp_buffers(ctx, (int64_t)nvox, spec->radius, &b));
+  // pinned staging: [map | stats | mask]
+  const size_t in_bytes = (nvox * es + 4095) & ~(size_t)4095;
+  void* pin = nullptr;
+  FM_TRY(fm_ctx_pinned(ctx, in_bytes + 256 + nvox, &pin));
+  host_copy(pin, pred, nvox * es);
+  FM_CUDA(cudaMemcpyAsync(b.field1, pin, nvox * es, cudaMemcpyHostToDevice, ctx->stream));
+  FM_TRY(k_postprocess(ctx, b, b.field1, dtype, (int64_t)dims[1] * dims[2], dims[2], dims, spec));
+  return pp_download(ctx, b, nvox, spec, (char*)pin + in_bytes, mask, n_components);
+}
+
+extern "C" int fm_op_gaussian3d(fm_ctx* ctx, const void* in, int dtype, const int32_t dims[3], int radius,
+                                const double* weights, void* out) {
+  FM_CHECK(ctx && in && dims && weights && out && radius >= 0, FM_EINVAL, "fm_op_gaussian3d: bad argument");
+  FM_CHECK(dtype == FM_DTYPE_FLOAT32 || dtype == FM_DTYPE_FLOAT64, FM_EINVAL, "fm_op_gaussian3d: dtype %d", dtype);
+  fm_postprocess_spec spec = {radius, weights, 0.0, 0, 0};
+  FM_TRY(check_pp_spec(&spec, dims));
+  FM_CUDA(cudaSetDevice(ctx->device));
+  const size_t nvox = (size_t)dims[0] * dims[1] * dims[2], es = dtype == FM_DTYPE_FLOAT64 ? 8 : 4;
+  PostprocBuffers b;
+  FM_TRY(pp_buffers(ctx, (int64_t)nvox, radius, &b));
+  FM_CUDA(cudaMemcpyAsync(b.field1, in, nvox * es, cudaMemcpyHostToDevice, ctx->stream));
+  FM_TRY(k_gaussian3d(ctx, b, b.field1, dtype, (int64_t)dims[1] * dims[2], dims[2], dims, radius, weights, b.field0));
+  FM_CUDA(cudaMemcpyAsync(out, b.field0, nvox * es, cudaMemcpyDeviceToHost, ctx->stream));
+  FM_CUDA(cudaStreamSynchronize(ctx->stream));
+  return FM_OK;
+}
+
 // reduce_root < 0: `out` receives this shard's result (the average for shard 0 of 1, the partial SUM otherwise).
 // reduce_root >= 0: the partial sums are reduced on the ctx communicator to that rank, which divides by the counts and
 // is the only one to copy anything back to the host.
+// pp != null (fm_patchwise_segment; single GPU): the cropped result is post-processed on the device into `pp_mask`;
+// `out` is then optional.
 static bool is_pinned_host(const void* p);
 static int patchwise_impl(fm_model* m, const float* vol, const int32_t vol_dims[3], const int32_t halo_pad[6],
                           const int32_t fit_pad[6], const double pad_value[2], const int32_t* idx, int64_t n, int batch,
                           int shard_rank, int shard_count, int reduce_root, const float* truth, int prev_truth_index,
-                          int prev_truth_size, double* out, int16_t* out_count) {
-  const bool want_out = reduce_root < 0 || shard_rank == reduce_root;
+                          int prev_truth_size, double* out, int16_t* out_count,
+                          const fm_postprocess_spec* pp = nullptr, uint8_t* pp_mask = nullptr,
+                          int64_t* pp_components = nullptr) {
+  const bool want_out = (reduce_root < 0 || shard_rank == reduce_root) && (out || !pp);
   FM_CHECK(m && vol && vol_dims && halo_pad && fit_pad && pad_value && idx && (out || !want_out) && n > 0 && batch > 0,
            FM_EINVAL, "fm_patchwise_predict: bad argument");
+  if (pp) {
+    FM_CHECK(pp_mask && shard_count == 1 && reduce_root < 0, FM_EINVAL,
+             "fm_patchwise_segment: needs a mask and a single shard");
+    FM_TRY(check_pp_spec(pp, vol_dims));
+  }
   FM_CHECK(shard_count >= 1 && shard_rank >= 0 && shard_rank < shard_count, FM_EINVAL,
            "fm_patchwise_predict: shard %d of %d", shard_rank, shard_count);
   fm_ctx* ctx = m->ctx;
@@ -2060,12 +2129,13 @@ static int patchwise_impl(fm_model* m, const float* vol, const int32_t vol_dims[
     t_start = t;
   };
   // host <-> device through the context's pinned staging buffer (pageable cudaMemcpy runs at a fraction of PCIe):
-  // [volume | truth | float64 result | int16 counts]
+  // [volume | truth | float64 result | int16 counts | post-processing stats + mask]
   const size_t in_bytes = (nv * sizeof(float) * (truth ? 2 : 1) + 4095) & ~(size_t)4095;
-  const size_t out_bytes = nout * sizeof(double), cnt_bytes = out_count ? nout * sizeof(int16_t) : 0;
+  const size_t out_bytes = pp && !out ? 0 : nout * sizeof(double), cnt_bytes = out_count ? nout * sizeof(int16_t) : 0;
   const size_t cnt_off = in_bytes + ((out_bytes + 4095) & ~(size_t)4095);
+  const size_t pp_off = cnt_off + ((cnt_bytes + 4095) & ~(size_t)4095);
   void* pin = nullptr;
-  FM_TRY(fm_ctx_pinned(ctx, cnt_off + cnt_bytes, &pin));
+  FM_TRY(fm_ctx_pinned(ctx, pp ? pp_off + 256 + nv : cnt_off + cnt_bytes, &pin));
   char* pin_in = (char*)pin;
   char* pin_out = (char*)pin + in_bytes;
   char* pin_cnt = (char*)pin + cnt_off;
@@ -2170,6 +2240,19 @@ static int patchwise_impl(fm_model* m, const float* vol, const int32_t vol_dims[
     unstage(false);
   }
   lap("enqueue (upload / gather / forward / overlap-add)");
+  if (pp) {
+    // the float64 map stays on the device: its pad_for_fit crop (prediction.py:198-207) is post-processed in place,
+    // while the slabs of `out` (when asked for) are still on their way back
+    PostprocBuffers b;
+    FM_TRY(pp_buffers(ctx, (int64_t)nv, pp->radius, &b));
+    const double* box = dout.p + (size_t)fit_pad[0] * plane + (size_t)fit_pad[2] * out_dims[2] + fit_pad[4];
+    FM_TRY(k_postprocess(ctx, b, box, FM_DTYPE_FLOAT64, (int64_t)plane, out_dims[2], vol_dims, pp));
+    if (stream_out) unstage(true);
+    FM_TRY(pp_download(ctx, b, nv, pp, (char*)pin + pp_off, pp_mask, pp_components));
+    lap("post-process + D2H");
+    m->fwd_valid = false;
+    return FM_OK;
+  }
   if (stream_out) {
     unstage(true);
     FM_CUDA(cudaStreamSynchronize(ctx->stream));
@@ -2228,6 +2311,15 @@ extern "C" int fm_patchwise_predict_dp(fm_model* m, const float* vol, const int3
   FM_CHECK(root >= 0 && root < ranks, FM_EINVAL, "fm_patchwise_predict_dp: root %d of %d ranks", root, ranks);
   return patchwise_impl(m, vol, vol_dims, halo_pad, fit_pad, pad_value, idx, n, batch, ctx->comm_rank, ranks, root, truth,
                         prev_truth_index, prev_truth_size, out, out_count);
+}
+
+extern "C" int fm_patchwise_segment(fm_model* m, const float* vol, const int32_t vol_dims[3], const int32_t halo_pad[6],
+                                    const int32_t fit_pad[6], const double pad_value[2], const int32_t* idx, int64_t n,
+                                    int batch, const float* truth, int prev_truth_index, int prev_truth_size,
+                                    const fm_postprocess_spec* spec, uint8_t* mask, double* prob, int64_t* n_components) {
+  FM_CHECK(spec && mask, FM_EINVAL, "fm_patchwise_segment: NULL spec or mask");
+  return patchwise_impl(m, vol, vol_dims, halo_pad, fit_pad, pad_value, idx, n, batch, 0, 1, -1, truth, prev_truth_index,
+                        prev_truth_size, prob, nullptr, spec, mask, n_components);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -74,6 +74,9 @@ struct fm_ctx {
   bool comm_enabled = true;  // false: collectives are skipped (bench.py measures the exposed communication time)
   cudaStream_t comm_stream = nullptr;
   cudaEvent_t comm_ev = nullptr;
+  // device workspace of the post-processing kernels (postprocess.cu), grown on demand
+  void* pp_ws = nullptr;
+  size_t pp_ws_bytes = 0;
 };
 
 // sampler.cu: cuts a batch of training samples out of device-resident cases into device buffers
@@ -328,6 +331,24 @@ void k_reassemble_release(ReasmPlan* plan);
 int k_reassemble_groups(const ReasmPlan* plan, const int32_t** xstarts, int* n_groups, int* patches_per_group);
 int k_reassemble_rows(fm_ctx*, const ReasmPlan* plan, const float* preds, int64_t shard_lo, int64_t shard_hi,
                       int64_t pred_base, double* out_dev, int16_t* count_dev, int divide, int x_lo, int x_hi);
+
+// postprocess.cu: postprocess_prediction (fetal_net/postprocess.py:13) on a float32 (dtype 0) / float64 (dtype 1) field.
+// Views of the ctx-owned workspace for volumes of up to nvox voxels and filters of up to `radius`.
+struct PostprocBuffers {
+  void *field0, *field1;      // nvox doubles each (float32 fields use the first half)
+  int32_t *labels, *aux;      // union-find parents; border marks / component sizes
+  uint8_t* mask;              // nvox result
+  double* weights;            // 2 radius + 1
+  unsigned long long* stats;  // [0] components found, [1] (size << 32 | ~root) of the kept component
+};
+int pp_buffers(fm_ctx*, int64_t nvox, int radius, PostprocBuffers* out);
+// gaussian_filter of the [dims] box of `src` (element strides sx, sy, 1) into the compact out_field (device); src may
+// be b.field1
+int k_gaussian3d(fm_ctx*, const PostprocBuffers& b, const void* src, int dtype, int64_t sx, int64_t sy,
+                 const int32_t dims[3], int radius, const double* weights_host, void* out_field);
+// the whole post-processing of the box: result in b.mask, component count and choice in b.stats
+int k_postprocess(fm_ctx*, const PostprocBuffers& b, const void* src, int dtype, int64_t sx, int64_t sy,
+                  const int32_t dims[3], const fm_postprocess_spec* spec);
 
 // conv_simt.cu
 // first layer: fp32 single/multi-channel input (channels-last), small Cin; out bf16 + ReLU

@@ -54,6 +54,12 @@ class UNet2DSpec(ctypes.Structure):
                 ("depth", ctypes.c_int32), ("n_base_filters", ctypes.c_int32), ("n_labels", ctypes.c_int32)]
 
 
+class PostprocessSpec(ctypes.Structure):
+    """fm_postprocess_spec: Gaussian weights (2 radius + 1), threshold and the two flags of postprocess_prediction."""
+    _fields_ = [("radius", ctypes.c_int32), ("weights", ctypes.POINTER(ctypes.c_double)), ("threshold", ctypes.c_double),
+                ("fill_holes", ctypes.c_int32), ("connected_component", ctypes.c_int32)]
+
+
 # name -> (restype, argtypes); exactly the symbols include/fetal_b200.h declares
 SIGNATURES = {
     "fm_ctx_create": (c_int, [c_int, ctypes.POINTER(c_vp)]),
@@ -94,6 +100,10 @@ SIGNATURES = {
                                      c_int, c_int, c_fp, c_int, c_int, c_dp, c_i16p]),
     "fm_reassemble": (c_int, [c_vp, c_fp, c_i32p, c_i64, c_i32p, c_int, c_i32p, c_dp, c_i16p]),
     "fm_gather_patches": (c_int, [c_vp, c_fp, c_i32p, c_i32p, c_i32p, c_dp, c_i32p, c_i64, c_i32p, c_fp]),
+    "fm_postprocess": (c_int, [c_vp, c_vp, c_int, c_i32p, ctypes.POINTER(PostprocessSpec), c_u8p, c_i64p]),
+    "fm_patchwise_segment": (c_int, [c_vp, c_fp, c_i32p, c_i32p, c_i32p, c_dp, c_i32p, c_i64, c_int, c_fp, c_int, c_int,
+                                     ctypes.POINTER(PostprocessSpec), c_u8p, c_dp, c_i64p]),
+    "fm_op_gaussian3d": (c_int, [c_vp, c_vp, c_int, c_i32p, c_int, c_dp, c_vp]),
     "fm_train_step": (c_int, [c_vp, c_fp, c_fp, c_int, c_f, c_fp]),
     "fm_train_forward": (c_int, [c_vp, c_fp, c_fp, c_int]),
     "fm_train_backward": (c_int, [c_vp]),

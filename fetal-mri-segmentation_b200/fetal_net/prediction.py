@@ -83,6 +83,25 @@ def _crop_fit(arr, fit):
     return arr
 
 
+def _native_truth(model, g, vol, truth_data, prev_truth_size):
+    """Checks the patch shape against a native Model's input; returns the float32 previous-truth volume of the 2.5D
+    path (or None)."""
+    if g["is3d"]:
+        assert tuple(g["patch_shape"]) == tuple(model.input_shape[2:]), \
+            "patch_shape %s != model input %s" % (g["patch_shape"], model.input_shape[2:])
+        assert truth_data is None, "truth_data conditions the 2.5D model only"
+        return None
+    n_truth = int(prev_truth_size) if truth_data is not None else 0
+    assert tuple(g["patch_shape"][:2]) == tuple(model.input_shape[1:3]) and \
+        g["patch_shape"][2] + n_truth == model.input_shape[3], \
+        "patch_shape %s (+%d truth slices) != model input %s" % (g["patch_shape"], n_truth, model.input_shape[1:])
+    if truth_data is None:
+        return None
+    truth = _lib.f32c(np.asarray(truth_data)[0])
+    assert truth.shape == vol.shape
+    return truth
+
+
 def patch_wise_prediction(model, data, patch_shape, overlap_factor=0, batch_size=5,
                           permute=False, truth_data=None, prev_truth_index=None, prev_truth_size=None,
                           shard=None, reduce_root=None):
@@ -118,19 +137,7 @@ def patch_wise_prediction(model, data, patch_shape, overlap_factor=0, batch_size
     cnt = np.empty(g["out_dims"], np.int16) if count > 1 else None
 
     if isinstance(model, Model):
-        truth = None
-        if g["is3d"]:
-            assert tuple(g["patch_shape"]) == tuple(model.input_shape[2:]), \
-                "patch_shape %s != model input %s" % (g["patch_shape"], model.input_shape[2:])
-            assert truth_data is None, "truth_data conditions the 2.5D model only"
-        else:
-            n_truth = int(prev_truth_size) if truth_data is not None else 0
-            assert tuple(g["patch_shape"][:2]) == tuple(model.input_shape[1:3]) and \
-                g["patch_shape"][2] + n_truth == model.input_shape[3], \
-                "patch_shape %s (+%d truth slices) != model input %s" % (g["patch_shape"], n_truth, model.input_shape[1:])
-            if truth_data is not None:
-                truth = _lib.f32c(np.asarray(truth_data)[0])
-                assert truth.shape == vol.shape
+        truth = _native_truth(model, g, vol, truth_data, prev_truth_size)
         if reduce_root is not None and count > 1:
             is_root = rank == int(reduce_root)
             _lib.check(lib.fm_patchwise_predict_dp(model._h, _lib.fptr(vol), _lib.i32ptr(vol_dims), _lib.i32ptr(halo),

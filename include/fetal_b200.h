@@ -248,6 +248,40 @@ int fm_gather_patches(fm_ctx* ctx, const float* vol, const int32_t vol_dims[3],
                       const double pad_value[2], const int32_t* idx, int64_t n,
                       const int32_t patch[3], float* out);
 
+/* ---- post-processing ---------------------------------------------------------------------- */
+
+/* Replaces: postprocess_prediction(pred, gaussian_std, threshold, fill_holes, connected_component)
+ * (fetal_net/postprocess.py:13): scipy.ndimage.gaussian_filter (mode 'reflect', truncate 4, axes 0, 1, 2, each pass
+ * rounded to the input dtype), `> threshold` in the input dtype, binary_fill_holes (6-connected background) and the
+ * largest 6-connected component (lowest first voxel in C order on a tie), bit-exact with scipy.
+ * `weights` are the 2 radius + 1 normalised Gaussian weights as scipy computes them with numpy.exp (so they are taken
+ * from the caller, not recomputed here); radius 0 with weight 1.0 is the identity (sigma 0). */
+typedef struct fm_postprocess_spec {
+  int32_t radius;
+  const double* weights; /* 2 radius + 1, host */
+  double threshold;
+  int32_t fill_holes;
+  int32_t connected_component;
+} fm_postprocess_spec;
+#define FM_DTYPE_FLOAT32 0
+#define FM_DTYPE_FLOAT64 1
+/* `pred` host [dims] of `dtype`, `mask` host uint8 [dims]. `n_components` (may be NULL) receives the number of
+ * foreground components before the largest one is selected, or -1 when connected_component is 0. With
+ * connected_component set and no foreground the mask is all zero and n_components 0 (the reference raises).
+ * Volumes of up to 2^31 - 1 voxels. */
+int fm_postprocess(fm_ctx* ctx, const void* pred, int dtype, const int32_t dims[3], const fm_postprocess_spec* spec,
+                   uint8_t* mask, int64_t* n_components);
+/* fm_patchwise_predict (single GPU, n_labels 1) followed by fm_postprocess of its cropped result, without the float64
+ * map leaving the device: `mask` host uint8 [vol_dims]; `prob` (may be NULL) receives exactly what `out` of
+ * fm_patchwise_predict would (the padded [X+fit, Y+fit, Z+fit, 1] float64 map). */
+int fm_patchwise_segment(fm_model* m, const float* vol, const int32_t vol_dims[3], const int32_t halo_pad[6],
+                         const int32_t fit_pad[6], const double pad_value[2], const int32_t* idx, int64_t n, int batch,
+                         const float* truth, int prev_truth_index, int prev_truth_size,
+                         const fm_postprocess_spec* spec, uint8_t* mask, double* prob, int64_t* n_components);
+/* Gaussian filter alone (test hook): `out` host [dims] of `dtype` = scipy.ndimage.gaussian_filter(in, sigma). */
+int fm_op_gaussian3d(fm_ctx* ctx, const void* in, int dtype, const int32_t dims[3], int radius, const double* weights,
+                     void* out);
+
 /* ---- training ----------------------------------------------------------------------------- */
 
 /* Replaces: model.train_on_batch(x, y) as driven by fit_generator (fetal_net/training.py:110-124):
