@@ -349,22 +349,17 @@ static Layer& L(fm_model* m, const char* fmt, int d) {
   return m->layers[layer_index(m, nm)];
 }
 
-// FETAL_B200_NO_MARCH=1 forces the per-tap kernel everywhere (A/B measurements, debugging)
-static bool use_march() {
-  const char* e = getenv("FETAL_B200_NO_MARCH");
-  return !(e && e[0] == '1');
-}
-
-// Training passes take the shared-accumulator marching kernel where it applies (N <= 32): 20-30 % faster, but the
-// order in which the three MMA warps' products land in an accumulator is not fixed, so activations differ in the
-// last bf16 bit from run to run. FETAL_B200_DETERMINISTIC=1 keeps training on the bit-reproducible kernel (the fp32
-// red.add order of the weight gradients is then the only run-to-run difference).
-static bool shared_march(const fm_model* m, int n_channels) {
+// Training passes (and fast inference) let the marching kernel issue its MMAs in three interleaved streams where it
+// applies (Cout <= 32): 20-30 % faster, but the order in which the three MMA warps' products land in an accumulator is
+// not fixed, so activations differ in the last bf16 bit from run to run. FETAL_B200_DETERMINISTIC=1 keeps training on
+// the bit-reproducible issue order (the fp32 red.add order of the weight gradients is then the only run-to-run
+// difference).
+static bool reproducible_pass(const fm_model* m) {
   static const bool det = [] {
     const char* e = getenv("FETAL_B200_DETERMINISTIC");
     return e && e[0] == '1';
   }();
-  return (m->train_pass || m->fast_inference) && n_channels <= 32 && !det;
+  return !(m->train_pass || m->fast_inference) || det;
 }
 
 static int build_unet(fm_ctx* ctx, const fm_unet3d_spec* spec, int kcode, int flags, fm_model** out);
@@ -512,35 +507,32 @@ static int build_unet(fm_ctx* ctx, const fm_unet3d_spec* spec, int kcode, int fl
     if (l.is_norm || l.k != 3 || l.c1 < 16) continue;
     const int X = spec->X >> l.level, Y = spec->Y >> l.level, Z = m->pz == 2 ? spec->Z >> l.level : spec->Z;
     const int cs[2] = {l.c1, l.c2};
-    if (use_march() && conv_march_supported(X, Y, Z, l.c1, l.c2, l.cout, l.k)) {
+    if (conv_march_supported(X, Y, Z, l.c1, l.c2, l.cout, l.k)) {
       l.march_f = true;
       for (int s = 0; s < (l.c2 ? 2 : 1); ++s)
         FM_CUDA(cudaMalloc((void**)&l.w_mf[s], (size_t)conv_march_pack_elems(cs[s], l.cout) * sizeof(bf16)));
     }
     for (int s = 0; s < (l.c2 ? 2 : 1); ++s)
-      if (use_march() && conv_march_supported(X, Y, Z, l.cout, 0, cs[s], l.k)) {
+      if (conv_march_supported(X, Y, Z, l.cout, 0, cs[s], l.k)) {
         l.march_d[s] = true;
         FM_CUDA(cudaMalloc((void**)&l.w_md[s], (size_t)conv_march_pack_elems(l.cout, cs[s]) * sizeof(bf16)));
       }
   }
   // decoder convs whose filter bank is too large for the marching kernel run at COARSE resolution on their upsampled
-  // source (dec1a, dec2a of the shipped model); FETAL_B200_NO_UP_COARSE=1 keeps the materialised upsampling
+  // source (dec1a, dec2a of the shipped model)
   for (auto& l : m->layers) {
     if (strncmp(l.name, "dec", 3) != 0 || l.c2 == 0 || l.k != 3 || m->pz != 2 || m->deconvolution || m->batch_norm ||
         l.is_norm)
       continue;
-    const char* e = getenv("FETAL_B200_NO_UP_COARSE");
-    if (e && e[0] == '1') continue;
     const int X = spec->X >> l.level, Y = spec->Y >> l.level, Z = spec->Z >> l.level;
     if (!conv_up_supported(X, Y, Z, l.c1, l.c2, l.cout)) continue;
     const size_t n = (size_t)l.cout * 64 * l.c1;
     FM_CUDA(cudaMalloc((void**)&l.w_up_d, n * sizeof(bf16)));
-    const char* all = getenv("FETAL_B200_UP_COARSE_ALL");
-    if (l.march_f && !(all && all[0] == '1')) {
+    if (l.march_f) {
       // small filter bank (dec0a): forward and weight gradient stay on the marching kernels over the materialised
       // upsampled tensor; the gradient towards the coarse tensor still drops from 27 fine taps + a sum-pool pass to
-      // 64 class taps per COARSE voxel. (FETAL_B200_UP_COARSE_ALL=1: all three passes at coarse resolution - A/B.)
-      l.up_dgrad = !(e && e[0] == '2');
+      // 64 class taps per COARSE voxel
+      l.up_dgrad = true;
       continue;
     }
     l.up_coarse = true;
@@ -835,48 +827,27 @@ static int refresh_packs(fm_model* m) {
     m->repack_blocks = blocks;
     m->repack_weights = weights;
   }
-  if (m->repack_n > 0 && !getenv("FETAL_B200_SPLIT_REPACK")) {
+  if (m->repack_n > 0)  // (0 only for a model without convs)
     FM_TRY(k_repack_all(m->ctx, m->params, m->repack_tab, m->repack_n, m->repack_blocks, m->repack_weights));
-    RepackUpTable ut;
-    memset(&ut, 0, sizeof(ut));
-    for (auto& l : m->layers) {
-      if (!(l.up_coarse || l.up_dgrad)) continue;
-      if (ut.n == 8) {
-        FM_TRY(k_repack_up_table(m->ctx, m->params, ut));
-        ut.n = 0;
-      }
-      RepackUpDesc& d = ut.d[ut.n];
-      d.w_off = l.w_off;
-      d.wf = l.w_up_f;
-      d.wd = l.w_up_d;
-      d.cout = l.cout;
-      d.cc = l.c1;
-      d.ct = l.cin();
-      d.block0 = ut.n ? ut.d[ut.n - 1].block0 + (int)ceil_div64((int64_t)ut.d[ut.n - 1].cout * 64 * ut.d[ut.n - 1].cc, 256) : 0;
-      ++ut.n;
-    }
-    FM_TRY(k_repack_up_table(m->ctx, m->params, ut));
-    m->packs_dirty = false;
-    return FM_OK;
-  }
+  RepackUpTable ut;
+  memset(&ut, 0, sizeof(ut));
   for (auto& l : m->layers) {
-    if (l.is_norm) continue;
-    if (l.k == 1 && l.cout == 1) continue;  // head reads fp32 weights directly
-    FM_TRY(k_repack_weights(m->ctx, m->params + l.w_off, l.w_f, l.w_d0, l.c2 ? l.w_d1 : nullptr,
-                            l.deconv ? l.cout * l.taps() : l.cout, l.deconv ? 1 : l.taps(), l.c1, l.c2));
-    const int cs[2] = {l.c1, l.c2};
-    int kofs = 0;
-    for (int s = 0; s < (l.c2 ? 2 : 1); ++s) {
-      if (l.march_f)
-        FM_TRY(k_repack_march(m->ctx, l.w_f, l.w_mf[s], l.cout, l.cin(), kofs, cs[s],
-                              conv_march_kc(l.c1, l.c2, l.cout, cs[s])));
-      if (l.march_d[s])
-        FM_TRY(k_repack_march(m->ctx, s == 0 ? l.w_d0 : l.w_d1, l.w_md[s], cs[s], l.cout, 0, l.cout,
-                              conv_march_kc(l.cout, 0, cs[s], l.cout)));
-      kofs += cs[s];
+    if (!(l.up_coarse || l.up_dgrad)) continue;
+    if (ut.n == 8) {
+      FM_TRY(k_repack_up_table(m->ctx, m->params, ut));
+      ut.n = 0;
     }
-    if (l.up_coarse || l.up_dgrad) FM_TRY(k_repack_up(m->ctx, m->params + l.w_off, l.w_up_f, l.w_up_d, l.cout, l.c1, l.cin()));
+    RepackUpDesc& d = ut.d[ut.n];
+    d.w_off = l.w_off;
+    d.wf = l.w_up_f;
+    d.wd = l.w_up_d;
+    d.cout = l.cout;
+    d.cc = l.c1;
+    d.ct = l.cin();
+    d.block0 = ut.n ? ut.d[ut.n - 1].block0 + (int)ceil_div64((int64_t)ut.d[ut.n - 1].cout * 64 * ut.d[ut.n - 1].cc, 256) : 0;
+    ++ut.n;
   }
+  FM_TRY(k_repack_up_table(m->ctx, m->params, ut));
   m->packs_dirty = false;
   return FM_OK;
 }
@@ -953,8 +924,8 @@ static int conv_fwd(fm_model* m, const Layer& l, const bf16* x1, const bf16* x2,
   const Dims5 d = m->dims(l.level, l.cout, B);
   const float* bias = m->params + l.b_off;
   if (l.march_f)
-    return (shared_march(m, l.cout) ? k_conv3d_march_shared : k_conv3d_march)(
-        ctx, x1, x2, l.w_mf[0], l.w_mf[1], bias, y, nullptr, B, d.X, d.Y, d.Z, l.c1, l.c2, l.cout, relu, l.cout, 0);
+    return k_conv3d_march(ctx, x1, x2, l.w_mf[0], l.w_mf[1], bias, y, nullptr, B, d.X, d.Y, d.Z, l.c1, l.c2, l.cout, relu,
+                          l.cout, 0, reproducible_pass(m));
   if (conv_tc_supported(l.c1, l.c2, l.cout, l.k))
     return k_conv3d_tc_fprop(ctx, x1, x2, l.w_f, bias, y, nullptr, B, d.X, d.Y, d.Z, l.c1, l.c2, l.cout,
                              l.k, relu, l.cout, 0);
@@ -1115,21 +1086,16 @@ static int conv_wgrad(fm_model* m, const Layer& l, const bf16* x1, const bf16* x
   const int cs[2] = {l.c1, l.c2};
   int cofs = 0;
   bool bias_done = false;
-  static const bool fold_bias = [] {
-    const char* e = getenv("FETAL_B200_SEPARATE_BIAS_GRAD");
-    return !(e && e[0] == '1');
-  }();
   for (int s = 0; s < (l.c2 ? 2 : 1); ++s) {
     if (only_src >= 0 && s != only_src) {
       cofs += cs[s];
       continue;
     }
-    if (use_march() && conv_wgrad_march_supported(d.X, d.Y, d.Z, cs[s], l.cout, l.k)) {
+    if (conv_wgrad_march_supported(d.X, d.Y, d.Z, cs[s], l.cout, l.k)) {
       // the marching kernel also sums dY over the voxels (bias gradient) while the tiles sit in shared memory
-      const bool with_bias = fold_bias && !bias_done;
       FM_TRY(k_conv3d_wgrad_march(ctx, xs[s], dy, dw, B, d.X, d.Y, d.Z, cs[s], l.cin(), cofs, l.cout,
-                                  with_bias ? m->grads + l.b_off : nullptr));
-      bias_done = bias_done || with_bias;
+                                  bias_done ? nullptr : m->grads + l.b_off));
+      bias_done = true;
     } else if (conv_tc_supported(cs[s], 0, l.cout, l.k))
       FM_TRY(k_conv3d_tc_wgrad(ctx, xs[s], dy, dw, B, d.X, d.Y, d.Z, cs[s], l.cin(), cofs, l.cout, l.k));
     else
@@ -1153,8 +1119,8 @@ static int conv_dgrad(fm_model* m, const Layer& l, int src, const bf16* dy, cons
   const int cs = src == 0 ? l.c1 : l.c2;
   const bf16* wd = src == 0 ? l.w_d0 : l.w_d1;
   if (l.march_d[src])
-    return (shared_march(m, cs) ? k_conv3d_march_shared : k_conv3d_march)(
-        ctx, dy, nullptr, l.w_md[src], nullptr, nullptr, dx, mask, B, d.X, d.Y, d.Z, l.cout, 0, cs, 0, cs, 0);
+    return k_conv3d_march(ctx, dy, nullptr, l.w_md[src], nullptr, nullptr, dx, mask, B, d.X, d.Y, d.Z, l.cout, 0, cs, 0,
+                          cs, 0, reproducible_pass(m));
   if (conv_tc_supported(l.cout, 0, cs, l.k))
     return k_conv3d_tc_fprop(ctx, dy, nullptr, wd, nullptr, dx, mask, B, d.X, d.Y, d.Z, l.cout, 0, cs, l.k,
                              0, cs, 0);
@@ -1501,13 +1467,13 @@ static int build_isensee(fm_ctx* ctx, const IsenseeBuild* spec, fm_model** out) 
     const int X = spec->X >> l.level, Y = spec->Y >> l.level, Z = spec->Z >> l.level;
     const int Xd = spec->X >> dl, Yd = spec->Y >> dl, Zd = spec->Z >> dl;
     const int cs[2] = {l.c1, l.c2};
-    if (l.stride == 1 && use_march() && conv_march_supported(X, Y, Z, l.c1, l.c2, l.cout, l.k)) {
+    if (l.stride == 1 && conv_march_supported(X, Y, Z, l.c1, l.c2, l.cout, l.k)) {
       l.march_f = true;
       for (int s = 0; s < (l.c2 ? 2 : 1); ++s)
         FM_CUDA(cudaMalloc((void**)&l.w_mf[s], (size_t)conv_march_pack_elems(cs[s], l.cout) * sizeof(bf16)));
     }
     for (int s = 0; s < (l.c2 ? 2 : 1); ++s)
-      if (use_march() && conv_march_supported(Xd, Yd, Zd, l.cout, 0, cs[s], l.k)) {
+      if (conv_march_supported(Xd, Yd, Zd, l.cout, 0, cs[s], l.k)) {
         l.march_d[s] = true;
         FM_CUDA(cudaMalloc((void**)&l.w_md[s], (size_t)conv_march_pack_elems(l.cout, cs[s]) * sizeof(bf16)));
       }
@@ -1615,8 +1581,8 @@ static int isensee_block(fm_model* m, const Layer& l, const Layer& nl, const bf1
     FM_TRY(k_conv3d_simt_fprop(ctx, x1, 1, nullptr, l.w_f, bias, raw, nullptr, B, d.X, d.Y, d.Z, 1, 0, l.cout, 3, 0,
                                nullptr));
   } else if (l.march_f) {
-    FM_TRY((shared_march(m, l.cout) ? k_conv3d_march_shared : k_conv3d_march)(
-        ctx, x1, x2, l.w_mf[0], l.w_mf[1], bias, raw, nullptr, B, d.X, d.Y, d.Z, l.c1, l.c2, l.cout, 0, l.cout, 0));
+    FM_TRY(k_conv3d_march(ctx, x1, x2, l.w_mf[0], l.w_mf[1], bias, raw, nullptr, B, d.X, d.Y, d.Z, l.c1, l.c2, l.cout, 0,
+                          l.cout, 0, reproducible_pass(m)));
   } else if (conv_tc_supported(l.c1, l.c2, l.cout, l.k)) {
     FM_TRY(k_conv3d_tc_fprop(ctx, x1, x2, l.w_f, bias, raw, nullptr, B, d.X, d.Y, d.Z, l.c1, l.c2, l.cout, l.k, 0,
                              l.cout, 0, l.stride, d.X * l.stride, d.Y * l.stride, m->pz == 2 ? d.Z * l.stride : d.Z));
@@ -1707,7 +1673,7 @@ static int is_wgrad(fm_model* m, const Layer& l, int level, const bf16* x1, cons
   // no bias gradient here: every Isensee conv feeds an InstanceNormalization, which removes a per-channel constant -
   // the gradient of such a bias is exactly zero (the heads, which have a live bias, are 1x1x1 kernels handled elsewhere)
   for (int s = 0; s < (l.c2 ? 2 : 1); ++s) {
-    if (use_march() && conv_wgrad_march_supported(d.X, d.Y, d.Z, cs[s], l.cout, l.k))
+    if (conv_wgrad_march_supported(d.X, d.Y, d.Z, cs[s], l.cout, l.k))
       FM_TRY(k_conv3d_wgrad_march(ctx, xs[s], dy, dw, B, d.X, d.Y, d.Z, cs[s], l.cin(), cofs, l.cout));
     else if (conv_tc_supported(cs[s], 0, l.cout, l.k))
       FM_TRY(k_conv3d_tc_wgrad(ctx, xs[s], dy, dw, B, d.X, d.Y, d.Z, cs[s], l.cin(), cofs, l.cout, l.k));
@@ -1724,8 +1690,8 @@ static int is_dgrad(fm_model* m, const Layer& l, int level, int src, const bf16*
   const int cs = src == 0 ? l.c1 : l.c2;
   const bf16* wd = src == 0 ? l.w_d0 : l.w_d1;
   if (l.march_d[src])
-    return (shared_march(m, cs) ? k_conv3d_march_shared : k_conv3d_march)(ctx, dy, nullptr, l.w_md[src], nullptr, nullptr, dx,
-                                                               nullptr, B, d.X, d.Y, d.Z, l.cout, 0, cs, 0, cs, 0);
+    return k_conv3d_march(ctx, dy, nullptr, l.w_md[src], nullptr, nullptr, dx, nullptr, B, d.X, d.Y, d.Z, l.cout, 0, cs, 0,
+                          cs, 0, reproducible_pass(m));
   if (conv_tc_supported(l.cout, 0, cs, l.k))
     return k_conv3d_tc_fprop(ctx, dy, nullptr, wd, nullptr, dx, nullptr, B, d.X, d.Y, d.Z, l.cout, 0, cs, l.k, 0, cs, 0);
   return k_conv3d_simt_fprop(ctx, dy, 0, nullptr, wd, nullptr, dx, nullptr, B, d.X, d.Y, d.Z, l.cout, 0, cs, l.k, 0,
@@ -2078,35 +2044,27 @@ static int patchwise_impl(fm_model* m, const float* vol, const int32_t vol_dims[
   // A large caller batch is therefore cut into sub-batches of whole x groups: the volume is uploaded slab by slab on
   // the copy stream just ahead of the patches that need it, and finished output slabs are overlap-added, copied back
   // and un-staged while the network still works on later patches. The network is bit-reproducible and batch-invariant,
-  // so the result does not depend on the cut. FETAL_B200_PW_SUB=0 keeps the caller's batch.
-  {
-    static const int sub_env = [] {
-      const char* e = getenv("FETAL_B200_PW_SUB");
-      return e ? atoi(e) : -1;
-    }();
-    if (sub_env > 0)
-      batch = std::min(batch, sub_env);
-    else if (sub_env < 0 && batch > ppg && ngroups >= 3) {
-      // cut so that a sub-batch fills the SMs in whole waves: the marching kernels run one 16 x 8 column per CTA, a
-      // patch has cpp columns, and q patches (q = SMs / gcd(SMs, cpp); 37 for 64^3 patches on 148 SMs) are a whole
-      // number of waves for them and for the 128-voxel tiles of the deeper levels. The first cut keeps ~3/4 of the
-      // patches (its finished output slabs travel back while the remainder runs); 2D models keep whole x groups.
-      const int64_t cpp = is2d ? 0 : (int64_t)(m->spec.Y / 16) * (m->spec.Z / 8);
-      int64_t q = 0;
-      if (cpp > 0) {
-        int64_t a = ctx->num_sms, b = cpp;
-        while (b) {
-          const int64_t t = a % b;
-          a = b;
-          b = t;
-        }
-        q = ctx->num_sms / a;
+  // so the result does not depend on the cut.
+  if (batch > ppg && ngroups >= 3) {
+    // cut so that a sub-batch fills the SMs in whole waves: the marching kernels run one 16 x 8 column per CTA, a
+    // patch has cpp columns, and q patches (q = SMs / gcd(SMs, cpp); 37 for 64^3 patches on 148 SMs) are a whole
+    // number of waves for them and for the 128-voxel tiles of the deeper levels. The first cut keeps ~3/4 of the
+    // patches (its finished output slabs travel back while the remainder runs); 2D models keep whole x groups.
+    const int64_t cpp = is2d ? 0 : (int64_t)(m->spec.Y / 16) * (m->spec.Z / 8);
+    int64_t q = 0;
+    if (cpp > 0) {
+      int64_t a = ctx->num_sms, b = cpp;
+      while (b) {
+        const int64_t t = a % b;
+        a = b;
+        b = t;
       }
-      if (q > 0 && nloc > q)
-        batch = (int)std::min<int64_t>(batch, q * std::max<int64_t>(1, std::min<int64_t>(2, (nloc * 3 / 4) / q)));
-      else if (q == 0)
-        batch = (int)std::min<int64_t>(batch, (int64_t)ppg * std::max(1, ngroups / 8));
+      q = ctx->num_sms / a;
     }
+    if (q > 0 && nloc > q)
+      batch = (int)std::min<int64_t>(batch, q * std::max<int64_t>(1, std::min<int64_t>(2, (nloc * 3 / 4) / q)));
+    else if (q == 0)
+      batch = (int)std::min<int64_t>(batch, (int64_t)ppg * std::max(1, ngroups / 8));
   }
   FM_TRY(ensure_capacity(m, batch, false));
   DevBuf<float>&dvol = m->pw_vol, &dpred = m->pw_pred;
@@ -2773,7 +2731,7 @@ extern "C" int fm_op_conv3d_fprop(fm_ctx* ctx, int impl, const float* x, const f
   FM_TRY(s.up_bf16(packed.data(), packed.size(), &dw));
   if (bias) FM_TRY(s.up_f32(bias, Cout, &dbias));
   FM_TRY(s.alloc(&dy, vox * Cout));
-  if (impl == 2 || impl == 3) {  // marching kernel: 2 = bit-reproducible, 3 = shared accumulators (training variant)
+  if (impl == 2 || impl == 3) {  // marching kernel: 2 = bit-reproducible, 3 = the issue order of training passes
     FM_CHECK(conv_march_supported(X, Y, Z, C1, C2, Cout, ksize), FM_EINVAL, "march kernel does not cover this shape");
     bf16 *wm1 = nullptr, *wm2 = nullptr;
     FM_TRY(s.alloc(&wm1, (size_t)conv_march_pack_elems(C1, Cout)));
@@ -2782,8 +2740,8 @@ extern "C" int fm_op_conv3d_fprop(fm_ctx* ctx, int impl, const float* x, const f
       FM_TRY(s.alloc(&wm2, (size_t)conv_march_pack_elems(C2, Cout)));
       FM_TRY(k_repack_march(ctx, dw, wm2, Cout, Ct, C1, C2, conv_march_kc(C1, C2, Cout, C2)));
     }
-    FM_TRY((impl == 3 && Cout <= 32 ? k_conv3d_march_shared : k_conv3d_march)(ctx, dx1, dx2, wm1, wm2, dbias, dy, nullptr,
-                                                                               N, X, Y, Z, C1, C2, Cout, relu, Cout, 0));
+    FM_TRY(k_conv3d_march(ctx, dx1, dx2, wm1, wm2, dbias, dy, nullptr, N, X, Y, Z, C1, C2, Cout, relu, Cout, 0,
+                          impl != 3));
   } else if (impl == 0)
     FM_TRY(k_conv3d_tc_fprop(ctx, dx1, dx2, dw, dbias, dy, nullptr, N, X, Y, Z, C1, C2, Cout, ksize, relu,
                              Cout, 0));
@@ -2816,8 +2774,8 @@ extern "C" int fm_op_conv3d_dgrad(fm_ctx* ctx, int impl, const float* dy, const 
     bf16* wm = nullptr;
     FM_TRY(s.alloc(&wm, (size_t)conv_march_pack_elems(Cout, Cin)));
     FM_TRY(k_repack_march(ctx, wd, wm, Cin, Cout, 0, Cout, conv_march_kc(Cout, 0, Cin, Cout)));
-    FM_TRY((impl == 3 && Cin <= 32 ? k_conv3d_march_shared : k_conv3d_march)(ctx, ddy, nullptr, wm, nullptr, nullptr, ddx,
-                                                                             dmask, N, X, Y, Z, Cout, 0, Cin, 0, Cin, 0));
+    FM_TRY(k_conv3d_march(ctx, ddy, nullptr, wm, nullptr, nullptr, ddx, dmask, N, X, Y, Z, Cout, 0, Cin, 0, Cin, 0,
+                          impl != 3));
   } else if (impl == 0)
     FM_TRY(k_conv3d_tc_fprop(ctx, ddy, nullptr, wd, nullptr, ddx, dmask, N, X, Y, Z, Cout, 0, Cin, ksize, 0,
                              Cin, 0));

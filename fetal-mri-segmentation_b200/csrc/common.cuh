@@ -134,29 +134,16 @@ static inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
 
 // ------------------------------------------------------------------------------------------
 // Work split of the plane-marching kernels. A problem is `cols` columns (sample, y tile, z tile) of X planes each; a CTA
-// marches along x inside a column.
-//   mode 0  equal ranges: the flat (column, x) sequence is cut into G contiguous ranges of T / G planes (+-1); a range
-//           that crosses a column boundary has several segments. Perfect balance, but neighbouring columns are walked at
-//           unrelated times, so the y / z halos they share are re-read from DRAM instead of L2.
-//   mode 1  lock-step chunks: every column is cut into nxc chunks of xchunk planes; work unit u = chunk * cols + column,
-//           CTA r takes units r, r + G, ... - a wave of G units covers neighbouring columns at the SAME x range, the
-//           halo re-reads hit L2 (DRAM traffic = algorithmic bytes); nxc is chosen on the host for wave efficiency.
-// `it` counts the CTA's segments / units from 0. Returns false when the CTA is done.
+// marches along x inside a column. Every column is cut into nxc chunks of xchunk planes; work unit u = chunk * cols +
+// column, CTA r of G takes units r, r + G, ... - a wave of G units covers neighbouring columns at the SAME x range, so
+// the y / z halos they share are re-read from L2 (DRAM traffic = algorithmic bytes); nxc is chosen on the host for wave
+// efficiency. `it` counts the CTA's units from 0. Returns false when the CTA is done.
 // ------------------------------------------------------------------------------------------
 struct PlaneSplit {
-  int mode, T, X, cols, nxc, xchunk;
+  int X, cols, nxc, xchunk;
 };
 #ifdef __CUDACC__
 __device__ __forceinline__ bool plane_split_next(const PlaneSplit& s, int rank, int G, int it, int& col, int& xa, int& xb) {
-  if (s.mode == 0) {
-    const int t_begin = (int)((int64_t)rank * s.T / G), t_end = (int)((int64_t)(rank + 1) * s.T / G);
-    col = t_begin / s.X + it;
-    const int lo = it == 0 ? t_begin : col * s.X;
-    if (lo >= t_end) return false;
-    xa = lo - col * s.X;
-    xb = min(s.X, t_end - col * s.X);
-    return true;
-  }
   const int u = rank + it * G;
   if (u >= s.cols * s.nxc) return false;
   const int xc = u / s.cols;
@@ -166,14 +153,8 @@ __device__ __forceinline__ bool plane_split_next(const PlaneSplit& s, int rank, 
   return true;
 }
 #endif
-// host side: fills `s` for `G` CTAs (halo = planes a chunk re-loads, in units of a plane's cost); FETAL_B200_SPLIT=0|1
+// host side: fills `s` for `G` CTAs (halo = planes a chunk re-loads, in units of a plane's cost)
 static inline void plane_split_setup(PlaneSplit* s, int cols, int X, int G, double halo) {
-  static const int forced = [] {
-    const char* e = getenv("FETAL_B200_SPLIT");
-    return e ? atoi(e) : -1;
-  }();
-  s->mode = forced >= 0 ? forced : 1;
-  s->T = cols * X;
   s->X = X;
   s->cols = cols;
   double best = -1.0;
@@ -423,48 +404,28 @@ int k_conv3d_up_wgrad(fm_ctx*, const bf16* coarse, const bf16* dy, float* dw_up,
                       int Cout);
 int k_fold_up_wgrad(fm_ctx*, const float* dw_up, float* dw_master, int Cout, int Cc, int Ct);
 
-// conv_first_tc.cu: first conv (Cin = 1, fp32 volume) and its weight gradient through an im2col tile + tcgen05;
-// FETAL_B200_SIMT_FIRST=1 keeps the SIMT kernels of conv_simt.cu
+// conv_first_tc.cu: first conv (Cin = 1, fp32 volume) and its weight gradient through an im2col tile + tcgen05
 int conv_first_tc_supported(int X, int Y, int Z, int Cout);
 int k_conv3d_first_tc(fm_ctx*, const float* x, const bf16* w_packed, const float* bias, bf16* y, int N, int X, int Y,
                       int Z, int Cout, int relu);
 int k_conv3d_first_tc_wgrad(fm_ctx*, const float* x, const bf16* dy, float* dw, int N, int X, int Y, int Z, int Cout);
 
-// conv_march.cu
+// conv_march.cu: plane-marching fprop / dgrad of 3x3x3 convs whose filter bank fits in shared memory
 int conv_march_supported(int X, int Y, int Z, int C1, int C2, int Cout, int ksize);
 int64_t conv_march_pack_elems(int Cs, int Cout);
 // K-chunk width of a source with Cs channels in a marching conv (C1 [+ C2] -> Cout): 64 (128-byte slab rows) unless the
 // resident filter bank leaves fewer than two slab slots per dz ring, then 32 (half-size slots, twice as many)
 int conv_march_kc(int C1, int C2, int Cout, int Cs);
 int k_repack_march(fm_ctx*, const bf16* P, bf16* Wm, int Nrows, int Ktot, int kofs, int Cs, int KC);
-int k_conv3d_march(fm_ctx*, const bf16* x1, const bf16* x2, const bf16* wm1, const bf16* wm2,
-                   const float* bias, bf16* y, const bf16* mask, int N, int X, int Y, int Z, int C1, int C2,
-                   int Cout, int relu, int out_C, int out_cofs);
-// conv_march_shared.cu: same contract, shared accumulators (training passes; not bit-reproducible run to run)
-int k_conv3d_march_shared(fm_ctx*, const bf16* x1, const bf16* x2, const bf16* wm1, const bf16* wm2,
-                          const float* bias, bf16* y, const bf16* mask, int N, int X, int Y, int Z, int C1, int C2,
-                          int Cout, int relu, int out_C, int out_cofs);
-
-// conv_march2.cu: second-generation marching kernel (tight issue loops, register-resident bias, one shared
-// accumulator ring). nissue = 1: single issuing warp, bit-reproducible; nissue = 3: one issuing warp per dz slab copy.
-// k_conv3d_march / k_conv3d_march_shared route here unless FETAL_B200_MARCH_V1=1 (A/B against the round-1 kernels).
-int k_conv3d_march2(fm_ctx*, const bf16* x1, const bf16* x2, const bf16* wm1, const bf16* wm2, const float* bias,
-                    bf16* y, const bf16* mask, int N, int X, int Y, int Z, int C1, int C2, int Cout, int relu,
-                    int out_C, int out_cofs, int nissue);
-static inline bool fm_march_v1() {
-  static const bool v1 = [] {
-    const char* e = getenv("FETAL_B200_MARCH_V1");
-    return e && e[0] == '1';
-  }();
-  return v1;
-}
+// reproducible: the MMAs reach the tensor pipe in a fixed order, so the output is identical run to run (predict /
+// evaluate / patch_wise_prediction); otherwise, for Cout <= 32, the order follows three interleaved issue streams
+// (training passes)
+int k_conv3d_march(fm_ctx*, const bf16* x1, const bf16* x2, const bf16* wm1, const bf16* wm2, const float* bias,
+                   bf16* y, const bf16* mask, int N, int X, int Y, int Z, int C1, int C2, int Cout, int relu,
+                   int out_C, int out_cofs, bool reproducible);
 
 // conv_wgrad_march.cu
 int conv_wgrad_march_supported(int X, int Y, int Z, int Cin, int Cout, int ksize);
 // db (optional): the bias gradient [Cout] = column sums of dY, accumulated (atomics) by the same launch
 int k_conv3d_wgrad_march(fm_ctx*, const bf16* x, const bf16* dy, float* dw_packed, int N, int X, int Y, int Z,
-                         int Cin, int Cin_total, int cin_ofs, int Cout, float* db = nullptr);
-// alternative (conv_wgrad_march3.cu, FETAL_B200_WGRAD_GEN=3): one z-haloed X slab per plane, the kz tap as a
-// descriptor start offset
-int k_conv3d_wgrad_march3(fm_ctx*, const bf16* x, const bf16* dy, float* dw_packed, int N, int X, int Y, int Z,
                          int Cin, int Cin_total, int cin_ofs, int Cout, float* db = nullptr);

@@ -13,7 +13,6 @@
 // Replaces: the first Conv3D of create_convolution_block (fetal_net/model/unet3d/unet.py:102) on the (1, X, Y, Z)
 // input and its TF autodiff weight gradient.
 #include <algorithm>
-#include <mutex>
 
 #include "tc_ptx.cuh"
 
@@ -341,22 +340,6 @@ __global__ void __launch_bounds__(kThreadsF, 1) conv3d_first_tc_kernel(const __g
   }
 }
 
-typedef CUresult (*PFN_encodeTiledF)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                     const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                     CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-PFN_encodeTiledF get_encode_f() {
-  static PFN_encodeTiledF fn = nullptr;
-  static std::once_flag once;
-  std::call_once(once, [] {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
-        qres == cudaDriverEntryPointSuccess)
-      fn = (PFN_encodeTiledF)p;
-  });
-  return fn;
-}
-
 size_t first_smem(int mode, int Cout) {
   return (size_t)(kABufs + 1) * kATile + (mode == 0 ? 32u * 128u : (size_t)kDyRingF * 128u * Cout * 2u) + 2 * kHaloBytes +
          1024 + 256 + 16;
@@ -378,11 +361,7 @@ int fill(FirstParams& p, int N, int X, int Y, int Z, int Cout) {
 }  // namespace
 
 int conv_first_tc_supported(int X, int Y, int Z, int Cout) {
-  static const bool off = [] {
-    const char* e = getenv("FETAL_B200_SIMT_FIRST");
-    return e && e[0] == '1';
-  }();
-  return !off && X > 0 && Y % kFY == 0 && Z % kFZ == 0 && (Cout == 16 || Cout == 32);
+  return X > 0 && Y % kFY == 0 && Z % kFZ == 0 && (Cout == 16 || Cout == 32);
 }
 
 int k_conv3d_first_tc(fm_ctx* ctx, const float* x, const bf16* w_packed, const float* bias, bf16* y, int N, int X, int Y,
@@ -418,7 +397,7 @@ int k_conv3d_first_tc_wgrad(fm_ctx* ctx, const float* x, const bf16* dy, float* 
   FM_TRY(fill(p, N, X, Y, Z, Cout));
   p.x = x;
   p.dw = dw;
-  PFN_encodeTiledF enc = get_encode_f();
+  EncodeTiledFn enc = encode_tiled();
   FM_CHECK(enc != nullptr, FM_ECUDA, "cuTensorMapEncodeTiled entry point not available");
   cuuint64_t dims[5] = {(cuuint64_t)Cout, (cuuint64_t)Z, (cuuint64_t)Y, (cuuint64_t)X, (cuuint64_t)N};
   cuuint64_t strides[4] = {(cuuint64_t)Cout * 2, (cuuint64_t)Z * Cout * 2, (cuuint64_t)Y * Z * Cout * 2,
@@ -426,7 +405,7 @@ int k_conv3d_first_tc_wgrad(fm_ctx* ctx, const float* x, const bf16* dy, float* 
   cuuint32_t box[5] = {(cuuint32_t)Cout, (cuuint32_t)kFZ, (cuuint32_t)kFY, 1, 1};
   cuuint32_t estr[5] = {1, 1, 1, 1, 1};
   CUresult r = enc(&p.tmDY, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, (void*)dy, dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, Cout == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B,
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for_row_bytes(Cout * 2),
                    CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   FM_CHECK(r == CUDA_SUCCESS, FM_ECUDA, "cuTensorMapEncodeTiled(first wgrad) failed: %d", (int)r);
   const size_t smem = first_smem(1, Cout);

@@ -19,7 +19,6 @@
 // Keras call site replaced: Conv3D(n_filters, kernel, padding='same') in create_convolution_block
 // (fetal_net/model/unet3d/unet.py:102) and its TF autodiff gradients.
 #include <algorithm>
-#include <mutex>
 
 #include "tc_ptx.cuh"
 
@@ -548,33 +547,10 @@ __global__ void __launch_bounds__(kThreadsTc, 1) conv3d_tc_wgrad_kernel(
 // ---------------------------------------------------------------------------------------------
 // host side: TMA descriptors and launch configuration
 // ---------------------------------------------------------------------------------------------
-typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*,
-                                    const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
-                                    const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                    CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-PFN_encodeTiled get_encode() {
-  static PFN_encodeTiled fn = nullptr;
-  static std::once_flag once;
-  std::call_once(once, [] {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
-        qres == cudaDriverEntryPointSuccess)
-      fn = (PFN_encodeTiled)p;
-  });
-  return fn;
-}
-
-CUtensorMapSwizzle swizzle_for(int row_bytes) {
-  return row_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B
-                          : (row_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
-}
-
 // 5-D map over a channels-last activation tensor [N][X][Y][Z][C] (bf16), box (cbox, bz, by, bx, 1)
 int make_act_tmap(CUtensorMap* tm, const bf16* base, int N, int X, int Y, int Z, int C, int cbox,
                   int bz, int by, int bx, int stride = 1, int stride_z = 0) {
-  PFN_encodeTiled enc = get_encode();
+  EncodeTiledFn enc = encode_tiled();
   FM_CHECK(enc != nullptr, FM_ECUDA, "cuTensorMapEncodeTiled entry point not available");
   cuuint64_t dims[5] = {(cuuint64_t)C, (cuuint64_t)Z, (cuuint64_t)Y, (cuuint64_t)X, (cuuint64_t)N};
   cuuint64_t strides[4] = {(cuuint64_t)C * 2, (cuuint64_t)Z * C * 2, (cuuint64_t)Y * Z * C * 2,
@@ -584,7 +560,7 @@ int make_act_tmap(CUtensorMap* tm, const bf16* base, int N, int X, int Y, int Z,
   cuuint32_t box[5] = {(cuuint32_t)cbox, (cuuint32_t)bz * stz, (cuuint32_t)by * st, (cuuint32_t)bx * st, 1};
   cuuint32_t estr[5] = {1, stz, st, st, 1};
   CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, (void*)base, dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for(cbox * 2), CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for_row_bytes(cbox * 2), CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   FM_CHECK(r == CUDA_SUCCESS, FM_ECUDA,
            "cuTensorMapEncodeTiled(act) failed: %d (N=%d %dx%dx%d C=%d box c=%d z=%d y=%d x=%d)", (int)r,
@@ -594,14 +570,14 @@ int make_act_tmap(CUtensorMap* tm, const bf16* base, int N, int X, int Y, int Z,
 
 // 3-D map over packed weights [Cout][taps][Ct] (bf16), box (kc, 1, nrows)
 int make_w_tmap(CUtensorMap* tm, const bf16* base, int Cout, int taps, int Ct, int kc, int nrows) {
-  PFN_encodeTiled enc = get_encode();
+  EncodeTiledFn enc = encode_tiled();
   FM_CHECK(enc != nullptr, FM_ECUDA, "cuTensorMapEncodeTiled entry point not available");
   cuuint64_t dims[3] = {(cuuint64_t)Ct, (cuuint64_t)taps, (cuuint64_t)Cout};
   cuuint64_t strides[2] = {(cuuint64_t)Ct * 2, (cuuint64_t)taps * Ct * 2};
   cuuint32_t box[3] = {(cuuint32_t)kc, 1, (cuuint32_t)nrows};
   cuuint32_t estr[3] = {1, 1, 1};
   CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, (void*)base, dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for(kc * 2), CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for_row_bytes(kc * 2), CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   FM_CHECK(r == CUDA_SUCCESS, FM_ECUDA, "cuTensorMapEncodeTiled(weights) failed: %d (Cout=%d taps=%d Ct=%d)",
            (int)r, Cout, taps, Ct);
@@ -627,7 +603,6 @@ void choose_box(int X, int Y, int Z, int* bx, int* by, int* bz) {
 bool chan_ok(int C) { return C > 0 && C % 16 == 0 && (C <= 64 ? (C == 16 || C == 32 || C == 64) : C % 64 == 0); }
 int chunk_of(int C) { return std::min(C, 64); }
 
-const int kMaxDynSmem = 227 * 1024;
 
 }  // namespace
 

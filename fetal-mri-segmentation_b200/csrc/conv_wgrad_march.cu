@@ -59,8 +59,6 @@ struct alignas(64) WgMarchParams {
   int Ct, cofs;        // dW layout [Cout][27][Ct], this source at channel offset cofs
   float* dw;
   float* db;           // bias gradient [Cout] (column sums of dY), or NULL
-  int debug;           // FETAL_B200_WGRAD_DEBUG ablation bits (timing only): 1 skip the flush atomics, 2 skip the MMAs,
-                       // 4 skip every plane (launch skeleton)
 };
 
 __global__ void __launch_bounds__(kThreadsW, 1) conv3d_wgrad_march_kernel(const __grid_constant__ WgMarchParams p) {
@@ -114,10 +112,9 @@ __global__ void __launch_bounds__(kThreadsW, 1) conv3d_wgrad_march_kernel(const 
   tmem_base = __shfl_sync(0xffffffffu, tmem_base, 0);
   const int warp_u = __shfl_sync(0xffffffffu, warp, 0);
 
-  // k-th segment / work unit of this CTA (see PlaneSplit in common.cuh)
+  // k-th work unit of this CTA (see PlaneSplit in common.cuh)
   auto next_seg = [&](int& it, int& n, int& iy, int& iz, int& xa, int& xb) -> bool {
     int col;
-    if (p.debug & 4) return false;  // ablation: the launch skeleton only (no planes at all)
     if (!plane_split_next(p.split, rank, p.ctas_per_pair, it, col, xa, xb)) return false;
     iz = col % p.nz;
     const int r = col / p.nz;
@@ -202,13 +199,11 @@ __global__ void __launch_bounds__(kThreadsW, 1) conv3d_wgrad_march_kernel(const 
         uint32_t a_lo = desc_lo(x_base + stage * p.xslot, a_sbo);          // M blocks (ky) one atom apart
         uint32_t bA = desc_lo(dy_base + rs * kDyTile, kDyTile);           // N blocks (kx) one ring slot apart
         const uint32_t dA = d_acc + j_lo * ncy;
-        if (!(p.debug & 2)) {
 #pragma unroll
-          for (int ks = 0; ks < (kBY * kBZ) / 16; ++ks) {
-            umma_bf16_lh_elect(dA, a_lo, a_hi32, bA, hi32, idA, 1u);
-            a_lo += a_kstep;
-            bA += kstep;
-          }
+        for (int ks = 0; ks < (kBY * kBZ) / 16; ++ks) {
+          umma_bf16_lh_elect(dA, a_lo, a_hi32, bA, hi32, idA, 1u);
+          a_lo += a_kstep;
+          bA += kstep;
         }
         umma_commit_elect(xempty_bar(stage));
         if (++sidx == (uint32_t)p.S3) {
@@ -302,12 +297,10 @@ __global__ void __launch_bounds__(kThreadsW, 1) conv3d_wgrad_march_kernel(const 
         const int col = c16 * 16;                      // kcy columns per kx block
         const int kx = 2 - col / p.kcy;
         const int tap = (kx * 3 + ky) * 3 + dz;
-        if (!(p.debug & 1)) {
 #pragma unroll
-          for (int j = 0; j < 16; ++j) {
-            const int co = coc * p.kcy + col % p.kcy + j;
-            atomicAdd(p.dw + ((int64_t)co * 27 + tap) * p.Ct + p.cofs + cic * p.kcx + ci, __uint_as_float(r[j]));
-          }
+        for (int j = 0; j < 16; ++j) {
+          const int co = coc * p.kcy + col % p.kcy + j;
+          atomicAdd(p.dw + ((int64_t)co * 27 + tap) * p.Ct + p.cofs + cic * p.kcx + ci, __uint_as_float(r[j]));
         }
       }
     }
@@ -321,24 +314,8 @@ __global__ void __launch_bounds__(kThreadsW, 1) conv3d_wgrad_march_kernel(const 
   }
 }
 
-typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                    const cuuint64_t*, const cuuint32_t*, const cuuint32_t*,
-                                    CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion,
-                                    CUtensorMapFloatOOBfill);
-PFN_encodeTiled get_encode_w() {
-  static PFN_encodeTiled fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
-        qres == cudaDriverEntryPointSuccess)
-      fn = (PFN_encodeTiled)p;
-  }
-  return fn;
-}
-
 int make_map(CUtensorMap* tm, const bf16* base, int N, int X, int Y, int Z, int C, int by, int cbox) {
-  PFN_encodeTiled enc = get_encode_w();
+  EncodeTiledFn enc = encode_tiled();
   FM_CHECK(enc != nullptr, FM_ECUDA, "cuTensorMapEncodeTiled entry point not available");
   cuuint64_t dims[5] = {(cuuint64_t)C, (cuuint64_t)Z, (cuuint64_t)Y, (cuuint64_t)X, (cuuint64_t)N};
   cuuint64_t strides[4] = {(cuuint64_t)C * 2, (cuuint64_t)Z * C * 2, (cuuint64_t)Y * Z * C * 2,
@@ -346,14 +323,11 @@ int make_map(CUtensorMap* tm, const bf16* base, int N, int X, int Y, int Z, int 
   cuuint32_t box[5] = {(cuuint32_t)cbox, (cuuint32_t)kBZ, (cuuint32_t)by, 1, 1};
   cuuint32_t estr[5] = {1, 1, 1, 1, 1};
   CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, (void*)base, dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, cbox == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B,
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for_row_bytes(cbox * 2),
                    CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   FM_CHECK(r == CUDA_SUCCESS, FM_ECUDA, "cuTensorMapEncodeTiled(wgrad march) failed: %d", (int)r);
   return FM_OK;
 }
-
-const int kMaxDynSmemW = 227 * 1024;
-const int kDefaultWgradGen = 1;
 
 }  // namespace
 
@@ -366,14 +340,6 @@ int conv_wgrad_march_supported(int X, int Y, int Z, int Cin, int Cout, int ksize
 
 int k_conv3d_wgrad_march(fm_ctx* ctx, const bf16* x, const bf16* dy, float* dw_packed, int N, int X, int Y, int Z,
                          int Cin, int Cin_total, int cin_ofs, int Cout, float* db) {
-  {
-    // FETAL_B200_WGRAD_GEN=3 selects the single-slab variant (A/B measurements); see conv_wgrad_march3.cu
-    static const int gen = [] {
-      const char* e = getenv("FETAL_B200_WGRAD_GEN");
-      return e ? atoi(e) : kDefaultWgradGen;
-    }();
-    if (gen == 3) return k_conv3d_wgrad_march3(ctx, x, dy, dw_packed, N, X, Y, Z, Cin, Cin_total, cin_ofs, Cout, db);
-  }
   FM_CHECK(conv_wgrad_march_supported(X, Y, Z, Cin, Cout, 3), FM_EINVAL,
            "conv3d wgrad march: unsupported shape %dx%dx%d Cin=%d Cout=%d", X, Y, Z, Cin, Cout);
   WgMarchParams p;
@@ -392,35 +358,23 @@ int k_conv3d_wgrad_march(fm_ctx* ctx, const bf16* x, const bf16* dy, float* dw_p
   p.cofs = cin_ofs;
   p.dw = dw_packed;
   p.db = db;
-  {
-    static const int dbg = [] {
-      const char* e = getenv("FETAL_B200_WGRAD_DEBUG");
-      return e ? atoi(e) : 0;
-    }();
-    p.debug = dbg;
-  }
   const int pairs = p.n_ci * p.n_co;
   const int cols = N * p.ny * p.nz;
   // CTAs per (ci, co) pair: at least 4 planes each; work units dealt as PlaneSplit describes (common.cuh)
   p.ctas_per_pair = std::max(1, std::min(ctx->num_sms / pairs, cols * X / 4));
   plane_split_setup(&p.split, cols, X, p.ctas_per_pair, 1.0);
-  if (p.split.mode == 1) p.ctas_per_pair = std::min(p.ctas_per_pair, cols * p.split.nxc);
+  p.ctas_per_pair = std::min(p.ctas_per_pair, cols * p.split.nxc);
   FM_TRY(make_map(&p.tmX, x, N, X, Y, Z, Cin, kBY + 128 / p.kcx - 1, p.kcx));  // halo + discarded M blocks
   FM_TRY(make_map(&p.tmDY, dy, N, X, Y, Z, Cout, kBY, p.kcy));
   // five slab slots per kz ring, packed at the slab's own 9728 bytes (512-byte aligned: enough for SWIZZLE_64B / 32B,
-  // whose pattern repeats every 512 / 256 bytes of shared-memory address); FETAL_B200_WGRAD_S3=4 is the 1 KB-aligned
-  // four-slot layout of the earlier captures
-  static const int s3_env = [] {
-    const char* e = getenv("FETAL_B200_WGRAD_S3");
-    return e ? atoi(e) : 5;
-  }();
-  p.S3 = s3_env == 4 ? 4 : 5;
-  p.xslot = p.S3 == 4 ? 10240u : kXSlotBytes;
+  // whose pattern repeats every 512 / 256 bytes of shared-memory address)
+  p.S3 = 5;
+  p.xslot = kXSlotBytes;
   const size_t smem = (size_t)3 * p.S3 * p.xslot + (size_t)(kDyRing + kDyMirror) * kDyTile + 1024 + 512;
   static bool attr_set = false;
   if (!attr_set) {
     FM_CUDA(cudaFuncSetAttribute(conv3d_wgrad_march_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 kMaxDynSmemW));
+                                 kMaxDynSmem));
     attr_set = true;
   }
   const double vox = (double)N * X * Y * Z;

@@ -262,4 +262,31 @@ __host__ __device__ constexpr uint32_t layout_code(int row_bytes) {
   return row_bytes == 128 ? 2u : (row_bytes == 64 ? 4u : 6u);
 }
 
+// ---------------------------------------------------------------------------------------------
+// host side
+// ---------------------------------------------------------------------------------------------
+constexpr int kMaxDynSmem = 227 * 1024;  // opt-in dynamic shared memory per block on sm_100
+
+// the same swizzle span for the TMA tensor map (rows of 128 / 64 / 32 bytes)
+inline CUtensorMapSwizzle swizzle_for_row_bytes(int row_bytes) {
+  return row_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B
+                          : (row_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
+}
+
+// cuTensorMapEncodeTiled through the runtime's driver entry-point query (no link against libcuda), looked up once;
+// nullptr when the driver does not provide it
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
+                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
+                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+inline EncodeTiledFn encode_tiled() {
+  static const EncodeTiledFn fn = [] {
+    void* p = nullptr;
+    cudaDriverEntryPointQueryResult qres;
+    const bool ok = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
+                    qres == cudaDriverEntryPointSuccess;
+    return ok ? (EncodeTiledFn)p : nullptr;
+  }();
+  return fn;
+}
+
 }  // namespace tcp

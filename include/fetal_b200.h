@@ -408,7 +408,12 @@ int fm_patchwise_predict_dp(fm_model* m, const float* vol, const int32_t vol_dim
  * All pointers are HOST pointers; tensors are channels-last (NDHWC) fp32 on the host and are
  * converted to the device storage type (bf16) inside the call. Each replaces one Keras layer
  * call of create_convolution_block / unet_model_3d (fetal_net/model/unet3d/unet.py:51,61,102,138)
- * or its TF autodiff counterpart. `impl`: 0 = tcgen05 tensor-core kernel, 1 = SIMT check kernel.
+ * or its TF autodiff counterpart. `impl`:
+ *   0 = tcgen05 per-tap tensor-core kernel;
+ *   1 = SIMT check kernel;
+ *   2 = plane-marching kernel, bit-reproducible issue order (predict / evaluate); for wgrad, the marching weight
+ *       gradient with the bias gradient folded in;
+ *   3 = plane-marching kernel in the issue order of training passes (fprop / dgrad; wgrad takes the SIMT kernel).
  */
 int fm_op_conv3d_fprop(fm_ctx* ctx, int impl, const float* x, const float* x2, const float* w_keras,
                        const float* bias, int N, int X, int Y, int Z, int C1, int C2, int Cout,

@@ -122,18 +122,3 @@ def test_keras_adam(ctx):
     ok, worst = gc.adam_case(ctx)
     assert ok, worst
 
-
-def test_wgrad_march_single_slab_variant_in_subprocess():
-    """conv_wgrad_march3.cu (ONE z-haloed X slab per plane, the kz tap as a start-address offset of the A descriptor on
-    10-row y-rows - valid because TMA and UMMA both swizzle on absolute shared-memory address bits;
-    FETAL_B200_WGRAD_GEN=3) is kept as a measured alternative to the default kernel: same parity bar, run in a
-    subprocess because the generation is read from the environment once per process."""
-    import os
-    import subprocess
-    import sys
-    env = dict(os.environ, FETAL_B200_WGRAD_GEN="3")
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.join(root, "tests", "test_gpu_ops.py"), "-q", "-m", "gpu",
-                        "-k", "wgrad_march and not single_slab", "-x", "-p", "no:cacheprovider"],
-                       env=env, cwd=root, capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
