@@ -1342,6 +1342,12 @@ struct IsenseeBuild {
 };
 static int build_isensee(fm_ctx* ctx, const IsenseeBuild* spec, fm_model** out);
 
+// whether the data gradient towards a source of cs channels (first source c1 channels) runs on the marching kernel;
+// decided once per layer when the model is built (X, Y, Z = the extent the dgrad runs at)
+static bool isensee_dgrad_marches(int X, int Y, int Z, int c1, int cs, int cout, int k) {
+  return k == 3 && c1 >= 16 && conv_march_supported(X, Y, Z, cout, 0, cs, k);
+}
+
 extern "C" int fm_model_create_isensee3d(fm_ctx* ctx, const fm_isensee3d_spec* spec, fm_model** out) {
   FM_CHECK(ctx && spec && out, FM_EINVAL, "fm_model_create_isensee3d: NULL argument");
   FM_CHECK(spec->in_channels == 1 && spec->n_labels == 1, FM_EINVAL, "isensee: in_channels and n_labels must be 1");
@@ -1473,7 +1479,7 @@ static int build_isensee(fm_ctx* ctx, const IsenseeBuild* spec, fm_model** out) 
         FM_CUDA(cudaMalloc((void**)&l.w_mf[s], (size_t)conv_march_pack_elems(cs[s], l.cout) * sizeof(bf16)));
     }
     for (int s = 0; s < (l.c2 ? 2 : 1); ++s)
-      if (conv_march_supported(Xd, Yd, Zd, l.cout, 0, cs[s], l.k)) {
+      if (isensee_dgrad_marches(Xd, Yd, Zd, l.c1, cs[s], l.cout, l.k)) {
         l.march_d[s] = true;
         FM_CUDA(cudaMalloc((void**)&l.w_md[s], (size_t)conv_march_pack_elems(l.cout, cs[s]) * sizeof(bf16)));
       }
@@ -1663,39 +1669,48 @@ static int forward_isensee(fm_model* m, int B) {
 // stride-1 dgrad / wgrad over the zero-inserted gradient (k_zero_insert), one level finer.
 // Gradients are produced in reverse layer-creation order, so the all-reduce buckets work as for the plain U-Net.
 // ---------------------------------------------------------------------------------------------
+// Kernel choice of the Isensee weight / data gradients, shared with the per-op hook fm_op_conv_strided so that the
+// hook runs what the model runs. Weight gradient of one source (cs of cin_total channels at cofs): marching, per-tap
+// tensor-core or SIMT kernel.
+static int isensee_wgrad_route(fm_ctx* ctx, const bf16* x, const bf16* dy, float* dw, int B, int X, int Y, int Z, int cs,
+                               int cin_total, int cofs, int cout, int k) {
+  if (conv_wgrad_march_supported(X, Y, Z, cs, cout, k))
+    return k_conv3d_wgrad_march(ctx, x, dy, dw, B, X, Y, Z, cs, cin_total, cofs, cout);
+  if (conv_tc_supported(cs, 0, cout, k))
+    return k_conv3d_tc_wgrad(ctx, x, dy, dw, B, X, Y, Z, cs, cin_total, cofs, cout, k);
+  return k_conv3d_simt_wgrad(ctx, x, 0, dy, dw, B, X, Y, Z, cs, cin_total, cofs, cout, k);
+}
+
+// data gradient towards one source: w_md = its marching pack (null: per-tap tensor-core or SIMT kernel on w_d)
+static int isensee_dgrad_route(fm_ctx* ctx, const bf16* dy, const bf16* w_md, const bf16* w_d, bf16* dx, int B, int X,
+                               int Y, int Z, int cout, int cs, int k, bool reproducible) {
+  if (w_md != nullptr)
+    return k_conv3d_march(ctx, dy, nullptr, w_md, nullptr, nullptr, dx, nullptr, B, X, Y, Z, cout, 0, cs, 0, cs, 0,
+                          reproducible);
+  if (conv_tc_supported(cout, 0, cs, k))
+    return k_conv3d_tc_fprop(ctx, dy, nullptr, w_d, nullptr, dx, nullptr, B, X, Y, Z, cout, 0, cs, k, 0, cs, 0);
+  return k_conv3d_simt_fprop(ctx, dy, 0, nullptr, w_d, nullptr, dx, nullptr, B, X, Y, Z, cout, 0, cs, k, 0, nullptr);
+}
+
 static int is_wgrad(fm_model* m, const Layer& l, int level, const bf16* x1, const bf16* x2, const bf16* dy, int B) {
-  fm_ctx* ctx = m->ctx;
   const Dims5 d = m->dims(level, l.cout, B);
-  float* dw = m->grads + l.w_off;
   const bf16* xs[2] = {x1, x2};
   const int cs[2] = {l.c1, l.c2};
   int cofs = 0;
   // no bias gradient here: every Isensee conv feeds an InstanceNormalization, which removes a per-channel constant -
   // the gradient of such a bias is exactly zero (the heads, which have a live bias, are 1x1x1 kernels handled elsewhere)
   for (int s = 0; s < (l.c2 ? 2 : 1); ++s) {
-    if (conv_wgrad_march_supported(d.X, d.Y, d.Z, cs[s], l.cout, l.k))
-      FM_TRY(k_conv3d_wgrad_march(ctx, xs[s], dy, dw, B, d.X, d.Y, d.Z, cs[s], l.cin(), cofs, l.cout));
-    else if (conv_tc_supported(cs[s], 0, l.cout, l.k))
-      FM_TRY(k_conv3d_tc_wgrad(ctx, xs[s], dy, dw, B, d.X, d.Y, d.Z, cs[s], l.cin(), cofs, l.cout, l.k));
-    else
-      FM_TRY(k_conv3d_simt_wgrad(ctx, xs[s], 0, dy, dw, B, d.X, d.Y, d.Z, cs[s], l.cin(), cofs, l.cout, l.k));
+    FM_TRY(isensee_wgrad_route(m->ctx, xs[s], dy, m->grads + l.w_off, B, d.X, d.Y, d.Z, cs[s], l.cin(), cofs, l.cout,
+                               l.k));
     cofs += cs[s];
   }
   return FM_OK;
 }
 
 static int is_dgrad(fm_model* m, const Layer& l, int level, int src, const bf16* dy, bf16* dx, int B) {
-  fm_ctx* ctx = m->ctx;
   const Dims5 d = m->dims(level, l.cout, B);
-  const int cs = src == 0 ? l.c1 : l.c2;
-  const bf16* wd = src == 0 ? l.w_d0 : l.w_d1;
-  if (l.march_d[src])
-    return k_conv3d_march(ctx, dy, nullptr, l.w_md[src], nullptr, nullptr, dx, nullptr, B, d.X, d.Y, d.Z, l.cout, 0, cs, 0,
-                          cs, 0, reproducible_pass(m));
-  if (conv_tc_supported(l.cout, 0, cs, l.k))
-    return k_conv3d_tc_fprop(ctx, dy, nullptr, wd, nullptr, dx, nullptr, B, d.X, d.Y, d.Z, l.cout, 0, cs, l.k, 0, cs, 0);
-  return k_conv3d_simt_fprop(ctx, dy, 0, nullptr, wd, nullptr, dx, nullptr, B, d.X, d.Y, d.Z, l.cout, 0, cs, l.k, 0,
-                             nullptr);
+  return isensee_dgrad_route(m->ctx, dy, l.march_d[src] ? l.w_md[src] : nullptr, src == 0 ? l.w_d0 : l.w_d1, dx, B, d.X,
+                             d.Y, d.Z, l.cout, src == 0 ? l.c1 : l.c2, l.k, reproducible_pass(m));
 }
 
 // norm + activation backward of block `li` -> m->gIsRaw (gradient of the raw conv output); gamma/beta/bias gradients
@@ -2751,14 +2766,13 @@ extern "C" int fm_op_conv3d_fprop(fm_ctx* ctx, int impl, const float* x, const f
   return s.down_bf16(dy, vox * Cout, y);
 }
 
-extern "C" int fm_op_conv3d_dgrad(fm_ctx* ctx, int impl, const float* dy, const float* w_keras,
-                                  const float* mask, int N, int X, int Y, int Z, int Cin, int Cout,
-                                  float* dx) {
-  FM_CHECK(ctx && dy && w_keras && dx, FM_EINVAL, "fm_op_conv3d_dgrad: NULL argument");
+extern "C" int fm_op_conv_dgrad(fm_ctx* ctx, int impl, const float* dy, const float* w_keras, const float* mask, int N,
+                                int X, int Y, int Z, int Cin, int Cout, int ksize, float* dx) {
+  FM_CHECK(ctx && dy && w_keras && dx, FM_EINVAL, "fm_op_conv_dgrad: NULL argument");
   FM_CUDA(cudaSetDevice(ctx->device));
   OpScratch s(ctx);
   const size_t vox = (size_t)N * X * Y * Z;
-  const int ksize = 3, taps = 27;
+  const int taps = kext_taps(ksize);
   std::vector<float> packed((size_t)Cout * taps * Cin);
   keras_to_packed(w_keras, packed.data(), ksize, Cin, Cout);
   float* dwm = nullptr;
@@ -2785,13 +2799,13 @@ extern "C" int fm_op_conv3d_dgrad(fm_ctx* ctx, int impl, const float* dy, const 
   return s.down_bf16(ddx, vox * Cin, dx);
 }
 
-extern "C" int fm_op_conv3d_wgrad(fm_ctx* ctx, int impl, const float* x, const float* dy, int N, int X,
-                                  int Y, int Z, int Cin, int Cout, float* dw_keras, float* dbias) {
-  FM_CHECK(ctx && x && dy && dw_keras, FM_EINVAL, "fm_op_conv3d_wgrad: NULL argument");
+extern "C" int fm_op_conv_wgrad(fm_ctx* ctx, int impl, const float* x, const float* dy, int N, int X, int Y, int Z,
+                                int Cin, int Cout, int ksize, float* dw_keras, float* dbias) {
+  FM_CHECK(ctx && x && dy && dw_keras, FM_EINVAL, "fm_op_conv_wgrad: NULL argument");
   FM_CUDA(cudaSetDevice(ctx->device));
   OpScratch s(ctx);
   const size_t vox = (size_t)N * X * Y * Z;
-  const int ksize = 3, taps = 27;
+  const int taps = kext_taps(ksize);
   bf16 *dx = nullptr, *ddy = nullptr;
   float *dw = nullptr, *db = nullptr;
   FM_TRY(s.up_bf16(x, vox * Cin, &dx));
@@ -2814,6 +2828,16 @@ extern "C" int fm_op_conv3d_wgrad(fm_ctx* ctx, int impl, const float* x, const f
   FM_CUDA(cudaStreamSynchronize(ctx->stream));
   packed_to_keras(packed.data(), dw_keras, ksize, Cin, Cout);
   return FM_OK;
+}
+
+// the 3x3x3 forms of the two hooks above
+extern "C" int fm_op_conv3d_dgrad(fm_ctx* ctx, int impl, const float* dy, const float* w_keras, const float* mask, int N,
+                                  int X, int Y, int Z, int Cin, int Cout, float* dx) {
+  return fm_op_conv_dgrad(ctx, impl, dy, w_keras, mask, N, X, Y, Z, Cin, Cout, 3, dx);
+}
+extern "C" int fm_op_conv3d_wgrad(fm_ctx* ctx, int impl, const float* x, const float* dy, int N, int X, int Y, int Z,
+                                  int Cin, int Cout, float* dw_keras, float* dbias) {
+  return fm_op_conv_wgrad(ctx, impl, x, dy, N, X, Y, Z, Cin, Cout, 3, dw_keras, dbias);
 }
 
 // First convolution of the network (one fp32 input channel): y = act(conv3x3x3(x) + bias) and / or the weight gradient
@@ -2918,57 +2942,79 @@ extern "C" int fm_op_conv3d_up_bwd(fm_ctx* ctx, const float* coarse, const float
   return FM_OK;
 }
 
-extern "C" int fm_op_maxpool3d(fm_ctx* ctx, const float* x, int N, int X, int Y, int Z, int C, float* y) {
-  FM_CHECK(ctx && x && y, FM_EINVAL, "fm_op_maxpool3d: NULL argument");
+// pz = pooling factor along z: 2 (MaxPooling3D / UpSampling3D) or 1 (the 2D models); X, Y, Z = the finer extent for
+// the pool hooks, the coarser one for the upsample hooks
+extern "C" int fm_op_maxpool(fm_ctx* ctx, const float* x, int N, int X, int Y, int Z, int C, int pz, float* y) {
+  FM_CHECK(ctx && x && y, FM_EINVAL, "fm_op_maxpool: NULL argument");
+  FM_CHECK(pz == 1 || pz == 2, FM_EINVAL, "fm_op_maxpool: pz=%d", pz);
   FM_CUDA(cudaSetDevice(ctx->device));
   OpScratch s(ctx);
-  const size_t n = (size_t)N * X * Y * Z * C;
+  const size_t n = (size_t)N * X * Y * Z * C, nc = n / (4 * pz);
   bf16 *dx = nullptr, *dy = nullptr;
   FM_TRY(s.up_bf16(x, n, &dx));
-  FM_TRY(s.alloc(&dy, n / 8));
-  FM_TRY(k_maxpool3d_fwd(ctx, dx, dy, Dims5{N, X, Y, Z, C}));
-  return s.down_bf16(dy, n / 8, y);
+  FM_TRY(s.alloc(&dy, nc));
+  FM_TRY(k_maxpool3d_fwd(ctx, dx, dy, Dims5{N, X, Y, Z, C}, pz));
+  return s.down_bf16(dy, nc, y);
 }
 
-extern "C" int fm_op_maxpool3d_bwd(fm_ctx* ctx, const float* x, const float* dy, const float* dskip,
-                                   int N, int X, int Y, int Z, int C, float* dx) {
-  FM_CHECK(ctx && x && dy && dx, FM_EINVAL, "fm_op_maxpool3d_bwd: NULL argument");
+extern "C" int fm_op_maxpool_bwd(fm_ctx* ctx, const float* x, const float* dy, const float* dskip,
+                                   int N, int X, int Y, int Z, int C, int pz, float* dx) {
+  FM_CHECK(ctx && x && dy && dx, FM_EINVAL, "fm_op_maxpool_bwd: NULL argument");
+  FM_CHECK(pz == 1 || pz == 2, FM_EINVAL, "fm_op_maxpool_bwd: pz=%d", pz);
   FM_CUDA(cudaSetDevice(ctx->device));
   OpScratch s(ctx);
-  const size_t n = (size_t)N * X * Y * Z * C;
+  const size_t n = (size_t)N * X * Y * Z * C, nc = n / (4 * pz);
   bf16 *bx = nullptr, *bdy = nullptr, *bsk = nullptr, *bdx = nullptr;
   FM_TRY(s.up_bf16(x, n, &bx));
-  FM_TRY(s.up_bf16(dy, n / 8, &bdy));
+  FM_TRY(s.up_bf16(dy, nc, &bdy));
   if (dskip) FM_TRY(s.up_bf16(dskip, n, &bsk));
   FM_TRY(s.alloc(&bdx, n));
-  FM_TRY(k_maxpool3d_bwd(ctx, bx, bdy, bsk, bdx, Dims5{N, X, Y, Z, C}, 1));
+  FM_TRY(k_maxpool3d_bwd(ctx, bx, bdy, bsk, bdx, Dims5{N, X, Y, Z, C}, 1, pz));
   return s.down_bf16(bdx, n, dx);
 }
 
-extern "C" int fm_op_upsample3d(fm_ctx* ctx, const float* x, int N, int X, int Y, int Z, int C, float* y) {
-  FM_CHECK(ctx && x && y, FM_EINVAL, "fm_op_upsample3d: NULL argument");
+extern "C" int fm_op_upsample(fm_ctx* ctx, const float* x, int N, int X, int Y, int Z, int C, int pz, float* y) {
+  FM_CHECK(ctx && x && y, FM_EINVAL, "fm_op_upsample: NULL argument");
+  FM_CHECK(pz == 1 || pz == 2, FM_EINVAL, "fm_op_upsample: pz=%d", pz);
   FM_CUDA(cudaSetDevice(ctx->device));
   OpScratch s(ctx);
-  const size_t n = (size_t)N * X * Y * Z * C;
+  const size_t n = (size_t)N * X * Y * Z * C, nf = n * 4 * pz;
   bf16 *dx = nullptr, *dy = nullptr;
   FM_TRY(s.up_bf16(x, n, &dx));
-  FM_TRY(s.alloc(&dy, n * 8));
-  FM_TRY(k_upsample3d_fwd(ctx, dx, dy, Dims5{N, X, Y, Z, C}));
-  return s.down_bf16(dy, n * 8, y);
+  FM_TRY(s.alloc(&dy, nf));
+  FM_TRY(k_upsample3d_fwd(ctx, dx, dy, Dims5{N, X, Y, Z, C}, pz));
+  return s.down_bf16(dy, nf, y);
 }
 
-extern "C" int fm_op_upsample3d_bwd(fm_ctx* ctx, const float* dy, const float* act, int N, int X, int Y,
-                                    int Z, int C, float* dx) {
-  FM_CHECK(ctx && dy && dx, FM_EINVAL, "fm_op_upsample3d_bwd: NULL argument");
+extern "C" int fm_op_upsample_bwd(fm_ctx* ctx, const float* dy, const float* act, int N, int X, int Y,
+                                    int Z, int C, int pz, float* dx) {
+  FM_CHECK(ctx && dy && dx, FM_EINVAL, "fm_op_upsample_bwd: NULL argument");
+  FM_CHECK(pz == 1 || pz == 2, FM_EINVAL, "fm_op_upsample_bwd: pz=%d", pz);
   FM_CUDA(cudaSetDevice(ctx->device));
   OpScratch s(ctx);
   const size_t n = (size_t)N * X * Y * Z * C;  // coarse elements
   bf16 *bdy = nullptr, *bact = nullptr, *bdx = nullptr;
-  FM_TRY(s.up_bf16(dy, n * 8, &bdy));
+  FM_TRY(s.up_bf16(dy, n * 4 * pz, &bdy));
   if (act) FM_TRY(s.up_bf16(act, n, &bact));
   FM_TRY(s.alloc(&bdx, n));
-  FM_TRY(k_upsample3d_bwd(ctx, bdy, bact, bdx, Dims5{N, X, Y, Z, C}, C, 0));
+  FM_TRY(k_upsample3d_bwd(ctx, bdy, bact, bdx, Dims5{N, X, Y, Z, C}, C, 0, pz));
   return s.down_bf16(bdx, n, dx);
+}
+
+// the MaxPooling3D / UpSampling3D forms (pz = 2) of the four hooks above
+extern "C" int fm_op_maxpool3d(fm_ctx* ctx, const float* x, int N, int X, int Y, int Z, int C, float* y) {
+  return fm_op_maxpool(ctx, x, N, X, Y, Z, C, 2, y);
+}
+extern "C" int fm_op_maxpool3d_bwd(fm_ctx* ctx, const float* x, const float* dy, const float* dskip, int N, int X, int Y,
+                                   int Z, int C, float* dx) {
+  return fm_op_maxpool_bwd(ctx, x, dy, dskip, N, X, Y, Z, C, 2, dx);
+}
+extern "C" int fm_op_upsample3d(fm_ctx* ctx, const float* x, int N, int X, int Y, int Z, int C, float* y) {
+  return fm_op_upsample(ctx, x, N, X, Y, Z, C, 2, y);
+}
+extern "C" int fm_op_upsample3d_bwd(fm_ctx* ctx, const float* dy, const float* act, int N, int X, int Y, int Z, int C,
+                                    float* dx) {
+  return fm_op_upsample_bwd(ctx, dy, act, N, X, Y, Z, C, 2, dx);
 }
 
 extern "C" int fm_op_dice(fm_ctx* ctx, const float* p, const float* t, int64_t n, double sums[8],
@@ -3033,6 +3079,349 @@ extern "C" int fm_op_adam(fm_ctx* ctx, float* p, const float* g, float* mm, floa
   FM_CUDA(cudaMemcpyAsync(p, dp, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
   FM_CUDA(cudaMemcpyAsync(mm, dm, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
   FM_CUDA(cudaMemcpyAsync(vv, dv, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  FM_CUDA(cudaStreamSynchronize(ctx->stream));
+  return FM_OK;
+}
+
+// Scratch of the normalisation kernels: per-(sample, block) partials for at most 1024 blocks per sample (norm_blocks)
+// plus the per-(sample, channel) coefficients of the forward (2) or backward (4) pass.
+static size_t norm_scratch_floats(int N, int C) { return (size_t)N * C * (2 * 1024 + 4); }
+
+// InstanceNormalization + LeakyReLU(0.3) of the Isensee blocks (isensee_block): y = act(norm(x)) * chan_scale + add.
+// add [N,vox,C] and chan_scale [N,C] may be NULL; stats [N,C,2] (optional) = (mean, 1/(std + eps)).
+extern "C" int fm_op_instnorm_lrelu(fm_ctx* ctx, const float* x, const float* gamma, const float* beta, const float* add,
+                                    const float* chan_scale, int N, int64_t vox, int C, float* y, float* stats) {
+  FM_CHECK(ctx && x && gamma && beta && y && N > 0 && vox > 0, FM_EINVAL, "fm_op_instnorm_lrelu: bad argument");
+  FM_CUDA(cudaSetDevice(ctx->device));
+  OpScratch s(ctx);
+  const size_t n = (size_t)N * vox * C, ns = norm_scratch_floats(N, C);
+  bf16 *bx = nullptr, *badd = nullptr, *by = nullptr;
+  float *dg = nullptr, *db = nullptr, *dcs = nullptr, *scratch = nullptr, *dst = nullptr;
+  FM_TRY(s.up_bf16(x, n, &bx));
+  if (add) FM_TRY(s.up_bf16(add, n, &badd));
+  if (chan_scale) FM_TRY(s.up_f32(chan_scale, (size_t)N * C, &dcs));
+  FM_TRY(s.up_f32(gamma, C, &dg));
+  FM_TRY(s.up_f32(beta, C, &db));
+  FM_TRY(s.alloc(&scratch, ns));
+  FM_TRY(s.alloc(&dst, (size_t)N * C * 2));
+  FM_TRY(s.alloc(&by, n));
+  FM_TRY(k_instnorm_lrelu(ctx, bx, dg, db, badd, by, N, vox, C, scratch, ns, dst, dcs));
+  if (stats) FM_CUDA(cudaMemcpyAsync(stats, dst, (size_t)N * C * 2 * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  return s.down_bf16(by, n, y);
+}
+
+// Its backward (is_block_bwd): the forward runs first for the device's own statistics; gy2 (the second incoming
+// gradient of a fan-out) and chan_scale may be NULL. dgamma / dbeta [C] are zeroed here (the kernel accumulates).
+extern "C" int fm_op_instnorm_lrelu_bwd(fm_ctx* ctx, const float* x, const float* gamma, const float* beta,
+                                        const float* gy, const float* gy2, const float* chan_scale, int N, int64_t vox,
+                                        int C, float* dx, float* dgamma, float* dbeta) {
+  FM_CHECK(ctx && x && gamma && beta && gy && dx && dgamma && dbeta && N > 0 && vox > 0, FM_EINVAL,
+           "fm_op_instnorm_lrelu_bwd: bad argument");
+  FM_CUDA(cudaSetDevice(ctx->device));
+  OpScratch s(ctx);
+  const size_t n = (size_t)N * vox * C, ns = norm_scratch_floats(N, C);
+  bf16 *bx = nullptr, *bgy = nullptr, *bgy2 = nullptr, *by = nullptr, *bdx = nullptr;
+  float *dg = nullptr, *db = nullptr, *dcs = nullptr, *scratch = nullptr, *dst = nullptr, *dgg = nullptr;
+  FM_TRY(s.up_bf16(x, n, &bx));
+  FM_TRY(s.up_bf16(gy, n, &bgy));
+  if (gy2) FM_TRY(s.up_bf16(gy2, n, &bgy2));
+  if (chan_scale) FM_TRY(s.up_f32(chan_scale, (size_t)N * C, &dcs));
+  FM_TRY(s.up_f32(gamma, C, &dg));
+  FM_TRY(s.up_f32(beta, C, &db));
+  FM_TRY(s.alloc(&scratch, ns));
+  FM_TRY(s.alloc(&dst, (size_t)N * C * 2));
+  FM_TRY(s.alloc(&dgg, 2 * (size_t)C));
+  FM_TRY(s.alloc(&by, n));
+  FM_TRY(s.alloc(&bdx, n));
+  FM_TRY(k_instnorm_lrelu(ctx, bx, dg, db, nullptr, by, N, vox, C, scratch, ns, dst, dcs));
+  FM_TRY(k_zero(ctx, dgg, 2 * (size_t)C * 4));
+  FM_TRY(k_instnorm_lrelu_bwd(ctx, bx, dst, dg, db, bgy, bgy2, dcs, bdx, dgg, dgg + C, N, vox, C, scratch, ns));
+  FM_CUDA(cudaMemcpyAsync(dgamma, dgg, (size_t)C * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  FM_CUDA(cudaMemcpyAsync(dbeta, dgg + C, (size_t)C * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  return s.down_bf16(bdx, n, dx);
+}
+
+// BatchNormalization + ReLU (bn_block_fwd): training = batch statistics, and moving_mean / moving_var [C] (in/out)
+// take the Keras moving-average step; inference = the moving statistics.
+extern "C" int fm_op_batchnorm_relu(fm_ctx* ctx, int training, const float* x, const float* gamma, const float* beta,
+                                    float* moving_mean, float* moving_var, int N, int64_t vox, int C, float* y) {
+  FM_CHECK(ctx && x && gamma && beta && moving_mean && moving_var && y && N > 0 && vox > 0, FM_EINVAL,
+           "fm_op_batchnorm_relu: bad argument");
+  FM_CUDA(cudaSetDevice(ctx->device));
+  OpScratch s(ctx);
+  const size_t n = (size_t)N * vox * C, ns = norm_scratch_floats(N, C);
+  bf16 *bx = nullptr, *by = nullptr;
+  float *dg = nullptr, *db = nullptr, *dmm = nullptr, *dmv = nullptr, *scratch = nullptr, *dst = nullptr;
+  FM_TRY(s.up_bf16(x, n, &bx));
+  FM_TRY(s.up_f32(gamma, C, &dg));
+  FM_TRY(s.up_f32(beta, C, &db));
+  FM_TRY(s.up_f32(moving_mean, C, &dmm));
+  FM_TRY(s.up_f32(moving_var, C, &dmv));
+  FM_TRY(s.alloc(&scratch, ns));
+  FM_TRY(s.alloc(&dst, (size_t)N * C * 2));
+  FM_TRY(s.alloc(&by, n));
+  FM_TRY(k_batchnorm_relu(ctx, bx, dg, db, dmm, dmv, by, N, vox, C, scratch, ns, training ? dst : nullptr,
+                          training ? 1 : 0));
+  FM_CUDA(cudaMemcpyAsync(moving_mean, dmm, (size_t)C * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  FM_CUDA(cudaMemcpyAsync(moving_var, dmv, (size_t)C * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  return s.down_bf16(by, n, y);
+}
+
+// Its backward (bn_block_bwd) after a training forward that supplies the batch statistics; gy2 may be NULL.
+// dgamma / dbeta [C] are zeroed here (the kernel adds into them).
+extern "C" int fm_op_batchnorm_relu_bwd(fm_ctx* ctx, const float* x, const float* gamma, const float* beta,
+                                        const float* gy, const float* gy2, int N, int64_t vox, int C, float* dx,
+                                        float* dgamma, float* dbeta) {
+  FM_CHECK(ctx && x && gamma && beta && gy && dx && dgamma && dbeta && N > 0 && vox > 0, FM_EINVAL,
+           "fm_op_batchnorm_relu_bwd: bad argument");
+  FM_CUDA(cudaSetDevice(ctx->device));
+  OpScratch s(ctx);
+  const size_t n = (size_t)N * vox * C, ns = norm_scratch_floats(N, C);
+  bf16 *bx = nullptr, *bgy = nullptr, *bgy2 = nullptr, *by = nullptr, *bdx = nullptr;
+  float *dg = nullptr, *db = nullptr, *scratch = nullptr, *dst = nullptr, *dgg = nullptr;
+  FM_TRY(s.up_bf16(x, n, &bx));
+  FM_TRY(s.up_bf16(gy, n, &bgy));
+  if (gy2) FM_TRY(s.up_bf16(gy2, n, &bgy2));
+  FM_TRY(s.up_f32(gamma, C, &dg));
+  FM_TRY(s.up_f32(beta, C, &db));
+  FM_TRY(s.alloc(&scratch, ns));
+  FM_TRY(s.alloc(&dst, (size_t)N * C * 2));
+  FM_TRY(s.alloc(&dgg, 2 * (size_t)C));
+  FM_TRY(s.alloc(&by, n));
+  FM_TRY(s.alloc(&bdx, n));
+  FM_TRY(k_batchnorm_relu(ctx, bx, dg, db, nullptr, nullptr, by, N, vox, C, scratch, ns, dst, 1));
+  FM_TRY(k_zero(ctx, dgg, 2 * (size_t)C * 4));
+  FM_TRY(k_batchnorm_relu_bwd(ctx, bx, dst, dg, db, bgy, bgy2, bdx, dgg, dgg + C, N, vox, C, scratch, ns));
+  FM_CUDA(cudaMemcpyAsync(dgamma, dgg, (size_t)C * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  FM_CUDA(cudaMemcpyAsync(dbeta, dgg + C, (size_t)C * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  return s.down_bf16(bdx, n, dx);
+}
+
+// Stride-2 TF-'SAME' convolution of the Isensee in-convs (isensee_block, relu 0): x [N,Xin,Yin,Zin,Cin] (even extents;
+// Zin is not strided for ksize 31), w_keras (3,3[,3],Cin,Cout), y [N,Xin/2,Yin/2,Zout,Cout]. With dy (same shape as y):
+// the backward of backward_isensee - zero insertion, then the stride-1 data gradient dx [N,Xin,Yin,Zin,Cin] and weight
+// gradient dw_keras on the kernels the model picks for that extent.
+extern "C" int fm_op_conv_strided(fm_ctx* ctx, const float* x, const float* w_keras, const float* bias, int N, int Xin,
+                                  int Yin, int Zin, int Cin, int Cout, int ksize, float* y, const float* dy, float* dx,
+                                  float* dw_keras) {
+  FM_CHECK(ctx && x && w_keras && (ksize == 3 || ksize == 31), FM_EINVAL, "fm_op_conv_strided: bad argument");
+  FM_CHECK(Xin % 2 == 0 && Yin % 2 == 0 && (ksize == 31 || Zin % 2 == 0), FM_EINVAL, "fm_op_conv_strided: odd extent");
+  FM_CHECK(!dy || (dx && dw_keras), FM_EINVAL, "fm_op_conv_strided: dy needs dx and dw_keras");
+  FM_CUDA(cudaSetDevice(ctx->device));
+  OpScratch s(ctx);
+  const int pz = ksize == 31 ? 1 : 2, X = Xin / 2, Y = Yin / 2, Z = Zin / pz, taps = kext_taps(ksize);
+  const size_t vin = (size_t)N * Xin * Yin * Zin, vout = (size_t)N * X * Y * Z, wn = (size_t)Cout * taps * Cin;
+  std::vector<float> packed(wn);
+  keras_to_packed(w_keras, packed.data(), ksize, Cin, Cout);
+  bf16 *bx = nullptr, *wf = nullptr, *wd = nullptr;
+  float* wm = nullptr;
+  FM_TRY(s.up_bf16(x, vin * Cin, &bx));
+  FM_TRY(s.up_f32(packed.data(), wn, &wm));
+  FM_TRY(s.alloc(&wf, wn));
+  FM_TRY(s.alloc(&wd, wn));
+  FM_TRY(k_repack_weights(ctx, wm, wf, wd, nullptr, Cout, taps, Cin, 0));
+  if (y) {
+    FM_CHECK(conv_tc_supported(Cin, 0, Cout, ksize), FM_EINVAL, "fm_op_conv_strided: no strided kernel for %d -> %d",
+             Cin, Cout);
+    bf16* by = nullptr;
+    float* db = nullptr;
+    if (bias) FM_TRY(s.up_f32(bias, Cout, &db));
+    FM_TRY(s.alloc(&by, vout * Cout));
+    FM_TRY(k_conv3d_tc_fprop(ctx, bx, nullptr, wf, db, by, nullptr, N, X, Y, Z, Cin, 0, Cout, ksize, 0, Cout, 0, 2, Xin,
+                             Yin, Zin));
+    FM_TRY(s.down_bf16(by, vout * Cout, y));
+  }
+  if (dy) {
+    bf16 *bdy = nullptr, *bz = nullptr, *bdx = nullptr, *wmd = nullptr;
+    float* dw = nullptr;
+    FM_TRY(s.up_bf16(dy, vout * Cout, &bdy));
+    FM_TRY(s.alloc(&bz, vin * Cout));
+    FM_TRY(s.alloc(&bdx, vin * Cin));
+    FM_TRY(s.alloc(&dw, wn));
+    FM_TRY(k_zero(ctx, dw, wn * 4));
+    FM_TRY(k_zero_insert(ctx, bdy, bz, Dims5{N, X, Y, Z, Cout}, pz));
+    FM_TRY(isensee_wgrad_route(ctx, bx, bz, dw, N, Xin, Yin, Zin, Cin, Cin, 0, Cout, ksize));
+    if (isensee_dgrad_marches(Xin, Yin, Zin, Cin, Cin, Cout, ksize)) {
+      FM_TRY(s.alloc(&wmd, (size_t)conv_march_pack_elems(Cout, Cin)));
+      FM_TRY(k_repack_march(ctx, wd, wmd, Cin, Cout, 0, Cout, conv_march_kc(Cout, 0, Cin, Cout)));
+    }
+    FM_TRY(isensee_dgrad_route(ctx, bz, wmd, wd, bdx, N, Xin, Yin, Zin, Cout, Cin, ksize, false));
+    FM_TRY(s.down_bf16(bdx, vin * Cin, dx));
+    std::vector<float> host(wn);
+    FM_CUDA(cudaMemcpyAsync(host.data(), dw, wn * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    FM_CUDA(cudaStreamSynchronize(ctx->stream));
+    packed_to_keras(host.data(), dw_keras, ksize, Cin, Cout);
+  }
+  return FM_OK;
+}
+
+// Deconvolution3D / Deconvolution2D (kernel 2, stride 2, C -> C channels) as the U-Nets run it: the 1x1x1 conv of the
+// coarse x [N,X,Y,Z,C] to 4*pz*C channels, then depth-to-space with the bias -> y [N,2X,2Y,pz*Z,C]. w_keras is the
+// Keras kernel (2,2[,2],C,C) = (..., Cout, Cin). With dy [N,2X,2Y,pz*Z,C]: the backward of backward_unet /
+// backward_unet_bn - bias gradient, space-to-depth, the 1x1x1 weight gradient and the data gradient dx (masked by
+// x > 0 when relu_mask, as behind a ReLU block of the plain U-Net).
+extern "C" int fm_op_deconv(fm_ctx* ctx, const float* x, const float* w_keras, const float* bias, int N, int X, int Y,
+                            int Z, int C, int pz, float* y, const float* dy, int relu_mask, float* dx, float* dw_keras,
+                            float* dbias) {
+  FM_CHECK(ctx && x && w_keras && (pz == 1 || pz == 2), FM_EINVAL, "fm_op_deconv: bad argument");
+  FM_CHECK(!dy || (dx && dw_keras && dbias), FM_EINVAL, "fm_op_deconv: dy needs dx, dw_keras and dbias");
+  FM_CUDA(cudaSetDevice(ctx->device));
+  OpScratch s(ctx);
+  const int c8 = 4 * pz * C;
+  const Dims5 dc{N, X, Y, Z, C};
+  const size_t vc = (size_t)N * X * Y * Z, nf = vc * c8, wn = (size_t)c8 * C;
+  bf16 *bx = nullptr, *wf = nullptr, *wd = nullptr, *bz = nullptr;
+  float* wm = nullptr;
+  FM_TRY(s.up_bf16(x, vc * C, &bx));
+  FM_TRY(s.up_f32(w_keras, wn, &wm));  // the Keras kernel is the master layout [class][Cout][Cin]
+  FM_TRY(s.alloc(&wf, wn));
+  FM_TRY(s.alloc(&wd, wn));
+  FM_TRY(k_repack_weights(ctx, wm, wf, wd, nullptr, c8, 1, C, 0));
+  FM_TRY(s.alloc(&bz, nf));
+  if (y) {
+    FM_CHECK(bias, FM_EINVAL, "fm_op_deconv: y needs the bias");
+    bf16* by = nullptr;
+    float* db = nullptr;
+    FM_TRY(s.up_f32(bias, C, &db));
+    FM_TRY(s.alloc(&by, nf));
+    FM_TRY(k_conv3d_tc_fprop(ctx, bx, nullptr, wf, nullptr, bz, nullptr, N, X, Y, Z, C, 0, c8, 1, 0, c8, 0));
+    FM_TRY(k_depth_to_space(ctx, bz, db, by, dc, pz));
+    FM_TRY(s.down_bf16(by, nf, y));
+  }
+  if (dy) {
+    bf16 *bdy = nullptr, *bdx = nullptr;
+    float *dw = nullptr, *db = nullptr;
+    FM_TRY(s.up_bf16(dy, nf, &bdy));
+    FM_TRY(s.alloc(&bdx, vc * C));
+    FM_TRY(s.alloc(&dw, wn));
+    FM_TRY(s.alloc(&db, C));
+    FM_TRY(k_zero(ctx, dw, wn * 4));
+    FM_TRY(k_zero(ctx, db, (size_t)C * 4));
+    FM_TRY(k_bias_grad(ctx, bdy, db, (int64_t)nf / C, C));
+    FM_TRY(k_space_to_depth(ctx, bdy, bz, dc, pz));
+    FM_TRY(k_conv3d_tc_wgrad(ctx, bx, bz, dw, N, X, Y, Z, C, C, 0, c8, 1));
+    FM_TRY(k_conv3d_tc_fprop(ctx, bz, nullptr, wd, nullptr, bdx, relu_mask ? bx : nullptr, N, X, Y, Z, c8, 0, C, 1, 0, C,
+                             0));
+    FM_CUDA(cudaMemcpyAsync(dw_keras, dw, wn * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    FM_CUDA(cudaMemcpyAsync(dbias, db, (size_t)C * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    FM_TRY(s.down_bf16(bdx, vc * C, dx));
+  }
+  return FM_OK;
+}
+
+// The raw shuffles of the deconvolution, without bias: depth-to-space of z8 [N,X,Y,Z,4*pz*C] -> fine
+// [N,2X,2Y,pz*Z,C] (to_space = 1) or its inverse (to_space = 0, fine -> z8).
+extern "C" int fm_op_depth_space(fm_ctx* ctx, int to_space, const float* in, int N, int X, int Y, int Z, int C, int pz,
+                                 float* out) {
+  FM_CHECK(ctx && in && out && (pz == 1 || pz == 2), FM_EINVAL, "fm_op_depth_space: bad argument");
+  FM_CUDA(cudaSetDevice(ctx->device));
+  OpScratch s(ctx);
+  const size_t n = (size_t)N * X * Y * Z * C * 4 * pz;
+  bf16 *bi = nullptr, *bo = nullptr;
+  FM_TRY(s.up_bf16(in, n, &bi));
+  FM_TRY(s.alloc(&bo, n));
+  if (to_space)
+    FM_TRY(k_depth_to_space(ctx, bi, nullptr, bo, Dims5{N, X, Y, Z, C}, pz));
+  else
+    FM_TRY(k_space_to_depth(ctx, bi, bo, Dims5{N, X, Y, Z, C}, pz));
+  return s.down_bf16(bo, n, out);
+}
+
+// Zero insertion of the strided-conv backward: coarse [N,X,Y,Z,C] -> fine [N,2X,2Y,pz*Z,C], fine[2v+1] = coarse[v].
+extern "C" int fm_op_zero_insert(fm_ctx* ctx, const float* coarse, int N, int X, int Y, int Z, int C, int pz,
+                                 float* fine) {
+  FM_CHECK(ctx && coarse && fine && (pz == 1 || pz == 2), FM_EINVAL, "fm_op_zero_insert: bad argument");
+  FM_CUDA(cudaSetDevice(ctx->device));
+  OpScratch s(ctx);
+  const size_t n = (size_t)N * X * Y * Z * C;
+  bf16 *bc = nullptr, *bf = nullptr;
+  FM_TRY(s.up_bf16(coarse, n, &bc));
+  FM_TRY(s.alloc(&bf, n * 4 * pz));
+  FM_TRY(k_zero_insert(ctx, bc, bf, Dims5{N, X, Y, Z, C}, pz));
+  return s.down_bf16(bf, n * 4 * pz, fine);
+}
+
+// The 1x1x1 single-output heads. Forward when p != NULL: p = [sigmoid](x . w + b) (k_head_fwd), or with targets t the
+// training form k_head_fwd_dice (always through the sigmoid) that also returns the 8 loss statistics in sums.
+// Backward when dz != NULL (k_head_bwd): dx = dz * w (mode 0: masked by x > 0; mode 1: plain; mode 2: added to dx, which
+// is then in/out), dw [C] = sum dz * x and db [1] = sum dz.
+extern "C" int fm_op_head(fm_ctx* ctx, const float* x, const float* w, const float* b, int64_t voxels, int C,
+                          int apply_sigmoid, const float* t, float* p, double sums[8], const float* dz, int mode, float* dx,
+                          float* dw, float* db) {
+  FM_CHECK(ctx && x && w && voxels > 0, FM_EINVAL, "fm_op_head: bad argument");
+  FM_CHECK(!p || b, FM_EINVAL, "fm_op_head: the forward needs b");
+  FM_CHECK(!t || (p && sums), FM_EINVAL, "fm_op_head: t needs p and sums");
+  FM_CHECK(!dz || (dx && dw && db && mode >= 0 && mode <= 2), FM_EINVAL, "fm_op_head: dz needs dx, dw, db, mode 0-2");
+  FM_CUDA(cudaSetDevice(ctx->device));
+  OpScratch s(ctx);
+  const size_t n = (size_t)voxels * C;
+  bf16* bx = nullptr;
+  float *dwt = nullptr, *dbias = nullptr;
+  FM_TRY(s.up_bf16(x, n, &bx));
+  FM_TRY(s.up_f32(w, C, &dwt));
+  if (p) {
+    float *dp = nullptr, *dt = nullptr;
+    FM_TRY(s.up_f32(b, 1, &dbias));
+    FM_TRY(s.alloc(&dp, (size_t)voxels));
+    if (t) {
+      double* ds = nullptr;
+      FM_TRY(s.up_f32(t, (size_t)voxels, &dt));
+      FM_TRY(s.alloc(&ds, kNumLossSums));
+      FM_TRY(k_head_fwd_dice(ctx, bx, dwt, dbias, dt, dp, voxels, C, ds));
+      FM_CUDA(cudaMemcpyAsync(sums, ds, 8 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    } else {
+      FM_TRY(k_head_fwd(ctx, bx, dwt, dbias, dp, voxels, C, apply_sigmoid));
+    }
+    FM_CUDA(cudaMemcpyAsync(p, dp, (size_t)voxels * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    FM_CUDA(cudaStreamSynchronize(ctx->stream));
+  }
+  if (dz) {
+    float *ddz = nullptr, *dg = nullptr;
+    bf16* bdx = nullptr;
+    FM_TRY(s.up_f32(dz, (size_t)voxels, &ddz));
+    if (mode == 2)
+      FM_TRY(s.up_bf16(dx, n, &bdx));
+    else
+      FM_TRY(s.alloc(&bdx, n));
+    FM_TRY(s.alloc(&dg, (size_t)C + 1));
+    FM_TRY(k_zero(ctx, dg, ((size_t)C + 1) * 4));
+    FM_TRY(k_head_bwd(ctx, bx, ddz, dwt, bdx, dg, dg + C, voxels, C, mode));
+    FM_CUDA(cudaMemcpyAsync(dw, dg, (size_t)C * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    FM_CUDA(cudaMemcpyAsync(db, dg + C, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    FM_TRY(s.down_bf16(bdx, n, dx));
+  }
+  return FM_OK;
+}
+
+// Deep-supervision plumbing of the Isensee nets (fp32 single-channel maps): out [N,X,Y,Z] = fine + the coarse map
+// [N,X/2,Y/2,Z/pz] upsampled, and the gradient of that upsampling: coarse [N,X,Y,Z] = 2x2(x2) sum-pool of fine
+// [N,2X,2Y,pz*Z].
+extern "C" int fm_op_seg_upsample_add(fm_ctx* ctx, const float* fine, const float* coarse, int N, int X, int Y, int Z,
+                                      int pz, float* out) {
+  FM_CHECK(ctx && fine && coarse && out && (pz == 1 || pz == 2), FM_EINVAL, "fm_op_seg_upsample_add: bad argument");
+  FM_CUDA(cudaSetDevice(ctx->device));
+  OpScratch s(ctx);
+  const size_t n = (size_t)N * X * Y * Z;
+  float *df = nullptr, *dc = nullptr, *dout = nullptr;
+  FM_TRY(s.up_f32(fine, n, &df));
+  FM_TRY(s.up_f32(coarse, n / (4 * pz), &dc));
+  FM_TRY(s.alloc(&dout, n));
+  FM_TRY(k_seg_upsample_add(ctx, df, dc, dout, N, X, Y, Z, pz));
+  FM_CUDA(cudaMemcpyAsync(out, dout, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  FM_CUDA(cudaStreamSynchronize(ctx->stream));
+  return FM_OK;
+}
+
+extern "C" int fm_op_sumpool_f32(fm_ctx* ctx, const float* fine, int N, int X, int Y, int Z, int pz, float* coarse) {
+  FM_CHECK(ctx && fine && coarse && (pz == 1 || pz == 2), FM_EINVAL, "fm_op_sumpool_f32: bad argument");
+  FM_CUDA(cudaSetDevice(ctx->device));
+  OpScratch s(ctx);
+  const size_t n = (size_t)N * X * Y * Z;
+  float *df = nullptr, *dc = nullptr;
+  FM_TRY(s.up_f32(fine, n * 4 * pz, &df));
+  FM_TRY(s.alloc(&dc, n));
+  FM_TRY(k_sumpool_f32(ctx, df, dc, N, X, Y, Z, pz));
+  FM_CUDA(cudaMemcpyAsync(coarse, dc, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
   FM_CUDA(cudaStreamSynchronize(ctx->stream));
   return FM_OK;
 }

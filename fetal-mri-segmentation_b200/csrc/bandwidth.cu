@@ -371,7 +371,9 @@ __global__ void __launch_bounds__(kThreads) instnorm_partial_kernel(const bf16* 
   }
 }
 
-// scale/shift per (n, c): y = x * scale + shift with scale = gamma / (sqrt(var) + eps), shift = beta - mean * scale.
+// coefficients per (n, c), ss[4 (n C + c) ...] = (scale, mean, beta, 0) with scale = gamma / (sqrt(var) + eps): the
+// apply pass forms y = (x - mean) * scale + beta. (A folded shift beta - mean * scale would leave y with an fp32 error
+// of ~|mean| * scale * 2^-24, which exceeds a bf16 ulp of y where the std is small against the mean.)
 // One warp per (n, c): lane l folds partials l, l+32, ... in fp64, then a fixed-order butterfly (deterministic).
 __global__ void instnorm_final_kernel(const float* __restrict__ part, const float* __restrict__ gamma,
                                       const float* __restrict__ beta, float* __restrict__ ss,
@@ -395,8 +397,10 @@ __global__ void instnorm_final_kernel(const float* __restrict__ part, const floa
   const double mean = s * inv_count;
   const double var = fmax(q * inv_count - mean * mean, 0.0);
   const double scale = (double)gamma[c] / (sqrt(var) + (double)eps);
-  ss[2 * i] = (float)scale;
-  ss[2 * i + 1] = (float)((double)beta[c] - mean * scale);
+  ss[4 * i] = (float)scale;
+  ss[4 * i + 1] = (float)mean;
+  ss[4 * i + 2] = beta[c];
+  ss[4 * i + 3] = 0.f;
   if (stats != nullptr) {  // kept for the backward pass: (mean, 1 / (sqrt(var) + eps))
     stats[2 * i] = (float)mean;
     stats[2 * i + 1] = (float)(1.0 / (sqrt(var) + (double)eps));
@@ -415,12 +419,12 @@ __global__ void __launch_bounds__(kThreads) instnorm_apply_kernel(const bf16* __
   const int c8 = threadIdx.x % c8n, l = threadIdx.x / c8n;
   if (l >= lanes) return;
   const int n = blockIdx.y;
-  float sc[8], sh[8], cs[8];
-  const float4* sp = reinterpret_cast<const float4*>(ss + ((int64_t)n * C + c8 * 8) * 2);
+  float sc[8], mu[8], be[8], cs[8];
+  const float4* sp = reinterpret_cast<const float4*>(ss + ((int64_t)n * C + c8 * 8) * 4);
 #pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const float4 t = __ldg(sp + i);  // (scale, shift) of two channels
-    sc[2 * i] = t.x, sh[2 * i] = t.y, sc[2 * i + 1] = t.z, sh[2 * i + 1] = t.w;
+  for (int i = 0; i < 8; ++i) {
+    const float4 t = __ldg(sp + i);  // (scale, mean, beta, 0) of one channel
+    sc[i] = t.x, mu[i] = t.y, be[i] = t.z;
   }
 #pragma unroll
   for (int i = 0; i < 8; ++i) cs[i] = chan_scale ? __ldg(chan_scale + (int64_t)n * C + c8 * 8 + i) : 1.f;
@@ -444,7 +448,7 @@ __global__ void __launch_bounds__(kThreads) instnorm_apply_kernel(const bf16* __
     unpack8(rx[u], f);
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
-      const float t = f[i] * sc[i] + sh[i];
+      const float t = (f[i] - mu[i]) * sc[i] + be[i];
       f[i] = (t > 0.f ? t : slope * t) * cs[i];
     }
     if (add != nullptr) {
@@ -459,7 +463,7 @@ __global__ void __launch_bounds__(kThreads) instnorm_apply_kernel(const bf16* __
     unpack8(ldg16(x + v * C + c8 * 8), f);
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
-      const float t = f[i] * sc[i] + sh[i];
+      const float t = (f[i] - mu[i]) * sc[i] + be[i];
       f[i] = (t > 0.f ? t : slope * t) * cs[i];
     }
     if (add != nullptr) {
@@ -1446,7 +1450,7 @@ int k_divide_by_count(fm_ctx* ctx, double* out, const int16_t* count, int64_t nv
   return FM_OK;
 }
 
-// x: raw conv output [N][vox][C] bf16 -> y = LeakyReLU(InstanceNorm(x)) (+ add). `scratch` >= N*C*2*(blocks+1) floats.
+// x: raw conv output [N][vox][C] bf16 -> y = LeakyReLU(InstanceNorm(x)) (+ add). `scratch` >= N*C*(2*blocks + 4) floats.
 static int norm_blocks(int64_t vox_per_sample, int64_t* vpb) {
   int bps = (int)std::min<int64_t>(std::max<int64_t>(1, vox_per_sample / 512), 1024);
   *vpb = ceil_div64(vox_per_sample, bps);
@@ -1600,7 +1604,7 @@ int k_instnorm_lrelu(fm_ctx* ctx, const bf16* x, const float* gamma, const float
   FM_CHECK(C >= 8 && C <= 512 && (C & (C - 1)) == 0, FM_EINVAL, "instnorm: C=%d must be a power of two in [8,512]", C);
   int64_t vpb;
   const int bps = norm_blocks(vox_per_sample, &vpb);
-  const size_t need = (size_t)N * C * 2 * ((size_t)bps + 1);
+  const size_t need = (size_t)N * C * (2 * (size_t)bps + 4);
   FM_CHECK(scratch_floats >= need, FM_EINVAL, "instnorm: scratch too small (%zu < %zu floats)", scratch_floats, need);
   float* part = scratch;
   float* ss = scratch + (size_t)N * C * 2 * bps;
@@ -1658,8 +1662,10 @@ __global__ void batchnorm_final_kernel(const float* __restrict__ part, const flo
   const double rstd = 1.0 / sqrt(var + (double)eps);
   const double scale = (double)gamma[c] * rstd;
   for (int n = lane; n < N; n += 32) {
-    ss[((int64_t)n * C + c) * 2] = (float)scale;
-    ss[((int64_t)n * C + c) * 2 + 1] = (float)((double)beta[c] - mean * scale);
+    ss[((int64_t)n * C + c) * 4] = (float)scale;
+    ss[((int64_t)n * C + c) * 4 + 1] = (float)mean;
+    ss[((int64_t)n * C + c) * 4 + 2] = beta[c];
+    ss[((int64_t)n * C + c) * 4 + 3] = 0.f;
     if (stats != nullptr) {
       stats[((int64_t)n * C + c) * 2] = (float)mean;
       stats[((int64_t)n * C + c) * 2 + 1] = (float)rstd;
@@ -1710,7 +1716,7 @@ int k_batchnorm_relu(fm_ctx* ctx, const bf16* x, const float* gamma, const float
   FM_CHECK(C >= 8 && C <= 512 && (C & (C - 1)) == 0, FM_EINVAL, "batchnorm: C=%d must be a power of two in [8,512]", C);
   int64_t vpb;
   const int bps = norm_blocks(vox_per_sample, &vpb);
-  const size_t need = (size_t)N * C * 2 * ((size_t)bps + 1);
+  const size_t need = (size_t)N * C * (2 * (size_t)bps + 4);
   FM_CHECK(scratch_floats >= need, FM_EINVAL, "batchnorm: scratch too small (%zu < %zu floats)", scratch_floats, need);
   float* part = scratch;
   float* ss = scratch + (size_t)N * C * 2 * bps;

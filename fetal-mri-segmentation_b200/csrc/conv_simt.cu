@@ -426,7 +426,7 @@ __global__ void __launch_bounds__(kThreads) head_fwd_dice_kernel(const bf16* __r
   }
 }
 
-// Thread-per-voxel form of the two head kernels for C <= 64 (every model of the BASELINE configs): one thread reads
+// Thread-per-voxel form of the two head kernels for C in {16, 32, 64} (every model of the BASELINE configs): one thread reads
 // its voxel's C channels with C/8 16-byte loads (the sectors a warp's loads share are consumed back to back out of L1),
 // keeps the weights in registers, and - in the training form - updates the loss statistics for its own voxel. The
 // lanes-per-voxel kernels above spend 13.7 warp instructions per voxel (shuffle folds, and the sigmoid / statistics
@@ -778,7 +778,7 @@ int k_head_fwd(fm_ctx* ctx, const bf16* x, const float* w, const float* b, float
   const int64_t vpb = kThreads / lpv;
   const int grid = (int)std::min<int64_t>(ceil_div64(voxels, vpb), (int64_t)ctx->num_sms * 32);
   ProfScope prof(ctx, "head_fwd", 2.0 * C * (double)voxels, (double)voxels * (C * 2.0 + 4.0));
-  if (C <= 64) {  // thread-per-voxel form
+  if (C >= 16 && C <= 64) {  // thread-per-voxel form (instantiated for 16, 32 and 64 channels)
     const int g2 = (int)std::min<int64_t>(ceil_div64(voxels, kThreads), (int64_t)ctx->num_sms * 16);
     const XentSpec none;
     if (C == 16)
@@ -808,7 +808,7 @@ int k_head_fwd_dice(fm_ctx* ctx, const bf16* x, const float* w, const float* b, 
   // one wave of resident blocks (64 registers x 256 threads: 4 blocks per SM): a grid-stride kernel launched with 1024
   // blocks on 592 slots ran 1.73 waves, the second one three-quarters empty
   const int grid = (int)std::min<int64_t>(ceil_div64(voxels, vpb * 4), (int64_t)std::min(1024, 4 * ctx->num_sms));
-  if (C <= 64) {  // thread-per-voxel form; one partial row per block of the reduction scratch
+  if (C >= 16 && C <= 64) {  // thread-per-voxel form; one partial row per block of the reduction scratch
     const int g2 = (int)std::min<int64_t>(ceil_div64(voxels, kThreads), (int64_t)std::min(kRedScratchRows, 16 * ctx->num_sms));
     {
       ProfScope prof(ctx, "head_fwd_dice", 2.0 * C * (double)voxels, (double)voxels * (C * 2.0 + 8.0));

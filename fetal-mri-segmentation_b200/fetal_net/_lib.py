@@ -141,6 +141,8 @@ SIGNATURES = {
     "fm_op_conv3d_fprop": (c_int, [c_vp, c_int, c_fp, c_fp, c_fp, c_fp] + [c_int] * 9 + [c_fp]),
     "fm_op_conv3d_dgrad": (c_int, [c_vp, c_int, c_fp, c_fp, c_fp] + [c_int] * 6 + [c_fp]),
     "fm_op_conv3d_wgrad": (c_int, [c_vp, c_int, c_fp, c_fp] + [c_int] * 6 + [c_fp, c_fp]),
+    "fm_op_conv_dgrad": (c_int, [c_vp, c_int, c_fp, c_fp, c_fp] + [c_int] * 7 + [c_fp]),
+    "fm_op_conv_wgrad": (c_int, [c_vp, c_int, c_fp, c_fp] + [c_int] * 7 + [c_fp, c_fp]),
     "fm_op_conv3d_first": (c_int, [c_vp, c_fp, c_fp, c_fp] + [c_int] * 6 + [c_fp, c_fp, c_fp]),
     "fm_op_conv3d_up_fprop": (c_int, [c_vp, c_fp, c_fp, c_fp, c_fp] + [c_int] * 8 + [c_fp]),
     "fm_op_conv3d_up_bwd": (c_int, [c_vp, c_fp, c_fp, c_fp] + [c_int] * 8 + [c_fp, c_fp]),
@@ -148,9 +150,26 @@ SIGNATURES = {
     "fm_op_maxpool3d_bwd": (c_int, [c_vp, c_fp, c_fp, c_fp] + [c_int] * 5 + [c_fp]),
     "fm_op_upsample3d": (c_int, [c_vp, c_fp] + [c_int] * 5 + [c_fp]),
     "fm_op_upsample3d_bwd": (c_int, [c_vp, c_fp, c_fp] + [c_int] * 5 + [c_fp]),
+    "fm_op_maxpool": (c_int, [c_vp, c_fp] + [c_int] * 6 + [c_fp]),
+    "fm_op_maxpool_bwd": (c_int, [c_vp, c_fp, c_fp, c_fp] + [c_int] * 6 + [c_fp]),
+    "fm_op_upsample": (c_int, [c_vp, c_fp] + [c_int] * 6 + [c_fp]),
+    "fm_op_upsample_bwd": (c_int, [c_vp, c_fp, c_fp] + [c_int] * 6 + [c_fp]),
     "fm_op_dice": (c_int, [c_vp, c_fp, c_fp, c_i64, c_dp, c_fp]),
     "fm_op_dice_xent": (c_int, [c_vp, c_fp, c_fp, c_fp, c_i64, ctypes.c_float, ctypes.c_float, c_dp, c_fp]),
     "fm_op_adam": (c_int, [c_vp, c_fp, c_fp, c_fp, c_fp, c_i64, c_int, c_f]),
+    "fm_op_instnorm_lrelu": (c_int, [c_vp, c_fp, c_fp, c_fp, c_fp, c_fp, c_int, c_i64, c_int, c_fp, c_fp]),
+    "fm_op_instnorm_lrelu_bwd": (c_int, [c_vp, c_fp, c_fp, c_fp, c_fp, c_fp, c_fp, c_int, c_i64, c_int, c_fp, c_fp,
+                                         c_fp]),
+    "fm_op_batchnorm_relu": (c_int, [c_vp, c_int, c_fp, c_fp, c_fp, c_fp, c_fp, c_int, c_i64, c_int, c_fp]),
+    "fm_op_batchnorm_relu_bwd": (c_int, [c_vp, c_fp, c_fp, c_fp, c_fp, c_fp, c_int, c_i64, c_int, c_fp, c_fp, c_fp]),
+    "fm_op_conv_strided": (c_int, [c_vp, c_fp, c_fp, c_fp] + [c_int] * 7 + [c_fp, c_fp, c_fp, c_fp]),
+    "fm_op_deconv": (c_int, [c_vp, c_fp, c_fp, c_fp] + [c_int] * 6 + [c_fp, c_fp, c_int, c_fp, c_fp, c_fp]),
+    "fm_op_depth_space": (c_int, [c_vp, c_int, c_fp] + [c_int] * 6 + [c_fp]),
+    "fm_op_zero_insert": (c_int, [c_vp, c_fp] + [c_int] * 6 + [c_fp]),
+    "fm_op_head": (c_int, [c_vp, c_fp, c_fp, c_fp, c_i64, c_int, c_int, c_fp, c_fp, c_dp, c_fp, c_int, c_fp, c_fp,
+                           c_fp]),
+    "fm_op_seg_upsample_add": (c_int, [c_vp, c_fp, c_fp] + [c_int] * 5 + [c_fp]),
+    "fm_op_sumpool_f32": (c_int, [c_vp, c_fp] + [c_int] * 5 + [c_fp]),
 }
 
 _lib = None

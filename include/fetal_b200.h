@@ -423,6 +423,12 @@ int fm_op_conv3d_dgrad(fm_ctx* ctx, int impl, const float* dy, const float* w_ke
                        float* dx);
 int fm_op_conv3d_wgrad(fm_ctx* ctx, int impl, const float* x, const float* dy, int N, int X, int Y,
                        int Z, int Cin, int Cout, float* dw_keras, float* dbias);
+/* The same two for any kernel code `ksize` (as in fm_op_conv3d_fprop: 3 = 3x3x3, 1 = 1x1x1, 31 = 3x3x1 Conv2D on a
+ * Z = 1 volume); the two above are their ksize = 3 forms. */
+int fm_op_conv_dgrad(fm_ctx* ctx, int impl, const float* dy, const float* w_keras, const float* mask, int N, int X, int Y,
+                     int Z, int Cin, int Cout, int ksize, float* dx);
+int fm_op_conv_wgrad(fm_ctx* ctx, int impl, const float* x, const float* dy, int N, int X, int Y, int Z, int Cin,
+                     int Cout, int ksize, float* dw_keras, float* dbias);
 /* First Conv3D of the network on the single-channel float32 input x [N,X,Y,Z] (create_convolution_block on the
  * (1, X, Y, Z) input, unet.py:102): y [N,X,Y,Z,Cout] = act(conv + bias) when y != NULL; the weight gradient
  * dw_keras (3,3,3,1,Cout) for dy [N,X,Y,Z,Cout] when both are != NULL. */
@@ -446,6 +452,14 @@ int fm_op_maxpool3d_bwd(fm_ctx* ctx, const float* x, const float* dy, const floa
 int fm_op_upsample3d(fm_ctx* ctx, const float* x, int N, int X, int Y, int Z, int C, float* y);
 int fm_op_upsample3d_bwd(fm_ctx* ctx, const float* dy, const float* act, int N, int X, int Y, int Z,
                          int C, float* dx);
+/* The same four pooling / upsampling by 2 in x and y and by `pz` in z: 2 (the four above) or 1 (the 2D models).
+ * X, Y, Z: the finer extent for the pool hooks, the coarser one for the upsample hooks. */
+int fm_op_maxpool(fm_ctx* ctx, const float* x, int N, int X, int Y, int Z, int C, int pz, float* y);
+int fm_op_maxpool_bwd(fm_ctx* ctx, const float* x, const float* dy, const float* dskip, int N, int X, int Y, int Z,
+                      int C, int pz, float* dx);
+int fm_op_upsample(fm_ctx* ctx, const float* x, int N, int X, int Y, int Z, int C, int pz, float* y);
+int fm_op_upsample_bwd(fm_ctx* ctx, const float* dy, const float* act, int N, int X, int Y, int Z, int C, int pz,
+                       float* dx);
 int fm_op_dice(fm_ctx* ctx, const float* p, const float* t, int64_t n, double sums[8],
                float* dloss_dp);
 /* dice_and_xent / dice_and_xent_mask (fetal_net/metrics.py:68-95) on probabilities p: sums[0..7] as fm_op_dice,
@@ -455,6 +469,48 @@ int fm_op_dice_xent(fm_ctx* ctx, const float* p, const float* t, const float* ma
                     float dist_sigma, double sums[9], float* dloss_dz);
 int fm_op_adam(fm_ctx* ctx, float* p, const float* g, float* mm, float* vv, int64_t n,
                int iterations, float lr);
+
+/* Normalisation blocks on x [N,vox,C] (C a power of two in [8, 512]).
+ * InstanceNormalization + LeakyReLU(0.3) of the Isensee blocks: y = act(norm(x)) * chan_scale + add; add [N,vox,C],
+ * chan_scale [N,C] (SpatialDropout keep / scale factors) and stats [N,C,2] = (mean, 1 / (std + eps)) may be NULL.
+ * The backward runs the forward first for its statistics; gy2 (a second incoming gradient) and chan_scale may be NULL. */
+int fm_op_instnorm_lrelu(fm_ctx* ctx, const float* x, const float* gamma, const float* beta, const float* add,
+                         const float* chan_scale, int N, int64_t vox, int C, float* y, float* stats);
+int fm_op_instnorm_lrelu_bwd(fm_ctx* ctx, const float* x, const float* gamma, const float* beta, const float* gy,
+                             const float* gy2, const float* chan_scale, int N, int64_t vox, int C, float* dx,
+                             float* dgamma, float* dbeta);
+/* BatchNormalization + ReLU (batch_normalization=True): training = batch statistics plus the Keras moving-average step
+ * of moving_mean / moving_var [C] (in/out); inference = the moving statistics. The backward follows a training
+ * forward; gy2 may be NULL. */
+int fm_op_batchnorm_relu(fm_ctx* ctx, int training, const float* x, const float* gamma, const float* beta,
+                         float* moving_mean, float* moving_var, int N, int64_t vox, int C, float* y);
+int fm_op_batchnorm_relu_bwd(fm_ctx* ctx, const float* x, const float* gamma, const float* beta, const float* gy,
+                             const float* gy2, int N, int64_t vox, int C, float* dx, float* dgamma, float* dbeta);
+/* Stride-2 TF-'SAME' convolution of the Isensee in-convs (no activation), ksize 3 or 31 (z not strided): x
+ * [N,Xin,Yin,Zin,Cin] -> y [N,Xin/2,Yin/2,Zin/2 (or Zin),Cout] when y != NULL; with dy (the shape of y) the data
+ * gradient dx [N,Xin,Yin,Zin,Cin] and weight gradient dw_keras through zero insertion and stride-1 kernels. */
+int fm_op_conv_strided(fm_ctx* ctx, const float* x, const float* w_keras, const float* bias, int N, int Xin, int Yin,
+                       int Zin, int Cin, int Cout, int ksize, float* y, const float* dy, float* dx, float* dw_keras);
+/* Deconvolution3D / 2D (kernel 2, stride 2, C -> C channels, pz = 2 / 1): x [N,X,Y,Z,C] -> y [N,2X,2Y,pz*Z,C] with
+ * the Keras kernel w_keras (2,2[,2],C,C) and bias [C]; with dy (the shape of y): dx (masked by x > 0 when relu_mask),
+ * dw_keras and dbias. */
+int fm_op_deconv(fm_ctx* ctx, const float* x, const float* w_keras, const float* bias, int N, int X, int Y, int Z,
+                 int C, int pz, float* y, const float* dy, int relu_mask, float* dx, float* dw_keras, float* dbias);
+/* The shuffles alone (no bias): to_space = 1: in [N,X,Y,Z,4*pz*C] -> out [N,2X,2Y,pz*Z,C]; 0: the inverse. */
+int fm_op_depth_space(fm_ctx* ctx, int to_space, const float* in, int N, int X, int Y, int Z, int C, int pz,
+                      float* out);
+/* coarse [N,X,Y,Z,C] -> fine [N,2X,2Y,pz*Z,C]: fine[2v+1] = coarse[v], zero elsewhere. */
+int fm_op_zero_insert(fm_ctx* ctx, const float* coarse, int N, int X, int Y, int Z, int C, int pz, float* fine);
+/* 1x1x1 single-output head on x [voxels,C] (C a power of two in [8, 256]). p != NULL: p = [sigmoid](x . w + b[0]), or,
+ * with targets t, the training form (sigmoid) that also returns the 8 loss statistics of fm_op_dice in sums.
+ * dz != NULL: dx = dz * w (mode 0: masked by x > 0; 1: plain; 2: added to dx, which is then in/out), dw [C], db [1]. */
+int fm_op_head(fm_ctx* ctx, const float* x, const float* w, const float* b, int64_t voxels, int C, int apply_sigmoid,
+               const float* t, float* p, double sums[8], const float* dz, int mode, float* dx, float* dw, float* db);
+/* Deep-supervision maps (fp32, one channel): out [N,X,Y,Z] = fine + upsample(coarse [N,X/2,Y/2,Z/pz]); and the
+ * gradient of the upsampling, coarse [N,X,Y,Z] = sum-pool of fine [N,2X,2Y,pz*Z]. */
+int fm_op_seg_upsample_add(fm_ctx* ctx, const float* fine, const float* coarse, int N, int X, int Y, int Z, int pz,
+                           float* out);
+int fm_op_sumpool_f32(fm_ctx* ctx, const float* fine, int N, int X, int Y, int Z, int pz, float* coarse);
 
 #ifdef __cplusplus
 }
