@@ -10,7 +10,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "fetal_net", "libfetalb200.so")
-SOURCES = ["api.cu", "bandwidth.cu", "conv_simt.cu", "conv_tc.cu", "conv_march.cu", "conv_wgrad_march.cu", "comm.cu", "sampler.cu", "conv_first_tc.cu", "postprocess.cu"]
+SOURCES = ["api.cu", "bandwidth.cu", "conv_simt.cu", "conv_tc.cu", "conv_march.cu", "conv_wgrad_march.cu", "comm.cu", "sampler.cu", "conv_first_tc.cu", "postprocess.cu", "tta.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
          "-Xcompiler", "-fPIC", "-Xcompiler", "-Wall", "--expt-relaxed-constexpr"]

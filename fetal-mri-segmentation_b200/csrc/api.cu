@@ -313,6 +313,9 @@ struct fm_model {
   DevBuf<double> pw_out;
   DevBuf<int16_t> pw_cnt;
   std::vector<cudaEvent_t> pw_events;  // [0] upload, [1] rows ready, [2..] one per finished output slab
+  // flip test-time augmentation (grow-only): the flipped copy of the volume, the un-flipped maps [passes][pitch]
+  DevBuf<float> tta_vol;
+  DevBuf<double> tta_stack;
 
   // backward bucket events (one per layer, reverse creation order)
   std::vector<cudaEvent_t> layer_done;
@@ -616,6 +619,8 @@ extern "C" int fm_model_destroy(fm_model* m) {
   m->pw_idx.release();
   m->pw_out.release();
   m->pw_cnt.release();
+  m->tta_vol.release();
+  m->tta_stack.release();
   m->x_in.release();
   m->bnRaw.release();
   m->bnGRaw.release();
@@ -2002,6 +2007,48 @@ extern "C" int fm_op_gaussian3d(fm_ctx* ctx, const void* in, int dtype, const in
 // pp != null (fm_patchwise_segment; single GPU): the cropped result is post-processed on the device into `pp_mask`;
 // `out` is then optional.
 static bool is_pinned_host(const void* p);
+
+// patch extent in the padded volume (`nslices` deep for the 2D model), the prediction extent it yields
+// (prediction.py:131-134) and the padded output extent (prediction.py:169); checks the halo pads against them
+static int pw_extents(const fm_model* m, int nslices, const int32_t vol_dims[3], const int32_t halo_pad[6],
+                      const int32_t fit_pad[6], int32_t patch[3], int32_t pred[3], int32_t out_dims[3]) {
+  const bool is2d = m->kcode == 31;
+  patch[0] = pred[0] = m->spec.X;
+  patch[1] = pred[1] = m->spec.Y;
+  patch[2] = nslices;
+  pred[2] = is2d ? 1 : m->spec.Z;
+  for (int a = 0; a < 3; ++a) {
+    FM_CHECK(halo_pad[2 * a] + halo_pad[2 * a + 1] == patch[a] - pred[a], FM_EINVAL,
+             "fm_patchwise_predict: halo pad on axis %d must total patch - prediction = %d", a, patch[a] - pred[a]);
+    out_dims[a] = vol_dims[a] + fit_pad[2 * a] + fit_pad[2 * a + 1];
+  }
+  return FM_OK;
+}
+
+// Patches per network launch for `nloc` patches in `ngroups` x groups of `ppg`, given the caller's `batch`.
+static int pw_sub_batch(const fm_model* m, int batch, int64_t nloc, int ngroups, int ppg) {
+  if (batch <= ppg || ngroups < 3) return batch;
+  // cut so that a sub-batch fills the SMs in whole waves: the marching kernels run one 16 x 8 column per CTA, a
+  // patch has cpp columns, and q patches (q = SMs / gcd(SMs, cpp); 37 for 64^3 patches on 148 SMs) are a whole
+  // number of waves for them and for the 128-voxel tiles of the deeper levels. The first cut keeps ~3/4 of the
+  // patches (its finished output slabs travel back while the remainder runs); 2D models keep whole x groups.
+  const int64_t cpp = m->kcode == 31 ? 0 : (int64_t)(m->spec.Y / 16) * (m->spec.Z / 8);
+  int64_t q = 0;
+  if (cpp > 0) {
+    int64_t a = m->ctx->num_sms, b = cpp;
+    while (b) {
+      const int64_t t = a % b;
+      a = b;
+      b = t;
+    }
+    q = m->ctx->num_sms / a;
+  }
+  if (q > 0 && nloc > q)
+    return (int)std::min<int64_t>(batch, q * std::max<int64_t>(1, std::min<int64_t>(2, (nloc * 3 / 4) / q)));
+  if (q == 0) return (int)std::min<int64_t>(batch, (int64_t)ppg * std::max(1, ngroups / 8));
+  return batch;
+}
+
 static int patchwise_impl(fm_model* m, const float* vol, const int32_t vol_dims[3], const int32_t halo_pad[6],
                           const int32_t fit_pad[6], const double pad_value[2], const int32_t* idx, int64_t n, int batch,
                           int shard_rank, int shard_count, int reduce_root, const float* truth, int prev_truth_index,
@@ -2030,15 +2077,8 @@ static int patchwise_impl(fm_model* m, const float* vol, const int32_t vol_dims[
   FM_CHECK(!truth || (prev_truth_index >= 0 && prev_truth_index + prev_truth_size <= nslices), FM_EINVAL,
            "fm_patchwise_predict: previous-truth slices [%d, %d) must lie inside the patch depth %d", prev_truth_index,
            prev_truth_index + prev_truth_size, nslices);
-  // patch extent in the padded volume and the prediction extent it yields (prediction.py:131-134)
-  const int32_t patch[3] = {m->spec.X, m->spec.Y, nslices};
-  const int32_t pred[3] = {m->spec.X, m->spec.Y, is2d ? 1 : m->spec.Z};
-  int32_t out_dims[3];
-  for (int a = 0; a < 3; ++a) {
-    FM_CHECK(halo_pad[2 * a] + halo_pad[2 * a + 1] == patch[a] - pred[a], FM_EINVAL,
-             "fm_patchwise_predict: halo pad on axis %d must total patch - prediction = %d", a, patch[a] - pred[a]);
-    out_dims[a] = vol_dims[a] + fit_pad[2 * a] + fit_pad[2 * a + 1];  // prediction.py:169
-  }
+  int32_t patch[3], pred[3], out_dims[3];
+  FM_TRY(pw_extents(m, nslices, vol_dims, halo_pad, fit_pad, patch, pred, out_dims));
   const size_t nv = (size_t)vol_dims[0] * vol_dims[1] * vol_dims[2];
   const size_t nout = (size_t)out_dims[0] * out_dims[1] * out_dims[2];
   const size_t pv = (size_t)pred[0] * pred[1] * pred[2];  // predicted voxels per patch
@@ -2060,27 +2100,7 @@ static int patchwise_impl(fm_model* m, const float* vol, const int32_t vol_dims[
   // the copy stream just ahead of the patches that need it, and finished output slabs are overlap-added, copied back
   // and un-staged while the network still works on later patches. The network is bit-reproducible and batch-invariant,
   // so the result does not depend on the cut.
-  if (batch > ppg && ngroups >= 3) {
-    // cut so that a sub-batch fills the SMs in whole waves: the marching kernels run one 16 x 8 column per CTA, a
-    // patch has cpp columns, and q patches (q = SMs / gcd(SMs, cpp); 37 for 64^3 patches on 148 SMs) are a whole
-    // number of waves for them and for the 128-voxel tiles of the deeper levels. The first cut keeps ~3/4 of the
-    // patches (its finished output slabs travel back while the remainder runs); 2D models keep whole x groups.
-    const int64_t cpp = is2d ? 0 : (int64_t)(m->spec.Y / 16) * (m->spec.Z / 8);
-    int64_t q = 0;
-    if (cpp > 0) {
-      int64_t a = ctx->num_sms, b = cpp;
-      while (b) {
-        const int64_t t = a % b;
-        a = b;
-        b = t;
-      }
-      q = ctx->num_sms / a;
-    }
-    if (q > 0 && nloc > q)
-      batch = (int)std::min<int64_t>(batch, q * std::max<int64_t>(1, std::min<int64_t>(2, (nloc * 3 / 4) / q)));
-    else if (q == 0)
-      batch = (int)std::min<int64_t>(batch, (int64_t)ppg * std::max(1, ngroups / 8));
-  }
+  batch = pw_sub_batch(m, batch, nloc, ngroups, ppg);
   FM_TRY(ensure_capacity(m, batch, false));
   DevBuf<float>&dvol = m->pw_vol, &dpred = m->pw_pred;
   DevBuf<int32_t>& didx = m->pw_idx;
@@ -2293,6 +2313,148 @@ extern "C" int fm_patchwise_segment(fm_model* m, const float* vol, const int32_t
   FM_CHECK(spec && mask, FM_EINVAL, "fm_patchwise_segment: NULL spec or mask");
   return patchwise_impl(m, vol, vol_dims, halo_pad, fit_pad, pad_value, idx, n, batch, 0, 1, -1, truth, prev_truth_index,
                         prev_truth_size, prob, nullptr, spec, mask, n_components);
+}
+
+// Flip test-time augmentation: `passes` sliding-window predictions of the volume flipped by in_flip[k], each cropped and
+// un-flipped by out_flip[k] into slot k of a device stack, then the per-voxel median and (spec) its post-processing.
+// Flipping keeps the volume's shape and multiset of values, so the pads, the patch list and the reassembly plan of the
+// unflipped volume serve every pass; the flip is applied to the unpadded volume and the gather pads it as usual.
+extern "C" int fm_patchwise_predict_flips(fm_model* m, const float* vol, const int32_t vol_dims[3],
+                                          const int32_t halo_pad[6], const int32_t fit_pad[6], const double pad_value[2],
+                                          const int32_t* idx, int64_t n, int batch, int passes, const int32_t* in_flip,
+                                          const int32_t* out_flip, double* maps, double* median,
+                                          const fm_postprocess_spec* spec, uint8_t* mask, int64_t* n_components) {
+  FM_CHECK(m && vol && vol_dims && halo_pad && fit_pad && pad_value && idx && in_flip && out_flip && n > 0 && batch > 0,
+           FM_EINVAL, "fm_patchwise_predict_flips: bad argument");
+  FM_CHECK(passes >= 1 && passes <= 8, FM_EINVAL, "fm_patchwise_predict_flips: %d passes (1 .. 8)", passes);
+  for (int k = 0; k < passes; ++k)
+    FM_CHECK(in_flip[k] >= 0 && in_flip[k] <= 7 && out_flip[k] >= 0 && out_flip[k] <= 7, FM_EINVAL,
+             "fm_patchwise_predict_flips: pass %d has flip masks %d / %d (0 .. 7)", k, in_flip[k], out_flip[k]);
+  FM_CHECK(vol_dims[0] > 0 && vol_dims[1] > 0 && vol_dims[2] > 0, FM_EINVAL,
+           "fm_patchwise_predict_flips: volume %d x %d x %d", vol_dims[0], vol_dims[1], vol_dims[2]);
+  if (spec) {
+    FM_CHECK(mask, FM_EINVAL, "fm_patchwise_predict_flips: post-processing needs a mask");
+    FM_TRY(check_pp_spec(spec, vol_dims));
+  }
+  fm_ctx* ctx = m->ctx;
+  FM_CUDA(cudaSetDevice(ctx->device));
+  const bool is2d = m->kcode == 31;
+  int32_t patch[3], pred[3], out_dims[3];
+  FM_TRY(pw_extents(m, is2d ? m->cin_real : m->spec.Z, vol_dims, halo_pad, fit_pad, patch, pred, out_dims));
+  const int32_t fit_lo[3] = {fit_pad[0], fit_pad[2], fit_pad[4]};
+  const size_t nv = (size_t)vol_dims[0] * vol_dims[1] * vol_dims[2];
+  const size_t nout = (size_t)out_dims[0] * out_dims[1] * out_dims[2];
+  const size_t pv = (size_t)pred[0] * pred[1] * pred[2];
+  const int64_t pitch = ((int64_t)nv + 3) & ~(int64_t)3;  // slot stride of the stack: whole 32-byte quads
+  ReasmPlan* plan = nullptr;
+  FM_TRY(k_reassemble_prepare(ctx, idx, n, pred, 1, out_dims, &plan));
+  struct PlanGuard {
+    ReasmPlan* p;
+    ~PlanGuard() { k_reassemble_release(p); }
+  } plan_guard{plan};
+  const int32_t* xstarts = nullptr;
+  int ngroups = 0, ppg = 0;
+  k_reassemble_groups(plan, &xstarts, &ngroups, &ppg);
+  batch = pw_sub_batch(m, (int)std::min<int64_t>(batch, n), n, ngroups, ppg);
+  FM_TRY(ensure_capacity(m, batch, false));
+  FM_TRY(m->pw_vol.ensure(nv));
+  FM_TRY(m->tta_vol.ensure(nv));
+  FM_TRY(m->pw_pred.ensure((size_t)n * pv));
+  FM_TRY(m->pw_idx.ensure((size_t)n * 3));
+  FM_TRY(m->pw_out.ensure(nout));
+  FM_TRY(m->pw_cnt.ensure(nout));
+  FM_TRY(m->tta_stack.ensure((size_t)passes * pitch));
+  if (m->pw_events.size() < 2) {
+    const size_t old = m->pw_events.size();
+    m->pw_events.resize(2, nullptr);
+    for (size_t i = old; i < 2; ++i) FM_CUDA(cudaEventCreateWithFlags(&m->pw_events[i], cudaEventDisableTiming));
+  }
+  cudaEvent_t ev_slot = m->pw_events[1];
+  double* stack = m->tta_stack.p;
+  double* dmed = m->pw_out.p;  // the median replaces the last pass's padded map once that is in the stack
+  // pinned staging: [volume | one float64 map (median / maps into pageable memory) | post-processing stats + mask]
+  const size_t in_bytes = (nv * sizeof(float) + 4095) & ~(size_t)4095;
+  const size_t map_bytes = (nv * sizeof(double) + 4095) & ~(size_t)4095;
+  void* pin = nullptr;
+  FM_TRY(fm_ctx_pinned(ctx, in_bytes + map_bytes + 256 + nv, &pin));
+  char* pin_map = (char*)pin + in_bytes;
+  host_copy(pin, vol, nv * sizeof(float));
+  FM_CUDA(cudaMemcpyAsync(m->pw_vol.p, pin, nv * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+  FM_CUDA(cudaMemcpyAsync(m->pw_idx.p, idx, (size_t)n * 12, cudaMemcpyHostToDevice, ctx->stream));
+  // a page-locked `maps` receives slot k on the copy-back stream while pass k + 1 computes
+  const bool maps_pinned = maps && is_pinned_host(maps);
+  for (int k = 0; k < passes; ++k) {
+    const float* src = m->pw_vol.p;
+    if (in_flip[k]) {
+      FM_TRY(k_flip_volume(ctx, m->pw_vol.p, m->tta_vol.p, vol_dims, in_flip[k]));
+      src = m->tta_vol.p;
+    }
+    for (int64_t b0 = 0; b0 < n; b0 += batch) {
+      const int nb = (int)std::min<int64_t>(batch, n - b0);
+      FM_TRY(k_gather_patches(ctx, src, vol_dims, halo_pad, fit_pad, (float)pad_value[0], (float)pad_value[1],
+                              m->pw_idx.p + b0 * 3, nb, patch, m->x_in.p, is2d ? m->cin_real : 0, 0, 0));
+      FM_TRY(forward(m, nb));
+      FM_CUDA(cudaMemcpyAsync(m->pw_pred.p + (size_t)b0 * pv, m->prob.p, (size_t)nb * pv * 4, cudaMemcpyDeviceToDevice,
+                              ctx->stream));
+    }
+    FM_TRY(k_reassemble_rows(ctx, plan, m->pw_pred.p, 0, n, 0, m->pw_out.p, m->pw_cnt.p, 1, 0, out_dims[0]));
+    double* slot = stack + (size_t)k * pitch;
+    FM_TRY(k_flip_crop(ctx, m->pw_out.p, out_dims, fit_lo, slot, vol_dims, out_flip[k]));
+    if (maps_pinned) {
+      FM_CUDA(cudaEventRecord(ev_slot, ctx->stream));
+      FM_CUDA(cudaStreamWaitEvent(ctx->d2h_stream, ev_slot, 0));
+      FM_CUDA(cudaMemcpyAsync(maps + (size_t)k * nv, slot, nv * sizeof(double), cudaMemcpyDeviceToHost,
+                              ctx->d2h_stream));
+    }
+  }
+  FM_TRY(k_median_passes(ctx, stack, pitch, passes, (int64_t)nv, dmed));
+  const bool median_pinned = median && is_pinned_host(median);
+  if (median)
+    FM_CUDA(cudaMemcpyAsync(median_pinned ? (void*)median : (void*)pin_map, dmed, nv * sizeof(double),
+                            cudaMemcpyDeviceToHost, ctx->stream));
+  if (spec) {
+    PostprocBuffers b;
+    FM_TRY(pp_buffers(ctx, (int64_t)nv, spec->radius, &b));
+    FM_TRY(k_postprocess(ctx, b, dmed, FM_DTYPE_FLOAT64, (int64_t)vol_dims[1] * vol_dims[2], vol_dims[2], vol_dims,
+                         spec));
+    FM_TRY(pp_download(ctx, b, nv, spec, pin_map + map_bytes, mask, n_components));
+  }
+  FM_CUDA(cudaStreamSynchronize(ctx->stream));
+  if (median && !median_pinned) host_copy(median, pin_map, nv * sizeof(double));
+  if (maps && !maps_pinned)
+    for (int k = 0; k < passes; ++k) {
+      FM_CUDA(cudaMemcpyAsync(pin_map, stack + (size_t)k * pitch, nv * sizeof(double), cudaMemcpyDeviceToHost,
+                              ctx->stream));
+      FM_CUDA(cudaStreamSynchronize(ctx->stream));
+      host_copy(maps + (size_t)k * nv, pin_map, nv * sizeof(double));
+    }
+  FM_CUDA(cudaStreamSynchronize(ctx->d2h_stream));
+  m->fwd_valid = false;
+  return FM_OK;
+}
+
+extern "C" int fm_op_median_passes(fm_ctx* ctx, const double* in, int passes, int64_t nvox, double* out) {
+  FM_CHECK(ctx && in && out && nvox > 0, FM_EINVAL, "fm_op_median_passes: bad argument");
+  FM_CHECK(passes >= 1 && passes <= 8, FM_EINVAL, "fm_op_median_passes: %d passes (1 .. 8)", passes);
+  FM_CUDA(cudaSetDevice(ctx->device));
+  const int64_t pitch = (nvox + 3) & ~(int64_t)3;
+  DevBuf<double> d;
+  FM_TRY(d.ensure((size_t)(passes + 1) * pitch));
+  int r = FM_OK;
+  cudaError_t e = cudaSuccess;
+  for (int k = 0; k < passes && e == cudaSuccess; ++k)
+    e = cudaMemcpyAsync(d.p + k * pitch, in + k * nvox, (size_t)nvox * 8, cudaMemcpyHostToDevice, ctx->stream);
+  if (e == cudaSuccess) r = k_median_passes(ctx, d.p, pitch, passes, nvox, d.p + passes * pitch);
+  if (e == cudaSuccess && r == FM_OK)
+    e = cudaMemcpyAsync(out, d.p + passes * pitch, (size_t)nvox * 8, cudaMemcpyDeviceToHost, ctx->stream);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+  if (e != cudaSuccess) {
+    fm_set_error("fm_op_median_passes: %s", cudaGetErrorString(e));
+    r = FM_ECUDA;
+  }
+  cudaStreamSynchronize(ctx->stream);
+  d.release();
+  return r;
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -331,6 +331,15 @@ int k_gaussian3d(fm_ctx*, const PostprocBuffers& b, const void* src, int dtype, 
 int k_postprocess(fm_ctx*, const PostprocBuffers& b, const void* src, int dtype, int64_t sx, int64_t sy,
                   const int32_t dims[3], const fm_postprocess_spec* spec);
 
+// tta.cu: flip test-time augmentation (predict_flips, fetal_net/prediction.py:65-85). Masks: bit a = axis a reversed.
+// out [dims] = in [dims] flipped by `mask`
+int k_flip_volume(fm_ctx*, const float* in, float* out, const int32_t dims[3], int mask);
+// out [dims] = the [dims] box at fit_lo of the [map_dims] map, flipped by `mask`
+int k_flip_crop(fm_ctx*, const double* map, const int32_t map_dims[3], const int32_t fit_lo[3], double* out,
+                const int32_t dims[3], int mask);
+// out[i] = np.median over k < passes (1 .. 8) of stack[k * pitch + i]; pitch % 4 == 0, stack and out 32-byte aligned
+int k_median_passes(fm_ctx*, const double* stack, int64_t pitch, int passes, int64_t nvox, double* out);
+
 // conv_simt.cu
 // first layer: fp32 single/multi-channel input (channels-last), small Cin; out bf16 + ReLU
 int k_conv3d_simt_fprop(fm_ctx*, const void* x, int x_is_f32, const bf16* x2, const bf16* w_packed,

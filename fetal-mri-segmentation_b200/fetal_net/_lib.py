@@ -104,6 +104,9 @@ SIGNATURES = {
     "fm_patchwise_segment": (c_int, [c_vp, c_fp, c_i32p, c_i32p, c_i32p, c_dp, c_i32p, c_i64, c_int, c_fp, c_int, c_int,
                                      ctypes.POINTER(PostprocessSpec), c_u8p, c_dp, c_i64p]),
     "fm_op_gaussian3d": (c_int, [c_vp, c_vp, c_int, c_i32p, c_int, c_dp, c_vp]),
+    "fm_patchwise_predict_flips": (c_int, [c_vp, c_fp, c_i32p, c_i32p, c_i32p, c_dp, c_i32p, c_i64, c_int, c_int, c_i32p,
+                                           c_i32p, c_dp, c_dp, ctypes.POINTER(PostprocessSpec), c_u8p, c_i64p]),
+    "fm_op_median_passes": (c_int, [c_vp, c_dp, c_int, c_i64, c_dp]),
     "fm_train_step": (c_int, [c_vp, c_fp, c_fp, c_int, c_f, c_fp]),
     "fm_train_forward": (c_int, [c_vp, c_fp, c_fp, c_int]),
     "fm_train_backward": (c_int, [c_vp]),

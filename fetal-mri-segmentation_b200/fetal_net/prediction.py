@@ -294,7 +294,12 @@ def predict_with_permutations(model, data):
 
 def predict_flips(data, model, overlap_factor, config):
     """prediction.py:65-85: the 8 axis-flip subsets in powerset order () (0,) (1,) (2,) (0,1) (0,2) (1,2) (0,1,2);
-    returns the list of un-flipped predictions [X,Y,Z] (the caller takes the median, predict_nifti2.py:86-87)."""
+    returns the list of un-flipped predictions [X,Y,Z] (the caller takes the median, predict_nifti2.py:86-87).
+    A native Model with a [X,Y,Z] or [1,X,Y,Z] volume runs all 8 passes in one device call (fetal_net.device_tta); its
+    entries are then views of one page-locked [8,X,Y,Z] array."""
+    from .device_tta import _device_flips, _native_route
+    if _native_route(model, data):
+        return list(_device_flips(data, model, overlap_factor, config, 5, maps=True)[0])
     patch_shape = list(config["patch_shape"]) + [config["patch_depth"]]
     axes_sets = itertools.chain.from_iterable(itertools.combinations([0, 1, 2], r) for r in range(4))
     predictions = []

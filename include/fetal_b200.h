@@ -282,6 +282,25 @@ int fm_patchwise_segment(fm_model* m, const float* vol, const int32_t vol_dims[3
 int fm_op_gaussian3d(fm_ctx* ctx, const void* in, int dtype, const int32_t dims[3], int radius, const double* weights,
                      void* out);
 
+/* ---- flip test-time augmentation ------------------------------------------------------------ */
+
+/* Replaces predict_flips (fetal_net/prediction.py:65-85), the caller's per-voxel median (predict_nifti2.py:86-87) and
+ * postprocess_prediction, for a single GPU and n_labels 1. Pass k predicts the volume flipped by in_flip[k] with the
+ * arguments of fm_patchwise_predict (no truth conditioning), crops pad_for_fit and flips the map by out_flip[k]; flip
+ * masks are 0 .. 7 with bit a reversing volume axis a (the two differ for a [1,X,Y,Z] input, whose reference flips act
+ * on (C,X,Y) going in and (X,Y,Z) coming out). 1 <= passes <= 8. `maps` (may be NULL) receives the host float64
+ * [passes][X][Y][Z] un-flipped predictions, `median` (may be NULL) np.median over them ([X][Y][Z]: NaN where any pass
+ * is NaN, the mean of the two middle values for an even count). With `spec` the median is post-processed as
+ * fm_postprocess does into `mask` / `n_components` (volumes of up to 2^31 - 1 voxels). Device memory: one float32
+ * volume copy and `passes` float64 maps beyond fm_patchwise_predict's. Page-locked `maps` (fm_host_alloc) receive
+ * each pass's map while the next one computes. */
+int fm_patchwise_predict_flips(fm_model* m, const float* vol, const int32_t vol_dims[3], const int32_t halo_pad[6],
+                               const int32_t fit_pad[6], const double pad_value[2], const int32_t* idx, int64_t n,
+                               int batch, int passes, const int32_t* in_flip, const int32_t* out_flip, double* maps,
+                               double* median, const fm_postprocess_spec* spec, uint8_t* mask, int64_t* n_components);
+/* The median alone (test hook): host float64 in [passes][nvox] -> out [nvox], 1 <= passes <= 8. */
+int fm_op_median_passes(fm_ctx* ctx, const double* in, int passes, int64_t nvox, double* out);
+
 /* ---- training ----------------------------------------------------------------------------- */
 
 /* Replaces: model.train_on_batch(x, y) as driven by fit_generator (fetal_net/training.py:110-124):
