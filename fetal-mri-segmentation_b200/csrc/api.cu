@@ -221,6 +221,8 @@ struct Layer {
   int stride = 1;       // 2: TF-'SAME' strided conv (Isensee in-convs)
   int deconv = 0;       // Deconvolution3D/2D (k = 2 or 21, stride 2): master kernel [class][Cout][Cin] = the Keras layout
   int cin() const { return c1 + c2; }
+  // the backward of a stride-2 conv runs as a stride-1 dgrad / wgrad over the zero-inserted gradient, one level finer
+  int bwd_level() const { return stride == 2 ? level - 1 : level; }
   int taps() const { return kext_taps(k); }
   int cin_keras() const { return cin_real ? cin_real : cin(); }
   int64_t wcount() const { return is_norm ? cout : (int64_t)cout * taps() * cin(); }
@@ -242,17 +244,23 @@ struct fm_model {
   // activations, allocated for `cap` samples
   int cap = 0;
   bool train_alloc = false;
-  int kind = 0;   // 0: plain U-Net (3D or 2D); 1: Isensee-2017 residual 3D U-Net (forward / inference only)
+  int kind = 0;   // 0: U-Net (3D or 2D, optionally batch-normalised); 1: Isensee-2017 residual U-Net (3D or 2D)
   int nseg = 1;   // Isensee: n_segmentation_levels
   std::vector<DevBuf<bf16>> isIn, isC1, isSum, isUp, isU, isLoc1, isLoc2;
   std::vector<DevBuf<float>> isSeg;
-  DevBuf<bf16> isRaw;
-  DevBuf<float> isScratch, isAcc;
-  // Isensee training: per-layer raw conv outputs + (mean, 1/std) for the norm backward, SpatialDropout3D scales per
-  // level, gradient scratch (three per level, the 2f-channel upsample gradient, zero-inserted strided gradients)
-  std::vector<DevBuf<bf16>> isRawL, gIsA, gIsB, gIsC, gIsUp;
-  std::vector<DevBuf<float>> isStatsL, isDropL, gSeg;
-  DevBuf<bf16> gIsRaw, gIsZero;
+  DevBuf<float> isAcc;
+  // Isensee training: SpatialDropout3D scales per level, gradient scratch (three per level, the 2f-channel upsample
+  // gradient, zero-inserted strided gradients)
+  std::vector<DevBuf<bf16>> gIsA, gIsB, gIsC, gIsUp;
+  std::vector<DevBuf<float>> isDropL, gSeg;
+  DevBuf<bf16> gIsZero;
+  // conv blocks with a normalisation (every Isensee block; every U-Net block under batch_normalization=True): raw conv
+  // outputs and the norm statistics per conv layer (training, indexed like `layers`), one raw scratch (inference), the
+  // gradient of a raw output, the norm kernels' scratch
+  std::vector<DevBuf<bf16>> normRawL;
+  std::vector<DevBuf<float>> normStatsL;
+  DevBuf<bf16> normRaw, normGRaw;
+  DevBuf<float> normScratch;
   float dropout_rate = 0.f;
   uint64_t dropout_seed = 0x5EEDull;
   // 2D U-Net: SpatialDropout2D keep/scale factors [B][C] after enc<d>a (slot d) and dec<d>a (slot depth + d)
@@ -261,14 +269,10 @@ struct fm_model {
   // shuffle, and the shuffled gradient on the way back
   bool deconvolution = false;
   DevBuf<bf16> dcZ, dcG;
-  // batch_normalization=True (create_convolution_block, unet3d/unet.py:103-104): every conv block is Conv -> BN -> ReLU.
-  // Raw conv outputs + batch statistics per layer (training), one raw scratch (inference), the gradient of a raw output
+  // batch_normalization=True (create_convolution_block, unet3d/unet.py:103-104): every conv block is Conv -> BN -> ReLU
   bool batch_norm = false;
-  std::vector<DevBuf<bf16>> bnRawL;
-  std::vector<DevBuf<float>> bnStatsL;
-  DevBuf<bf16> bnRaw, bnGRaw;
-  DevBuf<float> bnScratch;
-  bool unet_dropout() const { return kind == 0 && kcode == 31 && dropout_rate > 0.f; }
+  // (the Python builder refuses dropout with batch normalisation; a rate set through the C ABI is ignored)
+  bool unet_dropout() const { return kind == 0 && kcode == 31 && !batch_norm && dropout_rate > 0.f; }
   int kcode = 3;  // 3: Conv3D 3x3x3 (unet_model_3d); 31: Conv2D 3x3 on a Z = 1 volume (unet_model_2d)
   int pz = 2;     // pooling factor along z
   int cin_real = 1;
@@ -351,6 +355,7 @@ static Layer& L(fm_model* m, const char* fmt, int d) {
   snprintf(nm, sizeof(nm), fmt, d);
   return m->layers[layer_index(m, nm)];
 }
+static int layer_pos(const fm_model* m, const Layer& l) { return (int)(&l - m->layers.data()); }
 
 // Training passes (and fast inference) let the marching kernel issue its MMAs in three interleaved streams where it
 // applies (Cout <= 32): 20-30 % faster, but the order in which the three MMA warps' products land in an accumulator is
@@ -365,7 +370,127 @@ static bool reproducible_pass(const fm_model* m) {
   return !(m->train_pass || m->fast_inference) || det;
 }
 
+// ---------------------------------------------------------------------------------------------
+// layer table
+// ---------------------------------------------------------------------------------------------
+// Appends the conv layer named fmt % d to a family's layer list, followed by `norms` normalisation pseudo-layers
+// (1: "<name>_norm"; 2: also "<name>_moving"). build_model assigns the parameter offsets.
+static void add_layer(std::vector<Layer>& ls, const char* fmt, int d, int c1, int c2, int cout, int k, int level,
+                      int stride = 1, int norms = 0) {
+  Layer l;
+  memset(l.name, 0, sizeof(l.name));
+  snprintf(l.name, sizeof(l.name), fmt, d);
+  l.c1 = c1;
+  l.c2 = c2;
+  l.cout = cout;
+  l.k = k;
+  l.level = level;
+  l.stride = stride;
+  ls.push_back(l);
+  for (int kind = 1; kind <= norms; ++kind) {
+    Layer g;
+    memset(g.name, 0, sizeof(g.name));
+    snprintf(g.name, sizeof(g.name), kind == 1 ? "%s_norm" : "%s_moving", l.name);
+    g.is_norm = kind;
+    g.c1 = cout;
+    g.c2 = 0;
+    g.cout = cout;
+    g.k = 1;
+    g.level = level;
+    ls.push_back(g);
+  }
+}
+
+// Marching-kernel eligibility (conv_march.cu), decided once per layer when the model is built: 3x3x3 convs whose first
+// source has at least 16 channels, the forward only at stride 1. X, Y, Z = the extent the pass runs at.
+static bool march_fprop_ok(const Layer& l, int X, int Y, int Z) {
+  return l.k == 3 && l.c1 >= 16 && l.stride == 1 && conv_march_supported(X, Y, Z, l.c1, l.c2, l.cout, l.k);
+}
+static bool march_dgrad_ok(const Layer& l, int src, int X, int Y, int Z) {
+  return l.k == 3 && l.c1 >= 16 && conv_march_supported(X, Y, Z, l.cout, 0, src == 0 ? l.c1 : l.c2, l.k);
+}
+
+// The steps every family shares once its layer list is in m->layers (Keras creation order): the flat parameter
+// layout, the parameter, gradient and Adam buffers, the loss sums, the bf16 packs, the layer-done events and the
+// gradient buckets.
+static int build_layer_table(fm_model* m) {
+  for (auto& l : m->layers) {
+    l.w_off = m->nparams;
+    m->nparams += l.wcount();
+    l.b_off = m->nparams;
+    // keep every layer's block 16-byte aligned for the vectorised Adam / allreduce views
+    m->nparams = (m->nparams + l.cout + 3) & ~(int64_t)3;
+  }
+  const size_t pb = (size_t)m->nparams * sizeof(float);
+  for (float** b : {&m->params, &m->grads, &m->adam_m, &m->adam_v}) {
+    FM_CUDA(cudaMalloc((void**)b, pb));
+    FM_CUDA(cudaMemset(*b, 0, pb));
+  }
+  FM_CUDA(cudaMalloc((void**)&m->sums, kNumLossSums * sizeof(double)));
+  FM_CUDA(cudaMemset(m->sums, 0, kNumLossSums * sizeof(double)));
+  // bf16 packs: fprop + dgrad copies of every kernel (the norm parameters are read as fp32), plus the marching packs
+  int64_t pack_elems = 0;
+  for (auto& l : m->layers)
+    if (!l.is_norm) pack_elems += 2 * ((l.wcount() + 63) & ~(int64_t)63);
+  FM_CUDA(cudaMalloc((void**)&m->wpack, (size_t)pack_elems * sizeof(bf16)));
+  FM_CUDA(cudaMemset(m->wpack, 0, (size_t)pack_elems * sizeof(bf16)));
+  bf16* wp = m->wpack;
+  for (auto& l : m->layers) {
+    if (l.is_norm) continue;
+    const int64_t padded = (l.wcount() + 63) & ~(int64_t)63;
+    l.w_f = wp;
+    l.w_d0 = wp + padded;
+    l.w_d1 = l.w_d0 + (int64_t)l.c1 * l.taps() * l.cout;
+    wp += 2 * padded;
+    const int cs[2] = {l.c1, l.c2};
+    const Dims5 f = m->dims(l.level, l.cout, 1), b = m->dims(l.bwd_level(), l.cout, 1);
+    if (march_fprop_ok(l, f.X, f.Y, f.Z)) {
+      l.march_f = true;
+      for (int s = 0; s < (l.c2 ? 2 : 1); ++s)
+        FM_CUDA(cudaMalloc((void**)&l.w_mf[s], (size_t)conv_march_pack_elems(cs[s], l.cout) * sizeof(bf16)));
+    }
+    for (int s = 0; s < (l.c2 ? 2 : 1); ++s)
+      if (march_dgrad_ok(l, s, b.X, b.Y, b.Z)) {
+        l.march_d[s] = true;
+        FM_CUDA(cudaMalloc((void**)&l.w_md[s], (size_t)conv_march_pack_elems(l.cout, cs[s]) * sizeof(bf16)));
+      }
+  }
+  m->normRawL.resize(m->layers.size());
+  m->normStatsL.resize(m->layers.size());
+  m->layer_done.resize(m->layers.size());
+  for (auto& e : m->layer_done) FM_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+  FM_CUDA(cudaEventCreateWithFlags(&m->ev_tmp, cudaEventDisableTiming));
+  // gradient buckets: consecutive layers in backward (= reverse creation) order, ~1/4 of the
+  // parameters each; every bucket is one contiguous range of the flat buffer.
+  const int nl = (int)m->layers.size();
+  const int64_t target = m->nparams / 4 + 1;
+  int hi = nl - 1;
+  int64_t acc = 0;
+  for (int i = nl - 1; i >= 0; --i) {
+    acc += m->layers[i].wcount() + m->layers[i].cout;
+    if (acc >= target || i == 0) {
+      m->buckets.push_back({i, hi});
+      hi = i - 1;
+      acc = 0;
+    }
+  }
+  return FM_OK;
+}
+
+// the layer table, then what only the family has (`family`, may be null); on any error the half-built model is destroyed
+static int build_model(fm_model* m, int (*family)(fm_model*), fm_model** out) {
+  int rc = build_layer_table(m);
+  if (rc == FM_OK && family) rc = family(m);
+  if (rc != FM_OK) {
+    fm_model_destroy(m);
+    return rc;
+  }
+  *out = m;
+  return FM_OK;
+}
+
 static int build_unet(fm_ctx* ctx, const fm_unet3d_spec* spec, int kcode, int flags, fm_model** out);
+static int unet_up_packs(fm_model* m);
 
 extern "C" int fm_model_create_unet3d(fm_ctx* ctx, const fm_unet3d_spec* spec, fm_model** out) {
   return fm_model_create_unet3d_ex(ctx, spec, 0, out);
@@ -423,49 +548,16 @@ static int build_unet(fm_ctx* ctx, const fm_unet3d_spec* spec, int kcode, int fl
   m->deconvolution = (flags & FM_UNET_DECONVOLUTION) != 0;
   m->batch_norm = (flags & FM_UNET_BATCH_NORMALIZATION) != 0;
   const int D = spec->depth, nf = spec->n_base_filters;
-  auto add = [&](const char* fmt, int d, int c1, int c2, int cout, int k, int level) {
-    Layer l;
-    memset(l.name, 0, sizeof(l.name));
-    snprintf(l.name, sizeof(l.name), fmt, d);
-    l.c1 = c1;
-    l.c2 = c2;
-    l.cout = cout;
-    l.k = k;
-    l.level = level;
-    l.w_off = m->nparams;
-    m->nparams += l.wcount();
-    l.b_off = m->nparams;
-    m->nparams += cout;
-    // keep every layer's block 16-byte aligned for the vectorised Adam / allreduce views
-    m->nparams = (m->nparams + 3) & ~(int64_t)3;
-    m->layers.push_back(l);
-    if (m->batch_norm && (k == 3 || k == 31)) {
-      // BatchNormalization(axis=1) behind the conv of every block: (gamma, beta) and (moving_mean, moving_variance)
-      for (int kind = 1; kind <= 2; ++kind) {
-        Layer g;
-        memset(g.name, 0, sizeof(g.name));
-        snprintf(g.name, sizeof(g.name), kind == 1 ? "%s_norm" : "%s_moving", l.name);
-        g.is_norm = kind;
-        g.c1 = cout;
-        g.c2 = 0;
-        g.cout = cout;
-        g.k = 1;
-        g.level = level;
-        g.w_off = m->nparams;
-        m->nparams += cout;
-        g.b_off = m->nparams;
-        m->nparams = (m->nparams + cout + 3) & ~(int64_t)3;
-        m->layers.push_back(g);
-      }
-    }
-  };
+  // BatchNormalization(axis=1) behind the conv of every block: (gamma, beta) and (moving_mean, moving_variance)
+  const int norms = m->batch_norm ? 2 : 0;
+  std::vector<Layer>& ls = m->layers;
   // the 2D model feeds its first conv from a 16-channel zero-padded copy of the input (tensor-core K granule)
   int c = kcode == 31 ? 16 : spec->in_channels;
   std::vector<int> skipc;
   for (int d = 0; d < D; ++d) {
     const int f1 = nf << d, f2 = f1 * 2;
-    add("enc%da", d, c, 0, f1, kcode, d);
-    add("enc%db", d, f1, 0, f2, kcode, d);
+    add_layer(ls, "enc%da", d, c, 0, f1, kcode, d, 1, norms);
+    add_layer(ls, "enc%db", d, f1, 0, f2, kcode, d, 1, norms);
     skipc.push_back(f2);
     c = f2;
   }
@@ -473,61 +565,29 @@ static int build_unet(fm_ctx* ctx, const fm_unet3d_spec* spec, int kcode, int fl
     if (m->deconvolution) {
       // Deconvolution3D(filters = channels of the coarse tensor, kernel 2, strides 2), created before the block that
       // consumes it (unet.py:57-59): 8 (4 in 2D) parity-class 1x1x1 matrices, bias, no activation
-      add("up%d", d, c, 0, c, kcode == 31 ? 21 : 2, d + 1);
-      m->layers.back().deconv = 1;
+      add_layer(ls, "up%d", d, c, 0, c, kcode == 31 ? 21 : 2, d + 1);
+      ls.back().deconv = 1;
     }
-    add("dec%da", d, c, skipc[d], skipc[d], kcode, d);  // concat order [up, skip] (unet.py:61)
-    add("dec%db", d, skipc[d], 0, skipc[d], kcode, d);
+    add_layer(ls, "dec%da", d, c, skipc[d], skipc[d], kcode, d, 1, norms);  // concat order [up, skip] (unet.py:61)
+    add_layer(ls, "dec%db", d, skipc[d], 0, skipc[d], kcode, d, 1, norms);
     c = skipc[d];
   }
-  add("final", 0, c, 0, spec->n_labels, 1, 0);
-  if (kcode == 31) m->layers[0].cin_real = spec->in_channels;
+  add_layer(ls, "final", 0, c, 0, spec->n_labels, 1, 0);
+  if (kcode == 31) ls[0].cin_real = spec->in_channels;
+  for (auto* v : {&m->encA, &m->encB, &m->pool, &m->up, &m->decA, &m->decB, &m->gEncA, &m->gEncB, &m->gPool, &m->gUp,
+                  &m->gSkip, &m->gDecA, &m->gDecB})
+    v->resize(D);
+  return build_model(m, unet_up_packs, out);
+}
 
-  const size_t pb = (size_t)m->nparams * sizeof(float);
-  FM_CUDA(cudaMalloc((void**)&m->params, pb));
-  FM_CUDA(cudaMalloc((void**)&m->grads, pb));
-  FM_CUDA(cudaMalloc((void**)&m->adam_m, pb));
-  FM_CUDA(cudaMalloc((void**)&m->adam_v, pb));
-  FM_CUDA(cudaMemset(m->params, 0, pb));
-  FM_CUDA(cudaMemset(m->grads, 0, pb));
-  FM_CUDA(cudaMemset(m->adam_m, 0, pb));
-  FM_CUDA(cudaMemset(m->adam_v, 0, pb));
-  // bf16 packs: fprop + dgrad copies of every kernel
-  int64_t pack_elems = 0;
-  for (auto& l : m->layers) pack_elems += 2 * ((l.wcount() + 63) & ~(int64_t)63);
-  FM_CUDA(cudaMalloc((void**)&m->wpack, (size_t)pack_elems * sizeof(bf16)));
-  FM_CUDA(cudaMemset(m->wpack, 0, (size_t)pack_elems * sizeof(bf16)));
-  bf16* wp = m->wpack;
-  for (auto& l : m->layers) {
-    const int64_t padded = (l.wcount() + 63) & ~(int64_t)63;
-    l.w_f = wp;
-    wp += padded;
-    l.w_d0 = wp;
-    l.w_d1 = wp + (int64_t)l.c1 * l.taps() * l.cout;
-    wp += padded;
-  }
-  for (auto& l : m->layers) {
-    if (l.is_norm || l.k != 3 || l.c1 < 16) continue;
-    const int X = spec->X >> l.level, Y = spec->Y >> l.level, Z = m->pz == 2 ? spec->Z >> l.level : spec->Z;
-    const int cs[2] = {l.c1, l.c2};
-    if (conv_march_supported(X, Y, Z, l.c1, l.c2, l.cout, l.k)) {
-      l.march_f = true;
-      for (int s = 0; s < (l.c2 ? 2 : 1); ++s)
-        FM_CUDA(cudaMalloc((void**)&l.w_mf[s], (size_t)conv_march_pack_elems(cs[s], l.cout) * sizeof(bf16)));
-    }
-    for (int s = 0; s < (l.c2 ? 2 : 1); ++s)
-      if (conv_march_supported(X, Y, Z, l.cout, 0, cs[s], l.k)) {
-        l.march_d[s] = true;
-        FM_CUDA(cudaMalloc((void**)&l.w_md[s], (size_t)conv_march_pack_elems(l.cout, cs[s]) * sizeof(bf16)));
-      }
-  }
-  // decoder convs whose filter bank is too large for the marching kernel run at COARSE resolution on their upsampled
-  // source (dec1a, dec2a of the shipped model)
+// decoder convs whose filter bank is too large for the marching kernel run at COARSE resolution on their upsampled
+// source (dec1a, dec2a of the shipped model)
+static int unet_up_packs(fm_model* m) {
   for (auto& l : m->layers) {
     if (strncmp(l.name, "dec", 3) != 0 || l.c2 == 0 || l.k != 3 || m->pz != 2 || m->deconvolution || m->batch_norm ||
         l.is_norm)
       continue;
-    const int X = spec->X >> l.level, Y = spec->Y >> l.level, Z = spec->Z >> l.level;
+    const int X = m->spec.X >> l.level, Y = m->spec.Y >> l.level, Z = m->spec.Z >> l.level;
     if (!conv_up_supported(X, Y, Z, l.c1, l.c2, l.cout)) continue;
     const size_t n = (size_t)l.cout * 64 * l.c1;
     FM_CUDA(cudaMalloc((void**)&l.w_up_d, n * sizeof(bf16)));
@@ -542,43 +602,6 @@ static int build_unet(fm_ctx* ctx, const fm_unet3d_spec* spec, int kcode, int fl
     FM_CUDA(cudaMalloc((void**)&l.w_up_f, n * sizeof(bf16)));
     FM_CUDA(cudaMalloc((void**)&l.dw_up, n * sizeof(float)));
   }
-  FM_CUDA(cudaMalloc((void**)&m->sums, kNumLossSums * sizeof(double)));
-  FM_CUDA(cudaMemset(m->sums, 0, kNumLossSums * sizeof(double)));
-  m->encA.resize(D);
-  m->encB.resize(D);
-  m->pool.resize(D);
-  m->up.resize(D);
-  m->decA.resize(D);
-  m->decB.resize(D);
-  m->gEncA.resize(D);
-  m->gEncB.resize(D);
-  m->gPool.resize(D);
-  m->gUp.resize(D);
-  m->gSkip.resize(D);
-  m->gDecA.resize(D);
-  m->gDecB.resize(D);
-  m->bnRawL.resize(m->layers.size());
-  m->bnStatsL.resize(m->layers.size());
-  m->layer_done.resize(m->layers.size());
-  for (auto& e : m->layer_done) FM_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-  FM_CUDA(cudaEventCreateWithFlags(&m->ev_tmp, cudaEventDisableTiming));
-  // gradient buckets: consecutive layers in backward (= reverse creation) order, ~1/4 of the
-  // parameters each; every bucket is one contiguous range of the flat buffer.
-  {
-    const int nl = (int)m->layers.size();
-    const int64_t target = m->nparams / 4 + 1;
-    int hi = nl - 1;
-    int64_t acc = 0;
-    for (int i = nl - 1; i >= 0; --i) {
-      acc += m->layers[i].wcount() + m->layers[i].cout;
-      if (acc >= target || i == 0) {
-        m->buckets.push_back({i, hi});
-        hi = i - 1;
-        acc = 0;
-      }
-    }
-  }
-  *out = m;
   return FM_OK;
 }
 
@@ -605,14 +628,14 @@ extern "C" int fm_model_destroy(fm_model* m) {
   for (auto* v : {&m->isIn, &m->isC1, &m->isSum, &m->isUp, &m->isU, &m->isLoc1, &m->isLoc2})
     for (auto& b : *v) b.release();
   for (auto& b : m->isSeg) b.release();
-  for (auto* v : {&m->isRawL, &m->gIsA, &m->gIsB, &m->gIsC, &m->gIsUp})
+  for (auto* v : {&m->normRawL, &m->gIsA, &m->gIsB, &m->gIsC, &m->gIsUp})
     for (auto& b : *v) b.release();
-  for (auto* v : {&m->isStatsL, &m->isDropL, &m->gSeg, &m->dropU, &m->bnStatsL})
+  for (auto* v : {&m->normStatsL, &m->isDropL, &m->gSeg, &m->dropU})
     for (auto& b : *v) b.release();
-  m->gIsRaw.release();
+  m->normRaw.release();
+  m->normGRaw.release();
+  m->normScratch.release();
   m->gIsZero.release();
-  m->isRaw.release();
-  m->isScratch.release();
   m->isAcc.release();
   m->pw_vol.release();
   m->pw_pred.release();
@@ -622,10 +645,6 @@ extern "C" int fm_model_destroy(fm_model* m) {
   m->tta_vol.release();
   m->tta_stack.release();
   m->x_in.release();
-  m->bnRaw.release();
-  m->bnGRaw.release();
-  m->bnScratch.release();
-  for (auto& b : m->bnRawL) b.release();
   m->dcZ.release();
   m->dcG.release();
   m->mask_in.release();
@@ -636,7 +655,8 @@ extern "C" int fm_model_destroy(fm_model* m) {
   for (auto* v : {&m->encA, &m->encB, &m->pool, &m->up, &m->decA, &m->decB, &m->gEncA, &m->gEncB,
                   &m->gPool, &m->gUp, &m->gSkip, &m->gDecA, &m->gDecB})
     for (auto& b : *v) b.release();
-  for (auto& e : m->layer_done) cudaEventDestroy(e);
+  for (auto& e : m->layer_done)
+    if (e) cudaEventDestroy(e);
   for (auto& e : m->pw_events)
     if (e) cudaEventDestroy(e);
   for (int b = 0; b < 2; ++b) {
@@ -891,14 +911,14 @@ static int ensure_capacity(fm_model* m, int B, bool train) {
       const size_t n = (size_t)cap * m->vox(l.level) * l.cout;
       biggest = std::max(biggest, n);
       cmax = std::max(cmax, (size_t)l.cout);
-      if (train || m->train_alloc) {
-        FM_TRY(m->bnRawL[i].ensure(n));
-        FM_TRY(m->bnStatsL[i].ensure((size_t)cap * l.cout * 2));
+      if (train || m->train_alloc) {  // (the block's conv is the layer in front of its norm layer)
+        FM_TRY(m->normRawL[i - 1].ensure(n));
+        FM_TRY(m->normStatsL[i - 1].ensure((size_t)cap * l.cout * 2));
       }
     }
-    FM_TRY(m->bnRaw.ensure(biggest));
-    if (train || m->train_alloc) FM_TRY(m->bnGRaw.ensure(biggest));
-    FM_TRY(m->bnScratch.ensure((size_t)cap * cmax * 2 * 1030));
+    FM_TRY(m->normRaw.ensure(biggest));
+    if (train || m->train_alloc) FM_TRY(m->normGRaw.ensure(biggest));
+    FM_TRY(m->normScratch.ensure((size_t)cap * cmax * 2 * 1030));
   }
   if (train || m->train_alloc) {
     FM_TRY(m->t_in.ensure((size_t)cap * v0));  // (no dL/dz tensor: the head backward forms the Dice gradient itself)
@@ -923,84 +943,126 @@ static int ensure_capacity(fm_model* m, int B, bool train) {
   return FM_OK;
 }
 
-// conv block forward: Conv3D + bias + ReLU (create_convolution_block, unet.py:102-113)
-static int conv_fwd(fm_model* m, const Layer& l, const bf16* x1, const bf16* x2, bf16* y, int B, int relu = 1) {
-  fm_ctx* ctx = m->ctx;
-  const Dims5 d = m->dims(l.level, l.cout, B);
-  const float* bias = m->params + l.b_off;
+// ---------------------------------------------------------------------------------------------
+// conv-kernel routes: the one place that picks the kernel of a conv's forward, data gradient and weight gradient, for
+// every model family and for fm_op_conv_strided. `d` = the extent the pass runs at (d.N = batch): the output extent for
+// the forward, the finer zero-inserted extent for the gradients of a stride-2 conv.
+// ---------------------------------------------------------------------------------------------
+// y = conv(x1 [, x2]) + bias [, ReLU]. A single-channel first source is the fp32 model input.
+static int conv_fwd(fm_ctx* ctx, const Layer& l, const Dims5& d, const void* x1, const bf16* x2, const float* bias,
+                    bf16* y, int relu, bool reproducible) {
+  if (l.c1 == 1)  // Cin = 1: bandwidth kernel
+    return k_conv3d_simt_fprop(ctx, x1, 1, x2, l.w_f, bias, y, nullptr, d.N, d.X, d.Y, d.Z, l.c1, l.c2, l.cout, l.k,
+                               relu, nullptr);
+  const bf16* xb = (const bf16*)x1;
   if (l.march_f)
-    return k_conv3d_march(ctx, x1, x2, l.w_mf[0], l.w_mf[1], bias, y, nullptr, B, d.X, d.Y, d.Z, l.c1, l.c2, l.cout, relu,
-                          l.cout, 0, reproducible_pass(m));
-  if (conv_tc_supported(l.c1, l.c2, l.cout, l.k))
-    return k_conv3d_tc_fprop(ctx, x1, x2, l.w_f, bias, y, nullptr, B, d.X, d.Y, d.Z, l.c1, l.c2, l.cout,
-                             l.k, relu, l.cout, 0);
-  return k_conv3d_simt_fprop(ctx, x1, 0, x2, l.w_f, bias, y, nullptr, B, d.X, d.Y, d.Z, l.c1, l.c2,
-                             l.cout, l.k, relu, nullptr);
+    return k_conv3d_march(ctx, xb, x2, l.w_mf[0], l.w_mf[1], bias, y, nullptr, d.N, d.X, d.Y, d.Z, l.c1, l.c2, l.cout,
+                          relu, l.cout, 0, reproducible);
+  if (conv_tc_supported(l.c1, l.c2, l.cout, l.k)) {
+    const int sz = kext_z(l.k) == 1 ? 1 : l.stride;  // a 2D kernel does not stride along z
+    return k_conv3d_tc_fprop(ctx, xb, x2, l.w_f, bias, y, nullptr, d.N, d.X, d.Y, d.Z, l.c1, l.c2, l.cout, l.k, relu,
+                             l.cout, 0, l.stride, d.X * l.stride, d.Y * l.stride, d.Z * sz);
+  }
+  FM_CHECK(l.stride == 1, FM_EINVAL, "strided conv %s has no fallback", l.name);
+  return k_conv3d_simt_fprop(ctx, xb, 0, x2, l.w_f, bias, y, nullptr, d.N, d.X, d.Y, d.Z, l.c1, l.c2, l.cout, l.k, relu,
+                             nullptr);
 }
 
-// one conv block of a U-Net built with batch_normalization=True: Conv (+bias, no activation) -> raw ->
-// BatchNormalization + ReLU -> y. A training pass keeps the raw output and the batch statistics of every block.
-static int bn_block_fwd(fm_model* m, const Layer& l, const void* x1, int x1_f32, const bf16* x2, bf16* y, int B) {
-  fm_ctx* ctx = m->ctx;
-  const int li = (int)(&l - &m->layers[0]);
+// dx = conv(dy, W flipped^T) towards source `src` [* ReLU mask of `mask`]
+static int conv_dgrad(fm_ctx* ctx, const Layer& l, const Dims5& d, int src, const bf16* dy, const bf16* mask, bf16* dx,
+                      bool reproducible) {
+  const int cs = src == 0 ? l.c1 : l.c2;
+  const bf16* wd = src == 0 ? l.w_d0 : l.w_d1;
+  if (l.march_d[src])
+    return k_conv3d_march(ctx, dy, nullptr, l.w_md[src], nullptr, nullptr, dx, mask, d.N, d.X, d.Y, d.Z, l.cout, 0, cs,
+                          0, cs, 0, reproducible);
+  if (conv_tc_supported(l.cout, 0, cs, l.k))
+    return k_conv3d_tc_fprop(ctx, dy, nullptr, wd, nullptr, dx, mask, d.N, d.X, d.Y, d.Z, l.cout, 0, cs, l.k, 0, cs, 0);
+  return k_conv3d_simt_fprop(ctx, dy, 0, nullptr, wd, nullptr, dx, nullptr, d.N, d.X, d.Y, d.Z, l.cout, 0, cs, l.k, 0,
+                             mask);
+}
+
+// dw += weight gradient of each source against dy (only_src >= 0: that source alone). db: the bias gradient, which the
+// first marching source sums while its tiles sit in shared memory, else k_bias_grad after the sources; null: none.
+static int conv_wgrad(fm_ctx* ctx, const Layer& l, const Dims5& d, const void* x1, const bf16* x2, const bf16* dy,
+                      float* dw, float* db, int only_src = -1) {
+  const void* xs[2] = {x1, x2};
+  const int cs[2] = {l.c1, l.c2};
+  int cofs = 0;
+  for (int s = 0; s < (l.c2 ? 2 : 1); ++s) {
+    if (only_src < 0 || s == only_src) {
+      const bf16* x = (const bf16*)xs[s];
+      if (cs[s] == 1) {  // the fp32 single-channel model input
+        FM_TRY(k_conv3d_simt_wgrad(ctx, xs[s], 1, dy, dw, d.N, d.X, d.Y, d.Z, cs[s], l.cin(), cofs, l.cout, l.k));
+      } else if (conv_wgrad_march_supported(d.X, d.Y, d.Z, cs[s], l.cout, l.k)) {
+        FM_TRY(k_conv3d_wgrad_march(ctx, x, dy, dw, d.N, d.X, d.Y, d.Z, cs[s], l.cin(), cofs, l.cout, db));
+        db = nullptr;
+      } else if (conv_tc_supported(cs[s], 0, l.cout, l.k)) {
+        FM_TRY(k_conv3d_tc_wgrad(ctx, x, dy, dw, d.N, d.X, d.Y, d.Z, cs[s], l.cin(), cofs, l.cout, l.k));
+      } else {
+        FM_TRY(k_conv3d_simt_wgrad(ctx, x, 0, dy, dw, d.N, d.X, d.Y, d.Z, cs[s], l.cin(), cofs, l.cout, l.k));
+      }
+    }
+    cofs += cs[s];
+  }
+  return db ? k_bias_grad(ctx, dy, db, d.voxels(), l.cout) : FM_OK;
+}
+
+// The routes for a layer of model m (the gradients of a stride-2 conv run one level finer).
+static int conv_fwd(fm_model* m, const Layer& l, const void* x1, const bf16* x2, bf16* y, int B, int relu) {
+  return conv_fwd(m->ctx, l, m->dims(l.level, l.cout, B), x1, x2, m->params + l.b_off, y, relu, reproducible_pass(m));
+}
+static int conv_dgrad(fm_model* m, const Layer& l, int src, const bf16* dy, const bf16* mask, bf16* dx, int B) {
+  return conv_dgrad(m->ctx, l, m->dims(l.bwd_level(), l.cout, B), src, dy, mask, dx, reproducible_pass(m));
+}
+// The Isensee convs get no bias gradient: each feeds an InstanceNormalization, which removes a per-channel constant, so
+// the gradient of such a bias is exactly zero (the buffer was zeroed at the start of the backward pass; summing dY would
+// only return the rounding noise of a sum that vanishes analytically). The U-Nets sum theirs, as Keras does.
+static int conv_wgrad(fm_model* m, const Layer& l, const void* x1, const bf16* x2, const bf16* dy, int B,
+                      int only_src = -1) {
+  return conv_wgrad(m->ctx, l, m->dims(l.bwd_level(), l.cout, B), x1, x2, dy, m->grads + l.w_off,
+                    m->kind == 1 ? nullptr : m->grads + l.b_off, only_src);
+}
+
+static int conv_wgrad_source(fm_model* m, const Layer& l, int src, const bf16* x, const bf16* dy, int B) {
+  return conv_wgrad(m, l, src == 0 ? x : nullptr, src == 1 ? x : nullptr, dy, B, src);
+}
+
+// Deconvolution3D / 2D (kernel 2, stride 2, C -> C channels) of the coarse x (extent dc): the 1x1x1 conv to 4*pz*C
+// parity-class channels into z8, then depth-to-space with the bias -> the fine y.
+static int deconv_fwd(fm_ctx* ctx, const bf16* x, const bf16* w_f, const float* bias, bf16* z8, bf16* y,
+                      const Dims5& dc, int pz) {
+  const int c8 = 4 * pz * dc.C;
+  FM_TRY(k_conv3d_tc_fprop(ctx, x, nullptr, w_f, nullptr, z8, nullptr, dc.N, dc.X, dc.Y, dc.Z, dc.C, 0, c8, 1, 0, c8, 0));
+  return k_depth_to_space(ctx, z8, bias, y, dc, pz);
+}
+
+// Its backward from the fine gradient g: the bias gradient db (column sums of g); space-to-depth into z8, the dY of the
+// 1x1x1 conv; its weight gradient dw against x; then `wgrad_done` is recorded (when given) and the data gradient dx
+// runs through the transposed matrix w_d, masked by the ReLU of `mask` (when given).
+static int deconv_bwd(fm_ctx* ctx, const bf16* x, const bf16* g, const bf16* w_d, const bf16* mask, bf16* z8, bf16* dx,
+                      float* dw, float* db, const Dims5& dc, int pz, cudaEvent_t wgrad_done) {
+  const int c8 = 4 * pz * dc.C;
+  FM_TRY(k_bias_grad(ctx, g, db, dc.voxels() * 4 * pz, dc.C));
+  FM_TRY(k_space_to_depth(ctx, g, z8, dc, pz));
+  FM_TRY(k_conv3d_tc_wgrad(ctx, x, z8, dw, dc.N, dc.X, dc.Y, dc.Z, dc.C, dc.C, 0, c8, 1));
+  if (wgrad_done) FM_CUDA(cudaEventRecord(wgrad_done, ctx->stream));
+  return k_conv3d_tc_fprop(ctx, z8, nullptr, w_d, nullptr, dx, mask, dc.N, dc.X, dc.Y, dc.Z, c8, 0, dc.C, 1, 0, dc.C,
+                           0);
+}
+
+// One conv block of a U-Net: Conv + bias + ReLU (create_convolution_block, unet.py:102-113), or under
+// batch_normalization=True Conv (+bias, no activation) -> raw -> BatchNormalization + ReLU. A training pass keeps the
+// raw output and the batch statistics of every block.
+static int unet_block_fwd(fm_model* m, const Layer& l, const void* x1, const bf16* x2, bf16* y, int B) {
+  if (!m->batch_norm) return conv_fwd(m, l, x1, x2, y, B, 1);
+  const int li = layer_pos(m, l);
   const Layer &nl = m->layers[li + 1], &ml = m->layers[li + 2];
-  const Dims5 d = m->dims(l.level, l.cout, B);
-  bf16* raw = m->train_pass ? m->bnRawL[li + 1].p : m->bnRaw.p;
-  if (x1_f32)  // the first conv of the 3D model reads the fp32 single-channel input
-    FM_TRY(k_conv3d_simt_fprop(ctx, x1, 1, nullptr, l.w_f, m->params + l.b_off, raw, nullptr, B, d.X, d.Y, d.Z, l.c1, 0,
-                               l.cout, l.k, 0, nullptr));
-  else
-    FM_TRY(conv_fwd(m, l, (const bf16*)x1, x2, raw, B, 0));
-  return k_batchnorm_relu(ctx, raw, m->params + nl.w_off, m->params + nl.b_off, m->params + ml.w_off,
-                          m->params + ml.b_off, y, B, m->vox(l.level), l.cout, m->bnScratch.p, m->bnScratch.n,
-                          m->train_pass ? m->bnStatsL[li + 1].p : nullptr, m->train_pass ? 1 : 0);
-}
-
-static int forward_unet_bn(fm_model* m, int B) {
-  fm_ctx* ctx = m->ctx;
-  const int D = m->depth();
-  FM_TRY(refresh_packs(m));
-  const bf16* cur = nullptr;
-  for (int d = 0; d < D; ++d) {
-    const Layer &la = L(m, "enc%da", d), &lb = L(m, "enc%db", d);
-    if (d == 0 && m->kcode == 31) {
-      FM_TRY(k_pad_cast(ctx, m->x_in.p, m->x_pad.p, (int64_t)B * m->vox(0), m->cin_real, 16));
-      FM_TRY(bn_block_fwd(m, la, m->x_pad.p, 0, nullptr, m->encA[0].p, B));
-    } else if (d == 0) {
-      FM_TRY(bn_block_fwd(m, la, m->x_in.p, 1, nullptr, m->encA[0].p, B));
-    } else {
-      FM_TRY(bn_block_fwd(m, la, cur, 0, nullptr, m->encA[d].p, B));
-    }
-    FM_TRY(bn_block_fwd(m, lb, m->encA[d].p, 0, nullptr, m->encB[d].p, B));
-    cur = m->encB[d].p;
-    if (d < D - 1) {
-      FM_TRY(k_maxpool3d_fwd(ctx, m->encB[d].p, m->pool[d].p, m->dims(d, lb.cout, B), m->pz));
-      cur = m->pool[d].p;
-    }
-  }
-  for (int d = D - 2; d >= 0; --d) {
-    const Layer &da = L(m, "dec%da", d), &db = L(m, "dec%db", d);
-    if (m->deconvolution) {
-      const Layer& lu = L(m, "up%d", d);
-      const Dims5 dc = m->dims(d + 1, lu.cout, B);
-      FM_TRY(k_conv3d_tc_fprop(ctx, cur, nullptr, lu.w_f, nullptr, m->dcZ.p, nullptr, B, dc.X, dc.Y, dc.Z, lu.c1, 0,
-                               lu.cout * lu.taps(), 1, 0, lu.cout * lu.taps(), 0));
-      FM_TRY(k_depth_to_space(ctx, m->dcZ.p, m->params + lu.b_off, m->up[d].p, dc, m->pz));
-    } else {
-      FM_TRY(k_upsample3d_fwd(ctx, cur, m->up[d].p, m->dims(d + 1, da.c1, B), m->pz));
-    }
-    FM_TRY(bn_block_fwd(m, da, m->up[d].p, 0, m->encB[d].p, m->decA[d].p, B));
-    FM_TRY(bn_block_fwd(m, db, m->decA[d].p, 0, nullptr, m->decB[d].p, B));
-    cur = m->decB[d].p;
-  }
-  const Layer& lf = m->layers.back();
-  if (m->train_pass && m->targets_ready) {
-    FM_TRY(k_head_fwd_dice(ctx, cur, m->params + lf.w_off, m->params + lf.b_off, m->t_in.p, m->prob.p,
-                           (int64_t)B * m->vox(0), lf.c1, m->sums, m->xent()));
-    m->stats_done = true;
-    return FM_OK;
-  }
-  return k_head_fwd(ctx, cur, m->params + lf.w_off, m->params + lf.b_off, m->prob.p, (int64_t)B * m->vox(0), lf.c1);
+  bf16* raw = m->train_pass ? m->normRawL[li].p : m->normRaw.p;
+  FM_TRY(conv_fwd(m, l, x1, x2, raw, B, 0));
+  return k_batchnorm_relu(m->ctx, raw, m->params + nl.w_off, m->params + nl.b_off, m->params + ml.w_off,
+                          m->params + ml.b_off, y, B, m->vox(l.level), l.cout, m->normScratch.p, m->normScratch.n,
+                          m->train_pass ? m->normStatsL[li].p : nullptr, m->train_pass ? 1 : 0);
 }
 
 static int forward_isensee(fm_model* m, int B);
@@ -1020,25 +1082,19 @@ static int unet_dropout_fwd(fm_model* m, int slot, bf16* act, const Layer& l, in
 // forward pass on x_in (fp32 [B, X, Y, Z], C = 1) -> prob (fp32 [B, X, Y, Z])
 static int forward(fm_model* m, int B) {
   if (m->kind == 1) return forward_isensee(m, B);
-  if (m->batch_norm) return forward_unet_bn(m, B);
   fm_ctx* ctx = m->ctx;
   const int D = m->depth();
   FM_TRY(refresh_packs(m));
-  const bf16* cur = nullptr;
+  const void* cur = m->x_in.p;  // the 3D model's first conv reads the fp32 single-channel input
+  if (m->kcode == 31) {
+    FM_TRY(k_pad_cast(ctx, m->x_in.p, m->x_pad.p, (int64_t)B * m->vox(0), m->cin_real, 16));
+    cur = m->x_pad.p;
+  }
   for (int d = 0; d < D; ++d) {
     const Layer &la = L(m, "enc%da", d), &lb = L(m, "enc%db", d);
-    const Dims5 dd = m->dims(d, la.cout, B);
-    if (d == 0 && m->kcode == 31) {
-      FM_TRY(k_pad_cast(ctx, m->x_in.p, m->x_pad.p, dd.voxels(), m->cin_real, 16));
-      FM_TRY(conv_fwd(m, la, m->x_pad.p, nullptr, m->encA[0].p, B));
-    } else if (d == 0) {
-      FM_TRY(k_conv3d_simt_fprop(ctx, m->x_in.p, 1, nullptr, la.w_f, m->params + la.b_off, m->encA[0].p,
-                                 nullptr, B, dd.X, dd.Y, dd.Z, la.c1, 0, la.cout, la.k, 1, nullptr));
-    } else {
-      FM_TRY(conv_fwd(m, la, cur, nullptr, m->encA[d].p, B));
-    }
+    FM_TRY(unet_block_fwd(m, la, cur, nullptr, m->encA[d].p, B));
     if (m->train_pass && m->unet_dropout()) FM_TRY(unet_dropout_fwd(m, d, m->encA[d].p, la, B));
-    FM_TRY(conv_fwd(m, lb, m->encA[d].p, nullptr, m->encB[d].p, B));
+    FM_TRY(unet_block_fwd(m, lb, m->encA[d].p, nullptr, m->encB[d].p, B));
     cur = m->encB[d].p;
     if (d < D - 1) {
       FM_TRY(k_maxpool3d_fwd(ctx, m->encB[d].p, m->pool[d].p, m->dims(d, lb.cout, B), m->pz));
@@ -1047,202 +1103,90 @@ static int forward(fm_model* m, int B) {
   }
   for (int d = D - 2; d >= 0; --d) {
     const Layer &da = L(m, "dec%da", d), &db = L(m, "dec%db", d);
+    const bf16* coarse = (const bf16*)cur;
     if (da.up_coarse) {
       // no upsampled tensor: the conv reads the coarse tensor with class-combined weights (8 taps instead of 27)
       const Dims5 dd = m->dims(d, da.cout, B);
-      FM_TRY(k_conv3d_up_fprop(ctx, cur, m->encB[d].p, da.w_up_f, da.w_f, m->params + da.b_off, m->decA[d].p, B, dd.X,
-                               dd.Y, dd.Z, da.c1, da.c2, da.cout, 1));
-    } else if (m->deconvolution) {
-      // Deconvolution3D: 1x1x1 conv of the coarse tensor to (classes x C) channels, then depth-to-space (+ bias)
-      const Layer& lu = L(m, "up%d", d);
-      const Dims5 dc = m->dims(d + 1, lu.cout, B);
-      FM_TRY(k_conv3d_tc_fprop(ctx, cur, nullptr, lu.w_f, nullptr, m->dcZ.p, nullptr, B, dc.X, dc.Y, dc.Z, lu.c1, 0,
-                               lu.cout * lu.taps(), 1, 0, lu.cout * lu.taps(), 0));
-      FM_TRY(k_depth_to_space(ctx, m->dcZ.p, m->params + lu.b_off, m->up[d].p, dc, m->pz));
-      FM_TRY(conv_fwd(m, da, m->up[d].p, m->encB[d].p, m->decA[d].p, B));
+      FM_TRY(k_conv3d_up_fprop(ctx, coarse, m->encB[d].p, da.w_up_f, da.w_f, m->params + da.b_off, m->decA[d].p, B,
+                               dd.X, dd.Y, dd.Z, da.c1, da.c2, da.cout, 1));
     } else {
-      FM_TRY(k_upsample3d_fwd(ctx, cur, m->up[d].p, m->dims(d + 1, da.c1, B), m->pz));
-      FM_TRY(conv_fwd(m, da, m->up[d].p, m->encB[d].p, m->decA[d].p, B));
+      if (m->deconvolution) {
+        const Layer& lu = L(m, "up%d", d);
+        FM_TRY(deconv_fwd(ctx, coarse, lu.w_f, m->params + lu.b_off, m->dcZ.p, m->up[d].p, m->dims(d + 1, lu.cout, B),
+                          m->pz));
+      } else {
+        FM_TRY(k_upsample3d_fwd(ctx, coarse, m->up[d].p, m->dims(d + 1, da.c1, B), m->pz));
+      }
+      FM_TRY(unet_block_fwd(m, da, m->up[d].p, m->encB[d].p, m->decA[d].p, B));
     }
     if (m->train_pass && m->unet_dropout()) FM_TRY(unet_dropout_fwd(m, D + d, m->decA[d].p, da, B));
-    FM_TRY(conv_fwd(m, db, m->decA[d].p, nullptr, m->decB[d].p, B));
+    FM_TRY(unet_block_fwd(m, db, m->decA[d].p, nullptr, m->decB[d].p, B));
     cur = m->decB[d].p;
   }
   const Layer& lf = m->layers.back();
   if (m->train_pass && m->targets_ready) {
     // head + sigmoid + Dice / VOD / accuracy sums in one pass (unet.py:68-69 + metrics.py:11-28)
-    FM_TRY(k_head_fwd_dice(ctx, cur, m->params + lf.w_off, m->params + lf.b_off, m->t_in.p, m->prob.p,
+    FM_TRY(k_head_fwd_dice(ctx, (const bf16*)cur, m->params + lf.w_off, m->params + lf.b_off, m->t_in.p, m->prob.p,
                            (int64_t)B * m->vox(0), lf.c1, m->sums, m->xent()));
     m->stats_done = true;
     return FM_OK;
   }
-  FM_TRY(k_head_fwd(ctx, cur, m->params + lf.w_off, m->params + lf.b_off, m->prob.p,
-                    (int64_t)B * m->vox(0), lf.c1));
-  return FM_OK;
-}
-
-// wgrad + bias grad of one conv layer (only_src >= 0: the weight gradient of that source alone, plus the bias)
-static int conv_wgrad(fm_model* m, const Layer& l, const bf16* x1, const bf16* x2, const bf16* dy, int B,
-                      int only_src = -1) {
-  fm_ctx* ctx = m->ctx;
-  const Dims5 d = m->dims(l.level, l.cout, B);
-  float* dw = m->grads + l.w_off;
-  const bf16* xs[2] = {x1, x2};
-  const int cs[2] = {l.c1, l.c2};
-  int cofs = 0;
-  bool bias_done = false;
-  for (int s = 0; s < (l.c2 ? 2 : 1); ++s) {
-    if (only_src >= 0 && s != only_src) {
-      cofs += cs[s];
-      continue;
-    }
-    if (conv_wgrad_march_supported(d.X, d.Y, d.Z, cs[s], l.cout, l.k)) {
-      // the marching kernel also sums dY over the voxels (bias gradient) while the tiles sit in shared memory
-      FM_TRY(k_conv3d_wgrad_march(ctx, xs[s], dy, dw, B, d.X, d.Y, d.Z, cs[s], l.cin(), cofs, l.cout,
-                                  bias_done ? nullptr : m->grads + l.b_off));
-      bias_done = true;
-    } else if (conv_tc_supported(cs[s], 0, l.cout, l.k))
-      FM_TRY(k_conv3d_tc_wgrad(ctx, xs[s], dy, dw, B, d.X, d.Y, d.Z, cs[s], l.cin(), cofs, l.cout, l.k));
-    else
-      FM_TRY(k_conv3d_simt_wgrad(ctx, xs[s], 0, dy, dw, B, d.X, d.Y, d.Z, cs[s], l.cin(), cofs, l.cout,
-                                 l.k));
-    cofs += cs[s];
-  }
-  if (!bias_done) FM_TRY(k_bias_grad(ctx, dy, m->grads + l.b_off, d.voxels(), l.cout));
-  return FM_OK;
-}
-
-static int conv_wgrad_source(fm_model* m, const Layer& l, int src, const bf16* x, const bf16* dy, int B) {
-  return conv_wgrad(m, l, src == 0 ? x : nullptr, src == 1 ? x : nullptr, dy, B, src);
-}
-
-// dgrad of one source of a conv layer: dx = conv(dy, W flipped^T) [* ReLU mask of `mask`]
-static int conv_dgrad(fm_model* m, const Layer& l, int src, const bf16* dy, const bf16* mask, bf16* dx,
-                      int B) {
-  fm_ctx* ctx = m->ctx;
-  const Dims5 d = m->dims(l.level, l.cout, B);
-  const int cs = src == 0 ? l.c1 : l.c2;
-  const bf16* wd = src == 0 ? l.w_d0 : l.w_d1;
-  if (l.march_d[src])
-    return k_conv3d_march(ctx, dy, nullptr, l.w_md[src], nullptr, nullptr, dx, mask, B, d.X, d.Y, d.Z, l.cout, 0, cs, 0,
-                          cs, 0, reproducible_pass(m));
-  if (conv_tc_supported(l.cout, 0, cs, l.k))
-    return k_conv3d_tc_fprop(ctx, dy, nullptr, wd, nullptr, dx, mask, B, d.X, d.Y, d.Z, l.cout, 0, cs, l.k,
-                             0, cs, 0);
-  return k_conv3d_simt_fprop(ctx, dy, 0, nullptr, wd, nullptr, dx, nullptr, B, d.X, d.Y, d.Z, l.cout, 0,
-                             cs, l.k, 0, mask);
+  return k_head_fwd(ctx, (const bf16*)cur, m->params + lf.w_off, m->params + lf.b_off, m->prob.p,
+                    (int64_t)B * m->vox(0), lf.c1);
 }
 
 static int mark_layer_done(fm_model* m, const Layer& l) {
-  const int i = (int)(&l - &m->layers[0]);
-  FM_CUDA(cudaEventRecord(m->layer_done[i], m->ctx->stream));
+  FM_CUDA(cudaEventRecord(m->layer_done[layer_pos(m, l)], m->ctx->stream));
   return FM_OK;
 }
 
 static int backward_isensee(fm_model* m, int B);
 
-// BatchNormalization + ReLU backward of block `l` (gy [+ gy2] = gradient of the block's activation) -> m->bnGRaw, the
-// gradient of the raw conv output; gamma / beta gradients. The conv bias in front of the normalisation has an
-// analytically zero gradient (conv_wgrad still sums it: rounding noise, as in Keras).
-static int bn_block_bwd(fm_model* m, const Layer& l, const bf16* gy, const bf16* gy2, int B) {
-  const int li = (int)(&l - &m->layers[0]);
-  const Layer& nl = m->layers[li + 1];
-  FM_TRY(k_batchnorm_relu_bwd(m->ctx, m->bnRawL[li + 1].p, m->bnStatsL[li + 1].p, m->params + nl.w_off,
-                              m->params + nl.b_off, gy, gy2, m->bnGRaw.p, m->grads + nl.w_off, m->grads + nl.b_off, B,
-                              m->vox(l.level), l.cout, m->bnScratch.p, m->bnScratch.n));
-  FM_TRY(mark_layer_done(m, m->layers[li + 2]));
+// Backward of a U-Net block's epilogue from gy, the gradient of the block's activation: *dy = the gradient of its conv
+// output. Without batch normalisation that is gy (the ReLU mask was applied where gy was formed). With it: the
+// BatchNormalization + ReLU backward into normGRaw and the gamma / beta gradients; the moving statistics and then the
+// norm layer are done. The conv bias in front of the normalisation has an analytically zero gradient (conv_wgrad
+// still sums it: rounding noise, as in Keras).
+static int unet_block_bwd(fm_model* m, const Layer& l, const bf16* gy, int B, const bf16** dy) {
+  *dy = gy;
+  if (!m->batch_norm) return FM_OK;
+  const int li = layer_pos(m, l);
+  const Layer &nl = m->layers[li + 1], &ml = m->layers[li + 2];
+  FM_TRY(k_batchnorm_relu_bwd(m->ctx, m->normRawL[li].p, m->normStatsL[li].p, m->params + nl.w_off,
+                              m->params + nl.b_off, gy, nullptr, m->normGRaw.p, m->grads + nl.w_off,
+                              m->grads + nl.b_off, B, m->vox(l.level), l.cout, m->normScratch.p, m->normScratch.n));
+  *dy = m->normGRaw.p;
+  FM_TRY(mark_layer_done(m, ml));
   return mark_layer_done(m, nl);
-}
-
-// Backward pass of a U-Net built with batch_normalization=True: the ReLU derivative lives in the normalisation
-// backward (it is recomputed from the raw conv output and the batch statistics), so every dgrad / pooling / upsampling
-// gradient runs WITHOUT an activation mask; the decoder's upsampled source is materialised.
-static int backward_unet_bn(fm_model* m, int B) {
-  fm_ctx* ctx = m->ctx;
-  const int D = m->depth();
-  const int64_t n0 = (int64_t)B * m->vox(0);
-  FM_TRY(k_zero(ctx, m->grads, (size_t)m->nparams * sizeof(float)));
-  const Layer& lf = m->layers.back();
-  FM_TRY(k_head_bwd(ctx, m->decB[0].p, m->prob.p, m->params + lf.w_off, m->gDecB[0].p, m->grads + lf.w_off,
-                    m->grads + lf.b_off, n0, lf.c1, 1, m->t_in.p, m->sums, m->xent()));
-  FM_TRY(mark_layer_done(m, lf));
-  for (int d = 0; d <= D - 2; ++d) {
-    const Layer &da = L(m, "dec%da", d), &db = L(m, "dec%db", d);
-    FM_TRY(bn_block_bwd(m, db, m->gDecB[d].p, nullptr, B));
-    FM_TRY(conv_wgrad(m, db, m->decA[d].p, nullptr, m->bnGRaw.p, B));
-    FM_TRY(mark_layer_done(m, db));
-    FM_TRY(conv_dgrad(m, db, 0, m->bnGRaw.p, nullptr, m->gDecA[d].p, B));
-    FM_TRY(bn_block_bwd(m, da, m->gDecA[d].p, nullptr, B));
-    FM_TRY(conv_wgrad(m, da, m->up[d].p, m->encB[d].p, m->bnGRaw.p, B));
-    FM_TRY(mark_layer_done(m, da));
-    FM_TRY(conv_dgrad(m, da, 0, m->bnGRaw.p, nullptr, m->gUp[d].p, B));
-    FM_TRY(conv_dgrad(m, da, 1, m->bnGRaw.p, nullptr, m->gSkip[d].p, B));
-    const bool bottom = (d + 1 == D - 1);
-    const bf16* act = bottom ? m->encB[D - 1].p : m->decB[d + 1].p;
-    bf16* gdst = bottom ? m->gEncB[D - 1].p : m->gDecB[d + 1].p;
-    if (m->deconvolution) {
-      const Layer& lu = L(m, "up%d", d);
-      const Dims5 dc = m->dims(d + 1, lu.cout, B);
-      const int c8 = lu.cout * lu.taps();
-      FM_TRY(k_bias_grad(ctx, m->gUp[d].p, m->grads + lu.b_off, (int64_t)B * m->vox(d), lu.cout));
-      FM_TRY(k_space_to_depth(ctx, m->gUp[d].p, m->dcG.p, dc, m->pz));
-      FM_TRY(k_conv3d_tc_wgrad(ctx, act, m->dcG.p, m->grads + lu.w_off, B, dc.X, dc.Y, dc.Z, lu.c1, lu.c1, 0, c8, 1));
-      FM_TRY(mark_layer_done(m, lu));
-      FM_TRY(k_conv3d_tc_fprop(ctx, m->dcG.p, nullptr, lu.w_d0, nullptr, gdst, nullptr, B, dc.X, dc.Y, dc.Z, c8, 0, lu.c1,
-                               1, 0, lu.c1, 0));
-    } else {
-      FM_TRY(k_upsample3d_bwd(ctx, m->gUp[d].p, nullptr, gdst, m->dims(d + 1, da.c1, B), da.c1, 0, m->pz));
-    }
-  }
-  for (int d = D - 1; d >= 0; --d) {
-    const Layer &la = L(m, "enc%da", d), &lb = L(m, "enc%db", d);
-    if (d < D - 1)  // gradient of encB[d]: skip path + MaxPooling backward (no mask)
-      FM_TRY(k_maxpool3d_bwd(ctx, m->encB[d].p, m->gPool[d].p, m->gSkip[d].p, m->gEncB[d].p, m->dims(d, lb.cout, B), 0,
-                             m->pz));
-    FM_TRY(bn_block_bwd(m, lb, m->gEncB[d].p, nullptr, B));
-    FM_TRY(conv_wgrad(m, lb, m->encA[d].p, nullptr, m->bnGRaw.p, B));
-    FM_TRY(mark_layer_done(m, lb));
-    FM_TRY(conv_dgrad(m, lb, 0, m->bnGRaw.p, nullptr, m->gEncA[d].p, B));
-    FM_TRY(bn_block_bwd(m, la, m->gEncA[d].p, nullptr, B));
-    if (d > 0) {
-      FM_TRY(conv_wgrad(m, la, m->pool[d - 1].p, nullptr, m->bnGRaw.p, B));
-      FM_TRY(mark_layer_done(m, la));
-      FM_TRY(conv_dgrad(m, la, 0, m->bnGRaw.p, nullptr, m->gPool[d - 1].p, B));
-    } else if (m->kcode == 31) {
-      FM_TRY(conv_wgrad(m, la, m->x_pad.p, nullptr, m->bnGRaw.p, B));
-      FM_TRY(mark_layer_done(m, la));
-    } else {
-      const Dims5 dd = m->dims(0, la.cout, B);
-      FM_TRY(k_conv3d_simt_wgrad(ctx, m->x_in.p, 1, m->bnGRaw.p, m->grads + la.w_off, B, dd.X, dd.Y, dd.Z, la.c1, la.c1, 0,
-                                 la.cout, la.k));
-      FM_TRY(k_bias_grad(ctx, m->bnGRaw.p, m->grads + la.b_off, dd.voxels(), la.cout));
-      FM_TRY(mark_layer_done(m, la));
-    }
-  }
-  return FM_OK;
 }
 
 static int backward(fm_model* m, int B) {
   if (m->kind == 1) return backward_isensee(m, B);
-  if (m->batch_norm) return backward_unet_bn(m, B);
   fm_ctx* ctx = m->ctx;
   const int D = m->depth();
   const int64_t n0 = (int64_t)B * m->vox(0);
+  // under batch normalisation the ReLU derivative lives in the normalisation backward (recomputed from the raw conv
+  // output and the batch statistics): no gradient is masked by an activation
+  const bool bn = m->batch_norm;
+  auto relu_mask = [bn](const bf16* act) { return bn ? nullptr : act; };
+  const bf16* dy = nullptr;
   FM_TRY(k_zero(ctx, m->grads, (size_t)m->nparams * sizeof(float)));
   const Layer& lf = m->layers.back();
   // head backward with the soft-Dice gradient formed inside (closed form through the sigmoid with the GLOBAL sums):
-  // gradient lands masked by the ReLU of dec0b (or encB[0] when depth == 1)
+  // without batch normalisation the gradient lands masked by the ReLU of dec0b
   FM_TRY(k_head_bwd(ctx, m->decB[0].p, m->prob.p, m->params + lf.w_off, m->gDecB[0].p, m->grads + lf.w_off,
-                    m->grads + lf.b_off, n0, lf.c1, 0, m->t_in.p, m->sums, m->xent()));
+                    m->grads + lf.b_off, n0, lf.c1, bn ? 1 : 0, m->t_in.p, m->sums, m->xent()));
   FM_TRY(mark_layer_done(m, lf));
   for (int d = 0; d <= D - 2; ++d) {
     const Layer &da = L(m, "dec%da", d), &db = L(m, "dec%db", d);
     // dec_b: input decA[d]
-    FM_TRY(conv_wgrad(m, db, m->decA[d].p, nullptr, m->gDecB[d].p, B));
+    FM_TRY(unet_block_bwd(m, db, m->gDecB[d].p, B, &dy));
+    FM_TRY(conv_wgrad(m, db, m->decA[d].p, nullptr, dy, B));
     FM_TRY(mark_layer_done(m, db));
-    FM_TRY(conv_dgrad(m, db, 0, m->gDecB[d].p, m->decA[d].p, m->gDecA[d].p, B));
+    FM_TRY(conv_dgrad(m, db, 0, dy, relu_mask(m->decA[d].p), m->gDecA[d].p, B));
     if (m->unet_dropout()) FM_TRY(k_channel_scale(ctx, m->gDecA[d].p, m->dropU[D + d].p, B, m->vox(d), da.cout));
     // dec_a: inputs [up[d], encB[d]]; the coarser tensor that was upsampled and its ReLU mask
+    FM_TRY(unet_block_bwd(m, da, m->gDecA[d].p, B, &dy));
     const bool bottom = (d + 1 == D - 1);
     const bf16* act = bottom ? m->encB[D - 1].p : m->decB[d + 1].p;
     bf16* gdst = bottom ? m->gEncB[D - 1].p : m->gDecB[d + 1].p;
@@ -1252,65 +1196,52 @@ static int backward(fm_model* m, int B) {
       // straight from dY (no gUp tensor, no sum-pool pass)
       const Dims5 dd = m->dims(d, da.cout, B);
       FM_TRY(k_zero(ctx, da.dw_up, (size_t)da.cout * 64 * da.c1 * sizeof(float)));
-      FM_TRY(k_conv3d_up_wgrad(ctx, act, m->gDecA[d].p, da.dw_up, B, dd.X, dd.Y, dd.Z, da.c1, da.cout));
+      FM_TRY(k_conv3d_up_wgrad(ctx, act, dy, da.dw_up, B, dd.X, dd.Y, dd.Z, da.c1, da.cout));
       FM_TRY(k_fold_up_wgrad(ctx, da.dw_up, m->grads + da.w_off, da.cout, da.c1, da.cin()));
-      FM_TRY(conv_wgrad_source(m, da, 1, m->encB[d].p, m->gDecA[d].p, B));
+      FM_TRY(conv_wgrad_source(m, da, 1, m->encB[d].p, dy, B));
       FM_TRY(mark_layer_done(m, da));
-      FM_TRY(k_conv3d_up_dgrad(ctx, m->gDecA[d].p, da.w_up_d, gdst, act, B, dd.X, dd.Y, dd.Z, da.cout, da.c1));
-      FM_TRY(conv_dgrad(m, da, 1, m->gDecA[d].p, nullptr, m->gSkip[d].p, B));
+      FM_TRY(k_conv3d_up_dgrad(ctx, dy, da.w_up_d, gdst, act, B, dd.X, dd.Y, dd.Z, da.cout, da.c1));
+      FM_TRY(conv_dgrad(m, da, 1, dy, nullptr, m->gSkip[d].p, B));
       continue;
     }
-    FM_TRY(conv_wgrad(m, da, m->up[d].p, m->encB[d].p, m->gDecA[d].p, B));
+    FM_TRY(conv_wgrad(m, da, m->up[d].p, m->encB[d].p, dy, B));
     FM_TRY(mark_layer_done(m, da));
     if (da.up_dgrad) {
       const Dims5 dd = m->dims(d, da.cout, B);
-      FM_TRY(k_conv3d_up_dgrad(ctx, m->gDecA[d].p, da.w_up_d, gdst, act, B, dd.X, dd.Y, dd.Z, da.cout, da.c1));
-      FM_TRY(conv_dgrad(m, da, 1, m->gDecA[d].p, nullptr, m->gSkip[d].p, B));
+      FM_TRY(k_conv3d_up_dgrad(ctx, dy, da.w_up_d, gdst, act, B, dd.X, dd.Y, dd.Z, da.cout, da.c1));
+      FM_TRY(conv_dgrad(m, da, 1, dy, nullptr, m->gSkip[d].p, B));
       continue;
     }
-    FM_TRY(conv_dgrad(m, da, 0, m->gDecA[d].p, nullptr, m->gUp[d].p, B));
-    FM_TRY(conv_dgrad(m, da, 1, m->gDecA[d].p, nullptr, m->gSkip[d].p, B));
+    FM_TRY(conv_dgrad(m, da, 0, dy, nullptr, m->gUp[d].p, B));
+    FM_TRY(conv_dgrad(m, da, 1, dy, nullptr, m->gSkip[d].p, B));
     if (m->deconvolution) {
-      // Deconvolution3D backward: bias gradient = column sums of the fine gradient; the shuffled gradient is the dY
-      // of a 1x1x1 conv with (classes x C) outputs: weight gradient against the coarse activation, data gradient
-      // (+ ReLU mask of the coarse block) through the transposed matrix
       const Layer& lu = L(m, "up%d", d);
-      const Dims5 dc = m->dims(d + 1, lu.cout, B);
-      const int c8 = lu.cout * lu.taps();
-      FM_TRY(k_bias_grad(ctx, m->gUp[d].p, m->grads + lu.b_off, (int64_t)B * m->vox(d), lu.cout));
-      FM_TRY(k_space_to_depth(ctx, m->gUp[d].p, m->dcG.p, dc, m->pz));
-      FM_TRY(k_conv3d_tc_wgrad(ctx, act, m->dcG.p, m->grads + lu.w_off, B, dc.X, dc.Y, dc.Z, lu.c1, lu.c1, 0, c8, 1));
-      FM_TRY(mark_layer_done(m, lu));
-      FM_TRY(k_conv3d_tc_fprop(ctx, m->dcG.p, nullptr, lu.w_d0, nullptr, gdst, act, B, dc.X, dc.Y, dc.Z, c8, 0, lu.c1, 1,
-                               0, lu.c1, 0));
+      FM_TRY(deconv_bwd(ctx, act, m->gUp[d].p, lu.w_d0, relu_mask(act), m->dcG.p, gdst, m->grads + lu.w_off,
+                        m->grads + lu.b_off, m->dims(d + 1, lu.cout, B), m->pz, m->layer_done[layer_pos(m, lu)]));
       continue;
     }
     // through UpSampling3D into the coarser tensor that was upsampled (+ its ReLU mask)
-    FM_TRY(k_upsample3d_bwd(ctx, m->gUp[d].p, act, gdst, m->dims(d + 1, da.c1, B), da.c1, 0, m->pz));
+    FM_TRY(k_upsample3d_bwd(ctx, m->gUp[d].p, relu_mask(act), gdst, m->dims(d + 1, da.c1, B), da.c1, 0, m->pz));
   }
   for (int d = D - 1; d >= 0; --d) {
     const Layer &la = L(m, "enc%da", d), &lb = L(m, "enc%db", d);
     if (d < D - 1) {
       // gradient of encB[d]: skip path + MaxPooling3D backward, masked by its ReLU
       FM_TRY(k_maxpool3d_bwd(ctx, m->encB[d].p, m->gPool[d].p, m->gSkip[d].p, m->gEncB[d].p,
-                             m->dims(d, lb.cout, B), 1, m->pz));
+                             m->dims(d, lb.cout, B), bn ? 0 : 1, m->pz));
     }
-    FM_TRY(conv_wgrad(m, lb, m->encA[d].p, nullptr, m->gEncB[d].p, B));
+    FM_TRY(unet_block_bwd(m, lb, m->gEncB[d].p, B, &dy));
+    FM_TRY(conv_wgrad(m, lb, m->encA[d].p, nullptr, dy, B));
     FM_TRY(mark_layer_done(m, lb));
-    FM_TRY(conv_dgrad(m, lb, 0, m->gEncB[d].p, m->encA[d].p, m->gEncA[d].p, B));
+    FM_TRY(conv_dgrad(m, lb, 0, dy, relu_mask(m->encA[d].p), m->gEncA[d].p, B));
     if (m->unet_dropout()) FM_TRY(k_channel_scale(ctx, m->gEncA[d].p, m->dropU[d].p, B, m->vox(d), la.cout));
+    FM_TRY(unet_block_bwd(m, la, m->gEncA[d].p, B, &dy));
     if (d > 0) {
-      FM_TRY(conv_wgrad(m, la, m->pool[d - 1].p, nullptr, m->gEncA[d].p, B));
+      FM_TRY(conv_wgrad(m, la, m->pool[d - 1].p, nullptr, dy, B));
       FM_TRY(mark_layer_done(m, la));
-      FM_TRY(conv_dgrad(m, la, 0, m->gEncA[d].p, nullptr, m->gPool[d - 1].p, B));
-    } else if (m->kcode == 31) {
-      FM_TRY(conv_wgrad(m, la, m->x_pad.p, nullptr, m->gEncA[0].p, B));
-      FM_TRY(mark_layer_done(m, la));
+      FM_TRY(conv_dgrad(m, la, 0, dy, nullptr, m->gPool[d - 1].p, B));
     } else {
-      const Dims5 dd = m->dims(0, la.cout, B);
-      FM_TRY(k_conv3d_simt_wgrad(ctx, m->x_in.p, 1, m->gEncA[0].p, m->grads + la.w_off, B, dd.X, dd.Y, dd.Z,
-                                 la.c1, la.c1, 0, la.cout, la.k));
-      FM_TRY(k_bias_grad(ctx, m->gEncA[0].p, m->grads + la.b_off, dd.voxels(), la.cout));
+      FM_TRY(conv_wgrad(m, la, m->kcode == 31 ? (const void*)m->x_pad.p : m->x_in.p, nullptr, dy, B));
       FM_TRY(mark_layer_done(m, la));
     }
   }
@@ -1346,12 +1277,6 @@ struct IsenseeBuild {
   int X, Y, Z, in_channels, depth, n_base_filters, n_segmentation_levels, kcode;
 };
 static int build_isensee(fm_ctx* ctx, const IsenseeBuild* spec, fm_model** out);
-
-// whether the data gradient towards a source of cs channels (first source c1 channels) runs on the marching kernel;
-// decided once per layer when the model is built (X, Y, Z = the extent the dgrad runs at)
-static bool isensee_dgrad_marches(int X, int Y, int Z, int c1, int cs, int cout, int k) {
-  return k == 3 && c1 >= 16 && conv_march_supported(X, Y, Z, cout, 0, cs, k);
-}
 
 extern "C" int fm_model_create_isensee3d(fm_ctx* ctx, const fm_isensee3d_spec* spec, fm_model** out) {
   FM_CHECK(ctx && spec && out, FM_EINVAL, "fm_model_create_isensee3d: NULL argument");
@@ -1398,132 +1323,30 @@ static int build_isensee(fm_ctx* ctx, const IsenseeBuild* spec, fm_model** out) 
   m->spec.n_base_filters = spec->n_base_filters;
   m->spec.n_labels = 1;
   const int D = spec->depth, nf = spec->n_base_filters;
-  auto add_conv = [&](const char* fmt, int d, int c1, int c2, int cout, int k, int level, int stride, bool norm) {
-    Layer l;
-    memset(l.name, 0, sizeof(l.name));
-    snprintf(l.name, sizeof(l.name), fmt, d);
-    l.c1 = c1;
-    l.c2 = c2;
-    l.cout = cout;
-    l.k = k;
-    l.level = level;
-    l.stride = stride;
-    l.w_off = m->nparams;
-    m->nparams += l.wcount();
-    l.b_off = m->nparams;
-    m->nparams = (m->nparams + cout + 3) & ~(int64_t)3;
-    m->layers.push_back(l);
-    if (norm) {
-      Layer g;
-      memset(g.name, 0, sizeof(g.name));
-      snprintf(g.name, sizeof(g.name), "%s_norm", l.name);
-      g.is_norm = 1;
-      g.c1 = cout;
-      g.c2 = 0;
-      g.cout = cout;
-      g.k = 1;
-      g.level = level;
-      g.w_off = m->nparams;
-      m->nparams += cout;
-      g.b_off = m->nparams;
-      m->nparams = (m->nparams + cout + 3) & ~(int64_t)3;
-      m->layers.push_back(g);
-    }
-  };
+  std::vector<Layer>& ls = m->layers;
   // 2D: the first conv reads a 16-channel zero-padded bf16 copy of the input (tensor-core K granule)
   int c = kcode == 31 ? 16 : 1;
   for (int l = 0; l < D; ++l) {
     const int f = nf << l;
-    add_conv("l%d_in", l, c, 0, f, kcode, l, l == 0 ? 1 : 2, true);
-    if (l == 0 && kcode == 31) m->layers[m->layers.size() - 2].cin_real = spec->in_channels;
-    add_conv("l%d_ctx1", l, f, 0, f, kcode, l, 1, true);
-    add_conv("l%d_ctx2", l, f, 0, f, kcode, l, 1, true);
+    add_layer(ls, "l%d_in", l, c, 0, f, kcode, l, l == 0 ? 1 : 2, 1);
+    add_layer(ls, "l%d_ctx1", l, f, 0, f, kcode, l, 1, 1);
+    add_layer(ls, "l%d_ctx2", l, f, 0, f, kcode, l, 1, 1);
     c = f;
   }
   for (int l = D - 2; l >= 0; --l) {
     const int f = nf << l;
-    add_conv("u%d_up", l, c, 0, f, kcode, l, 1, true);
-    add_conv("u%d_loc1", l, f, f, f, kcode, l, 1, true);  // concat order [skip, up] (isensee2017.py:62)
-    add_conv("u%d_loc2", l, f, 0, f, 1, l, 1, true);
+    add_layer(ls, "u%d_up", l, c, 0, f, kcode, l, 1, 1);
+    add_layer(ls, "u%d_loc1", l, f, f, f, kcode, l, 1, 1);  // concat order [skip, up] (isensee2017.py:62)
+    add_layer(ls, "u%d_loc2", l, f, 0, f, 1, l, 1, 1);
     c = f;
-    if (l < m->nseg) add_conv("u%d_seg", l, f, 0, 1, 1, l, 1, false);
+    if (l < m->nseg) add_layer(ls, "u%d_seg", l, f, 0, 1, 1, l);
   }
-  const size_t pb = (size_t)m->nparams * sizeof(float);
-  float** bufs[4] = {&m->params, &m->grads, &m->adam_m, &m->adam_v};
-  for (auto b : bufs) {
-    FM_CUDA(cudaMalloc((void**)b, pb));
-    FM_CUDA(cudaMemset(*b, 0, pb));
-  }
-  FM_CUDA(cudaMalloc((void**)&m->sums, kNumLossSums * sizeof(double)));
-  FM_CUDA(cudaMemset(m->sums, 0, kNumLossSums * sizeof(double)));
-  int64_t pack_elems = 0;
-  for (auto& l : m->layers)
-    if (!l.is_norm) pack_elems += 2 * ((l.wcount() + 63) & ~(int64_t)63);
-  FM_CUDA(cudaMalloc((void**)&m->wpack, (size_t)pack_elems * sizeof(bf16)));
-  FM_CUDA(cudaMemset(m->wpack, 0, (size_t)pack_elems * sizeof(bf16)));
-  bf16* wp = m->wpack;
-  for (auto& l : m->layers) {
-    if (l.is_norm) continue;
-    const int64_t padded = (l.wcount() + 63) & ~(int64_t)63;
-    l.w_f = wp;
-    wp += padded;
-    if (l.c1 >= 16) {  // dgrad packs (none for the Cin = 1 first conv)
-      l.w_d0 = wp;
-      l.w_d1 = wp + (int64_t)l.c1 * l.taps() * l.cout;
-    }
-    wp += padded;
-    if (l.k != 3 || l.c1 < 16) continue;  // (the 2D family, k = 31, runs on the per-tap kernels)
-    // the backward of a stride-2 conv runs as a stride-1 dgrad over the zero-inserted gradient, one level finer
-    const int dl = l.stride == 2 ? l.level - 1 : l.level;
-    const int X = spec->X >> l.level, Y = spec->Y >> l.level, Z = spec->Z >> l.level;
-    const int Xd = spec->X >> dl, Yd = spec->Y >> dl, Zd = spec->Z >> dl;
-    const int cs[2] = {l.c1, l.c2};
-    if (l.stride == 1 && conv_march_supported(X, Y, Z, l.c1, l.c2, l.cout, l.k)) {
-      l.march_f = true;
-      for (int s = 0; s < (l.c2 ? 2 : 1); ++s)
-        FM_CUDA(cudaMalloc((void**)&l.w_mf[s], (size_t)conv_march_pack_elems(cs[s], l.cout) * sizeof(bf16)));
-    }
-    for (int s = 0; s < (l.c2 ? 2 : 1); ++s)
-      if (isensee_dgrad_marches(Xd, Yd, Zd, l.c1, cs[s], l.cout, l.k)) {
-        l.march_d[s] = true;
-        FM_CUDA(cudaMalloc((void**)&l.w_md[s], (size_t)conv_march_pack_elems(l.cout, cs[s]) * sizeof(bf16)));
-      }
-  }
-  m->layer_done.resize(m->layers.size());
-  for (auto& e : m->layer_done) FM_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-  {  // gradient buckets as for the plain U-Net: backward runs in reverse creation order
-    const int nl = (int)m->layers.size();
-    const int64_t target = m->nparams / 4 + 1;
-    int hi = nl - 1;
-    int64_t acc = 0;
-    for (int i = nl - 1; i >= 0; --i) {
-      acc += m->layers[i].wcount() + m->layers[i].cout;
-      if (acc >= target || i == 0) {
-        m->buckets.push_back({i, hi});
-        hi = i - 1;
-        acc = 0;
-      }
-    }
-  }
-  m->isRawL.resize(m->layers.size());
-  m->isStatsL.resize(m->layers.size());
-  m->gIsA.resize(D);
-  m->gIsB.resize(D);
-  m->gIsC.resize(D);
-  m->gIsUp.resize(D);
-  m->isDropL.resize(D);
-  m->gSeg.resize(D);
-  m->isIn.resize(D);
-  m->isC1.resize(D);
-  m->isSum.resize(D);
-  m->isUp.resize(D);
-  m->isU.resize(D);
-  m->isLoc1.resize(D);
-  m->isLoc2.resize(D);
-  m->isSeg.resize(D);
-  FM_CUDA(cudaEventCreateWithFlags(&m->ev_tmp, cudaEventDisableTiming));
-  *out = m;
-  return FM_OK;
+  if (kcode == 31) ls[0].cin_real = spec->in_channels;
+  for (auto* v : {&m->gIsA, &m->gIsB, &m->gIsC, &m->gIsUp, &m->isIn, &m->isC1, &m->isSum, &m->isUp, &m->isU,
+                  &m->isLoc1, &m->isLoc2})
+    v->resize(D);
+  for (auto* v : {&m->isDropL, &m->gSeg, &m->isSeg}) v->resize(D);
+  return build_model(m, nullptr, out);
 }
 
 static int ensure_capacity_isensee(fm_model* m, int B, bool train) {
@@ -1535,13 +1358,13 @@ static int ensure_capacity_isensee(fm_model* m, int B, bool train) {
   if (train || m->train_alloc) {
     FM_TRY(m->t_in.ensure((size_t)B * v0));
     FM_TRY(m->dz.ensure((size_t)B * v0));
-    FM_TRY(m->gIsRaw.ensure((size_t)B * v0 * nf));
+    FM_TRY(m->normGRaw.ensure((size_t)B * v0 * nf));
     FM_TRY(m->gIsZero.ensure((size_t)B * v0 * nf * 2));
     for (size_t i = 0; i < m->layers.size(); ++i) {
       const Layer& l = m->layers[i];
       if (l.is_norm || (l.k == 1 && l.cout == 1)) continue;
-      FM_TRY(m->isRawL[i].ensure((size_t)B * m->vox(l.level) * l.cout));
-      FM_TRY(m->isStatsL[i].ensure((size_t)B * l.cout * 2));
+      FM_TRY(m->normRawL[i].ensure((size_t)B * m->vox(l.level) * l.cout));
+      FM_TRY(m->normStatsL[i].ensure((size_t)B * l.cout * 2));
     }
     for (int l = 0; l < D; ++l) {
       const size_t n = (size_t)B * m->vox(l) * (nf << l);
@@ -1558,8 +1381,8 @@ static int ensure_capacity_isensee(fm_model* m, int B, bool train) {
   if (m->kcode == 31) FM_TRY(m->x_pad.ensure((size_t)B * v0 * 16));
   FM_TRY(m->prob.ensure((size_t)B * v0));
   FM_TRY(m->isAcc.ensure((size_t)B * v0));
-  FM_TRY(m->isRaw.ensure((size_t)B * v0 * nf));
-  FM_TRY(m->isScratch.ensure((size_t)B * (nf << (D - 1)) * 2 * 1028));
+  FM_TRY(m->normRaw.ensure((size_t)B * v0 * nf));
+  FM_TRY(m->normScratch.ensure((size_t)B * (nf << (D - 1)) * 2 * 1028));
   for (int l = 0; l < D; ++l) {
     const size_t n = (size_t)B * m->vox(l) * (nf << l);
     FM_TRY(m->isIn[l].ensure(n));
@@ -1579,54 +1402,29 @@ static int ensure_capacity_isensee(fm_model* m, int B, bool train) {
 
 // one Isensee conv block: Conv3D (+bias) -> raw -> InstanceNorm + LeakyReLU (* dropout scale) (+ residual add) -> y.
 // A training pass keeps the raw conv output and the norm statistics of every block for the backward pass.
-static int isensee_block(fm_model* m, const Layer& l, const Layer& nl, const bf16* x1, const bf16* x2, const bf16* add,
-                         bf16* y, int B, const float* chan_scale = nullptr) {
-  fm_ctx* ctx = m->ctx;
-  const Dims5 d = m->dims(l.level, l.cout, B);
-  const float* bias = m->params + l.b_off;
-  const int li = (int)(&l - &m->layers[0]);
-  bf16* raw = m->train_pass ? m->isRawL[li].p : m->isRaw.p;
-  float* stats = m->train_pass ? m->isStatsL[li].p : nullptr;
-  if (l.c1 == 1) {
-    // Cin = 1: bandwidth kernel, raw output (no activation)
-    FM_TRY(k_conv3d_simt_fprop(ctx, x1, 1, nullptr, l.w_f, bias, raw, nullptr, B, d.X, d.Y, d.Z, 1, 0, l.cout, 3, 0,
-                               nullptr));
-  } else if (l.march_f) {
-    FM_TRY(k_conv3d_march(ctx, x1, x2, l.w_mf[0], l.w_mf[1], bias, raw, nullptr, B, d.X, d.Y, d.Z, l.c1, l.c2, l.cout, 0,
-                          l.cout, 0, reproducible_pass(m)));
-  } else if (conv_tc_supported(l.c1, l.c2, l.cout, l.k)) {
-    FM_TRY(k_conv3d_tc_fprop(ctx, x1, x2, l.w_f, bias, raw, nullptr, B, d.X, d.Y, d.Z, l.c1, l.c2, l.cout, l.k, 0,
-                             l.cout, 0, l.stride, d.X * l.stride, d.Y * l.stride, m->pz == 2 ? d.Z * l.stride : d.Z));
-  } else {
-    FM_CHECK(l.stride == 1, FM_EINVAL, "isensee: strided conv %s has no fallback", l.name);
-    FM_TRY(k_conv3d_simt_fprop(ctx, x1, 0, x2, l.w_f, bias, raw, nullptr, B, d.X, d.Y, d.Z, l.c1, l.c2, l.cout, l.k, 0,
-                               nullptr));
-  }
-  return k_instnorm_lrelu(ctx, raw, m->params + nl.w_off, m->params + nl.b_off, add, y, B, m->vox(l.level), l.cout,
-                          m->isScratch.p, m->isScratch.n, stats, chan_scale);
+static int isensee_block(fm_model* m, const Layer& l, const void* x1, const bf16* x2, const bf16* add, bf16* y, int B,
+                         const float* chan_scale = nullptr) {
+  const int li = layer_pos(m, l);
+  const Layer& nl = m->layers[li + 1];
+  bf16* raw = m->train_pass ? m->normRawL[li].p : m->normRaw.p;
+  FM_TRY(conv_fwd(m, l, x1, x2, raw, B, 0));
+  return k_instnorm_lrelu(m->ctx, raw, m->params + nl.w_off, m->params + nl.b_off, add, y, B, m->vox(l.level), l.cout,
+                          m->normScratch.p, m->normScratch.n, m->train_pass ? m->normStatsL[li].p : nullptr,
+                          chan_scale);
 }
 
 static int forward_isensee(fm_model* m, int B) {
   fm_ctx* ctx = m->ctx;
   const int D = m->depth();
   FM_TRY(refresh_packs(m));
-  auto LI = [&](const char* fmt, int d) {
-    char nm[32];
-    snprintf(nm, sizeof(nm), fmt, d);
-    return layer_index(m, nm);
-  };
-  const bf16* cur = nullptr;
+  const void* cur = m->x_in.p;  // the 3D model's first conv reads the fp32 single-channel input
+  if (m->kcode == 31) {
+    FM_TRY(k_pad_cast(ctx, m->x_in.p, m->x_pad.p, (int64_t)B * m->vox(0), m->cin_real, 16));
+    cur = m->x_pad.p;
+  }
   for (int l = 0; l < D; ++l) {
-    const int i_in = LI("l%d_in", l), i_c1 = LI("l%d_ctx1", l), i_c2 = LI("l%d_ctx2", l);
-    const Layer &lin = m->layers[i_in], &lc1 = m->layers[i_c1], &lc2 = m->layers[i_c2];
-    const bf16* src = cur;
-    if (l == 0 && m->kcode == 31) {
-      FM_TRY(k_pad_cast(ctx, m->x_in.p, m->x_pad.p, (int64_t)B * m->vox(0), m->cin_real, 16));
-      src = m->x_pad.p;
-    } else if (l == 0) {
-      src = (const bf16*)m->x_in.p;  // fp32 single-channel input, read by the Cin = 1 kernel
-    }
-    FM_TRY(isensee_block(m, lin, m->layers[i_in + 1], src, nullptr, nullptr, m->isIn[l].p, B));
+    const Layer &lin = L(m, "l%d_in", l), &lc1 = L(m, "l%d_ctx1", l), &lc2 = L(m, "l%d_ctx2", l);
+    FM_TRY(isensee_block(m, lin, cur, nullptr, nullptr, m->isIn[l].p, B));
     // SpatialDropout3D between the two context convs (isensee2017.py:103-105): training passes only
     const float* drop = nullptr;
     if (m->train_pass && m->dropout_rate > 0.f) {
@@ -1634,23 +1432,22 @@ static int forward_isensee(fm_model* m, int B) {
                              m->dropout_seed + (uint64_t)m->iterations * 64 + (uint64_t)l));
       drop = m->isDropL[l].p;
     }
-    FM_TRY(isensee_block(m, lc1, m->layers[i_c1 + 1], m->isIn[l].p, nullptr, nullptr, m->isC1[l].p, B, drop));
+    FM_TRY(isensee_block(m, lc1, m->isIn[l].p, nullptr, nullptr, m->isC1[l].p, B, drop));
     // context output + residual: summation = in_conv + context (isensee2017.py:55)
-    FM_TRY(isensee_block(m, lc2, m->layers[i_c2 + 1], m->isC1[l].p, nullptr, m->isIn[l].p, m->isSum[l].p, B));
+    FM_TRY(isensee_block(m, lc2, m->isC1[l].p, nullptr, m->isIn[l].p, m->isSum[l].p, B));
     cur = m->isSum[l].p;
   }
   for (int l = D - 2; l >= 0; --l) {
-    const int i_up = LI("u%d_up", l), i_l1 = LI("u%d_loc1", l), i_l2 = LI("u%d_loc2", l);
-    const Layer& lup = m->layers[i_up];
-    FM_TRY(k_upsample3d_fwd(ctx, cur, m->isUp[l].p, m->dims(l + 1, lup.c1, B), m->pz));
-    FM_TRY(isensee_block(m, lup, m->layers[i_up + 1], m->isUp[l].p, nullptr, nullptr, m->isU[l].p, B));
-    FM_TRY(isensee_block(m, m->layers[i_l1], m->layers[i_l1 + 1], m->isSum[l].p, m->isU[l].p, nullptr, m->isLoc1[l].p, B));
-    FM_TRY(isensee_block(m, m->layers[i_l2], m->layers[i_l2 + 1], m->isLoc1[l].p, nullptr, nullptr, m->isLoc2[l].p, B));
+    const Layer& lup = L(m, "u%d_up", l);
+    FM_TRY(k_upsample3d_fwd(ctx, (const bf16*)cur, m->isUp[l].p, m->dims(l + 1, lup.c1, B), m->pz));
+    FM_TRY(isensee_block(m, lup, m->isUp[l].p, nullptr, nullptr, m->isU[l].p, B));
+    FM_TRY(isensee_block(m, L(m, "u%d_loc1", l), m->isSum[l].p, m->isU[l].p, nullptr, m->isLoc1[l].p, B));
+    FM_TRY(isensee_block(m, L(m, "u%d_loc2", l), m->isLoc1[l].p, nullptr, nullptr, m->isLoc2[l].p, B));
     cur = m->isLoc2[l].p;
     if (l < m->nseg) {
-      const Layer& ls = m->layers[LI("u%d_seg", l)];
-      FM_TRY(k_head_fwd(ctx, cur, m->params + ls.w_off, m->params + ls.b_off, m->isSeg[l].p, (int64_t)B * m->vox(l),
-                        ls.c1, 0));
+      const Layer& ls = L(m, "u%d_seg", l);
+      FM_TRY(k_head_fwd(ctx, m->isLoc2[l].p, m->params + ls.w_off, m->params + ls.b_off, m->isSeg[l].p,
+                        (int64_t)B * m->vox(l), ls.c1, 0));
     }
   }
   // deep-supervision sum, coarse to fine (isensee2017.py:68-77), then sigmoid (:79)
@@ -1668,78 +1465,27 @@ static int forward_isensee(fm_model* m, int B) {
 
 // ---------------------------------------------------------------------------------------------
 // Isensee backward. Per block: (InstanceNorm + LeakyReLU [+ dropout]) backward -> gradient of the raw conv output
-// (gIsRaw), bias / weight gradients, dgrad to the block input(s). Fan-outs: in_conv feeds ctx1 and the residual
+// (normGRaw), weight gradients, dgrad to the block input(s). Fan-outs: in_conv feeds ctx1 and the residual
 // add; summation[l] feeds the next level's stride-2 in_conv and the decoder's concat (or the first upsampling at
 // the bottom); loc2[l] feeds its segmentation head and the next upsampling. The stride-2 convs go backward as
 // stride-1 dgrad / wgrad over the zero-inserted gradient (k_zero_insert), one level finer.
 // Gradients are produced in reverse layer-creation order, so the all-reduce buckets work as for the plain U-Net.
 // ---------------------------------------------------------------------------------------------
-// Kernel choice of the Isensee weight / data gradients, shared with the per-op hook fm_op_conv_strided so that the
-// hook runs what the model runs. Weight gradient of one source (cs of cin_total channels at cofs): marching, per-tap
-// tensor-core or SIMT kernel.
-static int isensee_wgrad_route(fm_ctx* ctx, const bf16* x, const bf16* dy, float* dw, int B, int X, int Y, int Z, int cs,
-                               int cin_total, int cofs, int cout, int k) {
-  if (conv_wgrad_march_supported(X, Y, Z, cs, cout, k))
-    return k_conv3d_wgrad_march(ctx, x, dy, dw, B, X, Y, Z, cs, cin_total, cofs, cout);
-  if (conv_tc_supported(cs, 0, cout, k))
-    return k_conv3d_tc_wgrad(ctx, x, dy, dw, B, X, Y, Z, cs, cin_total, cofs, cout, k);
-  return k_conv3d_simt_wgrad(ctx, x, 0, dy, dw, B, X, Y, Z, cs, cin_total, cofs, cout, k);
-}
-
-// data gradient towards one source: w_md = its marching pack (null: per-tap tensor-core or SIMT kernel on w_d)
-static int isensee_dgrad_route(fm_ctx* ctx, const bf16* dy, const bf16* w_md, const bf16* w_d, bf16* dx, int B, int X,
-                               int Y, int Z, int cout, int cs, int k, bool reproducible) {
-  if (w_md != nullptr)
-    return k_conv3d_march(ctx, dy, nullptr, w_md, nullptr, nullptr, dx, nullptr, B, X, Y, Z, cout, 0, cs, 0, cs, 0,
-                          reproducible);
-  if (conv_tc_supported(cout, 0, cs, k))
-    return k_conv3d_tc_fprop(ctx, dy, nullptr, w_d, nullptr, dx, nullptr, B, X, Y, Z, cout, 0, cs, k, 0, cs, 0);
-  return k_conv3d_simt_fprop(ctx, dy, 0, nullptr, w_d, nullptr, dx, nullptr, B, X, Y, Z, cout, 0, cs, k, 0, nullptr);
-}
-
-static int is_wgrad(fm_model* m, const Layer& l, int level, const bf16* x1, const bf16* x2, const bf16* dy, int B) {
-  const Dims5 d = m->dims(level, l.cout, B);
-  const bf16* xs[2] = {x1, x2};
-  const int cs[2] = {l.c1, l.c2};
-  int cofs = 0;
-  // no bias gradient here: every Isensee conv feeds an InstanceNormalization, which removes a per-channel constant -
-  // the gradient of such a bias is exactly zero (the heads, which have a live bias, are 1x1x1 kernels handled elsewhere)
-  for (int s = 0; s < (l.c2 ? 2 : 1); ++s) {
-    FM_TRY(isensee_wgrad_route(m->ctx, xs[s], dy, m->grads + l.w_off, B, d.X, d.Y, d.Z, cs[s], l.cin(), cofs, l.cout,
-                               l.k));
-    cofs += cs[s];
-  }
-  return FM_OK;
-}
-
-static int is_dgrad(fm_model* m, const Layer& l, int level, int src, const bf16* dy, bf16* dx, int B) {
-  const Dims5 d = m->dims(level, l.cout, B);
-  return isensee_dgrad_route(m->ctx, dy, l.march_d[src] ? l.w_md[src] : nullptr, src == 0 ? l.w_d0 : l.w_d1, dx, B, d.X,
-                             d.Y, d.Z, l.cout, src == 0 ? l.c1 : l.c2, l.k, reproducible_pass(m));
-}
-
-// norm + activation backward of block `li` -> m->gIsRaw (gradient of the raw conv output); gamma/beta/bias gradients
-static int is_block_bwd(fm_model* m, int li, const bf16* gy, const bf16* gy2, const float* chan_scale, int B) {
-  const Layer &l = m->layers[li], &nl = m->layers[li + 1];
-  FM_TRY(k_instnorm_lrelu_bwd(m->ctx, m->isRawL[li].p, m->isStatsL[li].p, m->params + nl.w_off, m->params + nl.b_off, gy,
-                              gy2, chan_scale, m->gIsRaw.p, m->grads + nl.w_off, m->grads + nl.b_off, B, m->vox(l.level),
-                              l.cout, m->isScratch.p, m->isScratch.n));
-  FM_TRY(mark_layer_done(m, nl));
-  // no bias-gradient pass: the conv bias sits in front of an InstanceNormalization, which removes any per-channel
-  // constant - its gradient is exactly zero (the buffer was zeroed at the start of the backward pass); summing gIsRaw
-  // over the voxels would only return the rounding noise of a sum that vanishes analytically
-  return FM_OK;
+// norm + activation backward of block `l` -> m->normGRaw (gradient of the raw conv output); gamma / beta gradients
+static int is_block_bwd(fm_model* m, const Layer& l, const bf16* gy, const bf16* gy2, const float* chan_scale, int B) {
+  const int li = layer_pos(m, l);
+  const Layer& nl = m->layers[li + 1];
+  FM_TRY(k_instnorm_lrelu_bwd(m->ctx, m->normRawL[li].p, m->normStatsL[li].p, m->params + nl.w_off,
+                              m->params + nl.b_off, gy, gy2, chan_scale, m->normGRaw.p, m->grads + nl.w_off,
+                              m->grads + nl.b_off, B, m->vox(l.level), l.cout, m->normScratch.p, m->normScratch.n));
+  return mark_layer_done(m, nl);
 }
 
 static int backward_isensee(fm_model* m, int B) {
   fm_ctx* ctx = m->ctx;
   const int D = m->depth();
   const int64_t n0 = (int64_t)B * m->vox(0);
-  auto LI = [&](const char* fmt, int d) {
-    char nm[32];
-    snprintf(nm, sizeof(nm), fmt, d);
-    return layer_index(m, nm);
-  };
+  const bf16* g = m->normGRaw.p;
   FM_TRY(k_zero(ctx, m->grads, (size_t)m->nparams * sizeof(float)));
   // d(loss)/d(summed logits); the deep-supervision sum hands the same gradient, 2^3 sum-pooled, to every head
   FM_TRY(k_dice_bwd(ctx, m->prob.p, m->t_in.p, m->sums, n0, m->dz.p, 1, m->xent()));
@@ -1751,59 +1497,53 @@ static int backward_isensee(fm_model* m, int B) {
     gseg[l] = m->gSeg[l].p;
   }
   for (int l = 0; l <= D - 2; ++l) {
-    const int i_up = LI("u%d_up", l), i_l1 = LI("u%d_loc1", l), i_l2 = LI("u%d_loc2", l);
-    const Layer &lup = m->layers[i_up], &ll1 = m->layers[i_l1], &ll2 = m->layers[i_l2];
+    const Layer &lup = L(m, "u%d_up", l), &ll1 = L(m, "u%d_loc1", l), &ll2 = L(m, "u%d_loc2", l);
     // gradient of loc2[l] (gIsA[l]): upsampling path (already stored for l > 0) + segmentation head
     if (l < m->nseg) {
-      const Layer& ls = m->layers[LI("u%d_seg", l)];
+      const Layer& ls = L(m, "u%d_seg", l);
       FM_TRY(k_head_bwd(ctx, m->isLoc2[l].p, gseg[l], m->params + ls.w_off, m->gIsA[l].p, m->grads + ls.w_off,
                         m->grads + ls.b_off, (int64_t)B * m->vox(l), ls.c1, l > 0 ? 2 : 1));
       FM_TRY(mark_layer_done(m, ls));
     }
-    FM_TRY(is_block_bwd(m, i_l2, m->gIsA[l].p, nullptr, nullptr, B));
-    FM_TRY(is_wgrad(m, ll2, l, m->isLoc1[l].p, nullptr, m->gIsRaw.p, B));
+    FM_TRY(is_block_bwd(m, ll2, m->gIsA[l].p, nullptr, nullptr, B));
+    FM_TRY(conv_wgrad(m, ll2, m->isLoc1[l].p, nullptr, g, B));
     FM_TRY(mark_layer_done(m, ll2));
-    FM_TRY(is_dgrad(m, ll2, l, 0, m->gIsRaw.p, m->gIsB[l].p, B));
-    FM_TRY(is_block_bwd(m, i_l1, m->gIsB[l].p, nullptr, nullptr, B));
-    FM_TRY(is_wgrad(m, ll1, l, m->isSum[l].p, m->isU[l].p, m->gIsRaw.p, B));
+    FM_TRY(conv_dgrad(m, ll2, 0, g, nullptr, m->gIsB[l].p, B));
+    FM_TRY(is_block_bwd(m, ll1, m->gIsB[l].p, nullptr, nullptr, B));
+    FM_TRY(conv_wgrad(m, ll1, m->isSum[l].p, m->isU[l].p, g, B));
     FM_TRY(mark_layer_done(m, ll1));
-    FM_TRY(is_dgrad(m, ll1, l, 0, m->gIsRaw.p, m->gIsC[l].p, B));  // skip part of d(summation[l])
-    FM_TRY(is_dgrad(m, ll1, l, 1, m->gIsRaw.p, m->gIsA[l].p, B));  // d(up block output)
-    FM_TRY(is_block_bwd(m, i_up, m->gIsA[l].p, nullptr, nullptr, B));
-    FM_TRY(is_wgrad(m, lup, l, m->isUp[l].p, nullptr, m->gIsRaw.p, B));
+    FM_TRY(conv_dgrad(m, ll1, 0, g, nullptr, m->gIsC[l].p, B));  // skip part of d(summation[l])
+    FM_TRY(conv_dgrad(m, ll1, 1, g, nullptr, m->gIsA[l].p, B));  // d(up block output)
+    FM_TRY(is_block_bwd(m, lup, m->gIsA[l].p, nullptr, nullptr, B));
+    FM_TRY(conv_wgrad(m, lup, m->isUp[l].p, nullptr, g, B));
     FM_TRY(mark_layer_done(m, lup));
-    FM_TRY(is_dgrad(m, lup, l, 0, m->gIsRaw.p, m->gIsUp[l].p, B));
+    FM_TRY(conv_dgrad(m, lup, 0, g, nullptr, m->gIsUp[l].p, B));
     bf16* gdst = (l + 1 == D - 1) ? m->gIsC[D - 1].p : m->gIsA[l + 1].p;
     FM_TRY(k_upsample3d_bwd(ctx, m->gIsUp[l].p, nullptr, gdst, m->dims(l + 1, lup.c1, B), lup.c1, 0, m->pz));
   }
   for (int l = D - 1; l >= 0; --l) {
-    const int i_in = LI("l%d_in", l), i_c1 = LI("l%d_ctx1", l), i_c2 = LI("l%d_ctx2", l);
-    const Layer &lin = m->layers[i_in], &lc1 = m->layers[i_c1], &lc2 = m->layers[i_c2];
+    const Layer &lin = L(m, "l%d_in", l), &lc1 = L(m, "l%d_ctx1", l), &lc2 = L(m, "l%d_ctx2", l);
     const bf16* gsum = m->gIsC[l].p;  // complete d(summation[l])
-    FM_TRY(is_block_bwd(m, i_c2, gsum, nullptr, nullptr, B));
-    FM_TRY(is_wgrad(m, lc2, l, m->isC1[l].p, nullptr, m->gIsRaw.p, B));
+    FM_TRY(is_block_bwd(m, lc2, gsum, nullptr, nullptr, B));
+    FM_TRY(conv_wgrad(m, lc2, m->isC1[l].p, nullptr, g, B));
     FM_TRY(mark_layer_done(m, lc2));
-    FM_TRY(is_dgrad(m, lc2, l, 0, m->gIsRaw.p, m->gIsA[l].p, B));
+    FM_TRY(conv_dgrad(m, lc2, 0, g, nullptr, m->gIsA[l].p, B));
     const float* drop = m->dropout_rate > 0.f ? m->isDropL[l].p : nullptr;
-    FM_TRY(is_block_bwd(m, i_c1, m->gIsA[l].p, nullptr, drop, B));
-    FM_TRY(is_wgrad(m, lc1, l, m->isIn[l].p, nullptr, m->gIsRaw.p, B));
+    FM_TRY(is_block_bwd(m, lc1, m->gIsA[l].p, nullptr, drop, B));
+    FM_TRY(conv_wgrad(m, lc1, m->isIn[l].p, nullptr, g, B));
     FM_TRY(mark_layer_done(m, lc1));
-    FM_TRY(is_dgrad(m, lc1, l, 0, m->gIsRaw.p, m->gIsB[l].p, B));
+    FM_TRY(conv_dgrad(m, lc1, 0, g, nullptr, m->gIsB[l].p, B));
     // in_conv output feeds ctx1 and the residual add
-    FM_TRY(is_block_bwd(m, i_in, m->gIsB[l].p, gsum, nullptr, B));
-    if (l == 0 && m->kcode == 31) {
-      FM_TRY(is_wgrad(m, lin, 0, m->x_pad.p, nullptr, m->gIsRaw.p, B));  // the zero-padded 16-channel input copy
-      FM_TRY(mark_layer_done(m, lin));
-    } else if (l == 0) {
-      const Dims5 dd = m->dims(0, lin.cout, B);
-      FM_TRY(k_conv3d_simt_wgrad(ctx, m->x_in.p, 1, m->gIsRaw.p, m->grads + lin.w_off, B, dd.X, dd.Y, dd.Z, 1, 1, 0,
-                                 lin.cout, 3));
+    FM_TRY(is_block_bwd(m, lin, m->gIsB[l].p, gsum, nullptr, B));
+    if (l == 0) {
+      // the fp32 single-channel input (3D) or its zero-padded 16-channel copy (2D)
+      FM_TRY(conv_wgrad(m, lin, m->kcode == 31 ? (const void*)m->x_pad.p : m->x_in.p, nullptr, g, B));
       FM_TRY(mark_layer_done(m, lin));
     } else {
-      FM_TRY(k_zero_insert(ctx, m->gIsRaw.p, m->gIsZero.p, m->dims(l, lin.cout, B), m->pz));
-      FM_TRY(is_wgrad(m, lin, l - 1, m->isSum[l - 1].p, nullptr, m->gIsZero.p, B));
+      FM_TRY(k_zero_insert(ctx, g, m->gIsZero.p, m->dims(l, lin.cout, B), m->pz));
+      FM_TRY(conv_wgrad(m, lin, m->isSum[l - 1].p, nullptr, m->gIsZero.p, B));
       FM_TRY(mark_layer_done(m, lin));
-      FM_TRY(is_dgrad(m, lin, l - 1, 0, m->gIsZero.p, m->gIsA[l - 1].p, B));
+      FM_TRY(conv_dgrad(m, lin, 0, m->gIsZero.p, nullptr, m->gIsA[l - 1].p, B));
       FM_TRY(k_add_bf16(ctx, m->gIsC[l - 1].p, m->gIsA[l - 1].p, m->gIsC[l - 1].p,
                         (int64_t)B * m->vox(l - 1) * lin.c1));
     }
@@ -3303,7 +3043,7 @@ extern "C" int fm_op_instnorm_lrelu_bwd(fm_ctx* ctx, const float* x, const float
   return s.down_bf16(bdx, n, dx);
 }
 
-// BatchNormalization + ReLU (bn_block_fwd): training = batch statistics, and moving_mean / moving_var [C] (in/out)
+// BatchNormalization + ReLU (unet_block_fwd): training = batch statistics, and moving_mean / moving_var [C] (in/out)
 // take the Keras moving-average step; inference = the moving statistics.
 extern "C" int fm_op_batchnorm_relu(fm_ctx* ctx, int training, const float* x, const float* gamma, const float* beta,
                                     float* moving_mean, float* moving_var, int N, int64_t vox, int C, float* y) {
@@ -3369,6 +3109,8 @@ extern "C" int fm_op_conv_strided(fm_ctx* ctx, const float* x, const float* w_ke
   FM_CHECK(ctx && x && w_keras && (ksize == 3 || ksize == 31), FM_EINVAL, "fm_op_conv_strided: bad argument");
   FM_CHECK(Xin % 2 == 0 && Yin % 2 == 0 && (ksize == 31 || Zin % 2 == 0), FM_EINVAL, "fm_op_conv_strided: odd extent");
   FM_CHECK(!dy || (dx && dw_keras), FM_EINVAL, "fm_op_conv_strided: dy needs dx and dw_keras");
+  FM_CHECK(conv_tc_supported(Cin, 0, Cout, ksize), FM_EINVAL, "fm_op_conv_strided: no strided kernel for %d -> %d", Cin,
+           Cout);
   FM_CUDA(cudaSetDevice(ctx->device));
   OpScratch s(ctx);
   const int pz = ksize == 31 ? 1 : 2, X = Xin / 2, Y = Yin / 2, Z = Zin / pz, taps = kext_taps(ksize);
@@ -3382,19 +3124,26 @@ extern "C" int fm_op_conv_strided(fm_ctx* ctx, const float* x, const float* w_ke
   FM_TRY(s.alloc(&wf, wn));
   FM_TRY(s.alloc(&wd, wn));
   FM_TRY(k_repack_weights(ctx, wm, wf, wd, nullptr, Cout, taps, Cin, 0));
+  // the in-conv as a model holds it, with this call's packs
+  Layer l{};
+  snprintf(l.name, sizeof(l.name), "fm_op_conv_strided");
+  l.c1 = Cin;
+  l.cout = Cout;
+  l.k = ksize;
+  l.stride = 2;
+  l.w_f = wf;
+  l.w_d0 = wd;
   if (y) {
-    FM_CHECK(conv_tc_supported(Cin, 0, Cout, ksize), FM_EINVAL, "fm_op_conv_strided: no strided kernel for %d -> %d",
-             Cin, Cout);
     bf16* by = nullptr;
     float* db = nullptr;
     if (bias) FM_TRY(s.up_f32(bias, Cout, &db));
     FM_TRY(s.alloc(&by, vout * Cout));
-    FM_TRY(k_conv3d_tc_fprop(ctx, bx, nullptr, wf, db, by, nullptr, N, X, Y, Z, Cin, 0, Cout, ksize, 0, Cout, 0, 2, Xin,
-                             Yin, Zin));
+    FM_TRY(conv_fwd(ctx, l, Dims5{N, X, Y, Z, Cout}, bx, nullptr, db, by, 0, false));
     FM_TRY(s.down_bf16(by, vout * Cout, y));
   }
   if (dy) {
-    bf16 *bdy = nullptr, *bz = nullptr, *bdx = nullptr, *wmd = nullptr;
+    const Dims5 fine{N, Xin, Yin, Zin, Cout};
+    bf16 *bdy = nullptr, *bz = nullptr, *bdx = nullptr;
     float* dw = nullptr;
     FM_TRY(s.up_bf16(dy, vout * Cout, &bdy));
     FM_TRY(s.alloc(&bz, vin * Cout));
@@ -3402,12 +3151,13 @@ extern "C" int fm_op_conv_strided(fm_ctx* ctx, const float* x, const float* w_ke
     FM_TRY(s.alloc(&dw, wn));
     FM_TRY(k_zero(ctx, dw, wn * 4));
     FM_TRY(k_zero_insert(ctx, bdy, bz, Dims5{N, X, Y, Z, Cout}, pz));
-    FM_TRY(isensee_wgrad_route(ctx, bx, bz, dw, N, Xin, Yin, Zin, Cin, Cin, 0, Cout, ksize));
-    if (isensee_dgrad_marches(Xin, Yin, Zin, Cin, Cin, Cout, ksize)) {
-      FM_TRY(s.alloc(&wmd, (size_t)conv_march_pack_elems(Cout, Cin)));
-      FM_TRY(k_repack_march(ctx, wd, wmd, Cin, Cout, 0, Cout, conv_march_kc(Cout, 0, Cin, Cout)));
+    FM_TRY(conv_wgrad(ctx, l, fine, bx, nullptr, bz, dw, nullptr));
+    if (march_dgrad_ok(l, 0, Xin, Yin, Zin)) {
+      FM_TRY(s.alloc(&l.w_md[0], (size_t)conv_march_pack_elems(Cout, Cin)));
+      FM_TRY(k_repack_march(ctx, wd, l.w_md[0], Cin, Cout, 0, Cout, conv_march_kc(Cout, 0, Cin, Cout)));
+      l.march_d[0] = true;
     }
-    FM_TRY(isensee_dgrad_route(ctx, bz, wmd, wd, bdx, N, Xin, Yin, Zin, Cout, Cin, ksize, false));
+    FM_TRY(conv_dgrad(ctx, l, fine, 0, bz, nullptr, bdx, false));
     FM_TRY(s.down_bf16(bdx, vin * Cin, dx));
     std::vector<float> host(wn);
     FM_CUDA(cudaMemcpyAsync(host.data(), dw, wn * 4, cudaMemcpyDeviceToHost, ctx->stream));
@@ -3417,11 +3167,11 @@ extern "C" int fm_op_conv_strided(fm_ctx* ctx, const float* x, const float* w_ke
   return FM_OK;
 }
 
-// Deconvolution3D / Deconvolution2D (kernel 2, stride 2, C -> C channels) as the U-Nets run it: the 1x1x1 conv of the
-// coarse x [N,X,Y,Z,C] to 4*pz*C channels, then depth-to-space with the bias -> y [N,2X,2Y,pz*Z,C]. w_keras is the
-// Keras kernel (2,2[,2],C,C) = (..., Cout, Cin). With dy [N,2X,2Y,pz*Z,C]: the backward of backward_unet /
-// backward_unet_bn - bias gradient, space-to-depth, the 1x1x1 weight gradient and the data gradient dx (masked by
-// x > 0 when relu_mask, as behind a ReLU block of the plain U-Net).
+// Deconvolution3D / Deconvolution2D (kernel 2, stride 2, C -> C channels) as the U-Nets run it: deconv_fwd, the 1x1x1 conv of
+// the coarse x [N,X,Y,Z,C] to 4*pz*C channels, then depth-to-space with the bias -> y [N,2X,2Y,pz*Z,C]. w_keras is the
+// Keras kernel (2,2[,2],C,C) = (..., Cout, Cin). With dy [N,2X,2Y,pz*Z,C]: its backward as the U-Nets run it
+// (deconv_bwd) - bias gradient, space-to-depth, the 1x1x1 weight gradient and the data gradient dx (masked by x > 0
+// when relu_mask, as behind a ReLU block of the plain U-Net).
 extern "C" int fm_op_deconv(fm_ctx* ctx, const float* x, const float* w_keras, const float* bias, int N, int X, int Y,
                             int Z, int C, int pz, float* y, const float* dy, int relu_mask, float* dx, float* dw_keras,
                             float* dbias) {
@@ -3446,8 +3196,7 @@ extern "C" int fm_op_deconv(fm_ctx* ctx, const float* x, const float* w_keras, c
     float* db = nullptr;
     FM_TRY(s.up_f32(bias, C, &db));
     FM_TRY(s.alloc(&by, nf));
-    FM_TRY(k_conv3d_tc_fprop(ctx, bx, nullptr, wf, nullptr, bz, nullptr, N, X, Y, Z, C, 0, c8, 1, 0, c8, 0));
-    FM_TRY(k_depth_to_space(ctx, bz, db, by, dc, pz));
+    FM_TRY(deconv_fwd(ctx, bx, wf, db, bz, by, dc, pz));
     FM_TRY(s.down_bf16(by, nf, y));
   }
   if (dy) {
@@ -3459,11 +3208,7 @@ extern "C" int fm_op_deconv(fm_ctx* ctx, const float* x, const float* w_keras, c
     FM_TRY(s.alloc(&db, C));
     FM_TRY(k_zero(ctx, dw, wn * 4));
     FM_TRY(k_zero(ctx, db, (size_t)C * 4));
-    FM_TRY(k_bias_grad(ctx, bdy, db, (int64_t)nf / C, C));
-    FM_TRY(k_space_to_depth(ctx, bdy, bz, dc, pz));
-    FM_TRY(k_conv3d_tc_wgrad(ctx, bx, bz, dw, N, X, Y, Z, C, C, 0, c8, 1));
-    FM_TRY(k_conv3d_tc_fprop(ctx, bz, nullptr, wd, nullptr, bdx, relu_mask ? bx : nullptr, N, X, Y, Z, c8, 0, C, 1, 0, C,
-                             0));
+    FM_TRY(deconv_bwd(ctx, bx, bdy, wd, relu_mask ? bx : nullptr, bz, bdx, dw, db, dc, pz, nullptr));
     FM_CUDA(cudaMemcpyAsync(dw_keras, dw, wn * 4, cudaMemcpyDeviceToHost, ctx->stream));
     FM_CUDA(cudaMemcpyAsync(dbias, db, (size_t)C * 4, cudaMemcpyDeviceToHost, ctx->stream));
     FM_TRY(s.down_bf16(bdx, vc * C, dx));
