@@ -256,11 +256,13 @@ struct fm_model {
   DevBuf<bf16> gIsZero;
   // conv blocks with a normalisation (every Isensee block; every U-Net block under batch_normalization=True): raw conv
   // outputs and the norm statistics per conv layer (training, indexed like `layers`), one raw scratch (inference), the
-  // gradient of a raw output, the norm kernels' scratch
+  // gradient of a raw output, the norm kernels' scratch; under batch normalisation the per-channel sums of one layer
+  // (2 C + 1 doubles) that a data-parallel pass all-reduces
   std::vector<DevBuf<bf16>> normRawL;
   std::vector<DevBuf<float>> normStatsL;
   DevBuf<bf16> normRaw, normGRaw;
   DevBuf<float> normScratch;
+  DevBuf<double> normSums;
   float dropout_rate = 0.f;
   uint64_t dropout_seed = 0x5EEDull;
   // 2D U-Net: SpatialDropout2D keep/scale factors [B][C] after enc<d>a (slot d) and dec<d>a (slot depth + d)
@@ -330,6 +332,11 @@ struct fm_model {
   // training passes use the shared-accumulator marching kernel (faster; fp32 summation order not fixed), inference
   // the bit-reproducible one
   bool train_pass = false;
+  // the training pass is one rank's share of a data-parallel step (fm_train_step_dp, fm_train_step_sampled with a
+  // communicator of more than one rank): batch normalisation takes its statistics over the global batch.
+  // `stats_reduced` is recorded behind each statistics all-reduce of backward.
+  bool dp_pass = false;
+  cudaEvent_t stats_reduced = nullptr;
   // fm_model_set_inference_mode(m, 1): predict / evaluate / patch_wise_prediction also take the three-issuer mode
   // (about 25 % more conv throughput, results no longer bit-identical from run to run)
   bool fast_inference = false;
@@ -460,6 +467,7 @@ static int build_layer_table(fm_model* m) {
   m->layer_done.resize(m->layers.size());
   for (auto& e : m->layer_done) FM_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
   FM_CUDA(cudaEventCreateWithFlags(&m->ev_tmp, cudaEventDisableTiming));
+  if (m->batch_norm) FM_CUDA(cudaEventCreateWithFlags(&m->stats_reduced, cudaEventDisableTiming));
   // gradient buckets: consecutive layers in backward (= reverse creation) order, ~1/4 of the
   // parameters each; every bucket is one contiguous range of the flat buffer.
   const int nl = (int)m->layers.size();
@@ -635,6 +643,7 @@ extern "C" int fm_model_destroy(fm_model* m) {
   m->normRaw.release();
   m->normGRaw.release();
   m->normScratch.release();
+  m->normSums.release();
   m->gIsZero.release();
   m->isAcc.release();
   m->pw_vol.release();
@@ -672,6 +681,7 @@ extern "C" int fm_model_destroy(fm_model* m) {
     if (m->host_stage_done[b]) cudaEventDestroy(m->host_stage_done[b]);
   }
   if (m->ev_tmp) cudaEventDestroy(m->ev_tmp);
+  if (m->stats_reduced) cudaEventDestroy(m->stats_reduced);
   delete m;
   return FM_OK;
 }
@@ -919,6 +929,7 @@ static int ensure_capacity(fm_model* m, int B, bool train) {
     FM_TRY(m->normRaw.ensure(biggest));
     if (train || m->train_alloc) FM_TRY(m->normGRaw.ensure(biggest));
     FM_TRY(m->normScratch.ensure((size_t)cap * cmax * 2 * 1030));
+    if (train || m->train_alloc) FM_TRY(m->normSums.ensure(2 * cmax + 1));
   }
   if (train || m->train_alloc) {
     FM_TRY(m->t_in.ensure((size_t)cap * v0));  // (no dL/dz tensor: the head backward forms the Dice gradient itself)
@@ -1053,16 +1064,24 @@ static int deconv_bwd(fm_ctx* ctx, const bf16* x, const bf16* g, const bf16* w_d
 
 // One conv block of a U-Net: Conv + bias + ReLU (create_convolution_block, unet.py:102-113), or under
 // batch_normalization=True Conv (+bias, no activation) -> raw -> BatchNormalization + ReLU. A training pass keeps the
-// raw output and the batch statistics of every block.
+// raw output and the batch statistics of every block. In a data-parallel pass the statistics are those of the global
+// batch: this shard's per-channel sums are all-reduced over the ranks on the compute stream before the normalisation.
 static int unet_block_fwd(fm_model* m, const Layer& l, const void* x1, const bf16* x2, bf16* y, int B) {
   if (!m->batch_norm) return conv_fwd(m, l, x1, x2, y, B, 1);
+  fm_ctx* ctx = m->ctx;
   const int li = layer_pos(m, l);
   const Layer &nl = m->layers[li + 1], &ml = m->layers[li + 2];
   bf16* raw = m->train_pass ? m->normRawL[li].p : m->normRaw.p;
   FM_TRY(conv_fwd(m, l, x1, x2, raw, B, 0));
-  return k_batchnorm_relu(m->ctx, raw, m->params + nl.w_off, m->params + nl.b_off, m->params + ml.w_off,
+  const double* sums = nullptr;
+  if (m->dp_pass) {
+    FM_TRY(k_batchnorm_sums(ctx, raw, B, m->vox(l.level), l.cout, m->normScratch.p, m->normScratch.n, m->normSums.p));
+    FM_TRY(comm_allreduce(ctx, m->normSums.p, 2 * (size_t)l.cout + 1, 1, ctx->stream));
+    sums = m->normSums.p;
+  }
+  return k_batchnorm_relu(ctx, raw, m->params + nl.w_off, m->params + nl.b_off, m->params + ml.w_off,
                           m->params + ml.b_off, y, B, m->vox(l.level), l.cout, m->normScratch.p, m->normScratch.n,
-                          m->train_pass ? m->normStatsL[li].p : nullptr, m->train_pass ? 1 : 0);
+                          m->train_pass ? m->normStatsL[li].p : nullptr, m->train_pass ? 1 : 0, sums);
 }
 
 static int forward_isensee(fm_model* m, int B);
@@ -1146,15 +1165,28 @@ static int backward_isensee(fm_model* m, int B);
 // output. Without batch normalisation that is gy (the ReLU mask was applied where gy was formed). With it: the
 // BatchNormalization + ReLU backward into normGRaw and the gamma / beta gradients; the moving statistics and then the
 // norm layer are done. The conv bias in front of the normalisation has an analytically zero gradient (conv_wgrad
-// still sums it: rounding noise, as in Keras).
+// still sums it: rounding noise, as in Keras). In a data-parallel pass mean(g') and mean(g' * xh) are global (one
+// all-reduce of this shard's sums) while gamma / beta receive only this shard's sums: the gradient all-reduce adds the
+// other ranks' shares.
 static int unet_block_bwd(fm_model* m, const Layer& l, const bf16* gy, int B, const bf16** dy) {
   *dy = gy;
   if (!m->batch_norm) return FM_OK;
+  fm_ctx* ctx = m->ctx;
   const int li = layer_pos(m, l);
   const Layer &nl = m->layers[li + 1], &ml = m->layers[li + 2];
-  FM_TRY(k_batchnorm_relu_bwd(m->ctx, m->normRawL[li].p, m->normStatsL[li].p, m->params + nl.w_off,
+  const double* sums = nullptr;
+  if (m->dp_pass) {
+    FM_TRY(k_batchnorm_bwd_sums(ctx, m->normRawL[li].p, m->normStatsL[li].p, m->params + nl.w_off, m->params + nl.b_off,
+                                gy, nullptr, m->grads + nl.w_off, m->grads + nl.b_off, B, m->vox(l.level), l.cout,
+                                m->normScratch.p, m->normScratch.n, m->normSums.p));
+    FM_TRY(comm_allreduce(ctx, m->normSums.p, 2 * (size_t)l.cout + 1, 1, ctx->stream));
+    FM_CUDA(cudaEventRecord(m->stats_reduced, ctx->stream));
+    sums = m->normSums.p;
+  }
+  FM_TRY(k_batchnorm_relu_bwd(ctx, m->normRawL[li].p, m->normStatsL[li].p, m->params + nl.w_off,
                               m->params + nl.b_off, gy, nullptr, m->normGRaw.p, m->grads + nl.w_off,
-                              m->grads + nl.b_off, B, m->vox(l.level), l.cout, m->normScratch.p, m->normScratch.n));
+                              m->grads + nl.b_off, B, m->vox(l.level), l.cout, m->normScratch.p, m->normScratch.n,
+                              sums));
   *dy = m->normGRaw.p;
   FM_TRY(mark_layer_done(m, ml));
   return mark_layer_done(m, nl);
@@ -2446,14 +2478,19 @@ extern "C" int fm_train_step(fm_model* m, const float* x, const float* t, int ba
 // sums, backward, bucketed gradient all-reduce overlapped with it, Adam, metrics.
 static int dp_step_after_forward(fm_model* m, float lr, float out_metrics[4]);
 
+// Marks the passes of one data-parallel step (m->dp_pass) for the lifetime of the guard, whichever way the step returns.
+struct DpPassGuard {
+  fm_model* m;
+  DpPassGuard(fm_model* model, bool on) : m(model) { m->dp_pass = on; }
+  ~DpPassGuard() { m->dp_pass = false; }
+};
+
 extern "C" int fm_train_step_dp(fm_model* m, const float* x, const float* t, int batch, float lr,
                                 float out_metrics[4]) {
-  FM_CHECK(!(m && m->batch_norm), FM_EINVAL,
-           "fm_train_step_dp: batch_normalization=True needs batch statistics over the GLOBAL batch (not built): "
-           "a data-parallel step on local statistics would not equal the single-process reference");
   FM_CHECK(m && x && t && batch > 0 && out_metrics, FM_EINVAL, "fm_train_step_dp: bad argument");
   fm_ctx* ctx = m->ctx;
   if (!ctx->comm || ctx->comm_size == 1) return fm_train_step(m, x, t, batch, lr, out_metrics);
+  DpPassGuard dp(m, true);
   FM_TRY(fm_train_forward(m, x, t, batch));
   return dp_step_after_forward(m, lr, out_metrics);
 }
@@ -2483,8 +2520,10 @@ extern "C" int fm_train_step_sampled(fm_model* m, fm_volset* s, const int32_t* c
   FM_TRY(ensure_capacity(m, batch, true));
   FM_TRY(sampler_gather_device(s, cases, corners, aug, batch, patch, truth_index, truth_size, prev_truth_index,
                                prev_truth_size, m->x_in.p, m->t_in.p));
+  const bool dp = ctx->comm && ctx->comm_size > 1;
+  DpPassGuard dp_guard(m, dp);  // set before the forward pass: batch normalisation needs the global statistics there
   FM_TRY(train_forward_dev(m, batch));
-  if (ctx->comm && ctx->comm_size > 1) return dp_step_after_forward(m, lr, out_metrics);
+  if (dp) return dp_step_after_forward(m, lr, out_metrics);
   if (!pipeline_enabled()) {
     FM_TRY(fm_train_backward(m));
     return fm_train_apply(m, lr, 0, out_metrics);
@@ -2499,14 +2538,16 @@ extern "C" int fm_train_step_sampled(fm_model* m, fm_volset* s, const int32_t* c
 
 static int dp_step_after_forward(fm_model* m, float lr, float out_metrics[4]) {
   fm_ctx* ctx = m->ctx;
-  FM_CHECK(!m->batch_norm, FM_EINVAL,
-           "data-parallel step: batch_normalization=True needs batch statistics over the GLOBAL batch (not built)");
   // 8 float64: the GLOBAL Dice statistics every rank back-propagates (64 bytes; latency only)
   FM_TRY(comm_allreduce(ctx, m->sums, kNumLossSums, 1, ctx->stream));
   FM_TRY(fm_train_metrics_async(m));
   FM_TRY(fm_train_backward(m));
   // gradient buckets in completion order (backward runs in reverse creation order): each all-reduce waits only for
-  // the event of the bucket's first layer and overlaps whatever backward still has queued on the compute stream
+  // the event of the bucket's first layer and overlaps whatever backward still has queued on the compute stream.
+  // Under batch normalisation backward itself all-reduces statistics on the compute stream, over the same
+  // communicator, and one communicator's operations must not run concurrently: the buckets start behind the last of
+  // those all-reduces (they then overlap only the tail of backward).
+  if (m->batch_norm) FM_CUDA(cudaStreamWaitEvent(ctx->comm_stream, m->stats_reduced, 0));
   for (size_t b = 0; b < m->buckets.size(); ++b) {
     const Layer& first = m->layers[m->buckets[b].first];
     const int last_i = m->buckets[b].second;
@@ -3096,6 +3137,122 @@ extern "C" int fm_op_batchnorm_relu_bwd(fm_ctx* ctx, const float* x, const float
   FM_TRY(k_batchnorm_relu_bwd(ctx, bx, dst, dg, db, bgy, bgy2, bdx, dgg, dgg + C, N, vox, C, scratch, ns));
   FM_CUDA(cudaMemcpyAsync(dgamma, dgg, (size_t)C * 4, cudaMemcpyDeviceToHost, ctx->stream));
   FM_CUDA(cudaMemcpyAsync(dbeta, dgg + C, (size_t)C * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  return s.down_bf16(bdx, n, dx);
+}
+
+// The batch normalisation of a data-parallel step one stage at a time, for one shard x [N,vox,C] of the global batch
+// (unet_block_fwd / unet_block_bwd with m->dp_pass; the all-reduce in between is the caller's sum over the shards).
+// fm_op_batchnorm_sums: sums [2C + 1] = (sum x [C], sum x^2 [C], voxel count) of the shard.
+extern "C" int fm_op_batchnorm_sums(fm_ctx* ctx, const float* x, int N, int64_t vox, int C, double* sums) {
+  FM_CHECK(ctx && x && sums && N > 0 && vox > 0, FM_EINVAL, "fm_op_batchnorm_sums: bad argument");
+  FM_CUDA(cudaSetDevice(ctx->device));
+  OpScratch s(ctx);
+  const size_t n = (size_t)N * vox * C, ns = norm_scratch_floats(N, C);
+  bf16* bx = nullptr;
+  float* scratch = nullptr;
+  double* dsums = nullptr;
+  FM_TRY(s.up_bf16(x, n, &bx));
+  FM_TRY(s.alloc(&scratch, ns));
+  FM_TRY(s.alloc(&dsums, 2 * (size_t)C + 1));
+  FM_TRY(k_batchnorm_sums(ctx, bx, N, vox, C, scratch, ns, dsums));
+  FM_CUDA(cudaMemcpyAsync(sums, dsums, (2 * (size_t)C + 1) * 8, cudaMemcpyDeviceToHost, ctx->stream));
+  FM_CUDA(cudaStreamSynchronize(ctx->stream));
+  return FM_OK;
+}
+
+// fm_op_batchnorm_relu_global: the training forward of the shard with the global `sums` (every shard's sums added):
+// y, the moving-average step of moving_mean / moving_var [C] (in/out), and stats [C][2] = (mean, rsqrt(var + eps)).
+extern "C" int fm_op_batchnorm_relu_global(fm_ctx* ctx, const float* x, const float* gamma, const float* beta,
+                                           float* moving_mean, float* moving_var, int N, int64_t vox, int C,
+                                           const double* sums, float* y, float* stats) {
+  FM_CHECK(ctx && x && gamma && beta && moving_mean && moving_var && sums && y && stats && N > 0 && vox > 0, FM_EINVAL,
+           "fm_op_batchnorm_relu_global: bad argument");
+  FM_CUDA(cudaSetDevice(ctx->device));
+  OpScratch s(ctx);
+  const size_t n = (size_t)N * vox * C, ns = norm_scratch_floats(N, C);
+  bf16 *bx = nullptr, *by = nullptr;
+  float *dg = nullptr, *db = nullptr, *dmm = nullptr, *dmv = nullptr, *scratch = nullptr, *dst = nullptr;
+  double* dsums = nullptr;
+  FM_TRY(s.up_bf16(x, n, &bx));
+  FM_TRY(s.up_f32(gamma, C, &dg));
+  FM_TRY(s.up_f32(beta, C, &db));
+  FM_TRY(s.up_f32(moving_mean, C, &dmm));
+  FM_TRY(s.up_f32(moving_var, C, &dmv));
+  FM_TRY(s.alloc(&dsums, 2 * (size_t)C + 1));
+  FM_CUDA(cudaMemcpyAsync(dsums, sums, (2 * (size_t)C + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
+  FM_TRY(s.alloc(&scratch, ns));
+  FM_TRY(s.alloc(&dst, (size_t)N * C * 2));
+  FM_TRY(s.alloc(&by, n));
+  FM_TRY(k_batchnorm_relu(ctx, bx, dg, db, dmm, dmv, by, N, vox, C, scratch, ns, dst, 1, dsums));
+  FM_CUDA(cudaMemcpyAsync(moving_mean, dmm, (size_t)C * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  FM_CUDA(cudaMemcpyAsync(moving_var, dmv, (size_t)C * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  FM_CUDA(cudaMemcpyAsync(stats, dst, (size_t)C * 2 * 4, cudaMemcpyDeviceToHost, ctx->stream));  // sample 0's row
+  return s.down_bf16(by, n, y);
+}
+
+// Uploads stats [C][2] as the [N][C][2] rows (all equal) the backward kernels read.
+static int up_bn_stats(OpScratch& s, const float* stats, int N, int C, float** out) {
+  std::vector<float> rows((size_t)N * C * 2);
+  for (int i = 0; i < N; ++i) std::copy(stats, stats + 2 * (size_t)C, rows.begin() + (size_t)i * C * 2);
+  FM_TRY(s.up_f32(rows.data(), rows.size(), out));
+  FM_CUDA(cudaStreamSynchronize(s.ctx->stream));  // the copy reads `rows`, which leaves scope
+  return FM_OK;
+}
+
+// fm_op_batchnorm_bwd_sums: from the global stats [C][2] of fm_op_batchnorm_relu_global and the shard's gy (gy2 may be
+// NULL): sums [2C + 1] = (sum g' [C], sum g' * xh [C], voxel count), and this shard's dgamma / dbeta [C].
+extern "C" int fm_op_batchnorm_bwd_sums(fm_ctx* ctx, const float* x, const float* stats, const float* gamma,
+                                        const float* beta, const float* gy, const float* gy2, int N, int64_t vox, int C,
+                                        double* sums, float* dgamma, float* dbeta) {
+  FM_CHECK(ctx && x && stats && gamma && beta && gy && sums && dgamma && dbeta && N > 0 && vox > 0, FM_EINVAL,
+           "fm_op_batchnorm_bwd_sums: bad argument");
+  FM_CUDA(cudaSetDevice(ctx->device));
+  OpScratch s(ctx);
+  const size_t n = (size_t)N * vox * C, ns = norm_scratch_floats(N, C);
+  bf16 *bx = nullptr, *bgy = nullptr, *bgy2 = nullptr;
+  float *dg = nullptr, *db = nullptr, *scratch = nullptr, *dst = nullptr, *dgg = nullptr;
+  double* dsums = nullptr;
+  FM_TRY(s.up_bf16(x, n, &bx));
+  FM_TRY(s.up_bf16(gy, n, &bgy));
+  if (gy2) FM_TRY(s.up_bf16(gy2, n, &bgy2));
+  FM_TRY(s.up_f32(gamma, C, &dg));
+  FM_TRY(s.up_f32(beta, C, &db));
+  FM_TRY(up_bn_stats(s, stats, N, C, &dst));
+  FM_TRY(s.alloc(&scratch, ns));
+  FM_TRY(s.alloc(&dgg, 2 * (size_t)C));
+  FM_TRY(s.alloc(&dsums, 2 * (size_t)C + 1));
+  FM_TRY(k_zero(ctx, dgg, 2 * (size_t)C * 4));
+  FM_TRY(k_batchnorm_bwd_sums(ctx, bx, dst, dg, db, bgy, bgy2, dgg, dgg + C, N, vox, C, scratch, ns, dsums));
+  FM_CUDA(cudaMemcpyAsync(sums, dsums, (2 * (size_t)C + 1) * 8, cudaMemcpyDeviceToHost, ctx->stream));
+  FM_CUDA(cudaMemcpyAsync(dgamma, dgg, (size_t)C * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  FM_CUDA(cudaMemcpyAsync(dbeta, dgg + C, (size_t)C * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  FM_CUDA(cudaStreamSynchronize(ctx->stream));
+  return FM_OK;
+}
+
+// fm_op_batchnorm_relu_bwd_global: the shard's dx from the global stats and the global backward `sums`.
+extern "C" int fm_op_batchnorm_relu_bwd_global(fm_ctx* ctx, const float* x, const float* stats, const float* gamma,
+                                               const float* beta, const float* gy, const float* gy2, int N,
+                                               int64_t vox, int C, const double* sums, float* dx) {
+  FM_CHECK(ctx && x && stats && gamma && beta && gy && sums && dx && N > 0 && vox > 0, FM_EINVAL,
+           "fm_op_batchnorm_relu_bwd_global: bad argument");
+  FM_CUDA(cudaSetDevice(ctx->device));
+  OpScratch s(ctx);
+  const size_t n = (size_t)N * vox * C, ns = norm_scratch_floats(N, C);
+  bf16 *bx = nullptr, *bgy = nullptr, *bgy2 = nullptr, *bdx = nullptr;
+  float *dg = nullptr, *db = nullptr, *scratch = nullptr, *dst = nullptr;
+  double* dsums = nullptr;
+  FM_TRY(s.up_bf16(x, n, &bx));
+  FM_TRY(s.up_bf16(gy, n, &bgy));
+  if (gy2) FM_TRY(s.up_bf16(gy2, n, &bgy2));
+  FM_TRY(s.up_f32(gamma, C, &dg));
+  FM_TRY(s.up_f32(beta, C, &db));
+  FM_TRY(up_bn_stats(s, stats, N, C, &dst));
+  FM_TRY(s.alloc(&dsums, 2 * (size_t)C + 1));
+  FM_CUDA(cudaMemcpyAsync(dsums, sums, (2 * (size_t)C + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
+  FM_TRY(s.alloc(&scratch, ns));
+  FM_TRY(s.alloc(&bdx, n));
+  FM_TRY(k_batchnorm_relu_bwd(ctx, bx, dst, dg, db, bgy, bgy2, bdx, nullptr, nullptr, N, vox, C, scratch, ns, dsums));
   return s.down_bf16(bdx, n, dx);
 }
 

@@ -1632,26 +1632,61 @@ int k_instnorm_lrelu(fm_ctx* ctx, const bf16* x, const float* gamma, const float
 // the instance-norm kernels above (slope 0 = ReLU); only the folds differ: they run over the samples too, and
 // eps sits under the square root.
 // ---------------------------------------------------------------------------------------------
+// Per-channel fold of the (n, block) partial pairs part[b][C][2] in fp64, one warp per channel: lane l takes pairs l,
+// l + 32, ... in (n, block) order, then a fixed xor butterfly (deterministic; every lane ends with the same totals).
+// The single-pass final kernels and batchnorm_fold_kernel all fold through this function, so the statistics of a
+// data-parallel step with one rank are bit-identical to those of a single-process step.
+__device__ __forceinline__ void bn_fold(const float* __restrict__ part, int pairs, int C, int c, int lane, double& a,
+                                        double& b) {
+  a = 0.0, b = 0.0;
+  for (int i = lane; i < pairs; i += 32) {
+    const float2 o = *reinterpret_cast<const float2*>(part + ((int64_t)i * C + c) * 2);
+    a += (double)o.x;
+    b += (double)o.y;
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    a += __shfl_xor_sync(0xffffffffu, a, o);
+    b += __shfl_xor_sync(0xffffffffu, b, o);
+  }
+}
+
+// Global statistics (data-parallel training): this shard's per-channel totals into sums[2C + 1] = (sum_c a, sum_c b,
+// count), ready for a SUM all-reduce over the ranks. (a, b) = (x, x^2) forward, (g, g * xh) backward; the backward
+// also adds this shard's totals into dgamma / dbeta (the gradient all-reduce sums them over the ranks once).
+__global__ void batchnorm_fold_kernel(const float* __restrict__ part, int pairs, int C, double count,
+                                      double* __restrict__ sums, float* __restrict__ dgamma, float* __restrict__ dbeta) {
+  const int c = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+  if (c >= C) return;
+  double a, b;
+  bn_fold(part, pairs, C, c, lane, a, b);
+  if (lane != 0) return;
+  sums[c] = a;
+  sums[C + c] = b;
+  if (c == 0) sums[2 * C] = count;
+  if (dgamma != nullptr) {
+    dgamma[c] += (float)b;
+    dbeta[c] += (float)a;
+  }
+}
+
 // One warp per channel. ss / stats are written for every sample (identical rows) so that the apply kernels are shared.
-__global__ void batchnorm_final_kernel(const float* __restrict__ part, const float* __restrict__ gamma,
-                                       const float* __restrict__ beta, float* __restrict__ moving_mean,
-                                       float* __restrict__ moving_var, float* __restrict__ ss, float* __restrict__ stats,
-                                       int N, int C, int blocks_per_sample, double count, float eps, float momentum,
-                                       int training) {
+// Training folds the partials of this batch, or with `sums` != nullptr takes the (all-reduced) totals and count of the
+// global batch from sums[2C + 1].
+__global__ void batchnorm_final_kernel(const float* __restrict__ part, const double* __restrict__ sums,
+                                       const float* __restrict__ gamma, const float* __restrict__ beta,
+                                       float* __restrict__ moving_mean, float* __restrict__ moving_var,
+                                       float* __restrict__ ss, float* __restrict__ stats, int N, int C,
+                                       int blocks_per_sample, double count, float eps, float momentum, int training) {
   const int c = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (c >= C) return;
   double mean, var;
   if (training) {
-    double s = 0.0, q = 0.0;
-    for (int b = lane; b < N * blocks_per_sample; b += 32) {  // (n, block) pairs in a fixed order
-      const float2 o = *reinterpret_cast<const float2*>(part + ((int64_t)b * C + c) * 2);
-      s += (double)o.x;
-      q += (double)o.y;
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-      s += __shfl_xor_sync(0xffffffffu, s, o);
-      q += __shfl_xor_sync(0xffffffffu, q, o);
+    double s, q;
+    if (sums != nullptr) {
+      s = sums[c], q = sums[C + c], count = sums[2 * C];
+    } else {
+      bn_fold(part, N * blocks_per_sample, C, c, lane, s, q);
     }
     mean = s / count;
     var = fmax(q / count - mean * mean, 0.0);
@@ -1679,22 +1714,20 @@ __global__ void batchnorm_final_kernel(const float* __restrict__ part, const flo
 }
 
 // coef[n][c] = (gamma * rstd, mean(g), mean(g * xh)) for every sample; dgamma = sum g * xh, dbeta = sum g (stored).
-__global__ void batchnorm_bwd_final_kernel(const float* __restrict__ part, const float* __restrict__ stats,
-                                           const float* __restrict__ gamma, float* __restrict__ coef,
-                                           float* __restrict__ dgamma, float* __restrict__ dbeta, int N, int C,
-                                           int blocks_per_sample, double count) {
+// With `sums` the means are those of the global batch and dgamma / dbeta are left alone (batchnorm_fold_kernel added
+// this shard's totals).
+__global__ void batchnorm_bwd_final_kernel(const float* __restrict__ part, const double* __restrict__ sums,
+                                           const float* __restrict__ stats, const float* __restrict__ gamma,
+                                           float* __restrict__ coef, float* __restrict__ dgamma,
+                                           float* __restrict__ dbeta, int N, int C, int blocks_per_sample,
+                                           double count) {
   const int c = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (c >= C) return;
-  double s1 = 0.0, s2 = 0.0;
-  for (int b = lane; b < N * blocks_per_sample; b += 32) {
-    const float2 o = *reinterpret_cast<const float2*>(part + ((int64_t)b * C + c) * 2);
-    s1 += (double)o.x;
-    s2 += (double)o.y;
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    s1 += __shfl_xor_sync(0xffffffffu, s1, o);
-    s2 += __shfl_xor_sync(0xffffffffu, s2, o);
+  double s1, s2;
+  if (sums != nullptr) {
+    s1 = sums[c], s2 = sums[C + c], count = sums[2 * C];
+  } else {
+    bn_fold(part, N * blocks_per_sample, C, c, lane, s1, s2);
   }
   const float a = (float)((double)gamma[c] * (double)stats[2 * c + 1]);  // sample 0's row: all rows are equal
   for (int n = lane; n < N; n += 32) {
@@ -1704,31 +1737,57 @@ __global__ void batchnorm_bwd_final_kernel(const float* __restrict__ part, const
     o[2] = (float)(s2 / count);
     o[3] = 0.f;
   }
-  if (lane == 0) {
+  if (lane == 0 && sums == nullptr) {
     dgamma[c] += (float)s2;
     dbeta[c] += (float)s1;
   }
 }
 
+static int batchnorm_check(int C, int N, int64_t vox_per_sample, size_t scratch_floats, int64_t* vpb, int* bps) {
+  FM_CHECK(C >= 8 && C <= 512 && (C & (C - 1)) == 0, FM_EINVAL, "batchnorm: C=%d must be a power of two in [8,512]", C);
+  *bps = norm_blocks(vox_per_sample, vpb);
+  const size_t need = (size_t)N * C * (2 * (size_t)*bps + 4);
+  FM_CHECK(scratch_floats >= need, FM_EINVAL, "batchnorm: scratch too small (%zu < %zu floats)", scratch_floats, need);
+  return FM_OK;
+}
+
+int k_batchnorm_sums(fm_ctx* ctx, const bf16* x, int N, int64_t vox_per_sample, int C, float* scratch,
+                     size_t scratch_floats, double* sums) {
+  int64_t vpb;
+  int bps;
+  FM_TRY(batchnorm_check(C, N, vox_per_sample, scratch_floats, &vpb, &bps));
+  float* part = scratch;
+  ProfScope prof(ctx, "batchnorm_sums", 0.0, (double)N * vox_per_sample * C * 2.0);
+  instnorm_partial_kernel<<<dim3(bps, N), kThreads, kThreads * 16 * sizeof(float), ctx->stream>>>(x, part, vox_per_sample,
+                                                                                               C, vpb, bps);
+  FM_LAUNCH_OK(ctx);
+  batchnorm_fold_kernel<<<ceil_div(C * 32, 128), 128, 0, ctx->stream>>>(part, N * bps, C,
+                                                                      (double)N * (double)vox_per_sample, sums, nullptr,
+                                                                      nullptr);
+  FM_LAUNCH_OK(ctx);
+  return FM_OK;
+}
+
 int k_batchnorm_relu(fm_ctx* ctx, const bf16* x, const float* gamma, const float* beta, float* moving_mean,
                      float* moving_var, bf16* y, int N, int64_t vox_per_sample, int C, float* scratch,
-                     size_t scratch_floats, float* stats, int training) {
-  FM_CHECK(C >= 8 && C <= 512 && (C & (C - 1)) == 0, FM_EINVAL, "batchnorm: C=%d must be a power of two in [8,512]", C);
+                     size_t scratch_floats, float* stats, int training, const double* sums) {
   int64_t vpb;
-  const int bps = norm_blocks(vox_per_sample, &vpb);
-  const size_t need = (size_t)N * C * (2 * (size_t)bps + 4);
-  FM_CHECK(scratch_floats >= need, FM_EINVAL, "batchnorm: scratch too small (%zu < %zu floats)", scratch_floats, need);
+  int bps;
+  FM_TRY(batchnorm_check(C, N, vox_per_sample, scratch_floats, &vpb, &bps));
+  FM_CHECK(sums == nullptr || training, FM_EINVAL, "batchnorm: global sums need a training pass");
   float* part = scratch;
   float* ss = scratch + (size_t)N * C * 2 * bps;
-  ProfScope prof(ctx, "batchnorm_relu", 0.0, (double)N * vox_per_sample * C * (training ? 6.0 : 4.0));
-  if (training) {
+  const bool fold = training && sums == nullptr;
+  ProfScope prof(ctx, "batchnorm_relu", 0.0, (double)N * vox_per_sample * C * (fold ? 6.0 : 4.0));
+  if (fold) {
     instnorm_partial_kernel<<<dim3(bps, N), kThreads, kThreads * 16 * sizeof(float), ctx->stream>>>(x, part, vox_per_sample,
                                                                                                  C, vpb, bps);
     FM_LAUNCH_OK(ctx);
   }
-  batchnorm_final_kernel<<<ceil_div(C * 32, 128), 128, 0, ctx->stream>>>(part, gamma, beta, moving_mean, moving_var, ss, stats,
-                                                                       N, C, bps, (double)N * (double)vox_per_sample, 1e-3f,
-                                                                       0.99f, training);
+  batchnorm_final_kernel<<<ceil_div(C * 32, 128), 128, 0, ctx->stream>>>(part, sums, gamma, beta, moving_mean, moving_var,
+                                                                       ss, stats, N, C, bps,
+                                                                       (double)N * (double)vox_per_sample, 1e-3f, 0.99f,
+                                                                       training);
   FM_LAUNCH_OK(ctx);
   int64_t vpa;
   const int bpa = norm_apply_blocks(vox_per_sample, C, &vpa);
@@ -1737,22 +1796,41 @@ int k_batchnorm_relu(fm_ctx* ctx, const bf16* x, const float* gamma, const float
   return FM_OK;
 }
 
+int k_batchnorm_bwd_sums(fm_ctx* ctx, const bf16* x, const float* stats, const float* gamma, const float* beta,
+                         const bf16* gy, const bf16* gy2, float* dgamma, float* dbeta, int N, int64_t vox_per_sample,
+                         int C, float* scratch, size_t scratch_floats, double* sums) {
+  int64_t vpb;
+  int bps;
+  FM_TRY(batchnorm_check(C, N, vox_per_sample, scratch_floats, &vpb, &bps));
+  float* part = scratch;
+  NormBwdArgs a{x, stats, gamma, beta, gy, gy2, nullptr, vox_per_sample, C, 0.f};
+  ProfScope prof(ctx, "batchnorm_bwd_sums", 0.0, (double)N * vox_per_sample * C * (gy2 ? 6.0 : 4.0));
+  instnorm_bwd_partial_kernel<<<dim3(bps, N), kThreads, kThreads * 16 * sizeof(float), ctx->stream>>>(a, part, vpb, bps);
+  FM_LAUNCH_OK(ctx);
+  batchnorm_fold_kernel<<<ceil_div(C * 32, 128), 128, 0, ctx->stream>>>(part, N * bps, C,
+                                                                      (double)N * (double)vox_per_sample, sums, dgamma,
+                                                                      dbeta);
+  FM_LAUNCH_OK(ctx);
+  return FM_OK;
+}
+
 int k_batchnorm_relu_bwd(fm_ctx* ctx, const bf16* x, const float* stats, const float* gamma, const float* beta,
                          const bf16* gy, const bf16* gy2, bf16* dx, float* dgamma, float* dbeta, int N,
-                         int64_t vox_per_sample, int C, float* scratch, size_t scratch_floats) {
-  FM_CHECK(C >= 8 && C <= 512 && (C & (C - 1)) == 0, FM_EINVAL, "batchnorm bwd: C=%d must be a power of two in [8,512]", C);
+                         int64_t vox_per_sample, int C, float* scratch, size_t scratch_floats, const double* sums) {
   int64_t vpb;
-  const int bps = norm_blocks(vox_per_sample, &vpb);
-  const size_t need = (size_t)N * C * (2 * (size_t)bps + 4);
-  FM_CHECK(scratch_floats >= need, FM_EINVAL, "batchnorm bwd: scratch too small (%zu < %zu floats)", scratch_floats, need);
+  int bps;
+  FM_TRY(batchnorm_check(C, N, vox_per_sample, scratch_floats, &vpb, &bps));
   float* part = scratch;
   float* coef = scratch + (size_t)N * C * 2 * bps;
   NormBwdArgs a{x, stats, gamma, beta, gy, gy2, nullptr, vox_per_sample, C, 0.f};
-  ProfScope prof(ctx, "batchnorm_relu_bwd", 0.0, (double)N * vox_per_sample * C * (gy2 ? 14.0 : 10.0));
-  instnorm_bwd_partial_kernel<<<dim3(bps, N), kThreads, kThreads * 16 * sizeof(float), ctx->stream>>>(a, part, vpb, bps);
-  FM_LAUNCH_OK(ctx);
-  batchnorm_bwd_final_kernel<<<ceil_div(C * 32, 128), 128, 0, ctx->stream>>>(part, stats, gamma, coef, dgamma, dbeta, N, C, bps,
-                                                                           (double)N * (double)vox_per_sample);
+  ProfScope prof(ctx, "batchnorm_relu_bwd", 0.0,
+                 (double)N * vox_per_sample * C * ((gy2 ? 14.0 : 10.0) - (sums ? (gy2 ? 6.0 : 4.0) : 0.0)));
+  if (sums == nullptr) {
+    instnorm_bwd_partial_kernel<<<dim3(bps, N), kThreads, kThreads * 16 * sizeof(float), ctx->stream>>>(a, part, vpb, bps);
+    FM_LAUNCH_OK(ctx);
+  }
+  batchnorm_bwd_final_kernel<<<ceil_div(C * 32, 128), 128, 0, ctx->stream>>>(part, sums, stats, gamma, coef, dgamma, dbeta,
+                                                                           N, C, bps, (double)N * (double)vox_per_sample);
   FM_LAUNCH_OK(ctx);
   int64_t vpa;
   const int bpa = norm_apply_blocks(vox_per_sample, C, &vpa);

@@ -272,12 +272,24 @@ int k_instnorm_lrelu_bwd(fm_ctx*, const bf16* x, const float* stats, const float
 // BatchNormalization(axis=1) + ReLU of a raw conv output (create_convolution_block(batch_normalization=True)):
 // training = batch statistics (kept in `stats` [N][C][2] = (mean, rsqrt(var + eps)), identical rows) and the moving
 // averages are updated in place; inference = the moving statistics. Scratch as for the instance norm.
+// Global statistics (a data-parallel training pass): k_batchnorm_sums writes this shard's per-channel totals
+// sums[2C + 1] = (sum x [C], sum x^2 [C], count); once they are SUM all-reduced over the ranks, k_batchnorm_relu with
+// `sums` normalises with the statistics of the global batch (and skips its own partial pass). With one shard the result
+// is bit-identical to `sums` = nullptr.
+int k_batchnorm_sums(fm_ctx*, const bf16* x, int N, int64_t vox_per_sample, int C, float* scratch, size_t scratch_floats,
+                     double* sums);
 int k_batchnorm_relu(fm_ctx*, const bf16* x, const float* gamma, const float* beta, float* moving_mean, float* moving_var,
                      bf16* y, int N, int64_t vox_per_sample, int C, float* scratch, size_t scratch_floats, float* stats,
-                     int training);
+                     int training, const double* sums = nullptr);
+// The backward likewise: k_batchnorm_bwd_sums writes (sum g' [C], sum g' * xh [C], count) and adds this shard's totals
+// into dgamma / dbeta; k_batchnorm_relu_bwd with the all-reduced `sums` forms dx from the global means and leaves
+// dgamma / dbeta alone. The partials live in `scratch` only within one call.
+int k_batchnorm_bwd_sums(fm_ctx*, const bf16* x, const float* stats, const float* gamma, const float* beta,
+                         const bf16* gy, const bf16* gy2, float* dgamma, float* dbeta, int N, int64_t vox_per_sample,
+                         int C, float* scratch, size_t scratch_floats, double* sums);
 int k_batchnorm_relu_bwd(fm_ctx*, const bf16* x, const float* stats, const float* gamma, const float* beta, const bf16* gy,
                          const bf16* gy2, bf16* dx, float* dgamma, float* dbeta, int N, int64_t vox_per_sample, int C,
-                         float* scratch, size_t scratch_floats);
+                         float* scratch, size_t scratch_floats, const double* sums = nullptr);
 int k_zero_insert(fm_ctx*, const bf16* coarse, bf16* fine, Dims5 coarse_dims, int pz = 2);
 int k_add_bf16(fm_ctx*, const bf16* a, const bf16* b, bf16* out, int64_t n);
 int k_sumpool_f32(fm_ctx*, const float* fine, float* coarse, int N, int X, int Y, int Z, int pz = 2);

@@ -165,6 +165,12 @@ SIGNATURES = {
                                          c_fp]),
     "fm_op_batchnorm_relu": (c_int, [c_vp, c_int, c_fp, c_fp, c_fp, c_fp, c_fp, c_int, c_i64, c_int, c_fp]),
     "fm_op_batchnorm_relu_bwd": (c_int, [c_vp, c_fp, c_fp, c_fp, c_fp, c_fp, c_int, c_i64, c_int, c_fp, c_fp, c_fp]),
+    "fm_op_batchnorm_sums": (c_int, [c_vp, c_fp, c_int, c_i64, c_int, c_dp]),
+    "fm_op_batchnorm_relu_global": (c_int, [c_vp, c_fp, c_fp, c_fp, c_fp, c_fp, c_int, c_i64, c_int, c_dp, c_fp, c_fp]),
+    "fm_op_batchnorm_bwd_sums": (c_int, [c_vp, c_fp, c_fp, c_fp, c_fp, c_fp, c_fp, c_int, c_i64, c_int, c_dp, c_fp,
+                                         c_fp]),
+    "fm_op_batchnorm_relu_bwd_global": (c_int, [c_vp, c_fp, c_fp, c_fp, c_fp, c_fp, c_fp, c_int, c_i64, c_int, c_dp,
+                                                c_fp]),
     "fm_op_conv_strided": (c_int, [c_vp, c_fp, c_fp, c_fp] + [c_int] * 7 + [c_fp, c_fp, c_fp, c_fp]),
     "fm_op_deconv": (c_int, [c_vp, c_fp, c_fp, c_fp] + [c_int] * 6 + [c_fp, c_fp, c_int, c_fp, c_fp, c_fp]),
     "fm_op_depth_space": (c_int, [c_vp, c_int, c_fp] + [c_int] * 6 + [c_fp]),

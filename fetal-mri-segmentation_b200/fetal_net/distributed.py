@@ -9,7 +9,12 @@ gloo is enough) is only the CONTROL plane: it carries the 128-byte NCCL id from 
              every rank back-propagates the global Dice; the gradient of that one global scalar is the
              SUM (not the mean) of the ranks' local gradients. The flat fp32 gradient buffer is
              all-reduced bucket by bucket on a side stream while the rest of backward still runs,
-             then every rank applies the identical Adam step.
+             then every rank applies the identical Adam step. batch_normalization=True U-Nets take every
+             layer's batch statistics over the global batch: one float64 all-reduce of the per-channel
+             (sum, sum of squares, count) per layer in forward and of the gradient sums in backward, so
+             the step equals the single-process step on the concatenated batch (uneven shards too) and
+             the moving statistics stay identical on every rank. The gradient buckets then start after
+             backward's last statistics all-reduce instead of overlapping backward.
   inference  the patch list of patch_wise_prediction is split contiguously over ranks; each rank
              overlap-adds its patches into a private float64 partial sum on its GPU, one ncclReduce, then
              sum / count on the root. Counts are analytic (identical on every rank) and never communicated.

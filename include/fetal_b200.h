@@ -88,8 +88,12 @@ int fm_model_destroy(fm_model* m);
  * axis=1) -> ReLU (unet3d/unet.py:102-113). Keras semantics: batch statistics (biased variance, eps 1e-3 under the root)
  * in training passes, moving statistics (momentum 0.99, sample-size-corrected variance) at inference. The layer table
  * lists, behind every block's conv, a "<conv>_norm" pseudo-layer (kernel = gamma, bias = beta) and a "<conv>_moving"
- * pseudo-layer (kernel = moving_mean, bias = moving_variance; never touched by the optimizer). Single-process training
- * only: fm_train_step_dp refuses (the statistics would have to span the global batch). */
+ * pseudo-layer (kernel = moving_mean, bias = moving_variance; never touched by the optimizer). A data-parallel step
+ * (fm_train_step_dp, fm_train_step_sampled on more than one rank) takes every layer's statistics over the GLOBAL batch:
+ * one float64 all-reduce of (sum x, sum x^2, count) per layer in the forward pass and of (sum g', sum g' * xh, count)
+ * in the backward pass, so the step equals the single-process step on the concatenated batch and every rank computes
+ * the same moving averages (global count in the variance correction). Shards may be uneven. Outside such a step - and
+ * with fm_comm_enable(ctx, 0) - each process normalises with its own batch. */
 #define FM_UNET_DECONVOLUTION 1
 #define FM_UNET_BATCH_NORMALIZATION 2
 int fm_model_create_unet3d_ex(fm_ctx* ctx, const fm_unet3d_spec* spec, int flags, fm_model** out);
@@ -411,7 +415,9 @@ int fm_comm_broadcast_params(fm_model* m, int root);
  * communication stream, each as soon as its last layer's gradients are final (overlapping the rest of backward);
  * the identical Keras-Adam step on every rank. out_metrics are the GLOBAL loss / accuracy / VOD / Dice. With pinned
  * x / t the call returns when the statistics are on the host (like fm_train_step). Without a communicator it is
- * fm_train_step. */
+ * fm_train_step. Under FM_UNET_BATCH_NORMALIZATION every BatchNormalization takes its statistics over the global batch
+ * through small float64 all-reduces on the compute stream (2 per block and step); the gradient buckets then start after
+ * backward's last one, since one communicator runs its operations in issue order. */
 int fm_train_step_dp(fm_model* m, const float* x, const float* t, int batch, float lr, float out_metrics[4]);
 
 /* fm_patchwise_predict with the patch list sharded contiguously over the ranks of the ctx communicator: every rank
@@ -505,6 +511,25 @@ int fm_op_batchnorm_relu(fm_ctx* ctx, int training, const float* x, const float*
                          float* moving_mean, float* moving_var, int N, int64_t vox, int C, float* y);
 int fm_op_batchnorm_relu_bwd(fm_ctx* ctx, const float* x, const float* gamma, const float* beta, const float* gy,
                              const float* gy2, int N, int64_t vox, int C, float* dx, float* dgamma, float* dbeta);
+/* The same layer in a data-parallel step, one stage at a time for one shard x [N,vox,C] of the global batch; the
+ * caller sums the float64 sums [2C + 1] of all shards in between (what the all-reduce does).
+ * fm_op_batchnorm_sums: (sum x [C], sum x^2 [C], voxel count) of the shard.
+ * fm_op_batchnorm_relu_global: the training forward with the global sums: y, the moving-average step (in/out) and
+ * stats [C][2] = (mean, rsqrt(var + eps)).
+ * fm_op_batchnorm_bwd_sums: with those stats, (sum g' [C], sum g' * xh [C], voxel count) of the shard and the shard's
+ * own dgamma / dbeta [C] (their sum over the shards is the full-batch gradient); gy2 may be NULL.
+ * fm_op_batchnorm_relu_bwd_global: dx of the shard from the stats and the global backward sums.
+ * With one shard every output is bit-identical to fm_op_batchnorm_relu(_bwd). */
+int fm_op_batchnorm_sums(fm_ctx* ctx, const float* x, int N, int64_t vox, int C, double* sums);
+int fm_op_batchnorm_relu_global(fm_ctx* ctx, const float* x, const float* gamma, const float* beta, float* moving_mean,
+                                float* moving_var, int N, int64_t vox, int C, const double* sums, float* y,
+                                float* stats);
+int fm_op_batchnorm_bwd_sums(fm_ctx* ctx, const float* x, const float* stats, const float* gamma, const float* beta,
+                             const float* gy, const float* gy2, int N, int64_t vox, int C, double* sums, float* dgamma,
+                             float* dbeta);
+int fm_op_batchnorm_relu_bwd_global(fm_ctx* ctx, const float* x, const float* stats, const float* gamma,
+                                    const float* beta, const float* gy, const float* gy2, int N, int64_t vox, int C,
+                                    const double* sums, float* dx);
 /* Stride-2 TF-'SAME' convolution of the Isensee in-convs (no activation), ksize 3 or 31 (z not strided): x
  * [N,Xin,Yin,Zin,Cin] -> y [N,Xin/2,Yin/2,Zin/2 (or Zin),Cout] when y != NULL; with dy (the shape of y) the data
  * gradient dx [N,Xin,Yin,Zin,Cin] and weight gradient dw_keras through zero insertion and stride-1 kernels. */
