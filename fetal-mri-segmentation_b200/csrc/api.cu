@@ -409,7 +409,8 @@ static void add_layer(std::vector<Layer>& ls, const char* fmt, int d, int c1, in
 }
 
 // Marching-kernel eligibility (conv_march.cu), decided once per layer when the model is built: 3x3x3 convs whose first
-// source has at least 16 channels, the forward only at stride 1. X, Y, Z = the extent the pass runs at.
+// source has at least 16 channels and whose filter bank, or a 32-wide Cout slice of it, fits in shared memory
+// (conv_march_slices), the forward only at stride 1. X, Y, Z = the extent the pass runs at.
 static bool march_fprop_ok(const Layer& l, int X, int Y, int Z) {
   return l.k == 3 && l.c1 >= 16 && l.stride == 1 && conv_march_supported(X, Y, Z, l.c1, l.c2, l.cout, l.k);
 }
@@ -599,6 +600,11 @@ static int unet_up_packs(fm_model* m) {
     if (!conv_up_supported(X, Y, Z, l.c1, l.c2, l.cout)) continue;
     const size_t n = (size_t)l.cout * 64 * l.c1;
     FM_CUDA(cudaMalloc((void**)&l.w_up_d, n * sizeof(bf16)));
+    if (l.march_d[0]) {  // the gradient towards the coarse tensor never runs at fine resolution: no pack to refresh
+      FM_CUDA(cudaFree(l.w_md[0]));
+      l.w_md[0] = nullptr;
+      l.march_d[0] = false;
+    }
     if (l.march_f) {
       // small filter bank (dec0a): forward and weight gradient stay on the marching kernels over the materialised
       // upsampled tensor; the gradient towards the coarse tensor still drops from 27 fine taps + a sum-pool pass to
@@ -851,6 +857,9 @@ static int refresh_packs(fm_model* m) {
       d.kcf1 = l.c2 ? conv_march_kc(l.c1, l.c2, l.cout, l.c2) : 0;
       d.kcd0 = conv_march_kc(l.cout, 0, l.c1, l.cout);
       d.kcd1 = l.c2 ? conv_march_kc(l.cout, 0, l.c2, l.cout) : 0;
+      d.srf = l.march_f ? l.cout / conv_march_slices(l.c1, l.c2, l.cout) : l.cout;
+      d.srd0 = l.march_d[0] ? l.c1 / conv_march_slices(l.cout, 0, l.c1) : l.c1;
+      d.srd1 = l.march_d[1] ? l.c2 / conv_march_slices(l.cout, 0, l.c2) : l.c2;
       d.block0 = blocks;
       blocks += d.taps * ceil_div(d.cout, 32) * ceil_div(l.cin(), 32);  // 32 x 32 (co, c) tiles per tap
       weights += (double)l.wcount();
@@ -2693,10 +2702,11 @@ extern "C" int fm_op_conv3d_fprop(fm_ctx* ctx, int impl, const float* x, const f
     FM_CHECK(conv_march_supported(X, Y, Z, C1, C2, Cout, ksize), FM_EINVAL, "march kernel does not cover this shape");
     bf16 *wm1 = nullptr, *wm2 = nullptr;
     FM_TRY(s.alloc(&wm1, (size_t)conv_march_pack_elems(C1, Cout)));
-    FM_TRY(k_repack_march(ctx, dw, wm1, Cout, Ct, 0, C1, conv_march_kc(C1, C2, Cout, C1)));
+    const int srows = Cout / conv_march_slices(C1, C2, Cout);
+    FM_TRY(k_repack_march(ctx, dw, wm1, Cout, Ct, 0, C1, conv_march_kc(C1, C2, Cout, C1), srows));
     if (C2 > 0) {
       FM_TRY(s.alloc(&wm2, (size_t)conv_march_pack_elems(C2, Cout)));
-      FM_TRY(k_repack_march(ctx, dw, wm2, Cout, Ct, C1, C2, conv_march_kc(C1, C2, Cout, C2)));
+      FM_TRY(k_repack_march(ctx, dw, wm2, Cout, Ct, C1, C2, conv_march_kc(C1, C2, Cout, C2), srows));
     }
     FM_TRY(k_conv3d_march(ctx, dx1, dx2, wm1, wm2, dbias, dy, nullptr, N, X, Y, Z, C1, C2, Cout, relu, Cout, 0,
                           impl != 3));
@@ -2730,7 +2740,8 @@ extern "C" int fm_op_conv_dgrad(fm_ctx* ctx, int impl, const float* dy, const fl
     FM_CHECK(conv_march_supported(X, Y, Z, Cout, 0, Cin, ksize), FM_EINVAL, "march kernel does not cover this shape");
     bf16* wm = nullptr;
     FM_TRY(s.alloc(&wm, (size_t)conv_march_pack_elems(Cout, Cin)));
-    FM_TRY(k_repack_march(ctx, wd, wm, Cin, Cout, 0, Cout, conv_march_kc(Cout, 0, Cin, Cout)));
+    FM_TRY(k_repack_march(ctx, wd, wm, Cin, Cout, 0, Cout, conv_march_kc(Cout, 0, Cin, Cout),
+                          Cin / conv_march_slices(Cout, 0, Cin)));
     FM_TRY(k_conv3d_march(ctx, ddy, nullptr, wm, nullptr, nullptr, ddx, dmask, N, X, Y, Z, Cout, 0, Cin, 0, Cin, 0,
                           impl != 3));
   } else if (impl == 0)
@@ -3311,7 +3322,8 @@ extern "C" int fm_op_conv_strided(fm_ctx* ctx, const float* x, const float* w_ke
     FM_TRY(conv_wgrad(ctx, l, fine, bx, nullptr, bz, dw, nullptr));
     if (march_dgrad_ok(l, 0, Xin, Yin, Zin)) {
       FM_TRY(s.alloc(&l.w_md[0], (size_t)conv_march_pack_elems(Cout, Cin)));
-      FM_TRY(k_repack_march(ctx, wd, l.w_md[0], Cin, Cout, 0, Cout, conv_march_kc(Cout, 0, Cin, Cout)));
+      FM_TRY(k_repack_march(ctx, wd, l.w_md[0], Cin, Cout, 0, Cout, conv_march_kc(Cout, 0, Cin, Cout),
+                            Cin / conv_march_slices(Cout, 0, Cin)));
       l.march_d[0] = true;
     }
     FM_TRY(conv_dgrad(ctx, l, fine, 0, bz, nullptr, bdx, false));

@@ -376,12 +376,13 @@ int k_head_bwd(fm_ctx*, const bf16* x, const float* dz, const float* w, bf16* dx
 // weight repack: master fp32 [Cout][taps][Cin] -> bf16 fprop pack (same layout) and bf16 dgrad
 // pack(s) [Cin_s][taps flipped][Cout] per source
 // all layers in ONE launch (after every Adam step): per layer the fprop pack, the dgrad pack(s) and, where the
-// plane-marching kernels run, their packs [chunk][dz][dy][kx = 2,1,0][row][kc] — see k_repack_weights / k_repack_march
+// plane-marching kernels run, their packs (march_pack_index) — see k_repack_weights / k_repack_march
 struct RepackDesc {
   int64_t w_off;   // offset of the master kernel [Cout][taps][C1+C2] in the flat fp32 parameter buffer
   int cout, taps, c1, c2;
   bf16 *wf, *wd0, *wd1, *mf0, *mf1, *md0, *md1;  // null = not needed
   int kcf0, kcf1, kcd0, kcd1;                    // K-chunk widths of the four marching packs (conv_march_kc)
+  int srf, srd0, srd1;                           // rows per Cout slice of the fprop / dgrad marching packs
   int block0;      // first 256-thread block of this layer in the fused grid
 };
 int k_repack_all(fm_ctx*, const float* params, const RepackDesc* table_dev, int nlayers, int total_blocks,
@@ -431,13 +432,28 @@ int k_conv3d_first_tc(fm_ctx*, const float* x, const bf16* w_packed, const float
                       int Z, int Cout, int relu);
 int k_conv3d_first_tc_wgrad(fm_ctx*, const float* x, const bf16* dy, float* dw, int N, int X, int Y, int Z, int Cout);
 
-// conv_march.cu: plane-marching fprop / dgrad of 3x3x3 convs whose filter bank fits in shared memory
+// conv_march.cu: plane-marching fprop / dgrad of 3x3x3 convs whose filter bank, or a 32-wide Cout slice of it, fits in
+// shared memory
 int conv_march_supported(int X, int Y, int Z, int C1, int C2, int Cout, int ksize);
+// Cout slices of a marching conv (C1 [+ C2] -> Cout): 1 when the whole filter bank fits, Cout / 32 when only a 32-wide
+// slice of it does, 0 when neither does
+int conv_march_slices(int C1, int C2, int Cout);
 int64_t conv_march_pack_elems(int Cs, int Cout);
 // K-chunk width of a source with Cs channels in a marching conv (C1 [+ C2] -> Cout): 64 (128-byte slab rows) unless the
-// resident filter bank leaves fewer than two slab slots per dz ring, then 32 (half-size slots, twice as many)
+// resident filter bank (of one slice) leaves fewer than two slab slots per dz ring, then 32 (half-size slots, twice as
+// many)
 int conv_march_kc(int C1, int C2, int Cout, int Cs);
-int k_repack_march(fm_ctx*, const bf16* P, bf16* Wm, int Nrows, int Ktot, int kofs, int Cs, int KC);
+// march pack of one source (Ks input channels) of a conv with Cout slices of `srows` rows:
+// Wm[slice][chunk][dz][dy][kxr][row][kc] with tap = (kx*3 + ky)*3 + kz, kxr = 2 - kx, k = chunk * KC + kc. With one
+// slice (srows = all rows) the slice index is always 0.
+__host__ __device__ inline int64_t march_pack_index(int Ks, int srows, int row, int tap, int k, int KC) {
+  const int kx = tap / 9, ky = (tap / 3) % 3, kz = tap % 3;
+  const int sl = row / srows, r = row - sl * srows;
+  const int ch = k / KC, kc = k % KC;
+  return (int64_t)sl * 27 * Ks * srows + ((((int64_t)(ch * 3 + kz) * 3 + ky) * 3 + (2 - kx)) * srows + r) * KC + kc;
+}
+// P: bf16 pack [Nrows][27][Ktot]; writes the march pack (slices of srows rows) of channel range [kofs, kofs+Cs)
+int k_repack_march(fm_ctx*, const bf16* P, bf16* Wm, int Nrows, int Ktot, int kofs, int Cs, int KC, int srows);
 // reproducible: the MMAs reach the tensor pipe in a fixed order, so the output is identical run to run (predict /
 // evaluate / patch_wise_prediction); otherwise, for Cout <= 32, the order follows three interleaved issue streams
 // (training passes)

@@ -1,5 +1,6 @@
 // conv_march.cu — "plane-marching" implicit-GEMM Conv3D 3x3x3 (fprop + dgrad) for layers whose whole filter bank fits
-// in shared memory (the full-resolution layers that hold most of the U-Net's FLOPs).
+// in shared memory (the full-resolution layers that hold most of the U-Net's FLOPs), or whose bank fits in 32-wide Cout
+// slices (the 64 -> 64 and 64 -> 128 layers of the 32^3 and 16^3 levels: one slice per CTA, all slices in one launch).
 //
 // The per-tap kernel (conv_tc.cu) re-reads every activation tile 27x from L2 and, for Cout <= 64, is bound by the
 // A-operand read from shared memory. This kernel removes both limits:
@@ -54,6 +55,9 @@ struct alignas(64) March2Params {
   uint32_t wofs[2];  // byte offset of the source's resident weights inside the W region
   int N, X, Y, Z;
   int ny, nz;
+  // Cout slices of CN channels each (conv_march_slices); slice = the fastest-varying part of a split column and the
+  // grid a multiple of `slices`, so CTA r serves slice r mod slices for its whole life
+  int slices;
   PlaneSplit split;  // how the (column, x) plane-tiles are dealt to the CTAs (common.cuh)
   int R;       // accumulator ring blocks (power of two)
   int stages;  // slab slots, a multiple of 3 (one private ring per dz slab copy)
@@ -109,6 +113,7 @@ __global__ void __launch_bounds__(march2_threads(CN), 1) conv3d_march2_kernel(co
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem0 = (smem_u32(smem_raw) + 1023u) & ~1023u;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int slice = (int)blockIdx.x % p.slices;
 
   const uint32_t w_base = smem0;
   const uint32_t a_base = smem0 + p.w_region;
@@ -162,6 +167,7 @@ __global__ void __launch_bounds__(march2_threads(CN), 1) conv3d_march2_kernel(co
   auto decode = [&](int item, int& n, int& iy, int& iz, int& xa, int& xb) -> bool {
     int col;
     if (!plane_split_next(p.split, (int)blockIdx.x, (int)gridDim.x, item / (int)gridDim.x, col, xa, xb)) return false;
+    col /= p.slices;
     iz = col % p.nz;
     const int r = col / p.nz;
     iy = r % p.ny;
@@ -183,8 +189,9 @@ __global__ void __launch_bounds__(march2_threads(CN), 1) conv3d_march2_kernel(co
       mbar_expect_tx_elect(wfull_bar, p.w_bytes);
       for (int s = 0; s < p.nsrc; ++s) {
         const uint32_t tile = 3u * Cn * (uint32_t)p.KC[s] * 2u;
+        const int row0 = slice * p.nchunks[s] * 27 * CN;  // first pack row of this CTA's slice
         for (int t = 0; t < p.nchunks[s] * 9; ++t)
-          tma_load_2d_elect(w_base + p.wofs[s] + (uint32_t)t * tile, &p.tmW[s], wfull_bar, 0, t * 3 * CN);
+          tma_load_2d_elect(w_base + p.wofs[s] + (uint32_t)t * tile, &p.tmW[s], wfull_bar, 0, row0 + t * 3 * CN);
       }
     }
     // the weights do not depend on the previous kernel in the stream; the activation slabs do
@@ -384,7 +391,7 @@ __global__ void __launch_bounds__(march2_threads(CN), 1) conv3d_march2_kernel(co
     if (p.bias != nullptr) {
 #pragma unroll
       for (int j = 0; j < CW / 4; ++j) {
-        const float4 b4 = __ldg(reinterpret_cast<const float4*>(p.bias + half * CW) + j);
+        const float4 b4 = __ldg(reinterpret_cast<const float4*>(p.bias + slice * CN + half * CW) + j);
         bias_r[4 * j] = b4.x;
         bias_r[4 * j + 1] = b4.y;
         bias_r[4 * j + 2] = b4.z;
@@ -406,7 +413,7 @@ __global__ void __launch_bounds__(march2_threads(CN), 1) conv3d_march2_kernel(co
       it_xo = xa;
       it_xb = xb;
       const int64_t v0 = (((int64_t)n * p.X + xa) * p.Y + (iy * kBY + yl)) * p.Z + (iz * kBZ + zl);
-      it_off = v0 * p.out_C + p.out_cofs + half * CW;
+      it_off = v0 * p.out_C + p.out_cofs + slice * CN + half * CW;  // the dgrad mask is read at the same offset
       return true;
     };
     auto it_next = [&]() -> bool {
@@ -537,29 +544,22 @@ __global__ void __launch_bounds__(march2_threads(CN), 1) conv3d_march2_kernel(co
   }
 }
 
-// march pack: Wm[chunk][dz][dy][kxr][n][kc] = P[n][tap(kx = 2 - kxr, ky = dy, kz = dz)][kofs + chunk*KC + kc]
+// march pack (march_pack_index, common.cuh) of P[n][tap][kofs + k], k < Cs
 __global__ void repack_march_kernel(const bf16* __restrict__ P, bf16* __restrict__ Wm, int Nrows, int Ktot,
-                                    int kofs, int Cs, int KC) {
-  const int64_t total = (int64_t)(Cs / KC) * 27 * Nrows * KC;
+                                    int kofs, int Cs, int KC, int srows) {
+  const int64_t total = (int64_t)Nrows * 27 * Cs;
   const int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (g >= total) return;
-  const int kc = (int)(g % KC);
-  int64_t t = g / KC;
-  const int n = (int)(t % Nrows);
-  t /= Nrows;
-  const int kxr = (int)(t % 3);
-  t /= 3;
-  const int dy = (int)(t % 3);
-  t /= 3;
-  const int dz = (int)(t % 3);
-  const int ch = (int)(t / 3);
-  const int tap = ((2 - kxr) * 3 + dy) * 3 + dz;
-  Wm[g] = P[((int64_t)n * 27 + tap) * Ktot + kofs + ch * KC + kc];
+  const int k = (int)(g % Cs);
+  const int64_t t = g / Cs;
+  const int tap = (int)(t % 27), n = (int)(t / 27);
+  Wm[march_pack_index(Cs, srows, n, tap, k, KC)] = P[t * Ktot + kofs + k];
 }
 
 bool chan_ok_m(int C) { return C == 16 || C == 32 || C == 64 || (C > 64 && C % 64 == 0); }
 
-// resident filter bank: 27 taps * Cin * Cout * 2 B per source, each source region 1024-aligned
+// resident filter bank: 27 taps * Cin * Cn * 2 B per source (Cn = the output channels of one slice), each source region
+// 1024-aligned
 uint32_t march_w_region(int C1, int C2, int Cn) {
   const uint32_t a = ((uint32_t)27 * C1 * Cn * 2u + 1023u) & ~1023u;
   const uint32_t b = ((uint32_t)27 * C2 * Cn * 2u + 1023u) & ~1023u;
@@ -580,13 +580,21 @@ int launch_march2(fm_ctx* ctx, const March2Params& p, size_t smem, int grid) {
 
 }  // namespace
 
-// channels per source supported / whole filter bank + >= 3 slab stages fit in shared memory
+// A layer whose whole filter bank does not fit runs as Cout / 32 slices of 32 output channels in one launch (64 -> 64,
+// 64 -> 128): each CTA keeps one slice's bank resident.
+int conv_march_slices(int C1, int C2, int Cout) {
+  if (!chan_ok_m(C1) || (C2 != 0 && !chan_ok_m(C2))) return 0;
+  auto fits = [&](int cn) { return (int64_t)march_w_region(C1, C2, cn) + 3 * (int64_t)kSlot + 2048 <= kMaxDynSmem; };
+  if ((Cout == 16 || Cout == 32 || Cout == 64) && fits(Cout)) return 1;
+  if (Cout > 32 && Cout % 32 == 0 && fits(32)) return Cout / 32;
+  return 0;
+}
+
+// channels per source supported / the filter bank (of one slice) + >= 3 slab stages fit in shared memory
 int conv_march_supported(int X, int Y, int Z, int C1, int C2, int Cout, int ksize) {
   if (ksize != 3) return 0;
   if (Y % kBY != 0 || Z % kBZ != 0 || X < 2) return 0;
-  if (!(Cout == 16 || Cout == 32 || Cout == 64)) return 0;
-  if (!chan_ok_m(C1) || (C2 != 0 && !chan_ok_m(C2))) return 0;
-  return (int64_t)march_w_region(C1, C2, Cout) + 3 * (int64_t)kSlot + 2048 <= kMaxDynSmem;
+  return conv_march_slices(C1, C2, Cout) > 0;
 }
 
 int64_t conv_march_pack_elems(int Cs, int Cout) { return (int64_t)27 * Cs * Cout; }
@@ -594,15 +602,16 @@ int64_t conv_march_pack_elems(int Cs, int Cout) { return (int64_t)27 * Cs * Cout
 int conv_march_kc(int C1, int C2, int Cout, int Cs) {
   const int kc = std::min(Cs, 64);
   if (kc < 64) return kc;
-  const int full_slots = (kMaxDynSmem - 2048 - (int)march_w_region(C1, C2, Cout)) / (int)kSlot;
+  const int S = std::max(conv_march_slices(C1, C2, Cout), 1);
+  const int full_slots = (kMaxDynSmem - 2048 - (int)march_w_region(C1, C2, Cout / S)) / (int)kSlot;
   return full_slots < 6 ? 32 : 64;
 }
 
-// P: bf16 pack [Nrows][27][Ktot]; writes the march pack of channel range [kofs, kofs+Cs)
-int k_repack_march(fm_ctx* ctx, const bf16* P, bf16* Wm, int Nrows, int Ktot, int kofs, int Cs, int KC) {
+int k_repack_march(fm_ctx* ctx, const bf16* P, bf16* Wm, int Nrows, int Ktot, int kofs, int Cs, int KC, int srows) {
   const int64_t total = (int64_t)27 * Cs * Nrows;
   ProfScope prof(ctx, "repack_march", 0.0, (double)total * 4.0);
-  repack_march_kernel<<<(unsigned)ceil_div64(total, 256), 256, 0, ctx->stream>>>(P, Wm, Nrows, Ktot, kofs, Cs, KC);
+  repack_march_kernel<<<(unsigned)ceil_div64(total, 256), 256, 0, ctx->stream>>>(P, Wm, Nrows, Ktot, kofs, Cs, KC,
+                                                                                  srows);
   FM_LAUNCH_OK(ctx);
   return FM_OK;
 }
@@ -614,6 +623,7 @@ int k_conv3d_march(fm_ctx* ctx, const bf16* x1, const bf16* x2, const bf16* wm1,
            "conv3d march: unsupported shape %dx%dx%d C1=%d C2=%d Cout=%d", X, Y, Z, C1, C2, Cout);
   EncodeTiledFn enc = encode_tiled();
   FM_CHECK(enc != nullptr, FM_ECUDA, "cuTensorMapEncodeTiled entry point not available");
+  const int S = conv_march_slices(C1, C2, Cout), Cn = Cout / S;  // the kernel computes Cn output channels per CTA
   March2Params p;
   memset(&p, 0, sizeof(p));
   p.nsrc = C2 > 0 ? 2 : 1;
@@ -623,7 +633,8 @@ int k_conv3d_march(fm_ctx* ctx, const bf16* x1, const bf16* x2, const bf16* wm1,
   p.Z = Z;
   p.ny = Y / kBY;
   p.nz = Z / kBZ;
-  p.R = std::min(kMaxRing2, 512 / Cout);
+  p.slices = S;
+  p.R = std::min(kMaxRing2, 512 / Cn);
   p.out_C = out_C;
   p.out_cofs = out_cofs;
   p.relu = relu;
@@ -640,8 +651,8 @@ int k_conv3d_march(fm_ctx* ctx, const bf16* x1, const bf16* x2, const bf16* wm1,
     p.KC[s] = KC;
     p.nchunks[s] = Cs[s] / KC;
     p.wofs[s] = wofs;
-    wofs += ((uint32_t)27 * Cs[s] * Cout * 2u + 1023u) & ~1023u;
-    wbytes += (uint32_t)27 * Cs[s] * Cout * 2u;
+    wofs += ((uint32_t)27 * Cs[s] * Cn * 2u + 1023u) & ~1023u;
+    wbytes += (uint32_t)27 * Cs[s] * Cn * 2u;
     {
       cuuint64_t dims[5] = {(cuuint64_t)Cs[s], (cuuint64_t)Z, (cuuint64_t)Y, (cuuint64_t)X, (cuuint64_t)N};
       cuuint64_t strides[4] = {(cuuint64_t)Cs[s] * 2, (cuuint64_t)Z * Cs[s] * 2, (cuuint64_t)Y * Z * Cs[s] * 2,
@@ -657,7 +668,7 @@ int k_conv3d_march(fm_ctx* ctx, const bf16* x1, const bf16* x2, const bf16* wm1,
       const cuuint64_t rows = (cuuint64_t)p.nchunks[s] * 27 * Cout;
       cuuint64_t dims[2] = {(cuuint64_t)KC, rows};
       cuuint64_t strides[1] = {(cuuint64_t)KC * 2};
-      cuuint32_t box[2] = {(cuuint32_t)KC, (cuuint32_t)(3 * Cout)};
+      cuuint32_t box[2] = {(cuuint32_t)KC, (cuuint32_t)(3 * Cn)};
       cuuint32_t estr[2] = {1, 1};
       CUresult r = enc(&p.tmW[s], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (void*)wms[s], dims, strides, box, estr,
                        CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for_row_bytes(KC * 2), CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
@@ -681,18 +692,20 @@ int k_conv3d_march(fm_ctx* ctx, const bf16* x1, const bf16* x2, const bf16* wm1,
   p.stages = stages;
   const size_t smem = (size_t)wofs + (size_t)stages * p.slot + 2048;
   FM_CHECK(smem <= (size_t)kMaxDynSmem, FM_EINVAL, "conv3d march: %zu B of shared memory needed", smem);
-  int grid = std::max(1, std::min(N * p.ny * p.nz * X / 4, ctx->num_sms));
-  plane_split_setup(&p.split, N * p.ny * p.nz, X, grid, 1.4);
-  grid = std::min(grid, N * p.ny * p.nz * p.split.nxc);
+  // a split column = (sample, y tile, z tile, slice); the grid stays a multiple of S (one slice per CTA)
+  const int cols = N * p.ny * p.nz * S;
+  int grid = std::max(S, std::min(cols * X / 4, ctx->num_sms) / S * S);
+  plane_split_setup(&p.split, cols, X, grid, 1.4);
+  grid = std::min(grid, cols * p.split.nxc);
   const double vox = (double)N * X * Y * Z;
   ProfScope prof(ctx, mask != nullptr || bias == nullptr ? "conv3d_march_dgrad" : "conv3d_march_fprop",
                  2.0 * 27 * (C1 + C2) * Cout * vox, vox * (C1 + C2 + Cout) * 2.0);
-  // issue mode (see the kernel): one issuing warp keeps up with the 96-cycle MMAs of Cout = 64 (mode 0); narrower
-  // layers split the issue three ways, in a fixed order where the result has to be bit-reproducible (mode 2)
+  // issue mode (see the kernel): one issuing warp keeps up with the 96-cycle MMAs of Cn = 64 (mode 0); narrower
+  // layers and slices split the issue three ways, in a fixed order where the result has to be bit-reproducible (mode 2)
   int rc;
-  if (Cout == 64)
+  if (Cn == 64)
     rc = launch_march2<0, 64>(ctx, p, smem, grid);
-  else if (Cout == 32)
+  else if (Cn == 32)
     rc = reproducible ? launch_march2<2, 32>(ctx, p, smem, grid) : launch_march2<1, 32>(ctx, p, smem, grid);
   else
     rc = reproducible ? launch_march2<2, 16>(ctx, p, smem, grid) : launch_march2<1, 16>(ctx, p, smem, grid);

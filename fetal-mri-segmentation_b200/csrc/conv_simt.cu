@@ -613,13 +613,6 @@ __global__ void repack_weights_kernel(const float* __restrict__ w, bf16* __restr
   }
 }
 
-__device__ __forceinline__ int64_t march_pack_index(int rows, int row, int tap, int k, int KC) {
-  // Wm[chunk][dz][dy][kxr][row][kc] with tap = (kx*3 + ky)*3 + kz, kxr = 2 - kx
-  const int kx = tap / 9, ky = (tap / 3) % 3, kz = tap % 3;
-  const int ch = k / KC, kc = k % KC;
-  return ((((int64_t)(ch * 3 + kz) * 3 + ky) * 3 + (2 - kx)) * rows + row) * KC + kc;
-}
-
 // One block = one 32 (co) x 32 (c) tile of one tap of one layer: the master weights are read along c (coalesced), the
 // fprop pack and the marching fprop pack are written along c, and - through a shared-memory transpose - the dgrad pack
 // and the marching dgrad pack along co. (The first version wrote the transposed packs as scattered 2-byte stores:
@@ -655,7 +648,7 @@ __global__ void __launch_bounds__(kThreads) repack_all_kernel(const float* __res
         v = params[d.w_off + g];
         const bf16 b = __float2bfloat16(v);
         if (d.wf) d.wf[g] = b;
-        if (mf) mf[march_pack_index(d.cout, co, tap, cs, kcf)] = b;
+        if (mf) mf[march_pack_index(second ? d.c2 : d.c1, d.srf, co, tap, cs, kcf)] = b;
       }
       tile[ty + 8 * r][tx] = v;
     }
@@ -668,12 +661,12 @@ __global__ void __launch_bounds__(kThreads) repack_all_kernel(const float* __res
       const int c = ctile * 32 + ty + 8 * r;
       if (c >= Ct || co >= d.cout) continue;
       const bool second = c >= d.c1;
-      const int cs = second ? c - d.c1 : c, Cs = second ? d.c2 : d.c1;
+      const int cs = second ? c - d.c1 : c;
       const bf16 b = __float2bfloat16(tile[tx][ty + 8 * r]);
       bf16* wd = second ? d.wd1 : d.wd0;
       if (wd) wd[((int64_t)cs * d.taps + tf) * d.cout + co] = b;
       bf16* md = second ? d.md1 : d.md0;
-      if (md) md[march_pack_index(Cs, cs, tf, co, second ? d.kcd1 : d.kcd0)] = b;
+      if (md) md[march_pack_index(d.cout, second ? d.srd1 : d.srd0, cs, tf, co, second ? d.kcd1 : d.kcd0)] = b;
     }
   }
 }
