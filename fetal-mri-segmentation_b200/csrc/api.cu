@@ -2507,6 +2507,14 @@ extern "C" int fm_train_step_dp(fm_model* m, const float* x, const float* t, int
 extern "C" int fm_train_step_sampled(fm_model* m, fm_volset* s, const int32_t* cases, const int32_t* corners,
                                      const fm_sample_aug* aug, int batch, int truth_index, int truth_size,
                                      int prev_truth_index, int prev_truth_size, float lr, float out_metrics[4]) {
+  return fm_train_step_sampled_warp(m, s, cases, corners, aug, nullptr, batch, truth_index, truth_size,
+                                    prev_truth_index, prev_truth_size, lr, out_metrics);
+}
+
+extern "C" int fm_train_step_sampled_warp(fm_model* m, fm_volset* s, const int32_t* cases, const int32_t* corners,
+                                          const fm_sample_aug* aug, const fm_sample_warp* warp, int batch,
+                                          int truth_index, int truth_size, int prev_truth_index, int prev_truth_size,
+                                          float lr, float out_metrics[4]) {
   FM_CHECK(m && s && cases && corners && batch > 0 && out_metrics, FM_EINVAL, "fm_train_step_sampled: bad argument");
   fm_ctx* ctx = m->ctx;
   FM_CUDA(cudaSetDevice(ctx->device));
@@ -2527,7 +2535,7 @@ extern "C" int fm_train_step_sampled(fm_model* m, fm_volset* s, const int32_t* c
     patch[2] = m->spec.Z;
   }
   FM_TRY(ensure_capacity(m, batch, true));
-  FM_TRY(sampler_gather_device(s, cases, corners, aug, batch, patch, truth_index, truth_size, prev_truth_index,
+  FM_TRY(sampler_gather_device(s, cases, corners, aug, warp, batch, patch, truth_index, truth_size, prev_truth_index,
                                prev_truth_size, m->x_in.p, m->t_in.p));
   const bool dp = ctx->comm && ctx->comm_size > 1;
   DpPassGuard dp_guard(m, dp);  // set before the forward pass: batch normalisation needs the global statistics there

@@ -80,9 +80,10 @@ struct fm_ctx {
 };
 
 // sampler.cu: cuts a batch of training samples out of device-resident cases into device buffers
-int sampler_gather_device(fm_volset* s, const int32_t* cases, const int32_t* corners, const fm_sample_aug* aug, int batch,
-                          const int32_t patch[3], int truth_index, int truth_size, int prev_truth_index,
-                          int prev_truth_size, float* x_dev, float* y_dev);
+// (warp == NULL: the unwarped cut)
+int sampler_gather_device(fm_volset* s, const int32_t* cases, const int32_t* corners, const fm_sample_aug* aug,
+                          const fm_sample_warp* warp, int batch, const int32_t patch[3], int truth_index,
+                          int truth_size, int prev_truth_index, int prev_truth_size, float* x_dev, float* y_dev);
 
 // comm.cu: in-place SUM collectives on the ctx communicator (no-ops without one); dtype 0 = float32, 1 = float64
 int comm_allreduce(fm_ctx* ctx, void* buf, size_t count, int dtype, cudaStream_t stream);

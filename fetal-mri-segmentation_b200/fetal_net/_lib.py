@@ -43,6 +43,13 @@ class SampleAug(ctypes.Structure):
                 ("noise_seed", ctypes.c_uint32)]
 
 
+class SampleWarp(ctypes.Structure):
+    """fm_sample_warp: per-sample affine map (row-major matrix, offset in voxels about the centre of the data box) and
+    optional elastic displacement (alpha per axis, hash seed, control points per axis: 0 = none, else 2..8)."""
+    _fields_ = [("matrix", ctypes.c_float * 9), ("offset", ctypes.c_float * 3), ("elastic_alpha", ctypes.c_float * 3),
+                ("elastic_seed", ctypes.c_uint32), ("elastic_grid", ctypes.c_int32)]
+
+
 class Isensee2DSpec(ctypes.Structure):
     _fields_ = [("H", ctypes.c_int32), ("W", ctypes.c_int32), ("in_channels", ctypes.c_int32),
                 ("depth", ctypes.c_int32), ("n_base_filters", ctypes.c_int32),
@@ -130,6 +137,10 @@ SIGNATURES = {
                                  c_int, c_fp, c_fp]),
     "fm_train_step_sampled": (c_int, [c_vp, c_vp, c_i32p, c_i32p, ctypes.POINTER(SampleAug), c_int, c_int, c_int,
                                       c_int, c_int, c_f, c_fp]),
+    "fm_volset_gather_warp": (c_int, [c_vp, c_i32p, c_i32p, ctypes.POINTER(SampleAug), ctypes.POINTER(SampleWarp), c_int,
+                                      c_i32p, c_int, c_int, c_int, c_int, c_fp, c_fp]),
+    "fm_train_step_sampled_warp": (c_int, [c_vp, c_vp, c_i32p, c_i32p, ctypes.POINTER(SampleAug),
+                                           ctypes.POINTER(SampleWarp), c_int, c_int, c_int, c_int, c_int, c_f, c_fp]),
     "fm_comm_unique_id": (c_int, [c_u8p]),
     "fm_comm_init": (c_int, [c_vp, c_int, c_int, c_u8p]),
     "fm_comm_destroy": (c_int, [c_vp]),

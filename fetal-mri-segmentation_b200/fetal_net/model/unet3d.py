@@ -326,16 +326,21 @@ class Model:
                                            float(self.optimizer.lr), _lib.fptr(m)))
         return [float(v) for v in m[:len(self.metrics_names)]]
 
-    def train_on_sampled_batch(self, sampler, cases, corners):
+    def train_on_sampled_batch(self, sampler, cases, corners, aug=None, warp=None):
         """One training step on samples cut on the device by a `fetal_net.device_sampler.DeviceSampler`
-        (next(generator) + train_on_batch of fetal_net/training.py:110-124 with no host batch): fm_train_step_sampled."""
+        (next(generator) + train_on_batch of fetal_net/training.py:110-124 with no host batch): fm_train_step_sampled.
+        aug / warp: per-sample fm_sample_aug / fm_sample_warp arrays (a data-parallel rank passes its slice); with both
+        None the sampler draws them from its `device_augment`."""
+        from ..device_sampler import _c_array
         self._check_loss()
         cases, corners = _lib.i32x(cases), _lib.i32x(corners)
+        if aug is None and warp is None:
+            aug, warp = sampler.draw_augment(cases.size)
         ti, ts, pi, ps = sampler._args()
         m = np.zeros(4, np.float32)
-        _lib.check(self._lib.fm_train_step_sampled(self._h, sampler._handle, _lib.i32ptr(cases), _lib.i32ptr(corners),
-                                                   sampler._aug_array(cases.size), int(cases.size), ti, ts, pi, ps,
-                                                   float(self.optimizer.lr), _lib.fptr(m)))
+        _lib.check(self._lib.fm_train_step_sampled_warp(
+            self._h, sampler._handle, _lib.i32ptr(cases), _lib.i32ptr(corners), _c_array(_lib.SampleAug, aug),
+            _c_array(_lib.SampleWarp, warp), int(cases.size), ti, ts, pi, ps, float(self.optimizer.lr), _lib.fptr(m)))
         return [float(v) for v in m[:len(self.metrics_names)]]
 
     def test_on_batch(self, x, y, **kw):

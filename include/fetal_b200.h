@@ -387,6 +387,34 @@ int fm_volset_gather(fm_volset* s, const int32_t* cases, const int32_t* corners,
 int fm_train_step_sampled(fm_model* m, fm_volset* s, const int32_t* cases, const int32_t* corners,
                           const fm_sample_aug* aug, int batch, int truth_index, int truth_size, int prev_truth_index,
                           int prev_truth_size, float lr, float out_metrics[4]);
+/* Optional per-sample geometric warp applied while cutting: the library's own rotate / scale / translate / elastic
+ * augmentation, NOT the reference's nilearn / imgaug pipeline. Coordinates are voxels of the case volume, axes (x, y, z)
+ * = the array axes. An output element that the unwarped sampler reads at volume position q (after the flip step) reads
+ *   s = c + offset + matrix . (q + d(q) - c),   c = corner + (P - 1) / 2   (the centre of the data box)
+ * instead; c is shared by the data, target and previous-truth channels, so a 2.5D sample stays registered.
+ * d(q)[a] = elastic_alpha[a] * trilinear(G_a, (q - corner) / spacing), spacing = (P - 1) / (G - 1) per axis (grid
+ * coordinate 0 on an axis with P = 1, clamped to [0, G - 1]), G = elastic_grid; the control value at x-major index g of
+ * G_a is ((h >> 8) * 2^-23) - 1 with h = hash32(hash32(elastic_seed) ^ (3 g + a)) (the sampler's integer mixer).
+ * Data channels are interpolated trilinearly, target and previous-truth channels take the nearest sample floor(s + 0.5);
+ * every coordinate is clamped to [0, n - 1] (scipy.ndimage.map_coordinates(order=1 / 0, mode='nearest'), the edge
+ * replication of the unwarped cut). The intensity scale and noise of fm_sample_aug apply to the interpolated data. */
+typedef struct fm_sample_warp {
+  float matrix[9];          /* row-major 3x3 */
+  float offset[3];          /* voxels */
+  float elastic_alpha[3];   /* voxels, >= 0 */
+  uint32_t elastic_seed;
+  int32_t elastic_grid;     /* 0 = no elastic displacement, else 2..8 control points per axis */
+} fm_sample_warp;
+/* fm_volset_gather / fm_train_step_sampled with one fm_sample_warp per sample (warp == NULL: no warp, the two calls
+ * above). Rejected with FM_EINVAL: a non-finite matrix, offset or alpha, a negative alpha, elastic_grid outside
+ * {0, 2..8}. Data-parallel like fm_train_step_sampled: every rank passes its own samples and their warps. */
+int fm_volset_gather_warp(fm_volset* s, const int32_t* cases, const int32_t* corners, const fm_sample_aug* aug,
+                          const fm_sample_warp* warp, int batch, const int32_t patch[3], int truth_index, int truth_size,
+                          int prev_truth_index, int prev_truth_size, float* x_out, float* y_out);
+int fm_train_step_sampled_warp(fm_model* m, fm_volset* s, const int32_t* cases, const int32_t* corners,
+                               const fm_sample_aug* aug, const fm_sample_warp* warp, int batch, int truth_index,
+                               int truth_size, int prev_truth_index, int prev_truth_size, float lr,
+                               float out_metrics[4]);
 
 /* ---- data parallelism (one process per GPU; NCCL over NVLink 5 / NVSwitch) -----------------------------------
  * The reference is single-process (fetal_net/training.py:115-117: workers=1, use_multiprocessing=False); these entry
