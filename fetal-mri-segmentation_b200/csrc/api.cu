@@ -282,8 +282,14 @@ struct fm_model {
   DevBuf<float> x_in, t_in, prob, dz;
   std::vector<DevBuf<bf16>> encA, encB, pool, up, decA, decB;          // forward
   std::vector<DevBuf<bf16>> gEncA, gEncB, gPool, gUp, gSkip, gDecA, gDecB;  // gradients
-  double* sums = nullptr;  // kNumLossSums doubles (device): 7 Dice / VOD / accuracy sums, the count, sum w * bce
-  double sums_host[kNumLossSums];
+  // nsums() doubles (device): 7 Dice / VOD / accuracy sums, the count, sum w * bce; with n_labels > 1 then (tp, t, p)
+  // per label
+  double* sums = nullptr;
+  double sums_host[kNumLossSums + 3 * kMaxLabels];
+  float label_dice[kMaxLabels] = {};  // per-label Dice of the last training step / evaluation (fm_model_label_dice)
+  // n_labels > 1: prob / t_in / mask_in are [sample][voxel][label]; a 3D model's channels-first [sample][label][voxel]
+  // host arrays are transposed through `lab_tmp` on the way in and out
+  DevBuf<float> lab_tmp;
   // loss: 0 dice_coefficient_loss, 1 dice_and_xent, 2 dice_and_xent_mask (weight mask = second model input)
   int loss_kind = 0;
   float xent_weight = 0.f, xent_inv_sigma = 0.f;
@@ -344,6 +350,9 @@ struct fm_model {
   bool targets_ready = false, stats_done = false;
 
   int depth() const { return spec.depth; }
+  int labels() const { return spec.n_labels; }
+  int nsums() const { return kNumLossSums + (labels() > 1 ? 3 * labels() : 0); }
+  bool label_transpose() const { return kcode == 3 && labels() > 1; }
   Dims5 dims(int level, int C, int B) const {
     return Dims5{B, spec.X >> level, spec.Y >> level, pz == 2 ? spec.Z >> level : spec.Z, C};
   }
@@ -434,8 +443,8 @@ static int build_layer_table(fm_model* m) {
     FM_CUDA(cudaMalloc((void**)b, pb));
     FM_CUDA(cudaMemset(*b, 0, pb));
   }
-  FM_CUDA(cudaMalloc((void**)&m->sums, kNumLossSums * sizeof(double)));
-  FM_CUDA(cudaMemset(m->sums, 0, kNumLossSums * sizeof(double)));
+  FM_CUDA(cudaMalloc((void**)&m->sums, m->nsums() * sizeof(double)));
+  FM_CUDA(cudaMemset(m->sums, 0, m->nsums() * sizeof(double)));
   // bf16 packs: fprop + dgrad copies of every kernel (the norm parameters are read as fp32), plus the marching packs
   int64_t pack_elems = 0;
   for (auto& l : m->layers)
@@ -544,7 +553,8 @@ extern "C" int fm_model_create_unet2d_ex(fm_ctx* ctx, const fm_unet2d_spec* spec
 
 static int build_unet(fm_ctx* ctx, const fm_unet3d_spec* spec, int kcode, int flags, fm_model** out) {
   FM_CHECK(spec->depth >= 2 && spec->depth <= 6, FM_EINVAL, "depth %d unsupported", spec->depth);
-  FM_CHECK(spec->n_labels == 1, FM_EINVAL, "n_labels=%d: only 1 is built", spec->n_labels);
+  FM_CHECK(spec->n_labels >= 1 && spec->n_labels <= kMaxLabels, FM_EINVAL, "n_labels=%d: 1 .. %d are built",
+           spec->n_labels, kMaxLabels);
   FM_CHECK(spec->n_base_filters == 16 || spec->n_base_filters == 32, FM_EINVAL,
            "n_base_filters=%d: 16 or 32", spec->n_base_filters);
   FM_CUDA(cudaSetDevice(ctx->device));
@@ -667,6 +677,7 @@ extern "C" int fm_model_destroy(fm_model* m) {
   m->t_in.release();
   m->prob.release();
   m->dz.release();
+  m->lab_tmp.release();
   for (auto* v : {&m->encA, &m->encB, &m->pool, &m->up, &m->decA, &m->decB, &m->gEncA, &m->gEncB,
                   &m->gPool, &m->gUp, &m->gSkip, &m->gDecA, &m->gDecB})
     for (auto& b : *v) b.release();
@@ -804,17 +815,59 @@ extern "C" int fm_model_set_loss(fm_model* m, int kind, float xent_weight, float
   return FM_OK;
 }
 
+// `batch` samples of an array shaped like the model output (targets, weight mask) from `src` (host memory, or device
+// memory with src_dev) into `dst` on the compute stream, in the device's label-fastest layout: the channels-first
+// [B][L][V] of a 3D multi-label model is transposed on the way.
+static int upload_labels(fm_model* m, const float* src, bool src_dev, float* dst, int batch) {
+  const size_t n = (size_t)batch * m->vox(0) * m->labels();
+  if (!m->label_transpose()) {
+    FM_CUDA(cudaMemcpyAsync(dst, src, n * sizeof(float), src_dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice,
+                            m->ctx->stream));
+    return FM_OK;
+  }
+  if (!src_dev) {
+    if (n > m->lab_tmp.n) {
+      FM_CUDA(cudaStreamSynchronize(m->ctx->stream));  // an earlier transpose may still read the old buffer
+      FM_TRY(m->lab_tmp.ensure(n));
+    }
+    FM_CUDA(cudaMemcpyAsync(m->lab_tmp.p, src, n * sizeof(float), cudaMemcpyHostToDevice, m->ctx->stream));
+    src = m->lab_tmp.p;
+  }
+  return k_label_transpose(m->ctx, src, dst, batch, m->vox(0), m->labels(), 1);
+}
+
+// the model's probabilities of `batch` samples in its output layout (channels-first for a 3D multi-label model) on the
+// compute stream: a device pointer, or `nullptr` to get a device buffer holding them
+static int output_view(fm_model* m, int batch, float* dst, const float** out) {
+  const size_t n = (size_t)batch * m->vox(0) * m->labels();
+  if (!m->label_transpose()) {
+    if (dst) FM_CUDA(cudaMemcpyAsync(dst, m->prob.p, n * sizeof(float), cudaMemcpyDeviceToDevice, m->ctx->stream));
+    *out = dst ? dst : m->prob.p;
+    return FM_OK;
+  }
+  if (!dst) {
+    if (n > m->lab_tmp.n) {
+      FM_CUDA(cudaStreamSynchronize(m->ctx->stream));
+      FM_TRY(m->lab_tmp.ensure(n));
+    }
+    dst = m->lab_tmp.p;
+  }
+  FM_TRY(k_label_transpose(m->ctx, m->prob.p, dst, batch, m->vox(0), m->labels(), 0));
+  *out = dst;
+  return FM_OK;
+}
+
 extern "C" int fm_model_set_weight_mask(fm_model* m, const float* mask, int batch) {
   FM_CHECK(m && mask && batch > 0, FM_EINVAL, "fm_model_set_weight_mask: bad argument");
   FM_CHECK(m->loss_kind == 2, FM_EINVAL, "fm_model_set_weight_mask: the model's loss takes no weight mask");
   FM_CUDA(cudaSetDevice(m->ctx->device));
-  const size_t n = (size_t)batch * m->vox(0);
+  const size_t n = (size_t)batch * m->vox(0) * m->labels();
   if (n > m->mask_in.n) {
     // the previous step may still read the old buffer
     FM_CUDA(cudaStreamSynchronize(m->ctx->stream));
     FM_TRY(m->mask_in.ensure(n));
   }
-  FM_CUDA(cudaMemcpyAsync(m->mask_in.p, mask, n * sizeof(float), cudaMemcpyHostToDevice, m->ctx->stream));
+  FM_TRY(upload_labels(m, mask, false, m->mask_in.p, batch));
   m->mask_valid = true;
   m->mask_batch = batch;
   return FM_OK;
@@ -838,7 +891,8 @@ static int refresh_packs(fm_model* m) {
     int blocks = 0;
     double weights = 0.0;
     for (auto& l : m->layers) {
-      if (l.is_norm || (l.k == 1 && l.cout == 1)) continue;  // norm parameters / heads are read as fp32
+      // norm parameters / heads (the 1x1x1 convs to n_labels outputs) are read as fp32
+      if (l.is_norm || (l.k == 1 && l.cout == m->labels())) continue;
       RepackDesc d;
       d.w_off = l.w_off;
       // a deconvolution is repacked as the 1x1x1 conv it runs as: [class * Cout + co][1][Cin]
@@ -907,7 +961,7 @@ static int ensure_capacity(fm_model* m, int B, bool train) {
   const size_t v0 = (size_t)m->vox(0);
   FM_TRY(m->x_in.ensure((size_t)cap * v0 * m->cin_real));
   if (m->kcode == 31) FM_TRY(m->x_pad.ensure((size_t)cap * v0 * 16));
-  FM_TRY(m->prob.ensure((size_t)cap * v0));
+  FM_TRY(m->prob.ensure((size_t)cap * v0 * m->labels()));
   for (int d = 0; d < D; ++d) {
     const size_t v = (size_t)m->vox(d) * cap;
     const Layer &la = L(m, "enc%da", d), &lb = L(m, "enc%db", d);
@@ -941,7 +995,8 @@ static int ensure_capacity(fm_model* m, int B, bool train) {
     if (train || m->train_alloc) FM_TRY(m->normSums.ensure(2 * cmax + 1));
   }
   if (train || m->train_alloc) {
-    FM_TRY(m->t_in.ensure((size_t)cap * v0));  // (no dL/dz tensor: the head backward forms the Dice gradient itself)
+    // (no dL/dz tensor: the head backward forms the Dice gradient itself)
+    FM_TRY(m->t_in.ensure((size_t)cap * v0 * m->labels()));
     for (int d = 0; d < D; ++d) {
       const size_t v = (size_t)m->vox(d) * cap;
       const Layer &la = L(m, "enc%da", d), &lb = L(m, "enc%db", d);
@@ -1155,12 +1210,12 @@ static int forward(fm_model* m, int B) {
   if (m->train_pass && m->targets_ready) {
     // head + sigmoid + Dice / VOD / accuracy sums in one pass (unet.py:68-69 + metrics.py:11-28)
     FM_TRY(k_head_fwd_dice(ctx, (const bf16*)cur, m->params + lf.w_off, m->params + lf.b_off, m->t_in.p, m->prob.p,
-                           (int64_t)B * m->vox(0), lf.c1, m->sums, m->xent()));
+                           (int64_t)B * m->vox(0), lf.c1, m->sums, m->xent(), m->labels()));
     m->stats_done = true;
     return FM_OK;
   }
   return k_head_fwd(ctx, (const bf16*)cur, m->params + lf.w_off, m->params + lf.b_off, m->prob.p,
-                    (int64_t)B * m->vox(0), lf.c1);
+                    (int64_t)B * m->vox(0), lf.c1, 1, m->labels());
 }
 
 static int mark_layer_done(fm_model* m, const Layer& l) {
@@ -1216,7 +1271,7 @@ static int backward(fm_model* m, int B) {
   // head backward with the soft-Dice gradient formed inside (closed form through the sigmoid with the GLOBAL sums):
   // without batch normalisation the gradient lands masked by the ReLU of dec0b
   FM_TRY(k_head_bwd(ctx, m->decB[0].p, m->prob.p, m->params + lf.w_off, m->gDecB[0].p, m->grads + lf.w_off,
-                    m->grads + lf.b_off, n0, lf.c1, bn ? 1 : 0, m->t_in.p, m->sums, m->xent()));
+                    m->grads + lf.b_off, n0, lf.c1, bn ? 1 : 0, m->t_in.p, m->sums, m->xent(), m->labels()));
   FM_TRY(mark_layer_done(m, lf));
   for (int d = 0; d <= D - 2; ++d) {
     const Layer &da = L(m, "dec%da", d), &db = L(m, "dec%db", d);
@@ -1299,6 +1354,16 @@ static void metrics_from_sums(const double s[kNumLossSums], float out[4], float 
   out[3] = (float)dice;
 }
 
+// the four metrics of the loss sums `s`, and the per-label Dice behind them (smooth = 1, as dice_coefficient)
+static void model_metrics(fm_model* m, const double* s, float out[4]) {
+  metrics_from_sums(s, out, m->loss_kind ? m->xent_weight : 0.f);
+  m->label_dice[0] = out[3];
+  for (int l = 0; l < m->labels() && m->labels() > 1; ++l) {
+    const double* q = s + kNumLossSums + 3 * l;
+    m->label_dice[l] = (float)((2.0 * q[0] + 1.0) / (q[1] + q[2] + 1.0));
+  }
+}
+
 static int upload(fm_model* m, const float* src, float* dst, size_t count) {
   // pageable -> device through the runtime's own staging; callers that care pass pinned memory
   FM_CUDA(cudaMemcpyAsync(dst, src, count * sizeof(float), cudaMemcpyHostToDevice, m->ctx->stream));
@@ -1315,14 +1380,15 @@ static int upload(fm_model* m, const float* src, float* dst, size_t count) {
 // Layer table in Keras creation order, every conv followed by its norm pseudo-layer (gamma, beta).
 // ---------------------------------------------------------------------------------------------
 struct IsenseeBuild {
-  int X, Y, Z, in_channels, depth, n_base_filters, n_segmentation_levels, kcode;
+  int X, Y, Z, in_channels, depth, n_base_filters, n_segmentation_levels, kcode, n_labels;
 };
 static int build_isensee(fm_ctx* ctx, const IsenseeBuild* spec, fm_model** out);
 
 extern "C" int fm_model_create_isensee3d(fm_ctx* ctx, const fm_isensee3d_spec* spec, fm_model** out) {
   FM_CHECK(ctx && spec && out, FM_EINVAL, "fm_model_create_isensee3d: NULL argument");
-  FM_CHECK(spec->in_channels == 1 && spec->n_labels == 1, FM_EINVAL, "isensee: in_channels and n_labels must be 1");
-  IsenseeBuild b{spec->X, spec->Y, spec->Z, 1, spec->depth, spec->n_base_filters, spec->n_segmentation_levels, 3};
+  FM_CHECK(spec->in_channels == 1, FM_EINVAL, "isensee: in_channels must be 1");
+  IsenseeBuild b{spec->X, spec->Y, spec->Z, 1, spec->depth, spec->n_base_filters, spec->n_segmentation_levels, 3,
+                 spec->n_labels};
   return build_isensee(ctx, &b, out);
 }
 
@@ -1331,11 +1397,10 @@ extern "C" int fm_model_create_isensee3d(fm_ctx* ctx, const fm_isensee3d_spec* s
 // code 31 and no pooling along z, like the 2D U-Net. The input's `in_channels` slices are zero-padded to 16 channels.
 extern "C" int fm_model_create_isensee2d(fm_ctx* ctx, const fm_isensee2d_spec* spec, fm_model** out) {
   FM_CHECK(ctx && spec && out, FM_EINVAL, "fm_model_create_isensee2d: NULL argument");
-  FM_CHECK(spec->n_labels == 1, FM_EINVAL, "isensee2d: n_labels must be 1");
   FM_CHECK(spec->in_channels >= 1 && spec->in_channels <= 16, FM_EINVAL, "isensee2d: in_channels %d outside [1,16]",
            spec->in_channels);
   IsenseeBuild b{spec->H, spec->W, 1, spec->in_channels, spec->depth, spec->n_base_filters,
-                 spec->n_segmentation_levels, 31};
+                 spec->n_segmentation_levels, 31, spec->n_labels};
   return build_isensee(ctx, &b, out);
 }
 
@@ -1345,6 +1410,8 @@ static int build_isensee(fm_ctx* ctx, const IsenseeBuild* spec, fm_model** out) 
   FM_CHECK(spec->n_base_filters == 16 || spec->n_base_filters == 32, FM_EINVAL, "isensee: n_base_filters 16 or 32");
   FM_CHECK(spec->n_segmentation_levels >= 1 && spec->n_segmentation_levels <= spec->depth - 1, FM_EINVAL,
            "isensee: n_segmentation_levels %d out of range", spec->n_segmentation_levels);
+  FM_CHECK(spec->n_labels >= 1 && spec->n_labels <= kMaxLabels, FM_EINVAL, "isensee: n_labels=%d: 1 .. %d are built",
+           spec->n_labels, kMaxLabels);
   const int div = 1 << (spec->depth - 1);
   FM_CHECK(spec->X % div == 0 && spec->Y % div == 0 && (pz == 1 || spec->Z % div == 0) && spec->X > 0, FM_EINVAL,
            "isensee: input extent %dx%dx%d must be divisible by 2^(depth-1)=%d", spec->X, spec->Y, spec->Z, div);
@@ -1362,7 +1429,7 @@ static int build_isensee(fm_ctx* ctx, const IsenseeBuild* spec, fm_model** out) 
   m->spec.Z = spec->Z;
   m->spec.depth = spec->depth;
   m->spec.n_base_filters = spec->n_base_filters;
-  m->spec.n_labels = 1;
+  m->spec.n_labels = spec->n_labels;
   const int D = spec->depth, nf = spec->n_base_filters;
   std::vector<Layer>& ls = m->layers;
   // 2D: the first conv reads a 16-channel zero-padded bf16 copy of the input (tensor-core K granule)
@@ -1380,7 +1447,7 @@ static int build_isensee(fm_ctx* ctx, const IsenseeBuild* spec, fm_model** out) 
     add_layer(ls, "u%d_loc1", l, f, f, f, kcode, l, 1, 1);  // concat order [skip, up] (isensee2017.py:62)
     add_layer(ls, "u%d_loc2", l, f, 0, f, 1, l, 1, 1);
     c = f;
-    if (l < m->nseg) add_layer(ls, "u%d_seg", l, f, 0, 1, 1, l);
+    if (l < m->nseg) add_layer(ls, "u%d_seg", l, f, 0, spec->n_labels, 1, l);
   }
   if (kcode == 31) ls[0].cin_real = spec->in_channels;
   for (auto* v : {&m->gIsA, &m->gIsB, &m->gIsC, &m->gIsUp, &m->isIn, &m->isC1, &m->isSum, &m->isUp, &m->isU,
@@ -1397,13 +1464,13 @@ static int ensure_capacity_isensee(fm_model* m, int B, bool train) {
   const int D = m->depth(), nf = m->spec.n_base_filters;
   const size_t v0 = (size_t)m->vox(0);
   if (train || m->train_alloc) {
-    FM_TRY(m->t_in.ensure((size_t)B * v0));
-    FM_TRY(m->dz.ensure((size_t)B * v0));
+    FM_TRY(m->t_in.ensure((size_t)B * v0 * m->labels()));
+    FM_TRY(m->dz.ensure((size_t)B * v0 * m->labels()));
     FM_TRY(m->normGRaw.ensure((size_t)B * v0 * nf));
     FM_TRY(m->gIsZero.ensure((size_t)B * v0 * nf * 2));
     for (size_t i = 0; i < m->layers.size(); ++i) {
       const Layer& l = m->layers[i];
-      if (l.is_norm || (l.k == 1 && l.cout == 1)) continue;
+      if (l.is_norm || (l.k == 1 && l.cout == m->labels())) continue;  // heads
       FM_TRY(m->normRawL[i].ensure((size_t)B * m->vox(l.level) * l.cout));
       FM_TRY(m->normStatsL[i].ensure((size_t)B * l.cout * 2));
     }
@@ -1414,14 +1481,14 @@ static int ensure_capacity_isensee(fm_model* m, int B, bool train) {
       FM_TRY(m->gIsC[l].ensure(n));
       FM_TRY(m->isDropL[l].ensure((size_t)B * (nf << l)));
       if (l < D - 1) FM_TRY(m->gIsUp[l].ensure(2 * n));
-      if (l >= 1 && l < m->nseg) FM_TRY(m->gSeg[l].ensure((size_t)B * m->vox(l)));
+      if (l >= 1 && l < m->nseg) FM_TRY(m->gSeg[l].ensure((size_t)B * m->vox(l) * m->labels()));
     }
     m->train_alloc = true;
   }
   FM_TRY(m->x_in.ensure((size_t)B * v0 * m->cin_real));
   if (m->kcode == 31) FM_TRY(m->x_pad.ensure((size_t)B * v0 * 16));
-  FM_TRY(m->prob.ensure((size_t)B * v0));
-  FM_TRY(m->isAcc.ensure((size_t)B * v0));
+  FM_TRY(m->prob.ensure((size_t)B * v0 * m->labels()));
+  FM_TRY(m->isAcc.ensure((size_t)B * v0 * m->labels()));
   FM_TRY(m->normRaw.ensure((size_t)B * v0 * nf));
   FM_TRY(m->normScratch.ensure((size_t)B * (nf << (D - 1)) * 2 * 1028));
   for (int l = 0; l < D; ++l) {
@@ -1434,7 +1501,7 @@ static int ensure_capacity_isensee(fm_model* m, int B, bool train) {
       FM_TRY(m->isU[l].ensure(n));
       FM_TRY(m->isLoc1[l].ensure(n));
       FM_TRY(m->isLoc2[l].ensure(n));
-      if (l < m->nseg) FM_TRY(m->isSeg[l].ensure((size_t)B * m->vox(l)));
+      if (l < m->nseg) FM_TRY(m->isSeg[l].ensure((size_t)B * m->vox(l) * m->labels()));
     }
   }
   m->cap = B;
@@ -1488,7 +1555,7 @@ static int forward_isensee(fm_model* m, int B) {
     if (l < m->nseg) {
       const Layer& ls = L(m, "u%d_seg", l);
       FM_TRY(k_head_fwd(ctx, m->isLoc2[l].p, m->params + ls.w_off, m->params + ls.b_off, m->isSeg[l].p,
-                        (int64_t)B * m->vox(l), ls.c1, 0));
+                        (int64_t)B * m->vox(l), ls.c1, 0, m->labels()));
     }
   }
   // deep-supervision sum, coarse to fine (isensee2017.py:68-77), then sigmoid (:79)
@@ -1496,10 +1563,10 @@ static int forward_isensee(fm_model* m, int B) {
   for (int l = m->nseg - 2; l >= 0; --l) {
     const Dims5 d = m->dims(l, 1, B);
     float* dst = (l == 0) ? m->isAcc.p : m->isSeg[l].p;  // in place on the finer map is safe (element-wise)
-    FM_TRY(k_seg_upsample_add(ctx, m->isSeg[l].p, acc, dst, B, d.X, d.Y, d.Z, m->pz));
+    FM_TRY(k_seg_upsample_add(ctx, m->isSeg[l].p, acc, dst, B, d.X, d.Y, d.Z, m->pz, m->labels()));
     acc = dst;
   }
-  FM_TRY(k_sigmoid(ctx, acc, m->prob.p, (int64_t)B * m->vox(0)));
+  FM_TRY(k_sigmoid(ctx, acc, m->prob.p, (int64_t)B * m->vox(0) * m->labels()));
   return FM_OK;
 }
 
@@ -1529,12 +1596,12 @@ static int backward_isensee(fm_model* m, int B) {
   const bf16* g = m->normGRaw.p;
   FM_TRY(k_zero(ctx, m->grads, (size_t)m->nparams * sizeof(float)));
   // d(loss)/d(summed logits); the deep-supervision sum hands the same gradient, 2^3 sum-pooled, to every head
-  FM_TRY(k_dice_bwd(ctx, m->prob.p, m->t_in.p, m->sums, n0, m->dz.p, 1, m->xent()));
+  FM_TRY(k_dice_bwd(ctx, m->prob.p, m->t_in.p, m->sums, n0 * m->labels(), m->dz.p, 1, m->xent()));
   std::vector<const float*> gseg(D, nullptr);
   gseg[0] = m->dz.p;
   for (int l = 1; l < m->nseg; ++l) {
     const Dims5 d = m->dims(l, 1, B);
-    FM_TRY(k_sumpool_f32(ctx, gseg[l - 1], m->gSeg[l].p, B, d.X, d.Y, d.Z, m->pz));
+    FM_TRY(k_sumpool_f32(ctx, gseg[l - 1], m->gSeg[l].p, B, d.X, d.Y, d.Z, m->pz, m->labels()));
     gseg[l] = m->gSeg[l].p;
   }
   for (int l = 0; l <= D - 2; ++l) {
@@ -1543,7 +1610,8 @@ static int backward_isensee(fm_model* m, int B) {
     if (l < m->nseg) {
       const Layer& ls = L(m, "u%d_seg", l);
       FM_TRY(k_head_bwd(ctx, m->isLoc2[l].p, gseg[l], m->params + ls.w_off, m->gIsA[l].p, m->grads + ls.w_off,
-                        m->grads + ls.b_off, (int64_t)B * m->vox(l), ls.c1, l > 0 ? 2 : 1));
+                        m->grads + ls.b_off, (int64_t)B * m->vox(l), ls.c1, l > 0 ? 2 : 1, nullptr, nullptr, XentSpec(),
+                        m->labels()));
       FM_TRY(mark_layer_done(m, ls));
     }
     FM_TRY(is_block_bwd(m, ll2, m->gIsA[l].p, nullptr, nullptr, B));
@@ -1603,9 +1671,8 @@ extern "C" int fm_predict_device(fm_model* m, uint64_t x_dev, int batch, uint64_
   FM_CUDA(cudaMemcpyAsync(m->x_in.p, (const void*)(uintptr_t)x_dev, n * m->cin_real * 4, cudaMemcpyDeviceToDevice,
                           m->ctx->stream));
   FM_TRY(forward(m, batch));
-  if (y_dev)
-    FM_CUDA(cudaMemcpyAsync((void*)(uintptr_t)y_dev, m->prob.p, n * 4, cudaMemcpyDeviceToDevice,
-                            m->ctx->stream));
+  const float* y = nullptr;
+  if (y_dev) FM_TRY(output_view(m, batch, (float*)(uintptr_t)y_dev, &y));
   m->fwd_valid = false;
   return FM_OK;
 }
@@ -1617,7 +1684,9 @@ extern "C" int fm_predict(fm_model* m, const float* x, int batch, float* y) {
   const size_t n = (size_t)batch * m->vox(0);
   FM_TRY(upload(m, x, m->x_in.p, n * m->cin_real));
   FM_TRY(forward(m, batch));
-  FM_CUDA(cudaMemcpyAsync(y, m->prob.p, n * 4, cudaMemcpyDeviceToHost, m->ctx->stream));
+  const float* p = nullptr;
+  FM_TRY(output_view(m, batch, nullptr, &p));
+  FM_CUDA(cudaMemcpyAsync(y, p, n * m->labels() * 4, cudaMemcpyDeviceToHost, m->ctx->stream));
   FM_CUDA(cudaStreamSynchronize(m->ctx->stream));
   m->fwd_valid = false;
   return FM_OK;
@@ -1846,6 +1915,9 @@ static int patchwise_impl(fm_model* m, const float* vol, const int32_t vol_dims[
   }
   FM_CHECK(shard_count >= 1 && shard_rank >= 0 && shard_rank < shard_count, FM_EINVAL,
            "fm_patchwise_predict: shard %d of %d", shard_rank, shard_count);
+  FM_CHECK(!pp || m->labels() == 1, FM_EINVAL,
+           "fm_patchwise_segment: post-processing is defined on one probability map, the model has %d labels",
+           m->labels());
   fm_ctx* ctx = m->ctx;
   FM_CUDA(cudaSetDevice(ctx->device));
   const bool is2d = m->kcode == 31;
@@ -1860,15 +1932,18 @@ static int patchwise_impl(fm_model* m, const float* vol, const int32_t vol_dims[
            prev_truth_index + prev_truth_size, nslices);
   int32_t patch[3], pred[3], out_dims[3];
   FM_TRY(pw_extents(m, nslices, vol_dims, halo_pad, fit_pad, patch, pred, out_dims));
+  // the map is [x][y][z][label] (label fastest, as the network's output): `nout` and `pv` count values, the int16
+  // counts are one per voxel
+  const int L = m->labels();
   const size_t nv = (size_t)vol_dims[0] * vol_dims[1] * vol_dims[2];
-  const size_t nout = (size_t)out_dims[0] * out_dims[1] * out_dims[2];
-  const size_t pv = (size_t)pred[0] * pred[1] * pred[2];  // predicted voxels per patch
+  const size_t nvox_out = (size_t)out_dims[0] * out_dims[1] * out_dims[2], nout = nvox_out * L;
+  const size_t pv = (size_t)pred[0] * pred[1] * pred[2] * L;  // predicted values per patch
   const int64_t lo = n * shard_rank / shard_count, hi = n * (shard_rank + 1) / shard_count;
   const int64_t nloc = hi - lo;
   batch = (int)std::min<int64_t>(batch, std::max<int64_t>(nloc, 1));
   // the reassembly plan also validates the corner list (x-major Cartesian product, every voxel covered)
   ReasmPlan* plan = nullptr;
-  FM_TRY(k_reassemble_prepare(ctx, idx, n, pred, 1, out_dims, &plan));
+  FM_TRY(k_reassemble_prepare(ctx, idx, n, pred, L, out_dims, &plan));
   struct PlanGuard {
     ReasmPlan* p;
     ~PlanGuard() { k_reassemble_release(p); }
@@ -1891,7 +1966,7 @@ static int patchwise_impl(fm_model* m, const float* vol, const int32_t vol_dims[
   FM_TRY(dpred.ensure(std::max<size_t>(1, (size_t)nloc) * pv));
   FM_TRY(didx.ensure((size_t)n * 3));
   FM_TRY(dout.ensure(nout));
-  FM_TRY(dcnt.ensure(nout));
+  FM_TRY(dcnt.ensure(nvox_out));
   const bool trace = getenv("FETAL_B200_TRACE") != nullptr;
   auto now = [] { return std::chrono::steady_clock::now(); };
   auto t_start = now();
@@ -1905,7 +1980,7 @@ static int patchwise_impl(fm_model* m, const float* vol, const int32_t vol_dims[
   // host <-> device through the context's pinned staging buffer (pageable cudaMemcpy runs at a fraction of PCIe):
   // [volume | truth | float64 result | int16 counts | post-processing stats + mask]
   const size_t in_bytes = (nv * sizeof(float) * (truth ? 2 : 1) + 4095) & ~(size_t)4095;
-  const size_t out_bytes = pp && !out ? 0 : nout * sizeof(double), cnt_bytes = out_count ? nout * sizeof(int16_t) : 0;
+  const size_t out_bytes = pp && !out ? 0 : nout * sizeof(double), cnt_bytes = out_count ? nvox_out * sizeof(int16_t) : 0;
   const size_t cnt_off = in_bytes + ((out_bytes + 4095) & ~(size_t)4095);
   const size_t pp_off = cnt_off + ((cnt_bytes + 4095) & ~(size_t)4095);
   void* pin = nullptr;
@@ -1952,7 +2027,7 @@ static int patchwise_impl(fm_model* m, const float* vol, const int32_t vol_dims[
   };
   std::vector<Slab> slabs;
   size_t unstaged = 0;
-  const size_t plane = (size_t)out_dims[1] * out_dims[2];
+  const size_t plane = (size_t)out_dims[1] * out_dims[2];  // voxels of one output row
   const bool stream_out = want_out && shard_count == 1;  // slab-wise D2H only when no cross-rank reduce follows
   // a page-locked result (fm_host_alloc, what fetal_net.prediction hands in) receives the slabs directly: no staging
   // copy, no first-touch page faults of a fresh 33 MB array
@@ -1972,7 +2047,7 @@ static int patchwise_impl(fm_model* m, const float* vol, const int32_t vol_dims[
       }
       const size_t o = (size_t)sl.x0 * plane, c = (size_t)sl.rows * plane;
       if (!out_pinned) {
-        host_copy(out + o, pin_out + o * 8, c * 8);
+        host_copy(out + o * L, pin_out + o * L * 8, c * L * 8);
         if (out_count) host_copy(out_count + o, pin_cnt + o * 2, c * 2);
       }
       ++unstaged;
@@ -2002,7 +2077,7 @@ static int patchwise_impl(fm_model* m, const float* vol, const int32_t vol_dims[
         const size_t o = (size_t)x_done * plane, c = (size_t)(x_final - x_done) * plane;
         FM_CUDA(cudaEventRecord(ev_rows, ctx->stream));
         FM_CUDA(cudaStreamWaitEvent(ctx->d2h_stream, ev_rows, 0));
-        FM_CUDA(cudaMemcpyAsync(pin_out + o * 8, dout.p + o, c * 8, cudaMemcpyDeviceToHost, ctx->d2h_stream));
+        FM_CUDA(cudaMemcpyAsync(pin_out + o * L * 8, dout.p + o * L, c * L * 8, cudaMemcpyDeviceToHost, ctx->d2h_stream));
         if (out_count)
           FM_CUDA(cudaMemcpyAsync(pin_cnt + o * 2, dcnt.p + o, c * 2, cudaMemcpyDeviceToHost, ctx->d2h_stream));
         cudaEvent_t done = m->pw_events[2 + slabs.size() % (size_t)ngroups];
@@ -2036,7 +2111,7 @@ static int patchwise_impl(fm_model* m, const float* vol, const int32_t vol_dims[
   }
   if (reduce_root >= 0 && shard_count > 1) {
     FM_TRY(comm_reduce(ctx, dout.p, nout, 1, reduce_root, ctx->stream));
-    if (want_out) FM_TRY(k_divide_by_count(ctx, dout.p, dcnt.p, (int64_t)nout, 1));
+    if (want_out) FM_TRY(k_divide_by_count(ctx, dout.p, dcnt.p, (int64_t)nvox_out, L));
   }
   FM_CUDA(cudaStreamSynchronize(ctx->stream));
   lap("reduce");
@@ -2108,6 +2183,9 @@ extern "C" int fm_patchwise_predict_flips(fm_model* m, const float* vol, const i
   FM_CHECK(m && vol && vol_dims && halo_pad && fit_pad && pad_value && idx && in_flip && out_flip && n > 0 && batch > 0,
            FM_EINVAL, "fm_patchwise_predict_flips: bad argument");
   FM_CHECK(passes >= 1 && passes <= 8, FM_EINVAL, "fm_patchwise_predict_flips: %d passes (1 .. 8)", passes);
+  FM_CHECK(m->labels() == 1, FM_EINVAL,
+           "fm_patchwise_predict_flips: the median and post-processing are defined on one map, the model has %d labels",
+           m->labels());
   for (int k = 0; k < passes; ++k)
     FM_CHECK(in_flip[k] >= 0 && in_flip[k] <= 7 && out_flip[k] >= 0 && out_flip[k] <= 7, FM_EINVAL,
              "fm_patchwise_predict_flips: pass %d has flip masks %d / %d (0 .. 7)", k, in_flip[k], out_flip[k]);
@@ -2261,13 +2339,14 @@ static int train_forward_dev(fm_model* m, int batch, const float* t_host = nullp
   m->targets_ready = false;
   FM_TRY(rf);
   if (t_host) {
-    FM_CUDA(cudaMemcpyAsync(m->t_in.p, t_host, (size_t)batch * m->vox(0) * sizeof(float), cudaMemcpyHostToDevice,
-                            ctx->copy_stream));
+    FM_CUDA(cudaMemcpyAsync(m->t_in.p, t_host, (size_t)batch * m->vox(0) * m->labels() * sizeof(float),
+                            cudaMemcpyHostToDevice, ctx->copy_stream));
     FM_CUDA(cudaEventRecord(ctx->copy_done, ctx->copy_stream));
     FM_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->copy_done, 0));
   }
   if (!m->stats_done)
-    FM_TRY(k_dice_sums(m->ctx, m->prob.p, m->t_in.p, (int64_t)batch * m->vox(0), m->sums, 0, m->xent()));
+    FM_TRY(k_dice_sums(m->ctx, m->prob.p, m->t_in.p, (int64_t)batch * m->vox(0) * m->labels(), m->sums, 0, m->xent(),
+                       m->labels()));
   m->stats_done = false;
   m->last_batch = batch;
   m->fwd_valid = true;
@@ -2304,9 +2383,9 @@ static int stage_inputs(fm_model* m, const float* x, const float* t, int batch) 
       FM_CUDA(cudaEventCreateWithFlags(&m->stage_free[b], cudaEventDisableTiming));
     }
     FM_CUDA(cudaEventCreateWithFlags(&m->sums_ready, cudaEventDisableTiming));
-    FM_CUDA(cudaMallocHost((void**)&m->sums_pin, kNumLossSums * sizeof(double)));
+    FM_CUDA(cudaMallocHost((void**)&m->sums_pin, m->nsums() * sizeof(double)));
   }
-  const size_t n = (size_t)batch * m->vox(0), nx = n * m->cin_real;
+  const size_t nx = (size_t)batch * m->vox(0) * m->cin_real, n = (size_t)batch * m->vox(0) * m->labels();
   const int b = (m->stage_idx ^= 1);
   FM_TRY(m->stage_x[b].ensure(nx));
   FM_TRY(m->stage_t[b].ensure(n));
@@ -2337,7 +2416,7 @@ static int stage_inputs(fm_model* m, const float* x, const float* t, int batch) 
   if (pageable) FM_CUDA(cudaEventRecord(m->host_stage_done[b], ctx->copy_stream));
   FM_CUDA(cudaStreamWaitEvent(ctx->stream, m->stage_ready[b], 0));
   FM_CUDA(cudaMemcpyAsync(m->x_in.p, m->stage_x[b].p, nx * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
-  FM_CUDA(cudaMemcpyAsync(m->t_in.p, m->stage_t[b].p, n * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
+  FM_TRY(upload_labels(m, m->stage_t[b].p, true, m->t_in.p, batch));
   FM_CUDA(cudaEventRecord(m->stage_free[b], ctx->stream));
   return FM_OK;
 }
@@ -2352,6 +2431,10 @@ extern "C" int fm_train_forward(fm_model* m, const float* x, const float* t, int
     return train_forward_dev(m, batch);
   }
   FM_TRY(upload(m, x, m->x_in.p, n * m->cin_real));
+  if (m->label_transpose()) {  // the targets go through the transpose before the forward pass
+    FM_TRY(upload_labels(m, t, false, m->t_in.p, batch));
+    return train_forward_dev(m, batch);
+  }
   return train_forward_dev(m, batch, t);
 }
 
@@ -2368,9 +2451,9 @@ extern "C" int fm_train_metrics_async(fm_model* m) {
       FM_CUDA(cudaEventCreateWithFlags(&m->stage_free[b], cudaEventDisableTiming));
     }
     FM_CUDA(cudaEventCreateWithFlags(&m->sums_ready, cudaEventDisableTiming));
-    FM_CUDA(cudaMallocHost((void**)&m->sums_pin, kNumLossSums * sizeof(double)));
+    FM_CUDA(cudaMallocHost((void**)&m->sums_pin, m->nsums() * sizeof(double)));
   }
-  FM_CUDA(cudaMemcpyAsync(m->sums_pin, m->sums, kNumLossSums * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+  FM_CUDA(cudaMemcpyAsync(m->sums_pin, m->sums, m->nsums() * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
   FM_CUDA(cudaEventRecord(m->sums_ready, ctx->stream));
   m->metrics_pending = true;
   return FM_OK;
@@ -2380,7 +2463,7 @@ extern "C" int fm_train_metrics_wait(fm_model* m, float out_metrics[4]) {
   FM_CHECK(m->metrics_pending, FM_ESTATE, "fm_train_metrics_wait without fm_train_metrics_async");
   FM_CUDA(cudaSetDevice(m->ctx->device));
   FM_CUDA(cudaEventSynchronize(m->sums_ready));
-  metrics_from_sums(m->sums_pin, out_metrics, m->loss_kind ? m->xent_weight : 0.f);
+  model_metrics(m, m->sums_pin, out_metrics);
   m->metrics_pending = false;
   return FM_OK;
 }
@@ -2410,9 +2493,9 @@ extern "C" int fm_train_apply(fm_model* m, float lr, uint64_t after_stream, floa
   m->packs_dirty = true;
   FM_TRY(refresh_packs(m));
   if (out_metrics) {
-    FM_CUDA(cudaMemcpyAsync(m->sums_host, m->sums, kNumLossSums * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    FM_CUDA(cudaMemcpyAsync(m->sums_host, m->sums, m->nsums() * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
     FM_CUDA(cudaStreamSynchronize(ctx->stream));
-    metrics_from_sums(m->sums_host, out_metrics, m->loss_kind ? m->xent_weight : 0.f);
+    model_metrics(m, m->sums_host, out_metrics);
   }
   return FM_OK;
 }
@@ -2420,6 +2503,12 @@ extern "C" int fm_train_apply(fm_model* m, float lr, uint64_t after_stream, floa
 extern "C" int fm_model_loss_sums(fm_model* m, uint64_t* dev_ptr) {
   FM_CHECK(m && dev_ptr, FM_EINVAL, "NULL argument");
   *dev_ptr = (uint64_t)(uintptr_t)m->sums;
+  return FM_OK;
+}
+extern "C" int fm_model_label_dice(fm_model* m, float* out, int n) {
+  FM_CHECK(m && out, FM_EINVAL, "fm_model_label_dice: NULL argument");
+  FM_CHECK(n == m->labels(), FM_EINVAL, "fm_model_label_dice: n = %d, the model has %d labels", n, m->labels());
+  memcpy(out, m->label_dice, (size_t)n * sizeof(float));
   return FM_OK;
 }
 extern "C" int fm_model_grad_buffer(fm_model* m, uint64_t* dev_ptr, int64_t* n) {
@@ -2454,8 +2543,7 @@ extern "C" int fm_train_step_device(fm_model* m, uint64_t x_dev, uint64_t t_dev,
   const size_t n = (size_t)batch * m->vox(0);
   FM_CUDA(cudaMemcpyAsync(m->x_in.p, (const void*)(uintptr_t)x_dev, n * m->cin_real * 4, cudaMemcpyDeviceToDevice,
                           m->ctx->stream));
-  FM_CUDA(cudaMemcpyAsync(m->t_in.p, (const void*)(uintptr_t)t_dev, n * 4, cudaMemcpyDeviceToDevice,
-                          m->ctx->stream));
+  FM_TRY(upload_labels(m, (const float*)(uintptr_t)t_dev, true, m->t_in.p, batch));
   FM_TRY(train_forward_dev(m, batch));
   FM_TRY(fm_train_backward(m));
   return fm_train_apply(m, lr, 0, out_metrics);
@@ -2474,12 +2562,12 @@ extern "C" int fm_train_step(fm_model* m, const float* x, const float* t, int ba
   FM_TRY(ensure_capacity(m, batch, true));
   FM_TRY(stage_inputs(m, x, t, batch));
   FM_TRY(train_forward_dev(m, batch));
-  FM_CUDA(cudaMemcpyAsync(m->sums_pin, m->sums, kNumLossSums * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+  FM_CUDA(cudaMemcpyAsync(m->sums_pin, m->sums, m->nsums() * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
   FM_CUDA(cudaEventRecord(m->sums_ready, ctx->stream));
   FM_TRY(fm_train_backward(m));
   FM_TRY(fm_train_apply(m, lr, 0, nullptr));
   FM_CUDA(cudaEventSynchronize(m->sums_ready));  // the inputs were consumed long before: x / t may be reused
-  metrics_from_sums(m->sums_pin, out_metrics, m->loss_kind ? m->xent_weight : 0.f);
+  model_metrics(m, m->sums_pin, out_metrics);
   return FM_OK;
 }
 
@@ -2520,6 +2608,9 @@ extern "C" int fm_train_step_sampled_warp(fm_model* m, fm_volset* s, const int32
   FM_CUDA(cudaSetDevice(ctx->device));
   const bool is2d = m->kcode == 31;
   FM_CHECK(m->kind == 0 || !is2d, FM_EINVAL, "fm_train_step_sampled: unsupported model kind");
+  FM_CHECK(m->labels() == 1, FM_EINVAL,
+           "fm_train_step_sampled: the device sampler cuts one target channel; a model with %d labels trains through "
+           "fm_train_step with label-channel targets", m->labels());
   int32_t patch[3];
   if (is2d) {
     FM_CHECK(truth_size == 1 && prev_truth_size >= 0 && prev_truth_size < m->cin_real, FM_EINVAL,
@@ -2556,7 +2647,7 @@ extern "C" int fm_train_step_sampled_warp(fm_model* m, fm_volset* s, const int32
 static int dp_step_after_forward(fm_model* m, float lr, float out_metrics[4]) {
   fm_ctx* ctx = m->ctx;
   // 8 float64: the GLOBAL Dice statistics every rank back-propagates (64 bytes; latency only)
-  FM_TRY(comm_allreduce(ctx, m->sums, kNumLossSums, 1, ctx->stream));
+  FM_TRY(comm_allreduce(ctx, m->sums, m->nsums(), 1, ctx->stream));
   FM_TRY(fm_train_metrics_async(m));
   FM_TRY(fm_train_backward(m));
   // gradient buckets in completion order (backward runs in reverse creation order): each all-reduce waits only for
@@ -2628,15 +2719,15 @@ extern "C" int fm_evaluate(fm_model* m, const float* x, const float* t, int batc
   FM_TRY(ensure_capacity(m, batch, true));
   const size_t n = (size_t)batch * m->vox(0);
   FM_TRY(upload(m, x, m->x_in.p, n * m->cin_real));
-  FM_TRY(upload(m, t, m->t_in.p, n));
+  FM_TRY(upload_labels(m, t, false, m->t_in.p, batch));
   FM_CHECK(m->loss_kind != 2 || (m->mask_valid && m->mask_batch == batch), FM_ESTATE,
            "dice_and_xent_mask: call fm_model_set_weight_mask with this batch's weight mask before fm_evaluate");
   FM_TRY(forward(m, batch));  // inference kernels: same bits as fm_predict
-  FM_TRY(k_dice_sums(m->ctx, m->prob.p, m->t_in.p, (int64_t)n, m->sums, 0, m->xent()));
+  FM_TRY(k_dice_sums(m->ctx, m->prob.p, m->t_in.p, (int64_t)n * m->labels(), m->sums, 0, m->xent(), m->labels()));
   m->fwd_valid = false;
-  FM_CUDA(cudaMemcpyAsync(m->sums_host, m->sums, kNumLossSums * sizeof(double), cudaMemcpyDeviceToHost, m->ctx->stream));
+  FM_CUDA(cudaMemcpyAsync(m->sums_host, m->sums, m->nsums() * sizeof(double), cudaMemcpyDeviceToHost, m->ctx->stream));
   FM_CUDA(cudaStreamSynchronize(m->ctx->stream));
-  metrics_from_sums(m->sums_host, out_metrics, m->loss_kind ? m->xent_weight : 0.f);
+  model_metrics(m, m->sums_host, out_metrics);
   return FM_OK;
 }
 

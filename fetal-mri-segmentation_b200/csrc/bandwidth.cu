@@ -768,6 +768,49 @@ __global__ void seg_upsample_add_kernel(const float* __restrict__ fine, const fl
   const int64_t vc = (((int64_t)n * (X >> 1) + (x >> 1)) * (Y >> 1) + (y >> 1)) * Zc + zc;
   out[g] = fine[g] + __ldg(coarse + vc);
 }
+// the same two steps for L > 1 labels: maps [N][X][Y][Z][L] (label fastest); one thread per element, every label summed
+// with the arithmetic of the one-label kernels
+__global__ void seg_upsample_add_labels_kernel(const float* __restrict__ fine, const float* __restrict__ coarse,
+                                               float* __restrict__ out, int N, int X, int Y, int Z, int pz, int L) {
+  const int64_t total = (int64_t)N * X * Y * Z * L;
+  const int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (g >= total) return;
+  const int l = (int)(g % L);
+  int64_t r = g / L;
+  const int z = (int)(r % Z);
+  r /= Z;
+  const int y = (int)(r % Y);
+  r /= Y;
+  const int x = (int)(r % X);
+  const int n = (int)(r / X);
+  const int zc = pz == 2 ? (z >> 1) : z, Zc = pz == 2 ? (Z >> 1) : Z;
+  const int64_t vc = (((int64_t)n * (X >> 1) + (x >> 1)) * (Y >> 1) + (y >> 1)) * Zc + zc;
+  out[g] = fine[g] + __ldg(coarse + vc * L + l);
+}
+__global__ void sumpool_f32_labels_kernel(const float* __restrict__ fine, float* __restrict__ coarse, int N, int X,
+                                          int Y, int Z, int pz, int L) {  // coarse extents
+  const int64_t total = (int64_t)N * X * Y * Z * L;
+  const int64_t gi = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (gi >= total) return;
+  const int l = (int)(gi % L);
+  int64_t r = gi / L;
+  const int z = (int)(r % Z);
+  r /= Z;
+  const int y = (int)(r % Y);
+  r /= Y;
+  const int x = (int)(r % X);
+  const int n = (int)(r / X);
+  float acc = 0.f;
+#pragma unroll
+  for (int k = 0; k < 4; ++k) {
+    const int64_t vf = (((int64_t)n * 2 * X + 2 * x + (k >> 1)) * 2 * Y + 2 * y + (k & 1)) * pz * Z + pz * z;
+    if (pz == 2)
+      acc += __ldg(fine + vf * L + l) + __ldg(fine + (vf + 1) * L + l);
+    else
+      acc += __ldg(fine + vf * L + l);
+  }
+  coarse[gi] = acc;
+}
 __global__ void sigmoid_kernel(const float* __restrict__ z, float* __restrict__ p, int64_t n) {
   const int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (g < n) p[g] = 1.f / (1.f + __expf(-z[g]));
@@ -857,6 +900,78 @@ __global__ void __launch_bounds__(256) dice_final_kernel(const double* __restric
     sums[dst] = accumulate ? sums[dst] + s : s;
   } else if (threadIdx.x == 8) {
     sums[7] = accumulate ? sums[7] + n_elems : n_elems;
+  }
+}
+
+// Multi-label statistics (1 < L <= kMaxLabels, label of element i = i mod L): the 8 partials of dice_partial_kernel over
+// all elements, then (tp, t, p) per label; 8 + 3 L per block (write_label_partials).
+__global__ void __launch_bounds__(kThreads) dice_partial_labels_kernel(const float* __restrict__ p,
+                                                                       const float* __restrict__ t, int64_t n, int L,
+                                                                       double* __restrict__ part, XentSpec xs) {
+  FM_PDL_SYNC();
+  float s[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+  float sl[3 * kMaxLabels];
+#pragma unroll
+  for (int i = 0; i < 3 * kMaxLabels; ++i) sl[i] = 0.f;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const float pv = __ldg(p + i), tt = __ldg(t + i);
+    const float pb = pv > 0.5f ? 1.f : 0.f, tb = tt > 0.5f ? 1.f : 0.f;
+    s[0] += tt * pv;
+    s[1] += tt;
+    s[2] += pv;
+    s[3] += tb * pb;
+    s[4] += tb;
+    s[5] += pb;
+    s[6] += (tt == pb) ? 1.f : 0.f;
+    if (xs.weight != 0.f) s[7] += xent_voxel_weight(xs, i) * xent_term(tt, pv);
+    const int l = (int)(i % L);
+#pragma unroll
+    for (int k = 0; k < kMaxLabels; ++k)
+      if (k == l) {
+        sl[3 * k] += tt * pv;
+        sl[3 * k + 1] += tt;
+        sl[3 * k + 2] += pv;
+      }
+  }
+  write_label_partials<kThreads>(s, sl, L, part);
+}
+
+// fixed-order fold of nblocks rows of K = 8 + 3 L partials: 32 strided chains per statistic, then the chains in order.
+// Partial slot 7 (sum w * bce) -> sums[8], sums[7] = element count, slot 8 + j -> sums[kNumLossSums + j].
+__global__ void __launch_bounds__(1024) dice_final_labels_kernel(const double* __restrict__ part, int nblocks, int K,
+                                                                 double n_elems, double* __restrict__ sums) {
+  FM_PDL_SYNC();
+  __shared__ double sh[32][8 + 3 * kMaxLabels];
+  const int k = threadIdx.x & 31, j = threadIdx.x >> 5;
+  if (k < K) {
+    double a = 0.0;
+    for (int b = j; b < nblocks; b += 32) a += part[(int64_t)b * K + k];
+    sh[j][k] = a;
+  }
+  __syncthreads();
+  if ((int)threadIdx.x < K) {
+    double s = 0.0;
+    for (int g = 0; g < 32; ++g) s += sh[g][threadIdx.x];
+    sums[threadIdx.x < 7 ? threadIdx.x : threadIdx.x + 1] = s;
+  } else if ((int)threadIdx.x == K) {
+    sums[7] = n_elems;
+  }
+}
+
+// [B][L][V] -> [B][V][L] (to_device) or back; one thread per element of `out`
+__global__ void label_transpose_kernel(const float* __restrict__ in, float* __restrict__ out, int64_t V, int L,
+                                       int64_t total, int to_device) {
+  for (int64_t o = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; o < total; o += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t per = V * L, b = o / per, r = o - b * per;
+    int64_t v, l;
+    if (to_device) {
+      v = r / L;
+      l = r - v * L;
+    } else {
+      l = r / V;
+      v = r - l * V;
+    }
+    out[o] = __ldg(in + b * per + (to_device ? l * V + v : v * L + l));
   }
 }
 
@@ -1227,7 +1342,17 @@ int k_upsample3d_bwd(fm_ctx* ctx, const bf16* dy, const bf16* act, bf16* dx, Dim
   return FM_OK;
 }
 
-int k_dice_sums(fm_ctx* ctx, const float* p, const float* t, int64_t n, double* sums, int accumulate, XentSpec xs) {
+int k_dice_sums(fm_ctx* ctx, const float* p, const float* t, int64_t n, double* sums, int accumulate, XentSpec xs,
+                int L) {
+  if (L != 1) {
+    FM_CHECK(L >= 2 && L <= kMaxLabels && !accumulate && n % L == 0, FM_EINVAL,
+             "dice_sums: %d labels over %lld elements (accumulate %d)", L, (long long)n, accumulate);
+    ProfScope prof(ctx, "dice_sums_labels", 0.0, (double)n * (xs.mask ? 12.0 : 8.0));
+    FM_CUDA(launch_pdl(dice_partial_labels_kernel, dim3(kRedBlocks), dim3(kThreads), 0, ctx->stream, p, t, n, L,
+                       ctx->red_scratch, xs));
+    FM_LAUNCH_OK(ctx);
+    return k_dice_finalize_labels(ctx, kRedBlocks, (double)n, sums, L);
+  }
   ProfScope prof(ctx, "dice_sums", 0.0, (double)n * (xs.mask ? 12.0 : 8.0));
   FM_CUDA(launch_pdl(dice_partial_kernel, dim3(kRedBlocks), dim3(kThreads), 0, ctx->stream, p, t, n, ctx->red_scratch, xs));
   FM_LAUNCH_OK(ctx);
@@ -1239,6 +1364,19 @@ int k_dice_sums(fm_ctx* ctx, const float* p, const float* t, int64_t n, double* 
 // fixed-order fold of `nblocks` x 8 partial statistics in ctx->red_scratch (written by head_fwd_dice_kernel)
 int k_dice_finalize(fm_ctx* ctx, int nblocks, double n_elems, double* sums) {
   FM_CUDA(launch_pdl(dice_final_kernel, dim3(1), dim3(256), 0, ctx->stream, ctx->red_scratch, nblocks, n_elems, sums, 0));
+  FM_LAUNCH_OK(ctx);
+  return FM_OK;
+}
+int k_dice_finalize_labels(fm_ctx* ctx, int nblocks, double n_elems, double* sums, int L) {
+  FM_CUDA(launch_pdl(dice_final_labels_kernel, dim3(1), dim3(1024), 0, ctx->stream, ctx->red_scratch, nblocks, 8 + 3 * L,
+                     n_elems, sums));
+  FM_LAUNCH_OK(ctx);
+  return FM_OK;
+}
+int k_label_transpose(fm_ctx* ctx, const float* in, float* out, int B, int64_t V, int L, int to_device) {
+  const int64_t total = (int64_t)B * V * L;
+  ProfScope prof(ctx, "label_transpose", 0.0, (double)total * 8.0);
+  label_transpose_kernel<<<grid_for(total, 148 * 16), kThreads, 0, ctx->stream>>>(in, out, V, L, total, to_device);
   FM_LAUNCH_OK(ctx);
   return FM_OK;
 }
@@ -1507,7 +1645,14 @@ int k_add_bf16(fm_ctx* ctx, const bf16* a, const bf16* b, bf16* out, int64_t n) 
   return FM_OK;
 }
 
-int k_sumpool_f32(fm_ctx* ctx, const float* fine, float* coarse, int N, int X, int Y, int Z, int pz) {
+int k_sumpool_f32(fm_ctx* ctx, const float* fine, float* coarse, int N, int X, int Y, int Z, int pz, int L) {
+  if (L != 1) {
+    const int64_t total = (int64_t)N * X * Y * Z * L;
+    ProfScope prof(ctx, "sumpool_f32_labels", 0.0, (double)total * (4.0 + 16.0 * pz));
+    sumpool_f32_labels_kernel<<<grid_for(total), kThreads, 0, ctx->stream>>>(fine, coarse, N, X, Y, Z, pz, L);
+    FM_LAUNCH_OK(ctx);
+    return FM_OK;
+  }
   ProfScope prof(ctx, "sumpool_f32", 0.0, (double)N * X * Y * Z * (4.0 + 16.0 * pz));
   sumpool_f32_kernel<<<grid_for((int64_t)N * X * Y * Z), kThreads, 0, ctx->stream>>>(fine, coarse, N, X, Y, Z, pz);
   FM_LAUNCH_OK(ctx);
@@ -1840,7 +1985,13 @@ int k_batchnorm_relu_bwd(fm_ctx* ctx, const bf16* x, const float* stats, const f
 }
 
 int k_seg_upsample_add(fm_ctx* ctx, const float* fine, const float* coarse, float* out, int N, int X, int Y, int Z,
-                       int pz) {
+                       int pz, int L) {
+  if (L != 1) {
+    const int64_t total = (int64_t)N * X * Y * Z * L;
+    seg_upsample_add_labels_kernel<<<grid_for(total), kThreads, 0, ctx->stream>>>(fine, coarse, out, N, X, Y, Z, pz, L);
+    FM_LAUNCH_OK(ctx);
+    return FM_OK;
+  }
   const int64_t total = (int64_t)N * X * Y * Z;
   seg_upsample_add_kernel<<<grid_for(total), kThreads, 0, ctx->stream>>>(fine, coarse, out, N, X, Y, Z, pz);
   FM_LAUNCH_OK(ctx);

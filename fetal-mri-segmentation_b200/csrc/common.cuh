@@ -236,6 +236,9 @@ struct XentSpec {
   const float* mask = nullptr;
 };
 constexpr int kNumLossSums = 9;
+// Multi-label heads (n_labels = L > 1): probabilities, targets and weight masks are [voxel][label] (label fastest), and
+// the loss sums grow by 3 L per-label sums (tp, t, p) behind the kNumLossSums: sums[kNumLossSums + 3 l + {0, 1, 2}].
+constexpr int kMaxLabels = 8;
 constexpr int kRedScratchRows = 4096;  // rows of fm_ctx::red_scratch (one per block of the partial-sum kernels)
 #ifdef __CUDACC__
 // Keras K.binary_crossentropy on probabilities (TF backend): p is clipped to [1e-7, 1 - 1e-7] (fp32), turned back into
@@ -251,10 +254,37 @@ __device__ __forceinline__ float xent_grad(float t, float p) {
 __device__ __forceinline__ float xent_voxel_weight(const XentSpec& xs, int64_t i) {
   return xs.mask != nullptr ? __expf(-__ldg(xs.mask + i) * xs.inv_sigma) : 1.f;
 }
+// One block's partials of the multi-label loss statistics: the 8 of the one-label kernels (over all elements), then
+// (tp, t, p) of each of the L labels, written as 8 + 3 L doubles at part[blockIdx.x * (8 + 3 L)]. Warp shuffles, then a
+// fixed-order sum over the warps: deterministic. Every thread of the block must call it.
+template <int kBlock>
+__device__ __forceinline__ void write_label_partials(const float (&s)[8], const float (&sl)[3 * kMaxLabels], int L,
+                                                     double* __restrict__ part) {
+  constexpr int kMaxK = 8 + 3 * kMaxLabels;
+  __shared__ double shd[kBlock / 32][kMaxK];
+  const int K = 8 + 3 * L, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+#pragma unroll
+  for (int k = 0; k < kMaxK; ++k) {
+    if (k >= K) break;
+    double v = (double)(k < 8 ? s[k] : sl[k < 8 ? 0 : k - 8]);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    if (lane == 0) shd[warp][k] = v;
+  }
+  __syncthreads();
+  if ((int)threadIdx.x < K) {
+    double a = 0.0;
+    for (int wi = 0; wi < kBlock / 32; ++wi) a += shd[wi][threadIdx.x];
+    part[(int64_t)blockIdx.x * K + threadIdx.x] = a;
+  }
+}
 #endif
 // loss statistics over p,t (fp32): sums[9] (double) = {tp, t, p, tbpb, tb, pb, correct, count, sum w*bce}
+// With L > 1 (n = elements, label = index mod L) the 3 L per-label sums follow; `accumulate` must then be 0.
 int k_dice_sums(fm_ctx*, const float* p, const float* t, int64_t n, double* sums, int accumulate,
-                XentSpec xs = XentSpec());
+                XentSpec xs = XentSpec(), int L = 1);
+// [B][L][V] <-> [B][V][L] (channels-first host layout <-> the device's label-fastest layout); to_device selects the first
+int k_label_transpose(fm_ctx*, const float* in, float* out, int B, int64_t V, int L, int to_device);
 // dL/dz = dL/dp * p (1-p) with global sums (closed form, metrics.py:11-15) [+ weight/count * w * (p - t)]
 int k_dice_bwd(fm_ctx*, const float* p, const float* t, const double* sums, int64_t n, float* dz,
                int through_sigmoid, XentSpec xs = XentSpec());
@@ -293,7 +323,8 @@ int k_batchnorm_relu_bwd(fm_ctx*, const bf16* x, const float* stats, const float
                          float* scratch, size_t scratch_floats, const double* sums = nullptr);
 int k_zero_insert(fm_ctx*, const bf16* coarse, bf16* fine, Dims5 coarse_dims, int pz = 2);
 int k_add_bf16(fm_ctx*, const bf16* a, const bf16* b, bf16* out, int64_t n);
-int k_sumpool_f32(fm_ctx*, const float* fine, float* coarse, int N, int X, int Y, int Z, int pz = 2);
+// L > 1: maps [N][X][Y][Z][L], each label pooled / added on its own
+int k_sumpool_f32(fm_ctx*, const float* fine, float* coarse, int N, int X, int Y, int Z, int pz = 2, int L = 1);
 int k_dropout_scale(fm_ctx*, float* scale, int n, float rate, uint64_t seed);
 // Deconvolution3D/2D (kernel 2, stride 2) = a 1x1x1 conv to taps*C channels followed by a depth-to-space shuffle:
 // fine[n][2x+a][2y+b][pz*z+c][co] = z8[n][x][y][z][cls*C + co] + bias[co], cls = (a*2 + b)*pz + c. `coarse` = dims of z8
@@ -303,7 +334,7 @@ int k_space_to_depth(fm_ctx*, const bf16* fine, bf16* g8, Dims5 coarse, int pz);
 // x[n][v][c] *= scale[n][c] in place (SpatialDropout2D of the 2D U-Net, forward and backward)
 int k_channel_scale(fm_ctx*, bf16* x, const float* scale, int N, int64_t vox_per_sample, int C);
 int k_seg_upsample_add(fm_ctx*, const float* fine, const float* coarse, float* out, int N, int X, int Y, int Z,
-                       int pz = 2);
+                       int pz = 2, int L = 1);
 int k_sigmoid(fm_ctx*, const float* z, float* p, int64_t n);
 // out[(patch voxel (i,j)) * out_pitch + out_cofs + k]: with out_pitch = patch[2], out_cofs = 0 this is the plain
 // [n,P0,P1,P2] gather; the 2.5D path writes the slices and the previous-truth slices as channels of one row
@@ -362,18 +393,22 @@ int k_conv3d_simt_wgrad(fm_ctx*, const void* x, int x_is_f32, const bf16* dy, fl
                         int N, int X, int Y, int Z, int Cin, int Cin_total, int cin_ofs, int Cout,
                         int ksize);
 int k_bias_grad(fm_ctx*, const bf16* dy, float* db, int64_t voxels, int C);
-// 1x1x1 head: z = w.x + b ; p = sigmoid(z) (fp32 out)
+// 1x1x1 head: z = w.x + b ; p = sigmoid(z) (fp32 out). L outputs (w = [L][C], p = [voxel][L]): 1 <= L <= kMaxLabels;
+// the training form with L > 1 needs C in {16, 32, 64}; every label's map is bit-identical to a one-label head with that label's weights.
 int k_head_fwd(fm_ctx*, const bf16* x, const float* w, const float* b, float* p, int64_t voxels,
-               int C, int apply_sigmoid = 1);
+               int C, int apply_sigmoid = 1, int L = 1);
 // training forward: head + sigmoid + the 8 loss statistics of k_dice_sums in one pass over the activations
 int k_head_fwd_dice(fm_ctx*, const bf16* x, const float* w, const float* b, const float* t, float* p, int64_t voxels,
-                    int C, double* sums, XentSpec xs = XentSpec());
+                    int C, double* sums, XentSpec xs = XentSpec(), int L = 1);
 int k_dice_finalize(fm_ctx*, int nblocks, double n_elems, double* sums);
+// fixed-order fold of `nblocks` rows of 8 + 3 L partials in ctx->red_scratch into kNumLossSums + 3 L sums (L > 1)
+int k_dice_finalize_labels(fm_ctx*, int nblocks, double n_elems, double* sums, int L);
 // head backward: dx[v,c] = dz[v] * w[c] * (x[v,c] > 0); dw[c] = sum_v dz[v] x[v,c]; db = sum dz.
 // With `t` and `sums`: `dz` holds the probabilities and dL/dz of the soft-Dice loss is formed inside (fused dice_bwd)
+// L > 1 labels: dz / t are [voxel][L], dx[v,c] = sum_l g[v,l] w[l,c], dw[l,c] = sum_v g[v,l] x[v,c], db[l] = sum_v g[v,l]
 int k_head_bwd(fm_ctx*, const bf16* x, const float* dz, const float* w, bf16* dx, float* dw,
                float* db, int64_t voxels, int C, int mode = 0, const float* t = nullptr, const double* sums = nullptr,
-               XentSpec xs = XentSpec());
+               XentSpec xs = XentSpec(), int L = 1);
 // weight repack: master fp32 [Cout][taps][Cin] -> bf16 fprop pack (same layout) and bf16 dgrad
 // pack(s) [Cin_s][taps flipped][Cout] per source
 // all layers in ONE launch (after every Adam step): per layer the fprop pack, the dgrad pack(s) and, where the

@@ -491,6 +491,211 @@ __global__ void __launch_bounds__(kThreads) head_fwd_tpv_kernel(const bf16* __re
   }
 }
 
+// Multi-label form of head_fwd_tpv_kernel (1 < L <= kMaxLabels outputs per voxel, w = [L][C], p / t = [voxel][L]): the
+// voxel's C channels are read once, and label l accumulates them exactly as the one-label kernel does with w + l C and
+// b[l], so each label's map is bit-identical to a one-label head with that label's weights. The weights live in shared
+// memory; the label loops are unrolled to kMaxLabels behind a guard so the per-label sums stay in registers. The
+// training form writes 8 + 3 L partials per block (write_label_partials), folded by dice_final_labels_kernel.
+template <int C, bool DICE>
+__global__ void __launch_bounds__(kThreads) head_fwd_labels_kernel(const bf16* __restrict__ x, const float* __restrict__ w,
+                                                                   const float* __restrict__ b,
+                                                                   const float* __restrict__ t, float* __restrict__ p,
+                                                                   int64_t voxels, int L, int apply_sigmoid,
+                                                                   double* __restrict__ part, XentSpec xs) {
+  FM_PDL_SYNC();
+  __shared__ float wsh[kMaxLabels * C];
+  __shared__ float bsh[kMaxLabels];
+  for (int i = threadIdx.x; i < L * C; i += blockDim.x) wsh[i] = __ldg(w + i);
+  if ((int)threadIdx.x < L) bsh[threadIdx.x] = __ldg(b + threadIdx.x);
+  __syncthreads();
+  float s[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+  float sl[3 * kMaxLabels];
+#pragma unroll
+  for (int i = 0; i < 3 * kMaxLabels; ++i) sl[i] = 0.f;
+  for (int64_t v = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; v < voxels; v += (int64_t)gridDim.x * blockDim.x) {
+    uint4 r[C / 8];
+    const uint4* src = reinterpret_cast<const uint4*>(x + v * C);
+#pragma unroll
+    for (int j = 0; j < C / 8; ++j) r[j] = __ldg(src + j);
+#pragma unroll
+    for (int l = 0; l < kMaxLabels; ++l) {
+      if (l >= L) break;
+      const float* wl = wsh + l * C;
+      float acc = bsh[l];
+#pragma unroll
+      for (int j = 0; j < C / 8; ++j) {
+        const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&r[j]);
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+          const float2 f = __bfloat1622float2(h[i]);
+          acc += f.x * wl[j * 8 + 2 * i] + f.y * wl[j * 8 + 2 * i + 1];
+        }
+      }
+      const float pv = (DICE || apply_sigmoid) ? 1.f / (1.f + __expf(-acc)) : acc;
+      const int64_t e = v * L + l;
+      p[e] = pv;
+      if (DICE) {
+        const float tt = __ldg(t + e);
+        const float pb = pv > 0.5f ? 1.f : 0.f, tb = tt > 0.5f ? 1.f : 0.f;
+        s[0] += tt * pv;
+        s[1] += tt;
+        s[2] += pv;
+        s[3] += tb * pb;
+        s[4] += tb;
+        s[5] += pb;
+        s[6] += (tt == pb) ? 1.f : 0.f;
+        if (xs.weight != 0.f) s[7] += xent_voxel_weight(xs, e) * xent_term(tt, pv);
+        sl[3 * l] += tt * pv;
+        sl[3 * l + 1] += tt;
+        sl[3 * l + 2] += pv;
+      }
+    }
+  }
+  if (DICE) write_label_partials<kThreads>(s, sl, L, part);
+}
+
+// Multi-label inference form of head_fwd_kernel (C/8 lanes per voxel) for the channel counts the thread-per-voxel form
+// does not take (the Isensee heads of 128 or more channels): label l accumulates and shuffle-reduces exactly as the
+// one-label kernel does with w + l C and b[l].
+__global__ void __launch_bounds__(kThreads) head_fwd_labels_lpv_kernel(const bf16* __restrict__ x,
+                                                                       const float* __restrict__ w,
+                                                                       const float* __restrict__ b,
+                                                                       float* __restrict__ p, int64_t voxels, int C,
+                                                                       int L, int apply_sigmoid) {
+  FM_PDL_SYNC();
+  const int lpv = C >> 3;
+  const int sub = threadIdx.x % lpv;
+  const int64_t vpb = blockDim.x / lpv;
+  constexpr int U = 4;
+  for (int64_t base = (int64_t)blockIdx.x * vpb * U; base < voxels; base += (int64_t)gridDim.x * vpb * U) {
+    uint4 t[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      const int64_t v = base + u * vpb + threadIdx.x / lpv;
+      t[u] = v < voxels ? __ldg(reinterpret_cast<const uint4*>(x + v * C + sub * 8)) : make_uint4(0u, 0u, 0u, 0u);
+    }
+    for (int l = 0; l < L; ++l) {
+      float wv[8];
+#pragma unroll
+      for (int i = 0; i < 8; ++i) wv[i] = __ldg(w + l * C + sub * 8 + i);
+      const float bb = __ldg(b + l);
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        const int64_t v = base + u * vpb + threadIdx.x / lpv;
+        const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&t[u]);
+        float acc = 0.f;
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+          const float2 f = __bfloat1622float2(h[i]);
+          acc += f.x * wv[2 * i] + f.y * wv[2 * i + 1];
+        }
+        for (int s = lpv >> 1; s > 0; s >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, s);
+        if (sub == 0 && v < voxels) p[v * L + l] = apply_sigmoid ? 1.f / (1.f + __expf(-(acc + bb))) : acc + bb;
+      }
+    }
+  }
+}
+
+// Multi-label head backward (1 < L <= kMaxLabels, C a power of two in [8, 256]): C/8 lanes per voxel as in
+// head_bwd_kernel; g[l] is formed from p and t per label with the global sums, dx[c] = sum_l g[l] w[l][c] (labels in
+// ascending order), and each thread keeps dw / db partials for all labels of its 8 channels.
+__global__ void __launch_bounds__(kThreads) head_bwd_labels_kernel(const bf16* __restrict__ x,
+                                                                   const float* __restrict__ dz,
+                                                                   const float* __restrict__ w, bf16* __restrict__ dx,
+                                                                   float* __restrict__ dw, float* __restrict__ db,
+                                                                   int64_t voxels, int C, int L, int mode,
+                                                                   const float* __restrict__ pt,
+                                                                   const double* __restrict__ sums, XentSpec xs) {
+  FM_PDL_SYNC();
+  __shared__ float wsh[kMaxLabels * 256];
+  for (int i = threadIdx.x; i < L * C; i += blockDim.x) wsh[i] = __ldg(w + i);
+  float ga = 0.f, gbc = 0.f, xc = 0.f;
+  if (pt != nullptr) {
+    const double I = sums[0], S = sums[1] + sums[2] + 1.0;
+    ga = (float)(-2.0 / S);
+    gbc = (float)((2.0 * I + 1.0) / (S * S));
+    if (xs.weight != 0.f) xc = (float)((double)xs.weight / sums[7]);
+  }
+  const int lpv = C >> 3;
+  const int sub = threadIdx.x % lpv;
+  float gw[kMaxLabels][8], gb[kMaxLabels];
+#pragma unroll
+  for (int l = 0; l < kMaxLabels; ++l) {
+    gb[l] = 0.f;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) gw[l][i] = 0.f;
+  }
+  __syncthreads();
+  const int64_t vstride = (int64_t)gridDim.x * (blockDim.x / lpv);
+  for (int64_t v = (int64_t)blockIdx.x * (blockDim.x / lpv) + threadIdx.x / lpv; v < voxels; v += vstride) {
+    const uint4 xr = __ldg(reinterpret_cast<const uint4*>(x + v * C + sub * 8));
+    const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&xr);
+    float f[8], d[8];
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      const float2 q = __bfloat1622float2(h[i]);
+      f[2 * i] = q.x;
+      f[2 * i + 1] = q.y;
+    }
+#pragma unroll
+    for (int i = 0; i < 8; ++i) d[i] = 0.f;
+#pragma unroll
+    for (int l = 0; l < kMaxLabels; ++l) {
+      if (l >= L) break;
+      const int64_t e = v * L + l;
+      float g = __ldg(dz + e);
+      if (pt != nullptr) {
+        const float p0 = g, tv = __ldg(pt + e);
+        g = (ga * tv + gbc) * p0 * (1.f - p0);
+        if (xc != 0.f) g += xc * xent_voxel_weight(xs, e) * xent_grad(tv, p0);
+      }
+      const float* wl = wsh + l * C + sub * 8;
+#pragma unroll
+      for (int i = 0; i < 8; ++i) {
+        gw[l][i] += g * f[i];
+        d[i] += g * wl[i];
+      }
+      if (sub == 0) gb[l] += g;
+    }
+    uint4 o;
+    __nv_bfloat162* oh = reinterpret_cast<__nv_bfloat162*>(&o);
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+      oh[i] = __floats2bfloat162_rn(mode != 0 || f[2 * i] > 0.f ? d[2 * i] : 0.f,
+                                    mode != 0 || f[2 * i + 1] > 0.f ? d[2 * i + 1] : 0.f);
+    if (mode == 2) {
+      const uint4 prev = *reinterpret_cast<const uint4*>(dx + v * C + sub * 8);
+      const __nv_bfloat162* ph = reinterpret_cast<const __nv_bfloat162*>(&prev);
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        const float2 a = __bfloat1622float2(ph[i]), c = __bfloat1622float2(oh[i]);
+        oh[i] = __floats2bfloat162_rn(a.x + c.x, a.y + c.y);
+      }
+    }
+    *reinterpret_cast<uint4*>(dx + v * C + sub * 8) = o;
+  }
+  // block reduction, one label at a time: threads with equal `sub` hold partial sums of the same 8 channels
+  __shared__ float sh[kThreads][9];
+#pragma unroll
+  for (int l = 0; l < kMaxLabels; ++l) {
+    if (l >= L) break;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) sh[threadIdx.x][i] = gw[l][i];
+    sh[threadIdx.x][8] = gb[l];
+    __syncthreads();
+    if ((int)threadIdx.x < lpv) {
+      float a[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+      for (int tt = threadIdx.x; tt < kThreads; tt += lpv)
+#pragma unroll
+        for (int i = 0; i < 9; ++i) a[i] += sh[tt][i];
+#pragma unroll
+      for (int i = 0; i < 8; ++i) atomicAdd(dw + l * C + threadIdx.x * 8 + i, a[i]);
+      if (threadIdx.x == 0) atomicAdd(db + l, a[8]);
+    }
+    __syncthreads();
+  }
+}
+
 __global__ void __launch_bounds__(kThreads) head_bwd_kernel(const bf16* __restrict__ x,
                                                             const float* __restrict__ dz,
                                                             const float* __restrict__ w,
@@ -763,8 +968,51 @@ int k_bias_grad(fm_ctx* ctx, const bf16* dy, float* db, int64_t voxels, int C) {
   return FM_OK;
 }
 
+// the multi-label head forward (L > 1); with `t` the training form, whose partials land in ctx->red_scratch
+static int head_fwd_labels(fm_ctx* ctx, const bf16* x, const float* w, const float* b, const float* t, float* p,
+                           int64_t voxels, int C, int L, int apply_sigmoid, XentSpec xs, int* grid_out) {
+  FM_CHECK(L >= 2 && L <= kMaxLabels, FM_EINVAL, "head: %d labels (1 .. %d)", L, kMaxLabels);
+  FM_CHECK(C >= 8 && C <= 256 && (C & (C - 1)) == 0, FM_EINVAL,
+           "head: channel count %d must be a power of two in [8,256]", C);
+  if (!t && !(C >= 16 && C <= 64)) {  // inference form, lanes-per-voxel
+    const int64_t vpb = kThreads / (C / 8);
+    const int grid = (int)std::min<int64_t>(ceil_div64(voxels, vpb), (int64_t)ctx->num_sms * 32);
+    ProfScope prof(ctx, "head_fwd_labels", 2.0 * C * L * (double)voxels, (double)voxels * (C * 2.0 + L * 4.0));
+    FM_CUDA(launch_pdl(head_fwd_labels_lpv_kernel, dim3(grid), dim3(kThreads), 0, ctx->stream, x, w, b, p, voxels, C, L,
+                       apply_sigmoid));
+    FM_LAUNCH_OK(ctx);
+    return FM_OK;
+  }
+  FM_CHECK(C == 16 || C == 32 || C == 64, FM_EINVAL,
+           "head: the training form of %d labels needs 16, 32 or 64 input channels, not %d", L, C);
+  // one partial row of 8 + 3 L doubles per block in the reduction scratch
+  const int rows = kRedScratchRows * 8 / (8 + 3 * L);
+  const int grid = (int)std::min<int64_t>(ceil_div64(voxels, kThreads), (int64_t)std::min(rows, 16 * ctx->num_sms));
+  const bool dice = t != nullptr;
+  ProfScope prof(ctx, dice ? "head_fwd_dice_labels" : "head_fwd_labels", 2.0 * C * L * (double)voxels,
+                 (double)voxels * (C * 2.0 + L * (dice ? 8.0 : 4.0)));
+  double* part = dice ? ctx->red_scratch : nullptr;
+#define FM_HEAD_LABELS(CC)                                                                                           \
+  if (C == CC) {                                                                                                     \
+    if (dice)                                                                                                        \
+      FM_CUDA(launch_pdl(head_fwd_labels_kernel<CC, true>, dim3(grid), dim3(kThreads), 0, ctx->stream, x, w, b, t, p, \
+                         voxels, L, 1, part, xs));                                                                   \
+    else                                                                                                             \
+      FM_CUDA(launch_pdl(head_fwd_labels_kernel<CC, false>, dim3(grid), dim3(kThreads), 0, ctx->stream, x, w, b, t,   \
+                         p, voxels, L, apply_sigmoid, part, xs));                                                    \
+  }
+  FM_HEAD_LABELS(16)
+  FM_HEAD_LABELS(32)
+  FM_HEAD_LABELS(64)
+#undef FM_HEAD_LABELS
+  FM_LAUNCH_OK(ctx);
+  if (grid_out) *grid_out = grid;
+  return FM_OK;
+}
+
 int k_head_fwd(fm_ctx* ctx, const bf16* x, const float* w, const float* b, float* p, int64_t voxels,
-               int C, int apply_sigmoid) {
+               int C, int apply_sigmoid, int L) {
+  if (L != 1) return head_fwd_labels(ctx, x, w, b, nullptr, p, voxels, C, L, apply_sigmoid, XentSpec(), nullptr);
   FM_CHECK(C >= 8 && C <= 256 && (C & (C - 1)) == 0, FM_EINVAL,
            "head: channel count %d must be a power of two in [8,256]", C);
   const int lpv = C / 8;
@@ -793,7 +1041,12 @@ int k_head_fwd(fm_ctx* ctx, const bf16* x, const float* w, const float* b, float
 
 // head + sigmoid + Dice / VOD / accuracy partial sums in one pass; `sums` receives the 8 folded statistics
 int k_head_fwd_dice(fm_ctx* ctx, const bf16* x, const float* w, const float* b, const float* t, float* p,
-                    int64_t voxels, int C, double* sums, XentSpec xs) {
+                    int64_t voxels, int C, double* sums, XentSpec xs, int L) {
+  if (L != 1) {
+    int grid = 0;
+    FM_TRY(head_fwd_labels(ctx, x, w, b, t, p, voxels, C, L, 1, xs, &grid));
+    return k_dice_finalize_labels(ctx, grid, (double)voxels * L, sums, L);
+  }
   FM_CHECK(C >= 8 && C <= 256 && (C & (C - 1)) == 0, FM_EINVAL,
            "head: channel count %d must be a power of two in [8,256]", C);
   const int lpv = C / 8;
@@ -828,12 +1081,21 @@ int k_head_fwd_dice(fm_ctx* ctx, const bf16* x, const float* w, const float* b, 
 }
 
 int k_head_bwd(fm_ctx* ctx, const bf16* x, const float* dz, const float* w, bf16* dx, float* dw,
-               float* db, int64_t voxels, int C, int mode, const float* t, const double* sums, XentSpec xs) {
+               float* db, int64_t voxels, int C, int mode, const float* t, const double* sums, XentSpec xs, int L) {
   FM_CHECK(C >= 8 && C <= 256 && (C & (C - 1)) == 0, FM_EINVAL,
            "head_bwd: channel count %d must be a power of two in [8,256]", C);
   const int lpv = C / 8;
   const int64_t vpb = kThreads / lpv;
   const int grid = (int)std::min<int64_t>(ceil_div64(voxels, vpb), (int64_t)ctx->num_sms * 8);
+  if (L != 1) {
+    FM_CHECK(L >= 2 && L <= kMaxLabels, FM_EINVAL, "head_bwd: %d labels (1 .. %d)", L, kMaxLabels);
+    ProfScope prof(ctx, t ? "head_bwd_dice_labels" : "head_bwd_labels", 4.0 * C * L * (double)voxels,
+                   (double)voxels * (C * 4.0 + L * (t ? 8.0 : 4.0)));
+    FM_CUDA(launch_pdl(head_bwd_labels_kernel, dim3(grid), dim3(kThreads), 0, ctx->stream, x, dz, w, dx, dw, db, voxels,
+                       C, L, mode, t, sums, xs));
+    FM_LAUNCH_OK(ctx);
+    return FM_OK;
+  }
   ProfScope prof(ctx, t ? "head_bwd_dice" : "head_bwd", 4.0 * C * (double)voxels,
                  (double)voxels * (C * 4.0 + (t ? 8.0 : 4.0)));
   FM_CUDA(launch_pdl(head_bwd_kernel, dim3(grid), dim3(kThreads), 0, ctx->stream, x, dz, w, dx, dw, db, voxels, C, mode, t,

@@ -119,6 +119,7 @@ SIGNATURES = {
     "fm_train_backward": (c_int, [c_vp]),
     "fm_train_apply": (c_int, [c_vp, c_f, c_u64, c_fp]),
     "fm_model_loss_sums": (c_int, [c_vp, c_u64p]),
+    "fm_model_label_dice": (c_int, [c_vp, c_fp, c_int]),
     "fm_model_grad_buffer": (c_int, [c_vp, c_u64p, c_i64p]),
     "fm_model_num_buckets": (c_int, [c_vp]),
     "fm_model_bucket_range": (c_int, [c_vp, c_int, c_i64p, c_i64p]),

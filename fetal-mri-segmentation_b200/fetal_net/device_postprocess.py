@@ -73,6 +73,10 @@ def patch_wise_segmentation(model, data, patch_shape, overlap_factor=0, batch_si
                             connected_component=True, return_prediction=False):
     """postprocess_prediction(patch_wise_prediction(model, data, ...).squeeze(), ...) for a one-label model: the bool
     [X,Y,Z] mask, and with return_prediction also the [X,Y,Z,1] float64 map patch_wise_prediction returns."""
+    if getattr(model, "n_labels", 1) != 1:
+        raise NotImplementedError("patch_wise_segmentation post-processes one probability map; the model has %d labels "
+                                  "(segment each label of patch_wise_prediction with postprocess_prediction)"
+                                  % model.n_labels)
     if not isinstance(model, Model):
         prob = patch_wise_prediction(model, data, patch_shape, overlap_factor=overlap_factor, batch_size=batch_size,
                                      truth_data=truth_data, prev_truth_index=prev_truth_index,

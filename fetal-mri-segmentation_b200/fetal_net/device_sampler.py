@@ -186,6 +186,14 @@ def _c_array(cls, v):
     return (cls * len(v))(*v) if v else None
 
 
+def _check_one_label(model):
+    """The sampler cuts one target channel; expanding integer truth into label channels (the reference generator's
+    `labels` / `categorical` handling) is not built, so multi-label models train through train_on_batch."""
+    if getattr(model, "n_labels", 1) != 1:
+        raise NotImplementedError("the device sampler cuts one target channel; a model with %d labels trains through "
+                                  "train_on_batch with label-channel targets" % model.n_labels)
+
+
 class DeviceSampler(PatchDraws):
     """data_generator(data_file, index_list, ...) with the cases resident in HBM.
 
@@ -289,6 +297,7 @@ class DeviceSampler(PatchDraws):
     def train_on_next_batch(self, model):
         """next(generator) + model.train_on_batch(x, y) without the batch ever visiting the host. Returns the
         metrics of Model.train_on_batch ([loss, dice_coefficient, vod_coefficient, binary_accuracy])."""
+        _check_one_label(model)
         cases, corners = self.draw()
         aug, warp = self.draw_augment(len(cases))
         return model.train_on_sampled_batch(self, cases, corners, aug=aug, warp=warp)

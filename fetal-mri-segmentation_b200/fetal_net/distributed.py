@@ -82,14 +82,14 @@ class DataParallelTrainer:
 
     def train_on_batch(self, x, y):
         """x, y: this rank's shard of the global batch ([x, weight_mask] for a two-input model). Returns the GLOBAL
-        [loss, acc, vod(, dice)]."""
+        [loss, acc, vod(, dice)(, label-wise Dice)]."""
         self.model._check_loss()
         x = self.model._split_mask(x)
         x, y = _lib.f32c(x), _lib.f32c(y)
         m = np.zeros(4, np.float32)
         _lib.check(self.lib.fm_train_step_dp(self.model._h, _lib.fptr(x), _lib.fptr(y), int(x.shape[0]),
                                              float(self.model.optimizer.lr), _lib.fptr(m)))
-        return [float(v) for v in m[:len(self.model.metrics_names)]]
+        return self.model._metrics(m)
 
     def allreduce_bench(self, nbytes, iters=20):
         """(ms per all-reduce, bus GB/s = 2 (n-1)/n * bytes / t) of an in-place fp32 SUM all-reduce of `nbytes`."""

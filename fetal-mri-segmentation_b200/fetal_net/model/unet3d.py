@@ -32,7 +32,7 @@ class Model:
 
     def __init__(self, input_shape, depth, n_base_filters, n_labels, initial_learning_rate, loss_function,
                  device=None, ndim=3, isensee_levels=None, dropout_rate=0.0, dropout_seed=0x5EED, mask_shape=None,
-                 deconvolution=False, batch_normalization=False):
+                 deconvolution=False, batch_normalization=False, label_wise_dice=False):
         lib = _lib.load()
         self._ctx = _lib.get_context(device)
         self.ndim = int(ndim)
@@ -85,6 +85,11 @@ class Model:
         self.metrics_names = ['loss', 'binary_accuracy', 'vod_coefficient']
         if loss_function is not dice_coefficient_loss:
             self.metrics_names.append('dice_coefficient')
+        # include_label_wise_dice_coefficients (unet3d/unet.py:71-75): one dice_coefficient per label channel, after the
+        # others; 2D models take the label axis last ([B,H,W,n_labels]) - see label_dice_coefficient
+        self.label_wise_dice = bool(label_wise_dice) and self.n_labels > 1
+        if self.label_wise_dice:
+            self.metrics_names += ['label_%d_dice_coef' % i for i in range(self.n_labels)]
         self.stop_training = False
         self.deconvolution = bool(deconvolution)
         self.batch_normalization = bool(batch_normalization)
@@ -198,6 +203,7 @@ class Model:
         arrays["__isensee_levels__"] = np.array(int(getattr(self, "isensee_levels", 0) or 0))
         arrays["__deconvolution__"] = np.array(int(getattr(self, "deconvolution", False)))
         arrays["__batch_normalization__"] = np.array(int(getattr(self, "batch_normalization", False)))
+        arrays["__label_wise__"] = np.array(int(getattr(self, "label_wise_dice", False)))
         return arrays
 
     def save_weights(self, path):
@@ -324,15 +330,27 @@ class Model:
         m = np.zeros(4, np.float32)
         _lib.check(self._lib.fm_train_step(self._h, _lib.fptr(x), _lib.fptr(y), int(x.shape[0]),
                                            float(self.optimizer.lr), _lib.fptr(m)))
-        return [float(v) for v in m[:len(self.metrics_names)]]
+        return self._metrics(m)
+
+    def label_dice(self):
+        """Dice of each label over the batch of the last training step / evaluation (fm_model_label_dice)."""
+        d = np.zeros(self.n_labels, np.float32)
+        _lib.check(self._lib.fm_model_label_dice(self._h, _lib.fptr(d), self.n_labels))
+        return d
+
+    def _metrics(self, m):
+        """metrics_names' values from the four device metrics (+ the label-wise Dice)."""
+        out = [float(v) for v in m[:len(self.metrics_names) - (self.n_labels if self.label_wise_dice else 0)]]
+        return out + ([float(v) for v in self.label_dice()] if self.label_wise_dice else [])
 
     def train_on_sampled_batch(self, sampler, cases, corners, aug=None, warp=None):
         """One training step on samples cut on the device by a `fetal_net.device_sampler.DeviceSampler`
         (next(generator) + train_on_batch of fetal_net/training.py:110-124 with no host batch): fm_train_step_sampled.
         aug / warp: per-sample fm_sample_aug / fm_sample_warp arrays (a data-parallel rank passes its slice); with both
         None the sampler draws them from its `device_augment`."""
-        from ..device_sampler import _c_array
+        from ..device_sampler import _c_array, _check_one_label
         self._check_loss()
+        _check_one_label(self)
         cases, corners = _lib.i32x(cases), _lib.i32x(corners)
         if aug is None and warp is None:
             aug, warp = sampler.draw_augment(cases.size)
@@ -353,7 +371,7 @@ class Model:
         x, y = _lib.f32c(x), _lib.f32c(y)
         m = np.zeros(4, np.float32)
         _lib.check(self._lib.fm_evaluate(self._h, _lib.fptr(x), _lib.fptr(y), int(x.shape[0]), _lib.fptr(m)))
-        return [float(v) for v in m[:len(self.metrics_names)]]
+        return self._metrics(m)
 
     def evaluate(self, x, y, batch_size=32, verbose=0):
         """Keras semantics: per-batch metrics averaged with batch-size weights."""
@@ -439,7 +457,8 @@ def unet_model_3d(input_shape, pool_size=(2, 2, 2), n_labels=1, initial_learning
         raise NotImplementedError("activation_name %r: only 'sigmoid' is built" % activation_name)
     return Model(input_shape=input_shape, depth=depth, n_base_filters=n_base_filters, n_labels=n_labels,
                  initial_learning_rate=initial_learning_rate, loss_function=loss_function,
-                 device=kargs.get("device"), deconvolution=deconvolution, batch_normalization=batch_normalization)
+                 device=kargs.get("device"), deconvolution=deconvolution, batch_normalization=batch_normalization,
+                 label_wise_dice=include_label_wise_dice_coefficients)
 
 
 def unet_model_2d(input_shape, pool_size=(2, 2), n_labels=1, initial_learning_rate=0.00001, deconvolution=False,
@@ -460,7 +479,7 @@ def unet_model_2d(input_shape, pool_size=(2, 2), n_labels=1, initial_learning_ra
                  initial_learning_rate=initial_learning_rate, loss_function=loss_function,
                  device=kargs.get("device"), ndim=2, dropout_rate=dropout_rate or 0.0,
                  dropout_seed=kargs.get("dropout_seed", 0x5EED), deconvolution=deconvolution,
-                 batch_normalization=batch_normalization)
+                 batch_normalization=batch_normalization, label_wise_dice=include_label_wise_dice_coefficients)
 
 
 def isensee2017_model_3d(input_shape=(1, 128, 128, 128), n_base_filters=16, depth=5, dropout_rate=0.3,

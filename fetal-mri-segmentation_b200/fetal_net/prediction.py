@@ -53,6 +53,9 @@ def _geometry(model, data, patch_shape, overlap_factor):
     """Integer/percentile host logic of prediction.py:129-146,161-163,169-173."""
     out_shape = tuple(model.output_shape)
     is3d = int(np.sum(np.array(out_shape[1:]) > 1)) > 2
+    if getattr(model, "n_labels", 1) > 1 and getattr(model, "ndim", None) in (2, 3):
+        # the reference's shape rule (prediction.py:129) takes a [H, W, n_labels > 1] output for a 3D one
+        is3d = model.ndim == 3
     prediction_shape = tuple(out_shape[-3:]) if is3d else tuple(out_shape[-3:-1]) + (1,)
     patch_shape = tuple(int(v) for v in patch_shape)
     vol = data[0]

@@ -169,6 +169,7 @@ def load_old_model(model_file, verbose=True, config=None):
         levels = int(z["__isensee_levels__"]) if "__isensee_levels__" in z.files else 0
         deconv = bool(int(z["__deconvolution__"])) if "__deconvolution__" in z.files else False
         bnorm = bool(int(z["__batch_normalization__"])) if "__batch_normalization__" in z.files else False
+        label_wise = bool(int(z["__label_wise__"])) if "__label_wise__" in z.files else False
     loss = _metrics.dice_coefficient_loss
     lr = 1e-5
     if config is not None:
@@ -182,6 +183,8 @@ def load_old_model(model_file, verbose=True, config=None):
         kwargs['deconvolution'] = True
     if bnorm:
         kwargs['batch_normalization'] = True
+    if label_wise:
+        kwargs['include_label_wise_dice_coefficients'] = True
     if builder_name in ('isensee2017_model_3d', 'isensee2017_model'):
         kwargs['n_segmentation_levels'] = levels
         if builder_name == 'isensee2017_model':     # the 2D builder: `levels` heads reach the output only when summed

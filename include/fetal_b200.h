@@ -69,7 +69,7 @@ typedef struct fm_unet3d_spec {
   int32_t X, Y, Z;        /* patch extent; each divisible by 2^(depth-1)     */
   int32_t depth;          /* default 4                                       */
   int32_t n_base_filters; /* builder default 32; BASELINE configs use 16     */
-  int32_t n_labels;       /* 1                                               */
+  int32_t n_labels;       /* 1 .. 8: independent sigmoid maps (see below)    */
 } fm_unet3d_spec;
 
 /* Replaces: unet_model_3d(...) + model.compile(Adam, loss=dice_coefficient_loss)
@@ -106,7 +106,7 @@ typedef struct fm_unet2d_spec {
   int32_t in_channels;    /* patch_depth (+ prev_truth_size), 1..16                 */
   int32_t depth;          /* default 4                                              */
   int32_t n_base_filters; /* default 32                                             */
-  int32_t n_labels;       /* 1                                                      */
+  int32_t n_labels;       /* 1 .. 8                                                 */
 } fm_unet2d_spec;
 
 /* Replaces: unet_model_2d(...) + model.compile (fetal_net/model/unet/unet.py:49-88). Input [B,H,W,in_channels],
@@ -125,7 +125,7 @@ typedef struct fm_isensee3d_spec {
   int32_t depth;                  /* default 5                                */
   int32_t n_base_filters;         /* default 16                               */
   int32_t n_segmentation_levels;  /* default 1; BASELINE config 3 uses 3      */
-  int32_t n_labels;               /* 1                                        */
+  int32_t n_labels;               /* 1 .. 8                                   */
 } fm_isensee3d_spec;
 int fm_model_create_isensee3d(fm_ctx* ctx, const fm_isensee3d_spec* spec, fm_model** out);
 
@@ -142,7 +142,7 @@ typedef struct fm_isensee2d_spec {
   int32_t depth;                  /* default 5                                */
   int32_t n_base_filters;         /* default 16                               */
   int32_t n_segmentation_levels;  /* heads summed into the output (see above) */
-  int32_t n_labels;               /* 1                                        */
+  int32_t n_labels;               /* 1 .. 8                                   */
 } fm_isensee2d_spec;
 int fm_model_create_isensee2d(fm_ctx* ctx, const fm_isensee2d_spec* spec, fm_model** out);
 
@@ -203,7 +203,14 @@ int fm_model_set_weight_mask(fm_model* m, const float* mask, int batch);
 
 /* Replaces: model.predict(ndarray[B,Cin,X,Y,Z]) -> float32 [B,n_labels,X,Y,Z]
  * (fetal_net/prediction.py:354-361). Host pointers; H2D + forward + D2H inside the call.
- * With n_labels == 1 the channels-first and channels-last output layouts coincide. */
+ * With n_labels == 1 the channels-first and channels-last output layouts coincide.
+ * n_labels: every model family takes 1 .. 8 labels, each its own sigmoid of Conv(n_labels, 1) heads (unet.py:68-69;
+ * the Isensee nets sum their per-level heads label by label before the sigmoid); host and
+ * device arrays shaped like the output (predictions, targets, weight masks) follow the Keras layout,
+ * [B,n_labels,X,Y,Z] for 3D models and [B,H,W,n_labels] for 2D ones. The loss and its metrics are taken over all
+ * B * voxels * n_labels elements (dice_coefficient flattens, metrics.py:11-15); fm_model_label_dice gives the Dice of
+ * each label. The device sampler (fm_train_step_sampled*), fm_patchwise_segment and fm_patchwise_predict_flips take
+ * one-label models only and return FM_EINVAL otherwise. */
 int fm_predict(fm_model* m, const float* x, int batch, float* y);
 
 /* Page-locked host memory: a result array allocated here receives the device->host copies of fm_patchwise_predict
@@ -342,6 +349,11 @@ int fm_train_apply(fm_model* m, float lr, uint64_t after_stream, float out_metri
 int fm_train_metrics_async(fm_model* m);
 int fm_train_metrics_wait(fm_model* m, float out_metrics[4]);
 int fm_model_loss_sums(fm_model* m, uint64_t* dev_ptr);               /* 8 x float64, device */
+/* Per-label Dice (2 sum(t p) + 1) / (sum t + sum p + 1) over label l's elements of the batch of the last
+ * fm_train_step* / fm_evaluate (with one label: the Dice metric). n must equal n_labels. The device sums behind it follow
+ * the 9 loss sums at fm_model_loss_sums() as 3 n_labels float64 (sum t p, sum t, sum p per label) when n_labels > 1;
+ * a data-parallel step all-reduces them with the others. */
+int fm_model_label_dice(fm_model* m, float* out, int n);
 int fm_model_grad_buffer(fm_model* m, uint64_t* dev_ptr, int64_t* n); /* n x float32, device */
 int fm_model_num_buckets(fm_model* m);
 int fm_model_bucket_range(fm_model* m, int bucket, int64_t* offset, int64_t* count);
